@@ -8,6 +8,9 @@ data path: weak scaling).
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference algorithm on host CPU cores
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step computed as DIR/<name>.npy
+
+The inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 Vocabulary.  graph-step = one pocket graph through one denoiser forward + one reverse-diffusion step
 (sequence_model/sample.py:199-207).  One bench "step" = one complete T-step sampling of the rank's batch
@@ -133,6 +136,45 @@ class ClockSampler:
         return {"sm_mhz": statistics.median(sm), "sm_max_mhz": max(mx), "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 64 << 20  # all arrays of one --dump-outputs directory together
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: tensor} as out_dir/<name>.npy (float64 stays float64, everything else becomes float32), DUMP_BYTES in all.  Going
+    from the smallest array up, one larger than an even share of what is left is replaced by a fixed sample of its flattened elements
+    (seeded, ascending indices), so runs with the same arguments dump the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: (t.detach().cpu().double() if t.dtype == torch.float64 else t.detach().cpu().float()) for k, t in arrays.items()}
+    left = DUMP_BYTES - 256 * len(arrays)  # room for the .npy headers
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel() * kv[1].element_size())):
+        n = left // (len(arrays) - i) // t.element_size()
+        if t.numel() > n:
+            t = t.reshape(-1)[torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values]
+        left -= t.numel() * t.element_size()
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy())
+
+
+def training_outputs(sd, opt, loss, n_sample=1 << 20):
+    """What a caller holds after one optimizer step of the training path: the loss, the gradient norm the clip measured, and the same
+    fixed seeded sample of the flat gradient and of the updated fp32 weights (live parameters in name order)."""
+    import ctypes
+    flat = opt.flat
+    lib = sd.lib()
+    names = sorted(flat.table)
+    grads = torch.cat([flat.grads[flat.table[k][0]:flat.table[k][0] + flat.table[k][1]] for k in names])
+    weights = torch.empty_like(grads)
+    pos = 0
+    with torch.cuda.device(flat.device):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(flat.device).cuda_stream)
+        for k in names:
+            n = flat.table[k][1]
+            sd._cabi.check(lib.seqdiff_model_get_tensor(flat.handle, k.encode(), sd._cabi.ptr(weights[pos:pos + n]), n, stream))
+            pos += n
+    idx = torch.randperm(grads.numel(), generator=torch.Generator().manual_seed(0))[:n_sample].sort().values.to(grads.device)
+    return {"loss": loss.reshape(1), "grad_norm": opt.grad_norm, "grads_sample": grads[idx], "weights_sample": weights[idx]}
+
+
 def measured_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -142,10 +184,11 @@ def measured_peaks():
 
 
 # ----------------------------------------------------------------------------------------------------
-def cpu_reference_steps(state, batch, x_T, T, n_steps, n_warm, threads):
+def cpu_reference_steps(state, batch, x_T, T, n_steps, n_warm, threads, outputs=None):
     """The reference algorithm on host cores ("port": oracle/seqdiff_oracle.py, which restates
     sequence_model/model.py:200-237 + sample.py:141-179 incl. its Python multinomial loop).
-    One step = forward + reverse step over the whole batch at s_int = T-1, T-2, ..."""
+    One step = forward + reverse step over the whole batch at s_int = T-1, T-2, ...
+    `outputs` (a dict) receives the logits and the sampled x of the last step."""
     from oracle import seqdiff_oracle as O
     torch.set_num_threads(threads)
     cfg = O.OracleConfig(max_position_embeddings=L)
@@ -164,6 +207,8 @@ def cpu_reference_steps(state, batch, x_T, T, n_steps, n_warm, threads):
             dt = time.perf_counter() - t0
             if i >= n_warm:
                 times.append(dt)
+    if outputs is not None:
+        outputs.update(logits=logits, x=x)
     return times
 
 
@@ -189,7 +234,10 @@ def run_reference_arm(args):
     cfg_obj = workload_config(args.wl, args.batch, args.timesteps, int(os.environ.get("WORLD_SIZE", "1")))  # the product arm's config
     args.batch = cpu_b
     threads = os.cpu_count() or 1
-    times = cpu_reference_steps(state, batch, x_T, args.timesteps, args.steps, args.warmup, threads)
+    outputs = {} if args.dump_outputs else None
+    times = cpu_reference_steps(state, batch, x_T, args.timesteps, args.steps, args.warmup, threads, outputs)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     total = sum(times)
     value = args.batch * len(times) / total
     out = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -272,11 +320,13 @@ def cfg3_strong_record(sd, dev, world, rank, barrier, precision, steps=2, warmup
         L = keep_L
 
 
-def cfg4_train_record(sd, dev, world, rank, barrier, precision, steps=10, warmup=10, global_batch=128, grad_comm="fp32", weak=False):
+def cfg4_train_record(sd, dev, world, rank, barrier, precision, steps=10, warmup=10, global_batch=128, grad_comm="fp32", weak=False,
+                      outputs=None):
     """BASELINE configs[3]: one optimizer step of the sequence denoiser on a GLOBAL batch of 128 graphs (L = 128, T = 50, dropout 0.1,
     AdamW lr 5e-5 wd 0.1, clip 1.0: train_model.py:17-33), data-parallel over the ranks (128 / world graphs each), ONE gradient
     all-reduce per step over NCCL (61.06 M live parameters).  Reports whole steps (training_step + all-reduce + clip + AdamW), the
-    same without the all-reduce, and the all-reduce alone => exposed-communication fraction and achieved bus bandwidth."""
+    same without the all-reduce, and the all-reduce alone => exposed-communication fraction and achieved bus bandwidth.
+    `outputs` (a dict) receives training_outputs() of the last whole step."""
     import torch.distributed as dist
     global L
     keep_L = L
@@ -324,6 +374,8 @@ def cfg4_train_record(sd, dev, world, rank, barrier, precision, steps=10, warmup
         n0 = sd.lib().seqdiff_launch_count()  # counted over the timed steps (the warm-up steps also hold the GEMM tuner's candidate launches)
         ms_full, loss = timed(lambda i: step(i), steps)                       # bucketed all-reduce under the backward pass
         launches_per_step = (sd.lib().seqdiff_launch_count() - n0) // max(steps, 1)
+        if outputs is not None:  # outside the timed loops: timed() ends in a synchronise and the next one starts with one
+            outputs.update({k: v.cpu() for k, v in training_outputs(sd, opt, loss).items()})
         ms_block, _ = timed(lambda i: step(i, overlap=False), steps) if world > 1 else (ms_full, None)  # all-reduce after the backward pass
         ms_nocomm, _ = timed(lambda i: step(i, skip=True), steps)
         opt.overlap = True
@@ -354,9 +406,15 @@ def cfg4_train_record(sd, dev, world, rank, barrier, precision, steps=10, warmup
 
 # ----------------------------------------------------------------------------------------------------
 def main():
+    def positive_int(s):
+        v = int(s)
+        if v < 1:
+            raise argparse.ArgumentTypeError(f"needs at least 1, got {v}")
+        return v
+
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=0, help="pocket graphs per GPU (default: the workload's)")
@@ -365,6 +423,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="cfg2", choices=["cfg2", "cfg3", "cfg4"], help="cfg2 = headline (B=64/GPU, L=128); cfg3 = 256 ext-pockets of 512 residues sharded over the GPUs (strong scaling)")
     ap.add_argument("--no-extras", action="store_true", help="skip e2e / roofline / cpu legs (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0) as DIR/<name>.npy, "
+                                                          f"{DUMP_BYTES >> 20} MB at most")
     args = ap.parse_args()
     global L
     wl = WORKLOADS[args.workload]
@@ -412,8 +472,11 @@ def main():
             torch.cuda.synchronize(dev)
 
     if args.workload == "cfg4":  # the training configuration on its own: one line whose value is training graphs/s
+        outputs = {} if args.dump_outputs else None
         with ClockSampler(local) as clk:
-            rec = cfg4_train_record(sd, dev, world, rank, barrier0, args.precision, steps=max(args.steps, 1), warmup=max(args.warmup, 3))
+            rec = cfg4_train_record(sd, dev, world, rank, barrier0, args.precision, steps=args.steps, warmup=max(args.warmup, 3), outputs=outputs)
+        if rank == 0 and outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         if rank == 0:
             emit({"metric": "training graphs/s (forward + backward + gradient all-reduce + clip + AdamW; cfg4: global batch 128, L=128)",
                   "value": rec["value"], "unit": rec["unit"], "n_gpus": world, "steps": rec["steps"], "warmup": rec["warmup"],
@@ -471,6 +534,8 @@ def main():
     ms = ms.item()
     value = world * B * T * args.steps / (ms * 1e-3)
     assert torch.isfinite(out).all()
+    # denoise_tensors returns the final [B, L, 20] logits of the sampling (raw logits of the last step, as the reference's denoise)
+    outputs = {"final_logits": out.cpu()} if args.dump_outputs else None
 
     # ---- the same samplings with ragged packing (valid prefixes only; bit-identical at every position denoise() reads) ----
     packed_rec = None
@@ -493,6 +558,10 @@ def main():
         packed_rec = {"value": world * B * T * args.steps / (pms.item() * 1e-3), "unit": UNIT, "ms_per_step": pms.item() / args.steps,
                       "valid_token_frac": tok, "identical_to_padded_at_valid_positions": bool(torch.equal(outp[vmask], out[vmask])),
                       "note": "ragged packing (seqdiff_sample_ex flag 1): M = sum of lengths; `value` above is the padded computation"}
+        if outputs is not None:
+            outputs["final_logits_packed"] = outp.cpu()
+    if rank == 0 and outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
     result = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
               "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": wl["scaling"], "vs_baseline": None, "dtype": args.precision,

@@ -35,6 +35,26 @@ def test_reference_arm_prints_one_json_line():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_dump_outputs_same_arguments_same_arrays(tmp_path):
+    """--dump-outputs writes the last timed step's arrays as .npy; two runs with the same arguments dump identical arrays, and
+    --steps below 1 is refused rather than changed."""
+    import numpy as np
+    dumps = []
+    for k in range(2):
+        d = tmp_path / f"run{k}"
+        r = _run("--impl", "reference", "--steps", "2", "--warmup", "0", "--batch", "2", "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+        dumps.append({p.name: np.load(p) for p in sorted(d.glob("*.npy"))})
+    assert sorted(dumps[0]) == ["logits.npy", "x.npy"]
+    for name, a in dumps[0].items():
+        assert a.dtype == np.float32 and a.shape == (2, 128, 20) and np.isfinite(a).all()
+        assert np.array_equal(a, dumps[1][name]), name
+    assert sum(a.nbytes for a in dumps[0].values()) <= 64 << 20
+    r = _run("--impl", "reference", "--steps", "0", "--warmup", "0", "--batch", "2", timeout=120)
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_recorded_product_and_reference_lines_share_one_config():
     """the two lines of the last B200 verification of the round (profiles/): same metric, unit, direction and config object."""
     a = json.load(open(os.path.join(ROOT, "profiles", "bench_r02_final2.json")))

@@ -1,5 +1,5 @@
 """CPU tests: the oracle against the golden vectors produced from the unmodified reference
-(oracle/make_golden.py), and against the reference itself when /root/reference is present."""
+(oracle/make_golden.py)."""
 import glob
 import os
 
@@ -126,22 +126,19 @@ def test_identity_at_init_trap():
 
 
 def test_reference_live_pin():
-    """When the reference tree is present (build container only) re-run the live comparison."""
-    from oracle import ref_import as R
-    if not R.reference_available():
-        pytest.skip("reference tree not present on this box")
+    """The reference forward as installed (no relative_key term) on two graphs of L = 64, weight variant B: its stored logits
+    (forward_norel_L64_B.pt, the case test_forward_golden skips) against the oracle."""
+    g = _load("forward_norel_L64_B.pt")
+    assert (g["L"], g["B"], g["variant"], g["relative_key"]) == (64, 2, "B", False)
     cfg = O.OracleConfig(max_position_embeddings=64, relative_key=False)
-    sd = O.init_state_dict(cfg, 3, "B")
-    m = R.build_reference_model(64, relative_key=False)
-    m.load_state_dict(sd, strict=True)
-    b = O.synthetic_batch(2, 64, (5, 40), (16, 64), 5)
-    x_t = O.generate_discrete_noise(2, 64, generator=torch.Generator().manual_seed(1))
-    t = torch.full((2, 1), 11.0)
+    sd = O.init_state_dict(cfg, g["weight_seed"], "B")
+    b = O.synthetic_batch(2, 64, g["n_lig"], g["n_rec"], g["input_seed"])
+    x_t = F.one_hot(g["x_t_idx"].long(), 20).float()
+    t = torch.full((2, 1), g["timestep"])
     with torch.no_grad():
-        y = m(t, x_t, b["ligand_angles"], b["ligand_attn_mask"], b["receptor_seq"], b["receptor_angles"], b["receptor_attn_mask"])
         yo = O.denoiser_forward(sd, cfg, t, x_t, b["ligand_angles"], b["ligand_attn_mask"], b["receptor_seq"], b["receptor_angles"],
                                 b["receptor_attn_mask"])
-    assert (y - yo).abs().max().item() < 1e-5
+    assert (g["logits"] - yo).abs().max().item() < 1e-5
 
 
 def test_dataset_item_golden():
@@ -181,18 +178,9 @@ def test_structure_feed_cfg5_fixture_and_oracle():
 
 
 def test_structure_model_reference_shape_live():
-    """Same check against the reference structure model itself when /root/reference is present (build container only)."""
-    from oracle import ref_import as R
-    if not R.reference_available():
-        pytest.skip("reference tree not present")
-    from transformers.models.bert.modeling_bert import BertConfig
-    SM = R.load_structure_reference()
-    B, L = 2, 128
-    common = dict(max_position_embeddings=L, num_attention_heads=12, hidden_size=768, intermediate_size=1024, num_hidden_layers=2,
-                  position_embedding_type="relative_key")
-    m = SM.ConditionalBertForDiffusionBase(BertConfig(**common), BertConfig(**common, is_decoder=True, add_cross_attention=True), 8).eval()
-    batch = O.synthetic_batch(B, L, (5, 64), (16, 128), 7)
-    with torch.no_grad():
-        out = m(torch.randint(0, 1000, (B,)), torch.zeros(B, L, 8), batch["ligand_attn_mask"], batch["receptor_seq"],
-                batch["receptor_angles"], batch["receptor_attn_mask"])
-    assert out.shape == (B, L, 8) and out.dtype == torch.float32
+    """Same check on what the reference structure model itself returned for 128-residue graphs (its stored outputs, with and
+    without the relative_key term): [B, L, 8] fp32, the shape and dtype the sequence model takes as `ligand_angle`."""
+    for name in ("struct_forward_norel_L128_l12.pt", "struct_forward_rel_L128_l12.pt"):
+        g = _load(name)
+        out = g["out"]
+        assert out.shape == (g["B"], g["L"], 8) and g["L"] == 128 and out.dtype == torch.float32 and torch.isfinite(out).all()

@@ -118,42 +118,19 @@ def test_struct_mirror_schema_and_signatures():
 
 
 def test_struct_reference_live_pin():
-    """Build container only (the GPU box has no /root/reference): the UNMODIFIED structure_model module, its own p_sample and the
-    oracle on fresh inputs -- forward with the restored relative_key term, then one reverse step under torch.manual_seed."""
-    from oracle import ref_import as R
-    if not R.reference_available():
-        pytest.skip("reference tree not present on this box")
-    from transformers.models.bert.modeling_bert import BertConfig
-    SM, SS, SU = R.load_structure_sample_reference()
-    L, layers, B = 32, 1, 2
-    cfg = _cfg(L, layers, True)
-    state = S.init_struct_state_dict(cfg, 77)
-    common = dict(max_position_embeddings=L, num_attention_heads=12, hidden_size=768, intermediate_size=1024, num_hidden_layers=layers,
-                  position_embedding_type="relative_key", hidden_dropout_prob=0.1, attention_probs_dropout_prob=0.1, use_cache=False)
-    enc, dec = BertConfig(**common), BertConfig(**common, is_decoder=True, add_cross_attention=True)
-    for c in (enc, dec):
-        try:
-            c._attn_implementation = "eager"
-        except Exception:
-            pass
-    m = R.patch_relative_key_struct(SM.ConditionalBertForDiffusionBase(enc, dec, 8), L).eval()
-    m.load_state_dict(state, strict=True)
-    batch = O.synthetic_batch(B, L, (5, 32), (8, 32), 78)
-    g = torch.Generator().manual_seed(79)
-    x = (torch.rand(B, L, 8, generator=g) * 2 - 1) * math.pi
-    T, i = 50, 20
-    betas = SU.cosine_beta_schedule(T)
-    t = torch.full((B,), i, dtype=torch.long)
-    torch.manual_seed(80)
+    """The first reverse step of the UNMODIFIED structure_model's own p_sample_loop (struct_p_sample_loop_T4.pt: relative_key
+    term restored, the N(0,1) draw it made stored) against one oracle forward + p_sample_update + wrap from the same x_T."""
+    g = torch.load(os.path.join(GOLDEN, "struct_p_sample_loop_T4.pt"))
+    cfg = _cfg(g["L"], g["layers"], True)
+    state = S.init_struct_state_dict(cfg, g["weight_seed"])
+    batch = O.synthetic_batch(g["B"], g["L"], tuple(g["n_lig"]), tuple(g["n_rec"]), g["batch_seed"])
+    T, i = g["T"], g["T"] - 1
+    t = torch.full((g["B"],), i, dtype=torch.long)
     with torch.no_grad():
-        ref = SS.p_sample(model=m, ligand_mask=batch["ligand_attn_mask"], ligand_angle_noise=x, receptor_seq=batch["receptor_seq"],
-                          receptor_mask=batch["receptor_attn_mask"], receptor_angle=batch["receptor_angles"], timestep=t, betas=betas)
-        torch.manual_seed(80)
-        z = torch.randn(B, L, 8)
-        out = S.struct_forward(state, cfg, t, x, batch["ligand_attn_mask"], batch["receptor_seq"], batch["receptor_angles"], batch["receptor_attn_mask"])
-        got = S.p_sample_update(x, out, S.step_coefficients(S.cosine_beta_schedule(T)), i, z)
-    assert (ref - got).abs().max().item() < 1e-5
-    assert torch.equal(SU.modulo_with_wrapped_range(ref, -math.pi, math.pi), S.modulo_with_wrapped_range(ref, -math.pi, math.pi))
+        out = S.struct_forward(state, cfg, t, g["x_T"], batch["ligand_attn_mask"], batch["receptor_seq"], batch["receptor_angles"],
+                               batch["receptor_attn_mask"])
+    got = S.p_sample_update(g["x_T"], out, S.step_coefficients(S.cosine_beta_schedule(T)), i, g["noise"][i])
+    assert (S.modulo_with_wrapped_range(got, -math.pi, math.pi) - g["steps"][0]).abs().max().item() < 1e-5
 
 
 def test_struct_sample_driver_trims_and_batches():
