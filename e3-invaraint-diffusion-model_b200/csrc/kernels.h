@@ -43,7 +43,8 @@ int make_tmap_3d(const void* ptr, int fmt, int batch, int rows, int cols, int bo
 
 // ---- rowwise.cu -------------------------------------------------------------------------------------
 // GaussianFourierProjection (model.py:85-97): out[b, :] = [sin(x), cos(x)], x = ((t*W)*2)*pi in fp32.
-// t = timestep[b], or (float)*step_ptr for every b when step_ptr != NULL (sampling loop, quirk Q3).
+// t = timestep[b], or (float)*step_ptr for every b when step_ptr != NULL (sampling loop, quirk Q3), or (float)b when both are NULL
+// (the sampling loop's [T, H] table of steps 0 .. T-1).
 // out16 (optional): 16-bit copy in format fmt16 (0 = fp16, 1 = bf16).
 int timestep_embed(const float* timestep, const int* step_ptr, const float* W, int B, int H, float* out, void* out16, int fmt16,
                    cudaStream_t s);
@@ -64,6 +65,7 @@ struct EmbedJob {
   // the timestep features of graph row_graph[r]; NULL = identity / r / L
   const int* src_rows;
   const int* row_graph;
+  const int* te_row;  // sampling loop: every row takes te row *te_row (te is then the [T, H] table of the steps), else NULL
   int cta_begin, cta_count;  // filled by embed_ln_multi
 };
 struct EmbedJobs {
@@ -86,9 +88,12 @@ int layernorm(const float* in, int M, int H, const float* w, const float* b, flo
 //   out = x + gate * (LayerNorm_noaffine(y, 1e-5) * (1 + scale) + shift)
 // (shift, scale, gate) = mod[row / mod_div, (chunk0 + {0,1,2}) * H : ...], mod row pitch 6H.
 // row_graph (optional, packed mode with graph-level conditioning): row r uses mod row row_graph[r] instead of r / mod_div
+// mod_row (optional, sampling loop): every row uses mod row *mod_row (the step's row of a [T, 6H] modulation table)
+// in_hi / x_hi (optional, sampling loop): rows r >= split read `in` and `x` from row r - split of these instead
 template <typename T>
 int ln_modulate(const float* in, int M, int H, bool affine_first, const float* lnw, const float* lnb, float eps1, const float* x,
-                const T* mod, int mod_div, int chunk0, float* out32, T* outT, cudaStream_t s, const int* row_graph = nullptr);
+                const T* mod, int mod_div, int chunk0, float* out32, T* outT, cudaStream_t s, const int* row_graph = nullptr,
+                const int* mod_row = nullptr, int split = 0, const float* in_hi = nullptr, const float* x_hi = nullptr);
 // AminoAcidPredictor tail (model.py:151-152): logits = LayerNorm(y) @ W2^T + b2  (y is already GELU(dense1))
 // dst_rows (optional, packed mode): logits of row r are written to row dst_rows[r] of `logits` (the padded [B * L, F] layout)
 template <typename T>

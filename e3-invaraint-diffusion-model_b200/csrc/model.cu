@@ -252,6 +252,7 @@ Model::~Model() {
   for (void* p : packed_allocs) cudaFree(p);
   if (ws) { debug_guard_begin(ws); cudaFree(ws); }
   if (samp_in) { debug_guard_begin(samp_in); cudaFree(samp_in); }
+  if (samp_inv) { debug_guard_begin(samp_inv); cudaFree(samp_inv); }
   if (d_tables) cudaFree(d_tables);
   if (d_pack) cudaFree(d_pack);
   if (tws) { debug_guard_begin(tws); cudaFree(tws); }
@@ -760,36 +761,99 @@ template <typename T> struct SEBufs {
   Act<T> x1;
 };
 
+// Sampling loop: what se_layer takes from the per-sampling invariants (LoopInv).  o_hi != NULL: only rows [0, Ma) go through the
+// attention sublayer (segs cover just those); rows r >= Ma take its output (dense + residual, before the LayerNorm) and their
+// residual x from row r - Ma of o_hi / x_hi.  mod != NULL: the adaLN GEMMs are skipped and every row takes row *mod_row of mod.
+template <typename T> struct SEHoist {
+  int Ma;
+  const float* o_hi;
+  const float* x_hi;
+  const T* mod;
+  const int* mod_row;
+};
+
 // SELayer.forward (model.py:52-63).  x:[M,H]; c:[Mc,H] with token row r using c row r / mod_div.
 // packs (optional, one per segment): ragged batch -- the segment's graphs are addressed through offset / length arrays (absolute rows
 // of the token matrix) and seg.L is the largest length; row_graph: graph of every row (conditioning broadcast over a graph).
 template <typename T>
 static int se_layer(const Model& m, int wfmt, const SEW& w, const Act<T>& x, const T* c, int Mc, int mod_div, int M,
                     const std::vector<Segment>& segs, const SEBufs<T>& b, const Act<T>& out, cudaStream_t s,
-                    const std::vector<AttnPack>* packs = nullptr, const int* row_graph = nullptr) {
+                    const std::vector<AttnPack>* packs = nullptr, const int* row_graph = nullptr, const SEHoist<T>* hz = nullptr) {
   const int H = m.cfg.hidden_size, P = m.cfg.max_position_embeddings, heads = m.cfg.num_attention_heads;
-  SD_TRY(gemm_T(wfmt, Mc, H, H, c, w.ada0, w.ada0_b, 2, b.u, s));          // SiLU(Linear(c))
-  SD_TRY(gemm_T(wfmt, Mc, 6 * H, H, b.u, w.ada2, w.ada2_b, 0, b.mod, s));   // -> 6 chunks
-  SD_TRY(gemm_T(wfmt, M, 3 * H, H, x.t, w.attn.qkv, w.attn.qkv_b, 0, b.qkv, s));
+  const int Ma = hz && hz->o_hi ? hz->Ma : M;
+  const T* mod = hz && hz->mod ? hz->mod : b.mod;
+  const int* mod_row = hz ? hz->mod_row : nullptr;
+  if (mod == b.mod) {
+    SD_TRY(gemm_T(wfmt, Mc, H, H, c, w.ada0, w.ada0_b, 2, b.u, s));          // SiLU(Linear(c))
+    SD_TRY(gemm_T(wfmt, Mc, 6 * H, H, b.u, w.ada2, w.ada2_b, 0, b.mod, s));   // -> 6 chunks
+  }
+  SD_TRY(gemm_T(wfmt, Ma, 3 * H, H, x.t, w.attn.qkv, w.attn.qkv_b, 0, b.qkv, s));
   for (size_t gi = 0; gi < segs.size(); ++gi) {
     const Segment& g = segs[gi];
     const T* base = b.qkv + static_cast<size_t>(g.row0) * 3 * H;
     SD_TRY(attention<T>(g.B, heads, g.L, g.L, base, 3 * H, base + H, 3 * H, base + 2 * H, 3 * H, pick<T>(w.attn.E), P, g.mask,
                         b.ctx + static_cast<size_t>(g.row0) * H, s, packs ? &(*packs)[gi] : nullptr));
   }
-  SD_TRY(gemm_S(wfmt, M, H, H, b.ctx, w.attn.out, w.attn.out_b, x.s, b.o, s));  // dense + residual (fp32)
-  SD_TRY(ln_modulate<T>(b.o, M, H, true, w.attn.ln_w, w.attn.ln_b, m.cfg.layer_norm_eps, x.s, b.mod, mod_div, 0, b.x1.s, b.x1.t_out(), s, row_graph));
+  SD_TRY(gemm_S(wfmt, Ma, H, H, b.ctx, w.attn.out, w.attn.out_b, x.s, b.o, s));  // dense + residual (fp32)
+  SD_TRY(ln_modulate<T>(b.o, M, H, true, w.attn.ln_w, w.attn.ln_b, m.cfg.layer_norm_eps, x.s, mod, mod_div, 0, b.x1.s, b.x1.t_out(), s, row_graph,
+                        mod_row, Ma, hz ? hz->o_hi : nullptr, hz ? hz->x_hi : nullptr));
   SD_TRY(gemm_T(wfmt, M, 4 * H, H, b.x1.t, w.m0, w.m0_b, 1, b.m1, s));        // GELU
   SD_TRY(gemm_S(wfmt, M, H, 4 * H, b.m1, w.m3, w.m3_b, nullptr, b.m2, s));
-  SD_TRY(ln_modulate<T>(b.m2, M, H, false, nullptr, nullptr, 0.f, b.x1.s, b.mod, mod_div, 3, out.s, out.t_out(), s, row_graph));
+  SD_TRY(ln_modulate<T>(b.m2, M, H, false, nullptr, nullptr, 0.f, b.x1.s, mod, mod_div, 3, out.s, out.t_out(), s, row_graph, mod_row));
   return SEQDIFF_OK;
+}
+
+// The forward's workspace carve.  loop_invariants_t takes its scratch from the same carve, so the debug build's guard bands stay
+// the ones the replayed step writes around.
+template <typename T> struct FwdBufs {
+  float* te;
+  T* teT;
+  float* maskcat;
+  Act<T> x;   // embeddings; reused as the decoder_normalize output
+  Act<T> x2;  // ligand_feature_emb output: [lig | rec]
+  SEBufs<T> sb;
+  T *ccat, *kv_all;
+  Act<T> hbuf[2];
+  float* obuf3;     // third rotating pre-LN buffer (16-bit modes)
+  float2* lnstats;  // (mean, rstd) of the three LayerNorms of a layer
+  T *cq, *y, *ffn;
+};
+template <typename T>
+static FwdBufs<T> carve_forward(uint8_t* ws, cudaStream_t s, int B, int H, int I, int NL, int Mlp, int Mrp, int Ml, int Mr) {
+  constexpr bool k16 = !std::is_same<T, float>::value;
+  const size_t MtH = static_cast<size_t>(Ml + Mr) * H, MlH = static_cast<size_t>(Ml) * H;
+  Bump bp(ws, s);
+  FwdBufs<T> f;
+  f.te = bp.take<float>(static_cast<size_t>(B) * H);
+  f.teT = k16 ? bp.take<T>(static_cast<size_t>(B) * H) : reinterpret_cast<T*>(f.te);
+  f.maskcat = bp.take<float>(static_cast<size_t>(Mlp) + Mrp);
+  f.x = take_act<T>(bp, MtH);
+  f.x2 = take_act<T>(bp, MtH);
+  f.sb.x1 = take_act<T>(bp, MtH);
+  f.sb.o = bp.take<float>(MtH);
+  f.sb.m2 = bp.take<float>(MtH);
+  f.ccat = bp.take<T>(MtH);
+  f.sb.u = bp.take<T>(MtH);
+  f.sb.ctx = bp.take<T>(MtH);
+  f.sb.mod = bp.take<T>(MtH * 6);
+  f.sb.qkv = bp.take<T>(MtH * 3);
+  f.sb.m1 = bp.take<T>(MtH * 4);
+  f.kv_all = bp.take<T>(static_cast<size_t>(Mr) * NL * 2 * H);
+  f.hbuf[0] = take_act<T>(bp, MlH);
+  f.hbuf[1] = take_act<T>(bp, MlH);
+  f.obuf3 = bp.take<float>(MlH);
+  f.lnstats = bp.take<float2>(3 * static_cast<size_t>(Ml));
+  f.cq = bp.take<T>(MlH);
+  f.y = bp.take<T>(MlH);
+  f.ffn = bp.take<T>(static_cast<size_t>(Ml) * I);
+  return f;
 }
 
 
 template <typename T>
 int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t,
                      const float* lig_angle, const float* lig_mask, const float* rec_seq_in, const float* rec_angle,
-                     const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk) {
+                     const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk, const LoopInv* inv) {
   constexpr bool k16 = !std::is_same<T, float>::value;
   const int H = cfg.hidden_size, I = cfg.intermediate_size, NL = cfg.num_hidden_layers, heads = cfg.num_attention_heads;
   const int P = cfg.max_position_embeddings;
@@ -797,38 +861,27 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
   // packed (ragged) batch: only the valid prefix of every graph is a row; inputs, masks and logits keep their padded layouts
   const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : B * Lr, Mt = Ml + Mr;
   const int Mlp = B * Ll, Mrp = B * Lr;  // padded row counts (input tensors, key masks)
-  const size_t MtH = static_cast<size_t>(Mt) * H, MlH = static_cast<size_t>(Ml) * H;
-  Bump bp(ws, s);
-  float* te = bp.take<float>(static_cast<size_t>(B) * H);
-  T* teT = k16 ? bp.take<T>(static_cast<size_t>(B) * H) : reinterpret_cast<T*>(te);
-  float* maskcat = bp.take<float>(static_cast<size_t>(Mlp) + Mrp);
-  Act<T> x = take_act<T>(bp, MtH);   // embeddings; reused as the decoder_normalize output
-  Act<T> x2 = take_act<T>(bp, MtH);  // ligand_feature_emb output: [lig | rec]
-  SEBufs<T> sb;
-  sb.x1 = take_act<T>(bp, MtH);
-  sb.o = bp.take<float>(MtH);
-  sb.m2 = bp.take<float>(MtH);
-  T* ccat = bp.take<T>(MtH);
-  sb.u = bp.take<T>(MtH);
-  sb.ctx = bp.take<T>(MtH);
-  sb.mod = bp.take<T>(MtH * 6);
-  sb.qkv = bp.take<T>(MtH * 3);
-  sb.m1 = bp.take<T>(MtH * 4);
-  T* kv_all = bp.take<T>(static_cast<size_t>(Mr) * NL * 2 * H);
-  Act<T> hbuf[2] = {take_act<T>(bp, MlH), take_act<T>(bp, MlH)};
-  float* obuf3 = bp.take<float>(MlH);                                   // third rotating pre-LN buffer (16-bit modes)
-  float2* lnstats = bp.take<float2>(3 * static_cast<size_t>(Ml));        // (mean, rstd) of the three LayerNorms of a layer
-  T* cq = bp.take<T>(MlH);
-  T* y = bp.take<T>(MlH);
-  T* ffn = bp.take<T>(static_cast<size_t>(Ml) * I);
+  const size_t MlH = static_cast<size_t>(Ml) * H;
+  const FwdBufs<T> f = carve_forward<T>(ws, s, B, H, I, NL, Mlp, Mrp, Ml, Mr);
+  float* te = f.te;
+  T* teT = f.teT;
+  const Act<T> x = f.x, x2 = f.x2;
+  SEBufs<T> sb = f.sb;
+  T *ccat = f.ccat, *kv_all = f.kv_all, *cq = f.cq, *y = f.y, *ffn = f.ffn;
+  const Act<T>* hbuf = f.hbuf;
+  float2* lnstats = f.lnstats;
 
-  // timestep features + the four BertEmbeddings (model.py:211-213,219-220)
-  SD_TRY(timestep_embed(timestep, step_ptr, ts_W, B, H, te, k16 ? static_cast<void*>(teT) : nullptr, Fmt<T>::v, s));
+  // timestep features + the four BertEmbeddings (model.py:211-213,219-220).  Sampling loop (inv): the receptor sequence embedding
+  // and the timestep features of every step are in inv; the angle embeddings stay here, because c = LN(Linear(angles)) + te is
+  // rounded to the operand type after the add.
+  if (!inv) SD_TRY(timestep_embed(timestep, step_ptr, ts_W, B, H, te, k16 ? static_cast<void*>(teT) : nullptr, Fmt<T>::v, s));
   const Act<T> xr = offset(x, MlH);
   {
-    auto job = [&](const float* in, int M, const EmbW& e, const float* te_, int L, float* o32, T* oT, bool lig) {
+    const float* te_ = inv ? inv->te : te;
+    auto job = [&](const float* in, int M, const EmbW& e, bool cond, int L, float* o32, T* oT, bool lig) {
       EmbedJob jb{};
-      jb.x = in; jb.Wt = e.Wt_; jb.b = e.b; jb.lnw = e.ln_w; jb.lnb = e.ln_b; jb.te = te_;
+      jb.x = in; jb.Wt = e.Wt_; jb.b = e.b; jb.lnw = e.ln_w; jb.lnb = e.ln_b; jb.te = cond ? te_ : nullptr;
+      jb.te_row = cond && inv ? step_ptr : nullptr;
       jb.out32 = o32; jb.outT = oT; jb.M = M; jb.fin = e.fin; jb.L = L;
       if (pk) {
         jb.src_rows = lig ? pk->src_l : pk->src_r;
@@ -837,26 +890,34 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
       return jb;
     };
     EmbedJobs jobs{};
-    jobs.n = 4;
-    jobs.j[0] = job(x_t, Ml, lig_seq, nullptr, Ll, x.s, x.t_out(), true);
-    jobs.j[1] = job(rec_seq_in, Mr, rec_seq, nullptr, Lr, xr.s, xr.t_out(), false);
+    jobs.j[jobs.n++] = job(x_t, Ml, lig_seq, false, Ll, x.s, x.t_out(), true);
+    if (!inv) jobs.j[jobs.n++] = job(rec_seq_in, Mr, rec_seq, false, Lr, xr.s, xr.t_out(), false);
     // the conditioning c = LN(Linear(angles)) + te only ever feeds a GEMM: operand type only
-    jobs.j[2] = job(lig_angle, Ml, lig_ang, te, Ll, k16 ? nullptr : reinterpret_cast<float*>(ccat), k16 ? ccat : nullptr, true);
-    jobs.j[3] = job(rec_angle, Mr, rec_ang, te, Lr, k16 ? nullptr : reinterpret_cast<float*>(ccat + MlH), k16 ? ccat + MlH : nullptr, false);
-    if (Ll == Lr) {  // stacked [lig | rec] key mask for the one-pass ligand_feature_emb attention (always the PADDED masks)
-      jobs.cat_dst = maskcat; jobs.cat_a = lig_mask; jobs.cat_b = rec_mask; jobs.cat_na = Mlp; jobs.cat_nb = Mrp;
+    jobs.j[jobs.n++] = job(lig_angle, Ml, lig_ang, true, Ll, k16 ? nullptr : reinterpret_cast<float*>(ccat), k16 ? ccat : nullptr, true);
+    jobs.j[jobs.n++] = job(rec_angle, Mr, rec_ang, true, Lr, k16 ? nullptr : reinterpret_cast<float*>(ccat + MlH), k16 ? ccat + MlH : nullptr, false);
+    if (Ll == Lr && !inv) {  // stacked [lig | rec] key mask for the one-pass ligand_feature_emb attention (always the PADDED masks)
+      jobs.cat_dst = f.maskcat; jobs.cat_a = lig_mask; jobs.cat_b = rec_mask; jobs.cat_na = Mlp; jobs.cat_nb = Mrp;
     }
     SD_TRY(embed_ln_multi<T>(jobs, eps, H, s));
   }
 
-  // ligand_feature_emb on ligand AND receptor tokens in one pass (model.py:214-224, quirk Q1)
+  // ligand_feature_emb on ligand AND receptor tokens in one pass (model.py:214-224, quirk Q1).  Sampling loop: its attention
+  // sublayer sees the receptor embedding alone (the conditioning enters after it), so only the ligand rows run through it here and
+  // the receptor rows of its output come from inv->o.
   std::vector<Segment> segs;
   std::vector<AttnPack> packs;
   AttnPack pk_self{}, pk_cross{};
   if (pk) {
+    pk_self = AttnPack{pk->off_l, pk->off_l, pk->len_l, Ml, Ml, Ll};
+    pk_cross = AttnPack{pk->off_l, pk->off_r, pk->len_l, Ml, Mr, Lr};
+  }
+  if (inv) {
+    segs.push_back({0, B, pk ? pk->max_l : Ll, lig_mask});
+    if (pk) packs.push_back(pk_self);
+  } else if (pk) {
     // offsets are absolute rows of the stacked matrix, so every segment starts at row 0
     if (Ll == Lr) {
-      segs.push_back({0, 2 * B, pk->max_l > pk->max_r ? pk->max_l : pk->max_r, maskcat});
+      segs.push_back({0, 2 * B, pk->max_l > pk->max_r ? pk->max_l : pk->max_r, f.maskcat});
       packs.push_back(AttnPack{pk->off_cat, pk->off_cat, pk->len_cat, Mt, Mt, Ll});
     } else {
       segs.push_back({0, B, pk->max_l, lig_mask});
@@ -864,10 +925,8 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
       segs.push_back({0, B, pk->max_r, rec_mask});
       packs.push_back(AttnPack{pk->off_cat + B, pk->off_cat + B, pk->len_cat + B, Mt, Mt, Lr});
     }
-    pk_self = AttnPack{pk->off_l, pk->off_l, pk->len_l, Ml, Ml, Ll};
-    pk_cross = AttnPack{pk->off_l, pk->off_r, pk->len_l, Ml, Mr, Lr};
   } else if (Ll == Lr) {
-    segs.push_back({0, 2 * B, Ll, maskcat});
+    segs.push_back({0, 2 * B, Ll, f.maskcat});
   } else {
     segs.push_back({0, B, Ll, lig_mask});
     segs.push_back({Ml, B, Lr, rec_mask});
@@ -875,7 +934,8 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
   const int Lq_self = pk ? pk->max_l : Ll, Lk_cross = pk ? pk->max_r : Lr;
   const AttnPack* aps = pk ? &pk_self : nullptr;
   const AttnPack* apc = pk ? &pk_cross : nullptr;
-  SD_TRY(se_layer<T>(*this, wfmt, se_lig, x, ccat, Mt, 1, Mt, segs, sb, x2, s, pk ? &packs : nullptr, nullptr));
+  const SEHoist<T> hz_lig{Ml, inv ? inv->o : nullptr, inv ? inv->xr : nullptr, nullptr, nullptr};
+  SD_TRY(se_layer<T>(*this, wfmt, se_lig, x, ccat, Mt, 1, Mt, segs, sb, x2, s, pk ? &packs : nullptr, nullptr, inv ? &hz_lig : nullptr));
   const T* rec = x2.t + MlH;
 
   // decoder: 6 x (self-attn -> cross-attn -> FFN), post-LN (HF BertLayer; model.py:226-231)
@@ -887,7 +947,7 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
     // (mean, rstd) the LN kernel emits and the LN affine -- the same fp32 formula, so bit-identical -- which lets the LN kernel
     // skip its 3 KB/row fp32 copy.  o needs three buffers with fixed roles (oA, oB, oC): every GEMM reads its residual from a
     // different buffer than the one it writes (attn_out: oC of the previous layer -> oA; cross_out: oA -> oB; ffn_down: oB -> oC).
-    float* obuf[3] = {sb.o, sb.m2, obuf3};
+    float* obuf[3] = {sb.o, sb.m2, f.obuf3};
     LnResid prev{};        // how to rebuild the current residual-stream value from `o_prev` (layer >= 1)
     const float* o_prev = nullptr;
     for (int i = 0; i < NL; ++i) {
@@ -940,11 +1000,13 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
     }
   }
 
-  // decoder_normalize: SELayer conditioned on the timestep only (c broadcast over L; model.py:232-235)
+  // decoder_normalize: SELayer conditioned on the timestep only (c broadcast over L; model.py:232-235).  Sampling loop: its
+  // modulation is row *step_ptr of inv->mod.
   std::vector<Segment> lseg{{0, B, Lq_self, lig_mask}};
   std::vector<AttnPack> lpack;
   if (pk) lpack.push_back(pk_self);
-  SD_TRY(se_layer<T>(*this, wfmt, se_dec, h, teT, B, Ll, Ml, lseg, sb, x, s, pk ? &lpack : nullptr, pk ? pk->graph : nullptr));
+  const SEHoist<T> hz_dec{Ml, nullptr, nullptr, inv ? static_cast<const T*>(inv->mod) : nullptr, step_ptr};
+  SD_TRY(se_layer<T>(*this, wfmt, se_dec, h, teT, B, Ll, Ml, lseg, sb, x, s, pk ? &lpack : nullptr, pk ? pk->graph : nullptr, inv ? &hz_dec : nullptr));
 
   // AminoAcidPredictor (model.py:148-153)
   if constexpr (std::is_same<T, bf16>::value) {
@@ -966,12 +1028,13 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
 
 int Model::forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t,
                    const float* lig_angle, const float* lig_mask, const float* rec_seq_in, const float* rec_angle,
-                   const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk) {
+                   const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk, const LoopInv* inv) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
   SD_CHECK(arch == kArchSequence, "handle holds a structure model: use seqdiff_struct_forward");
   SD_CHECK(!pk || precision != SEQDIFF_FP32, "ragged packing runs in the 16-bit modes");
   SD_CHECK(precision >= SEQDIFF_FP32 && precision <= SEQDIFF_FP16, "unknown precision mode");
   SD_CHECK(B > 0 && Ll > 0 && Lr > 0, "empty batch");
+  SD_CHECK(!inv || step_ptr, "the sampling-loop invariants are indexed by the device step counter");
   if (cfg.relative_key) SD_CHECK(Ll <= cfg.max_position_embeddings && Lr <= cfg.max_position_embeddings, "Length exceed");
   SD_CUDA(cudaSetDevice(device));
   SD_TRY(ensure_workspace(workspace_need(precision, B, Ll, Lr)));
@@ -979,12 +1042,46 @@ int Model::forward(int precision, int B, int Ll, int Lr, const float* timestep, 
   const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * (Ll + Lr)));
   switch (precision) {
     case SEQDIFF_FP32:
-      return forward_t<float>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, nullptr);
+      return forward_t<float>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, nullptr, inv);
     case SEQDIFF_BF16:
-      return forward_t<bf16>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk);
+      return forward_t<bf16>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk, inv);
     default:  // SEQDIFF_FP16
-      return forward_t<f16>(0, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk);
+      return forward_t<f16>(0, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk, inv);
   }
+}
+
+// The per-sampling part of the loop (LoopInv): the kernels forward_t runs on the same inputs, so every value is the one the
+// stand-alone forward computes at every step.  None of them splits K, so a GEMM row's result does not depend on M (T rows of steps
+// here, B rows of one step there), and attention items are per (graph, head), so the receptor graphs give the same result without
+// the ligand graphs next to them.
+template <typename T>
+int Model::loop_invariants_t(int wfmt, int B, int Ll, int Lr, int T_, const float* rec_seq_in, const float* rec_mask, const LoopInv& iv,
+                             cudaStream_t s, const PackInfo* pk) {
+  constexpr bool k16 = !std::is_same<T, float>::value;
+  const int H = cfg.hidden_size, heads = cfg.num_attention_heads, P = cfg.max_position_embeddings;
+  const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : B * Lr;
+  const FwdBufs<T> f = carve_forward<T>(ws, s, B, H, cfg.intermediate_size, cfg.num_hidden_layers, B * Ll, B * Lr, Ml, Mr);
+  // timestep features of steps 0 .. T-1 (row i: t = i, as (float)*step_ptr gives it) and decoder_normalize's adaLN GEMMs on them
+  SD_TRY(timestep_embed(nullptr, nullptr, ts_W, T_, H, iv.te, k16 ? iv.teT : nullptr, Fmt<T>::v, s));
+  SD_TRY(gemm_T(wfmt, T_, H, H, static_cast<const T*>(iv.teT), se_dec.ada0, se_dec.ada0_b, 2, static_cast<T*>(iv.u), s));
+  SD_TRY(gemm_T(wfmt, T_, 6 * H, H, static_cast<const T*>(iv.u), se_dec.ada2, se_dec.ada2_b, 0, static_cast<T*>(iv.mod), s));
+  // receptor sequence embedding
+  EmbedJobs jobs{};
+  jobs.n = 1;
+  EmbedJob& jb = jobs.j[0];
+  jb.x = rec_seq_in; jb.Wt = rec_seq.Wt_; jb.b = rec_seq.b; jb.lnw = rec_seq.ln_w; jb.lnb = rec_seq.ln_b;
+  jb.out32 = iv.xr; jb.outT = k16 ? iv.xrT : nullptr; jb.M = Mr; jb.fin = rec_seq.fin; jb.L = Lr;
+  if (pk) jb.src_rows = pk->src_r;
+  SD_TRY(embed_ln_multi<T>(jobs, cfg.layer_norm_eps, H, s));
+  // receptor rows of ligand_feature_emb's attention sublayer up to its output dense + residual (se_layer)
+  const AttnW& a = se_lig.attn;
+  T* qkv = f.sb.qkv;
+  SD_TRY(gemm_T(wfmt, Mr, 3 * H, H, static_cast<const T*>(iv.xrT), a.qkv, a.qkv_b, 0, qkv, s));
+  const AttnPack ap = pk ? AttnPack{pk->off_r, pk->off_r, pk->len_r, Mr, Mr, Lr} : AttnPack{};
+  const int Lk = pk ? pk->max_r : Lr;
+  SD_TRY(attention<T>(B, heads, Lk, Lk, qkv, 3 * H, qkv + H, 3 * H, qkv + 2 * H, 3 * H, pick<T>(a.E), P, rec_mask, f.sb.ctx, s, pk ? &ap : nullptr));
+  SD_TRY(gemm_S(wfmt, Mr, H, H, f.sb.ctx, a.out, a.out_b, iv.xr, iv.o, s));
+  return SEQDIFF_OK;
 }
 
 // =====================================================================================================
@@ -1122,14 +1219,44 @@ int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_ta
     }
   }
 
+  // The per-sampling invariants (LoopInv), computed here by every call, outside the graph: the graph only holds their addresses.
+  // Receptor rows first (B * Lr, the packed rows are a prefix), then the step tables with a grow-only capacity, so a cached graph
+  // serves any T up to it.
+  {
+    inv.rows = T > inv.rows ? T : inv.rows;
+    const size_t es = precision == SEQDIFF_FP32 ? 4 : 2, NrH = Nr * cfg.hidden_size, tH = static_cast<size_t>(inv.rows) * cfg.hidden_size;
+    const size_t need_inv = 2 * align256(NrH * 4) + align256(NrH * 2) + align256(tH * 4) + align256(tH * 2) + align256(tH * es) +
+                            align256(tH * 6 * es) + 8 * kGuardBytes;
+    if (need_inv > samp_inv_bytes) {
+      if (samp_inv) { SD_CUDA(cudaDeviceSynchronize()); debug_guard_begin(samp_inv); SD_CUDA(cudaFree(samp_inv)); samp_inv = nullptr; samp_inv_bytes = 0; }
+      SD_CUDA(cudaMalloc(reinterpret_cast<void**>(&samp_inv), need_inv));
+      samp_inv_bytes = need_inv;
+    }
+    Bump bi(samp_inv, s);
+    inv.xr = bi.take<float>(NrH);
+    inv.xrT = es == 2 ? static_cast<void*>(bi.take<uint16_t>(NrH)) : inv.xr;
+    inv.o = bi.take<float>(NrH);
+    inv.te = bi.take<float>(tH);
+    inv.teT = es == 2 ? static_cast<void*>(bi.take<uint16_t>(tH)) : inv.te;
+    inv.u = bi.take<uint8_t>(tH * es);
+    inv.mod = bi.take<uint8_t>(tH * 6 * es);
+    const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * (Ll + Lr)));
+    switch (precision) {
+      case SEQDIFF_FP32: SD_TRY(loop_invariants_t<float>(1, B, Ll, Lr, T, c_rseq, c_rmask, inv, s, nullptr)); break;
+      case SEQDIFF_BF16: SD_TRY(loop_invariants_t<bf16>(1, B, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
+      default: SD_TRY(loop_invariants_t<f16>(0, B, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
+    }
+  }
+
   GraphKey key;
   key.pack_hash = pk ? pk->hash : 0;
   key.precision = precision; key.B = B; key.Ll = Ll; key.Lr = Lr; key.diverse = diverse; key.noise = noise_E;
   key.ws_ptr = ws; key.in_ptr = samp_in; key.tab_ptr = d_tables;  // (seed, gid0) are NOT part of the key: device memory, see arm_loop_kernel
+  key.inv_ptr = samp_inv; key.inv_rows = inv.rows;
   uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
   auto one_step = [&](cudaStream_t st) -> int {
     const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * (Ll + Lr)));
-    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, st, pk));
+    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, st, pk, &inv));
     SD_TRY(reverse_step(d_tables, 1, B, Ll, x_cur, logits, diverse, noise_E, 0, 0, 0, d_step, x_cur, nullptr, st, d_step + 1, d_rng));
     return SEQDIFF_OK;
   };
@@ -1138,7 +1265,7 @@ int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_ta
     // un-captured dry run of the forward: sets kernel attributes and fills the TMA descriptor cache
     SD_CUDA(launch_k(set_int_kernel, dim3(1), dim3(1), 0, s, d_step, T - 1));
     SD_LAUNCHED("set_int", s);
-    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, s, pk));
+    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, s, pk, &inv));
     SD_CUDA(cudaStreamSynchronize(s));
     cudaGraph_t graph = nullptr;
     const uint64_t l0 = g_launches.load();

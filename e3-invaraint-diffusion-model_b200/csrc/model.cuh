@@ -89,6 +89,22 @@ struct PackInfo {
   uint64_t hash = 0;              // of the length vectors (part of the CUDA-graph key)
 };
 
+// What the sequence model's sampling loop computes once per sampling instead of once per step (Model::sample).  Every graph of the
+// batch shares the step index and x_t is the only other input that changes between steps, so the receptor embedding, the receptor
+// half of ligand_feature_emb's attention sublayer (its input is the receptor embedding alone), the timestep features and
+// decoder_normalize's modulation (a function of the timestep features alone) are the same at every step.  The buffers are carved
+// from the handle's samp_inv block; receptor rows are [Mr, H] in the row order of the step's token matrix (packed or padded).
+struct LoopInv {
+  int rows = 0;          // table capacity in steps (>= T of the sampling)
+  float* xr = nullptr;   // [Mr, H] receptor embedding, fp32 stream
+  void* xrT = nullptr;   // [Mr, H] its operand copy (== xr in fp32 mode)
+  float* o = nullptr;    // [Mr, H] receptor rows of ligand_feature_emb's attention output (dense + residual, before its LayerNorm)
+  float* te = nullptr;   // [rows, H] timestep features of step i in row i
+  void* teT = nullptr;   // [rows, H] operand copy (== te in fp32 mode)
+  void* u = nullptr;     // [rows, H] SiLU(adaLN_modulation.0) of decoder_normalize (scratch of the table)
+  void* mod = nullptr;   // [rows, 6H] decoder_normalize's modulation (shift, scale, gate) x 2 of step i in row i
+};
+
 enum Arch { kArchSequence = 0, kArchStructure = 1 };
 
 struct Model {
@@ -120,6 +136,9 @@ struct Model {
   size_t tables_cap = 0;
   uint8_t* samp_in = nullptr;  // persistent copies of the loop inputs + x_t + logits
   size_t samp_in_bytes = 0;
+  uint8_t* samp_inv = nullptr;  // the LoopInv buffers (grow-only)
+  size_t samp_inv_bytes = 0;
+  LoopInv inv;
   cudaGraphExec_t graph_exec = nullptr;
   int graph_kernels = 0;
   cudaStream_t loop_stream = nullptr;  // private stream: graphs cannot be captured on the legacy default stream
@@ -131,11 +150,13 @@ struct Model {
     const void* in_ptr = nullptr;
     const void* tab_ptr = nullptr;
     const void* aux_ptr = nullptr;
+    const void* inv_ptr = nullptr;
+    int inv_rows = 0;  // with B, Lr and the precision: the layout of the LoopInv buffers
     int T = 0;
     uint64_t pack_hash = 0;
     bool operator==(const GraphKey& o) const {
       return pack_hash == o.pack_hash && aux_ptr == o.aux_ptr && T == o.T && precision == o.precision && B == o.B && Ll == o.Ll && Lr == o.Lr && diverse == o.diverse && noise == o.noise &&
-             ws_ptr == o.ws_ptr && in_ptr == o.in_ptr && tab_ptr == o.tab_ptr;
+             ws_ptr == o.ws_ptr && in_ptr == o.in_ptr && tab_ptr == o.tab_ptr && inv_ptr == o.inv_ptr && inv_rows == o.inv_rows;
     }
   } graph_key;
 
@@ -143,9 +164,11 @@ struct Model {
   int init(const seqdiff_config_t& c, int dev, int arch_ = kArchSequence);
   int set_tensor(const char* name, const float* data, int64_t numel, cudaStream_t s);
   int finalize(cudaStream_t s);
+  // inv != NULL (sampling loop, with step_ptr): the step reads what loop_invariants_t() left in `inv` instead of recomputing it;
+  // rec_seq is not read then
   int forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t,
               const float* lig_angle, const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask,
-              float* logits, cudaStream_t s, const PackInfo* pk = nullptr);
+              float* logits, cudaStream_t s, const PackInfo* pk = nullptr, const LoopInv* inv = nullptr);
   // flags bit 0: ragged packing (valid positions bit-identical to the padded computation; padded positions of final_out are 0)
   int sample(int precision, int B, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
              const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, int diverse,
@@ -212,7 +235,11 @@ struct Model {
   template <typename T>
   int forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t, const float* lig_angle,
                 const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, float* logits,
-                cudaStream_t s, const PackInfo* pk);
+                cudaStream_t s, const PackInfo* pk, const LoopInv* inv);
+  // fills `inv` for a sampling of T_ <= inv.rows steps (Model::sample); scratch from the forward's workspace
+  template <typename T>
+  int loop_invariants_t(int wfmt, int B, int Ll, int Lr, int T_, const float* rec_seq, const float* rec_mask, const LoopInv& inv, cudaStream_t s,
+                        const PackInfo* pk);
 };
 
 }  // namespace seqdiff

@@ -54,7 +54,7 @@ __global__ void timestep_embed_kernel(const float* __restrict__ timestep, const 
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * half) return;
   const int b = i / half, j = i % half;
-  const float t = step_ptr ? static_cast<float>(*step_ptr) : timestep[b];
+  const float t = step_ptr ? static_cast<float>(*step_ptr) : (timestep ? timestep[b] : static_cast<float>(b));
   // x[:, None] * W[None, :] * 2 * torch.pi  -> three separately rounded fp32 multiplies (model.py:95)
   const float x = __fmul_rn(__fmul_rn(__fmul_rn(t, W[j]), 2.0f), 3.14159274101257324f);
   const float sv = sinf(x), cv = cosf(x);
@@ -175,7 +175,8 @@ __global__ void __launch_bounds__(kRowThreads, 2) embed_ln_multi_kernel(const __
       }
       float mean, rstd;
       row_stats<VPL>(v, H, eps, mean, rstd);
-      const float* terow = job.te ? job.te + static_cast<size_t>(job.row_graph ? __ldg(job.row_graph + tok0 + t) : (tok0 + t) / job.L) * H : nullptr;
+      const int te_r = job.te_row ? *job.te_row : (job.row_graph ? __ldg(job.row_graph + tok0 + t) : (tok0 + t) / job.L);
+      const float* terow = job.te ? job.te + static_cast<size_t>(te_r) * H : nullptr;
 #pragma unroll
       for (int i = 0; i < VPL; ++i) {
         float g8[8], b8[8];
@@ -315,14 +316,17 @@ template <typename T, int VPL, bool AFFINE_FIRST>
 __global__ void __launch_bounds__(kRowThreads) ln_modulate_kernel(const float* __restrict__ in, int M, int H, const float* __restrict__ lnw,
                                                                   const float* __restrict__ lnb, float eps1, const float* __restrict__ x,
                                                                   const T* __restrict__ mod, int mod_div, int chunk0,
-                                                                  float* __restrict__ out32, T* __restrict__ outT, const int* __restrict__ row_graph) {
+                                                                  float* __restrict__ out32, T* __restrict__ outT, const int* __restrict__ row_graph,
+                                                                  const int* __restrict__ mod_row, int split, const float* __restrict__ in_hi,
+                                                                  const float* __restrict__ x_hi) {
   pdl_trigger();
   pdl_wait();  // predecessor grid complete + flushed before any dependent global access
   const int lane = threadIdx.x & 31;
   const int row = (blockIdx.x * kRowThreads + threadIdx.x) >> 5;
   if (row >= M) return;
+  const bool hi = in_hi && row >= split;
   float v[VPL][8];
-  load_row<float, VPL>(in + static_cast<size_t>(row) * H, lane, v);
+  load_row<float, VPL>(hi ? in_hi + static_cast<size_t>(row - split) * H : in + static_cast<size_t>(row) * H, lane, v);
   float mean, rstd;
   if (AFFINE_FIRST) {  // BertSelfOutput.LayerNorm (eps 1e-12, affine) -- output of self.attn(x, mask)[0]
     row_stats<VPL>(v, H, eps1, mean, rstd);
@@ -337,8 +341,10 @@ __global__ void __launch_bounds__(kRowThreads) ln_modulate_kernel(const float* _
   }
   row_stats<VPL>(v, H, 1e-5f, mean, rstd);  // SELayer.norm1/norm2: elementwise_affine=False, default eps
   SD_DEV_ASSERT(!row_graph || __ldg(row_graph + row) >= 0);
-  const T* mrow = mod + static_cast<size_t>(row_graph ? __ldg(row_graph + row) : row / mod_div) * (6 * H);
-  const float* xrow = x + static_cast<size_t>(row) * H;
+  SD_DEV_ASSERT(!mod_row || *mod_row >= 0);
+  const int mr = mod_row ? *mod_row : (row_graph ? __ldg(row_graph + row) : row / mod_div);
+  const T* mrow = mod + static_cast<size_t>(mr) * (6 * H);
+  const float* xrow = hi ? x_hi + static_cast<size_t>(row - split) * H : x + static_cast<size_t>(row) * H;
 #pragma unroll
   for (int i = 0; i < VPL; ++i) {
     const int e = (i * 32 + lane) * 8;
@@ -359,18 +365,23 @@ __global__ void __launch_bounds__(kRowThreads) ln_modulate_kernel(const float* _
 
 template <typename T>
 int ln_modulate(const float* in, int M, int H, bool affine_first, const float* lnw, const float* lnb, float eps1, const float* x,
-                const T* mod, int mod_div, int chunk0, float* out32, T* outT, cudaStream_t s, const int* row_graph) {
+                const T* mod, int mod_div, int chunk0, float* out32, T* outT, cudaStream_t s, const int* row_graph, const int* mod_row, int split,
+                const float* in_hi, const float* x_hi) {
+  SD_CHECK(!in_hi == !x_hi && (!in_hi || (split >= 0 && split <= M)), "ln_modulate: split sources need both in_hi and x_hi and 0 <= split <= M");
   const int grid = ceil_div(M * 32, kRowThreads);
   if (affine_first) {
-    SD_VPL_DISPATCH(H, SD_CUDA(launch_k(ln_modulate_kernel<T, VPL, true>, dim3(grid), dim3(kRowThreads), 0, s, in, M, H, lnw, lnb, eps1, x, mod, mod_div, chunk0, out32, outT, row_graph)));
+    SD_VPL_DISPATCH(H, SD_CUDA(launch_k(ln_modulate_kernel<T, VPL, true>, dim3(grid), dim3(kRowThreads), 0, s, in, M, H, lnw, lnb, eps1, x, mod, mod_div, chunk0, out32, outT, row_graph,
+                                        mod_row, split, in_hi, x_hi)));
   } else {
-    SD_VPL_DISPATCH(H, SD_CUDA(launch_k(ln_modulate_kernel<T, VPL, false>, dim3(grid), dim3(kRowThreads), 0, s, in, M, H, lnw, lnb, eps1, x, mod, mod_div, chunk0, out32, outT, row_graph)));
+    SD_VPL_DISPATCH(H, SD_CUDA(launch_k(ln_modulate_kernel<T, VPL, false>, dim3(grid), dim3(kRowThreads), 0, s, in, M, H, lnw, lnb, eps1, x, mod, mod_div, chunk0, out32, outT, row_graph,
+                                        mod_row, split, in_hi, x_hi)));
   }
   SD_LAUNCHED("ln_modulate", s);
   return SEQDIFF_OK;
 }
-#define SD_INST_LNMOD(T) \
-  template int ln_modulate<T>(const float*, int, int, bool, const float*, const float*, float, const float*, const T*, int, int, float*, T*, cudaStream_t, const int*)
+#define SD_INST_LNMOD(T)                                                                                                                                  \
+  template int ln_modulate<T>(const float*, int, int, bool, const float*, const float*, float, const float*, const T*, int, int, float*, T*, cudaStream_t, \
+                              const int*, const int*, int, const float*, const float*)
 SD_INST_LNMOD(float);
 SD_INST_LNMOD(bf16);
 SD_INST_LNMOD(f16);
