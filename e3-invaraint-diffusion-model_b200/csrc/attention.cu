@@ -360,43 +360,44 @@ static int attn_choice() {
 #endif
 template <typename T>
 static int attention_any16(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const T* dist_emb,
-                           int P, const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack) {
+                           int P, const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack, int kv_div) {
 #ifdef SEQDIFF_AB_KERNELS
   const int c = attn_choice();
   if (c != 0 && !pack) {
+    SD_CHECK(kv_div == 1, "the A/B reference attention kernels read the keys of their own graph only");
     // "auto_r1": the per-shape choice before the pipelined kernel existed (legacy for one-key-block relative_key, tc otherwise)
     const bool legacy = c == 2 || (c == 3 && dist_emb != nullptr && Lk <= kKB);
     if (legacy) return attention_16<T>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s);
     return attention_tc<T>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s);
   }
 #endif
-  return attention_pipe<T>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack);
+  return attention_pipe<T>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack, kv_div);
 }
 template <>
 int attention<bf16>(int B, int heads, int Lq, int Lk, const bf16* q, int ldq, const bf16* k, int ldk, const bf16* v, int ldv,
-                    const bf16* dist_emb, int P, const float* key_mask, bf16* out, cudaStream_t s, const AttnPack* pack) {
-  return attention_any16<bf16>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack);
+                    const bf16* dist_emb, int P, const float* key_mask, bf16* out, cudaStream_t s, const AttnPack* pack, int kv_div) {
+  return attention_any16<bf16>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack, kv_div);
 }
 template <>
 int attention<f16>(int B, int heads, int Lq, int Lk, const f16* q, int ldq, const f16* k, int ldk, const f16* v, int ldv,
-                   const f16* dist_emb, int P, const float* key_mask, f16* out, cudaStream_t s, const AttnPack* pack) {
-  return attention_any16<f16>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack);
+                   const f16* dist_emb, int P, const float* key_mask, f16* out, cudaStream_t s, const AttnPack* pack, int kv_div) {
+  return attention_any16<f16>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack, kv_div);
 }
 
 // ---------------------------------------------------------------------------------------------------
-// fp32 parity kernel: one warp per query row; scores for the whole row live in smem.
+// fp32 parity kernel: one warp per query row; scores for the whole row live in smem.  Query graph b reads key graph b / kv_div.
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restrict__ q, int ldq, const float* __restrict__ k, int ldk,
                                                             const float* __restrict__ v, int ldv, const float* __restrict__ E, int P,
                                                             const float* __restrict__ key_mask, float* __restrict__ out, int heads,
-                                                            int Lq, int Lk) {
+                                                            int Lq, int Lk, int kv_div) {
   extern __shared__ float sm[];
   pdl_trigger();
   pdl_wait();  // predecessor grid complete + flushed before any dependent global access
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float* sq = sm + warp * 64;
   float* sc = sm + 8 * 64 + warp * Lk;
-  const int l = blockIdx.x * 8 + warp, h = blockIdx.y, b = blockIdx.z;
+  const int l = blockIdx.x * 8 + warp, h = blockIdx.y, b = blockIdx.z, kg = b / kv_div;
   if (l >= Lq) return;
   const float* qrow = q + (static_cast<size_t>(b) * Lq + l) * ldq + h * 64;
   sq[lane] = qrow[lane];
@@ -404,7 +405,7 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restr
   __syncwarp();
   float mx = -INFINITY;
   for (int r = lane; r < Lk; r += 32) {
-    const float* kr = k + (static_cast<size_t>(b) * Lk + r) * ldk + h * 64;
+    const float* kr = k + (static_cast<size_t>(kg) * Lk + r) * ldk + h * 64;
     float acc = 0.f, rel = 0.f;
 #pragma unroll 4
     for (int d = 0; d < 64; d += 4) {
@@ -421,7 +422,7 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restr
         rel = fmaf(sq[d + 2], ee.z, rel); rel = fmaf(sq[d + 3], ee.w, rel);
       }
     }
-    const float sv = (acc + rel) / 8.0f + (1.0f - key_mask[static_cast<size_t>(b) * Lk + r]) * -10000.0f;
+    const float sv = (acc + rel) / 8.0f + (1.0f - key_mask[static_cast<size_t>(kg) * Lk + r]) * -10000.0f;
     sc[r] = sv;
     mx = fmaxf(mx, sv);
   }
@@ -437,7 +438,7 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restr
   float a0 = 0.f, a1 = 0.f;
   for (int r = 0; r < Lk; ++r) {
     const float p = sc[r] / sum;
-    const float* vr = v + (static_cast<size_t>(b) * Lk + r) * ldv + h * 64;
+    const float* vr = v + (static_cast<size_t>(kg) * Lk + r) * ldv + h * 64;
     a0 = fmaf(p, vr[lane], a0);
     a1 = fmaf(p, vr[lane + 32], a1);
   }
@@ -448,15 +449,16 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restr
 
 template <>
 int attention<float>(int B, int heads, int Lq, int Lk, const float* q, int ldq, const float* k, int ldk, const float* v, int ldv,
-                     const float* dist_emb, int P, const float* key_mask, float* out, cudaStream_t s, const AttnPack* pack) {
+                     const float* dist_emb, int P, const float* key_mask, float* out, cudaStream_t s, const AttnPack* pack, int kv_div) {
   SD_CHECK(pack == nullptr, "packed batches run in the 16-bit modes only");
   SD_CHECK(B > 0 && heads > 0 && Lq > 0 && Lk > 0, "empty attention");
+  SD_CHECK(kv_div >= 1 && B % kv_div == 0, "every key graph must serve kv_div whole query graphs");
   SD_CHECK(ldq % 4 == 0 && ldk % 4 == 0 && ldv % 4 == 0, "row strides must be multiples of 4 elements");
   SD_CHECK(!dist_emb || (Lq <= P && Lk <= P), "sequence longer than max_position_embeddings");
   const size_t smem = (8 * 64 + 8 * static_cast<size_t>(Lk)) * sizeof(float);
   SD_CHECK(smem <= 48 * 1024, "fp32 attention: Lk too large");
   dim3 grid(ceil_div(Lq, 8), heads, B);
-  SD_CUDA(launch_k(attention_f32_kernel, dim3(grid), dim3(256), smem, s, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, heads, Lq, Lk));
+  SD_CUDA(launch_k(attention_f32_kernel, dim3(grid), dim3(256), smem, s, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, heads, Lq, Lk, kv_div));
   SD_LAUNCHED("attention_f32", s);
   return SEQDIFF_OK;
 }

@@ -74,11 +74,13 @@ __device__ __forceinline__ PipeItem decode_item(int item, int nqb, int heads) {
 }
 // Walks this CTA's step list (item = blockIdx.x + it * gridDim.x; kb = 0..nkb-1) without divisions in the loop: the item
 // stride is decomposed once into (db, dh, dqb) and applied with carries.  (An integer division per step sat on the softmax
-// threads' critical path: ~800 cycles per item in the timeline.)
+// threads' critical path: ~800 cycles per item in the timeline.)  KV: the key graph kg = b / kv_div is carried the same way
+// (kr = b % kv_div); otherwise the key graph is b.
+template <bool KV>
 struct StepCursor {
-  int b, h, qb, kb, it;
-  int db, dh, dqb, nqb, heads, nkb;
-  __device__ __forceinline__ void init(int first_item, int stride, int nqb_, int heads_, int nkb_) {
+  int b, h, qb, kb, it, kg_, kr;
+  int db, dh, dqb, nqb, heads, nkb, dkg, dkr, kv_div;
+  __device__ __forceinline__ void init(int first_item, int stride, int nqb_, int heads_, int nkb_, int kv_div_) {
     nqb = nqb_; heads = heads_; nkb = nkb_;
     const PipeItem w = decode_item(first_item, nqb, heads);
     b = w.b; h = w.h; qb = w.q0 / kPQ; kb = 0; it = 0;
@@ -86,15 +88,32 @@ struct StepCursor {
     const int sh = stride / nqb;
     dh = sh % heads;
     db = sh / heads;
+    if constexpr (KV) {
+      kv_div = kv_div_;
+      kg_ = b / kv_div; kr = b % kv_div;
+      dkg = db / kv_div; dkr = db % kv_div;
+    }
   }
   __device__ __forceinline__ void next_item() {
     qb += dqb;
     if (qb >= nqb) { qb -= nqb; ++h; }
     h += dh;
-    if (h >= heads) { h -= heads; ++b; }
+    if (h >= heads) {
+      h -= heads; ++b;
+      if constexpr (KV) ++kr;
+    }
     b += db;
+    if constexpr (KV) {
+      kr += dkr;
+      kg_ += dkg;
+      if (kr >= kv_div) { kr -= kv_div; ++kg_; }  // kr <= 2 kv_div - 1 here: one subtraction suffices
+    }
     kb = 0;
     ++it;
+  }
+  __device__ __forceinline__ int kg() const {
+    if constexpr (KV) return kg_;
+    else return b;
   }
   __device__ __forceinline__ void next_step() {
     if (++kb == nkb) next_item();
@@ -111,13 +130,16 @@ __global__ void __launch_bounds__(kPipeThreads, 1)
 attention_pipe_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV,
                       const __grid_constant__ CUtensorMap tmE, const __grid_constant__ CUtensorMap tmO, const float* __restrict__ key_mask, int heads, int Lq,
                       int Lk, int P, uint32_t fmt, int nqb, int n_items, unsigned long long* __restrict__ trace, const int* __restrict__ q_off,
-                      const int* __restrict__ k_off, const int* __restrict__ q_len, int Lk_mask, T* __restrict__ out_raw, const DropSpec dr,
-                      uint32_t* __restrict__ keep_out) {
+                      const int* __restrict__ k_off, const int* __restrict__ q_len, int Lk_mask, int kv_div, T* __restrict__ out_raw,
+                      const DropSpec dr, uint32_t* __restrict__ keep_out) {
   // keep_out (DROP, Lq / Lk <= 128, optional): the dropout mask of item (b, h) as bits -- word ((b * heads + h) * 128 + row) * 4 + kc holds
   // keys 32 kc .. 32 kc + 31 of query `row` -- so that the backward kernel reads 8 bytes per thread instead of regenerating 16 Philox calls
   // q_off != NULL: packed (ragged) batch -- graph b's rows start at q_off[b] / k_off[b] of the packed q / k / v matrices, Lq / Lk are
   // the largest lengths of the batch, key_mask keeps its padded pitch Lk_mask, and output rows are stored per thread with a
   // q_len[b] predicate (a bulk tile store would spill into the next graph's rows).
+  // kv_div: query graph b reads the keys, values and key-mask row of graph b / kv_div (carried by the step cursors, no division
+  // per step).  The training-mode kernels (DROP) always read their own graph and leave the cursor without that bookkeeping.
+  using Cursor = StepCursor<!DROP>;
   using C = PipeCfg<REL>;
   constexpr int NKS = C::kNKS, NS = C::kNS, NVS = C::kNVS;
   constexpr float kScale2 = 0.125f * kLog2e;
@@ -183,15 +205,15 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     // (whole warp runs the loop, one elected lane issues: common.cuh "warp-uniform single-issuer variants")
     {
       int g = 0;
-      StepCursor cur;
-      cur.init(static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nqb, heads, nkb);
+      Cursor cur;
+      cur.init(static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nqb, heads, nkb, kv_div);
       for (int it = 0; it < my_items; ++it, cur.next_item()) {
         const PipeItem w = cur.item();
         const int qs = it & 1;
         mbar_wait(&q_empty[qs], ((it >> 1) & 1) ^ 1);
         mbar_expect_tx_e(&q_full[qs], 16384);
         const int q_row0 = q_off ? __ldg(q_off + w.b) : w.b * Lq;
-        const int k_row0 = q_off ? __ldg(k_off + w.b) : w.b * Lk;
+        const int k_row0 = q_off ? __ldg(k_off + cur.kg()) : cur.kg() * Lk;
         tma_load_2d_e(smem + C::kQ + qs * 16384, &tmQ, &q_full[qs], w.h * 64, q_row0 + w.q0);
         for (int kb = 0; kb < nkb; ++kb, ++g) {
           const int ks = g % NKS;
@@ -271,11 +293,11 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     // whole step, so its latency never shows), stored to smem one step ahead, published by that step's barrier
     auto mask_cvt = [&](float raw, bool in_range) -> float { return in_range ? (1.0f - raw) * (-10000.0f * kLog2e) : -INFINITY; };
     // raw mask value of key 128 kb + st for the step the cursor points at (false past the end of the list / for st >= 128)
-    auto mask_fetch = [&](const StepCursor& c, float& raw, bool& in_range) -> bool {
+    auto mask_fetch = [&](const Cursor& c, float& raw, bool& in_range) -> bool {
       if (c.it >= my_items || st >= kPK) return false;
       const int r = c.kb * kPK + st;
       in_range = r < Lk_mask;
-      raw = in_range ? __ldg(key_mask + static_cast<size_t>(c.b) * Lk_mask + r) : 0.f;
+      raw = in_range ? __ldg(key_mask + static_cast<size_t>(c.kg()) * Lk_mask + r) : 0.f;
       return true;
     };
     // O of a finished item -> global.  Each thread scales its 32 of the row's 64 output columns and drops them as 16-bit into
@@ -328,8 +350,8 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
       if (lane == 0) sFlag[parity * 4 + (st >> 5)] = (any != 0u || (first_step_of_item && st < 32)) ? 1 : 0;
     };
     PipeItem prev{0, 0, 0};
-    StepCursor cur, ahead;  // current step / the step two ahead (mask prefetch)
-    cur.init(static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nqb, heads, nkb);
+    Cursor cur, ahead;  // current step / the step two ahead (mask prefetch)
+    cur.init(static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nqb, heads, nkb, kv_div);
     ahead = cur;
     if (my_items > 0) {
       float raw; bool inr;
@@ -345,6 +367,7 @@ attention_pipe_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_cons
     for (int it = 0; it < my_items; ++it, cur.next_item()) {
       const PipeItem w = cur.item();
       SD_DEV_ASSERT(w.b >= 0 && w.h >= 0 && w.h < heads && (w.b * heads + w.h) * nqb + w.q0 / kPQ < n_items);  // the division-free cursor stays on the item list
+      SD_DEV_ASSERT(cur.kg() == w.b / kv_div);  // ... and on the key graph
       SD_DEV_ASSERT(!q_off || (__ldg(q_len + w.b) > 0 && __ldg(q_len + w.b) <= Lq && __ldg(q_off + w.b) >= 0));
       float m_run = -INFINITY, l_run = 0.f;
       for (int kb = 0; kb < nkb; ++kb, ++g) {
@@ -541,7 +564,7 @@ template <> struct PipeFmt<bf16> { static constexpr int v = 1; };
 template <typename T, bool REL, bool DROP = false>
 static int launch_pipe(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const T* E, int P,
                        const float* mask, T* out, cudaStream_t s, const AttnPack* pk, const DropSpec dr = DropSpec{0.f, 0u, 0u, 0ull},
-                       uint32_t* keep_out = nullptr) {
+                       uint32_t* keep_out = nullptr, int kv_div = 1) {
   using C = PipeCfg<REL>;
   auto kfn = attention_pipe_kernel<T, REL, DROP>;
   static bool configured = false;
@@ -554,8 +577,8 @@ static int launch_pipe(int B, int heads, int Lq, int Lk, const T* q, int ldq, co
   SD_TRY(make_tmap(q, fmt, pk ? pk->q_rows : B * Lq, ldq, 128, &tq));
   if (pk) to = tq;  // packed: per-thread predicated stores, no tile store
   else SD_TRY(make_tmap_3d(out, fmt, B, Lq, heads * 64, 128, &to));
-  SD_TRY(make_tmap(k, fmt, pk ? pk->k_rows : B * Lk, ldk, 128, &tk));
-  SD_TRY(make_tmap(v, fmt, pk ? pk->k_rows : B * Lk, ldv, 128, &tv));
+  SD_TRY(make_tmap(k, fmt, pk ? pk->k_rows : B / kv_div * Lk, ldk, 128, &tk));
+  SD_TRY(make_tmap(v, fmt, pk ? pk->k_rows : B / kv_div * Lk, ldv, 128, &tv));
   if (REL) SD_TRY(make_tmap(E, fmt, 2 * P - 1, 64, 256, &te));
   else te = tq;
   const int nqb = ceil_div(Lq, kPQ);
@@ -565,21 +588,23 @@ static int launch_pipe(int B, int heads, int Lq, int Lk, const T* q, int ldq, co
   int grid = n_items < num_sms() ? n_items : num_sms();
   if (grid_cap > 0 && grid > grid_cap) grid = grid_cap;
   SD_CUDA(launch_k(kfn, dim3(grid), dim3(kPipeThreads), C::kBytes, s, tq, tk, tv, te, to, mask, heads, Lq, Lk, P, static_cast<uint32_t>(fmt), nqb,
-                   n_items, g_attn_trace, pk ? pk->q_off : nullptr, pk ? pk->k_off : nullptr, pk ? pk->q_len : nullptr, pk ? pk->Lk_mask : Lk, out, dr, keep_out));
+                   n_items, g_attn_trace, pk ? pk->q_off : nullptr, pk ? pk->k_off : nullptr, pk ? pk->q_len : nullptr, pk ? pk->Lk_mask : Lk, kv_div, out, dr, keep_out));
   SD_LAUNCHED(DROP ? (REL ? "attention_pipe_rel_drop" : "attention_pipe_norel_drop") : (REL ? "attention_pipe_rel" : "attention_pipe_norel"), s);
   return SEQDIFF_OK;
 }
 
 template <typename T>
 int attention_pipe(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const T* dist_emb, int P,
-                   const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack) {
+                   const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack, int kv_div) {
   SD_CHECK(B > 0 && heads > 0 && Lq > 0 && Lk > 0, "empty attention");
+  SD_CHECK(kv_div >= 1 && B % kv_div == 0, "every key graph must serve kv_div whole query graphs");
   SD_CHECK(ldq % 8 == 0 && ldk % 8 == 0 && ldv % 8 == 0, "row strides must be multiples of 8 elements");
   SD_CHECK((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(v)) % 16 == 0, "q/k/v must be 16B aligned");
   SD_CHECK(!dist_emb || (Lq <= P && Lk <= P), "sequence longer than max_position_embeddings");
   SD_CHECK(!pack || (pack->q_off && pack->k_off && pack->q_len && pack->Lk_mask >= Lk && pack->q_rows > 0 && pack->k_rows > 0), "bad packed-attention descriptor");
-  if (dist_emb) return launch_pipe<T, true>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack);
-  return launch_pipe<T, false>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack);
+  const DropSpec none{0.f, 0u, 0u, 0ull};
+  if (dist_emb) return launch_pipe<T, true>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack, none, nullptr, kv_div);
+  return launch_pipe<T, false>(B, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, dist_emb, P, key_mask, out, s, pack, none, nullptr, kv_div);
 }
 // training-mode forward (attention-probability dropout inside the kernel); needs Lk % 4 == 0
 template <typename T>
@@ -597,7 +622,7 @@ int attention_pipe_dropout(int B, int heads, int Lq, int Lk, const T* q, int ldq
 }
 template int attention_pipe_dropout<bf16>(int, int, int, int, const bf16*, int, const bf16*, int, const bf16*, int, const bf16*, int, const float*, DropSpec, bf16*, cudaStream_t, uint32_t*);
 template int attention_pipe_dropout<f16>(int, int, int, int, const f16*, int, const f16*, int, const f16*, int, const f16*, int, const float*, DropSpec, f16*, cudaStream_t, uint32_t*);
-template int attention_pipe<bf16>(int, int, int, int, const bf16*, int, const bf16*, int, const bf16*, int, const bf16*, int, const float*, bf16*, cudaStream_t, const AttnPack*);
-template int attention_pipe<f16>(int, int, int, int, const f16*, int, const f16*, int, const f16*, int, const f16*, int, const float*, f16*, cudaStream_t, const AttnPack*);
+template int attention_pipe<bf16>(int, int, int, int, const bf16*, int, const bf16*, int, const bf16*, int, const bf16*, int, const float*, bf16*, cudaStream_t, const AttnPack*, int);
+template int attention_pipe<f16>(int, int, int, int, const f16*, int, const f16*, int, const f16*, int, const f16*, int, const float*, f16*, cudaStream_t, const AttnPack*, int);
 
 }  // namespace seqdiff

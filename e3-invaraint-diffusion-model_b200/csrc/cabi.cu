@@ -156,7 +156,7 @@ int seqdiff_sample(seqdiff_model_t* m, int precision, int B, int L_lig, int L_re
   SD_GUARD_BEGIN
   SD_CHECK(m && q_tables_steps && x_T && ligand_angle && ligand_mask && receptor_seq && receptor_angle && receptor_mask && final_out,
            "null argument");
-  return m->impl.sample(precision, B, L_lig, L_rec, T, q_tables_steps, x_T, ligand_angle, ligand_mask, receptor_seq, receptor_angle,
+  return m->impl.sample(precision, B, 1, L_lig, L_rec, T, q_tables_steps, x_T, ligand_angle, ligand_mask, receptor_seq, receptor_angle,
                         receptor_mask, diverse, noise_E_steps, seed, graph_id0, final_out, static_cast<cudaStream_t>(stream));
   SD_GUARD_END
 }
@@ -253,7 +253,23 @@ int seqdiff_sample_ex(seqdiff_model_t* m, int precision, int B, int L_lig, int L
   SD_CHECK(m && q_tables_steps && x_T && ligand_angle && ligand_mask && receptor_seq && receptor_angle && receptor_mask && final_out,
            "null argument");
   SD_CHECK((flags & ~1) == 0, "unknown sampling flag");
-  return m->impl.sample(precision, B, L_lig, L_rec, T, q_tables_steps, x_T, ligand_angle, ligand_mask, receptor_seq, receptor_angle,
+  return m->impl.sample(precision, B, 1, L_lig, L_rec, T, q_tables_steps, x_T, ligand_angle, ligand_mask, receptor_seq, receptor_angle,
+                        receptor_mask, diverse, noise_E_steps, seed, graph_id0, final_out, static_cast<cudaStream_t>(stream), flags);
+  SD_GUARD_END
+}
+
+int seqdiff_sample_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T, const float* q_tables_steps,
+                         const float* x_T, const float* ligand_angle, const float* ligand_mask, const float* receptor_seq,
+                         const float* receptor_angle, const float* receptor_mask, int diverse, const float* noise_E_steps, uint64_t seed,
+                         uint64_t graph_id0, int flags, float* final_out, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(m && q_tables_steps && x_T && ligand_angle && ligand_mask && receptor_seq && receptor_angle && receptor_mask && final_out,
+           "null argument");
+  SD_CHECK(P >= 1 && K >= 1, "need at least one pocket and one sample per pocket");
+  SD_CHECK(L_lig > 0 && L_rec > 0 && static_cast<int64_t>(P) * K * (L_lig > L_rec ? L_lig : L_rec) <= INT32_MAX,
+           "pockets x samples x length overflows the row counts");
+  SD_CHECK((flags & ~1) == 0, "unknown sampling flag");
+  return m->impl.sample(precision, P, K, L_lig, L_rec, T, q_tables_steps, x_T, ligand_angle, ligand_mask, receptor_seq, receptor_angle,
                         receptor_mask, diverse, noise_E_steps, seed, graph_id0, final_out, static_cast<cudaStream_t>(stream), flags);
   SD_GUARD_END
 }

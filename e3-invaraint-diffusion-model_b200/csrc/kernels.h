@@ -115,9 +115,11 @@ struct AttnPack {
   int q_rows, k_rows;  // total rows of the packed q / k matrices
   int Lk_mask;
 };
+// kv_div > 1 (B % kv_div == 0): query graph b attends to key graph b / kv_div -- its K / V rows (padded: (b / kv_div) * Lk, packed:
+// k_off[b / kv_div]) and its key-mask row.  The sampler's K samples per pocket share one pocket's cross K|V this way.
 template <typename T>
 int attention(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const T* dist_emb,
-              int P, const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack = nullptr);
+              int P, const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack = nullptr, int kv_div = 1);
 
 // ---- collate.cu ---------------------------------------------------------------------------------------
 // LigandBindingSiteDataset.__getitem__ for G ragged complexes (dataset.py:97-129); lengths[g] = (n_lig, n_rec) BEFORE clamping.
@@ -132,7 +134,7 @@ extern unsigned long long* g_attn_trace;  // debug timeline buffer of the pipeli
 // ---- attention_pipe.cu: persistent, warp-specialised version (TMA / MMA / softmax roles pipelined over work items) -----
 template <typename T>
 int attention_pipe(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const T* dist_emb,
-                   int P, const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack = nullptr);
+                   int P, const float* key_mask, T* out, cudaStream_t s, const AttnPack* pack = nullptr, int kv_div = 1);
 // ---- attention_bwd_pipe.cu: backward of the attention core on tcgen05 (Lq, Lk <= 128; dE += gradient of the distance embedding) ----
 bool attention_bwd_pipe_usable(int Lq, int Lk, const void* dist_emb, float p_drop);
 template <typename T>

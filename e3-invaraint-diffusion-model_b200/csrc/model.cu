@@ -853,14 +853,15 @@ static FwdBufs<T> carve_forward(uint8_t* ws, cudaStream_t s, int B, int H, int I
 template <typename T>
 int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t,
                      const float* lig_angle, const float* lig_mask, const float* rec_seq_in, const float* rec_angle,
-                     const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk, const LoopInv* inv) {
+                     const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk, const LoopInv* inv, int K) {
   constexpr bool k16 = !std::is_same<T, float>::value;
   const int H = cfg.hidden_size, I = cfg.intermediate_size, NL = cfg.num_hidden_layers, heads = cfg.num_attention_heads;
   const int P = cfg.max_position_embeddings;
   const float eps = cfg.layer_norm_eps;
-  // packed (ragged) batch: only the valid prefix of every graph is a row; inputs, masks and logits keep their padded layouts
-  const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : B * Lr, Mt = Ml + Mr;
-  const int Mlp = B * Ll, Mrp = B * Lr;  // padded row counts (input tensors, key masks)
+  // packed (ragged) batch: only the valid prefix of every graph is a row; inputs, masks and logits keep their padded layouts.
+  // The receptor rows are those of the B / K pockets.
+  const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : B / K * Lr, Mt = Ml + Mr;
+  const int Mlp = B * Ll, Mrp = B / K * Lr;  // padded row counts (input tensors, key masks)
   const size_t MlH = static_cast<size_t>(Ml) * H;
   const FwdBufs<T> f = carve_forward<T>(ws, s, B, H, I, NL, Mlp, Mrp, Ml, Mr);
   float* te = f.te;
@@ -963,7 +964,7 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
                         w.self.ln_b, eps, h1.t, lnstats, s));
       SD_TRY(gemm_T(wfmt, Ml, H, H, h1.t, w.cq, w.cq_b, 0, cq, s));
       const T* kbase = kv_all + static_cast<size_t>(i) * 2 * H;
-      SD_TRY(attention<T>(B, heads, Lq_self, Lk_cross, cq, H, kbase, NL * 2 * H, kbase + H, NL * 2 * H, static_cast<const T*>(nullptr), P, rec_mask, sb.ctx, s, apc));
+      SD_TRY(attention<T>(B, heads, Lq_self, Lk_cross, cq, H, kbase, NL * 2 * H, kbase + H, NL * 2 * H, static_cast<const T*>(nullptr), P, rec_mask, sb.ctx, s, apc, K));
       const LnResid r1{lnstats, w.self.ln_w, w.self.ln_b};
       SD_TRY(gemm_ln<T>(wfmt, Ml, H, H, sb.ctx, w.cout, w.cout_b, oA, oB, &r1, w.cln_w, w.cln_b, eps, h2.t, lnstats + Ml, s));
       SD_TRY(gemm_T(wfmt, Ml, I, H, h2.t, w.inter, w.inter_b, 1, ffn, s));
@@ -990,7 +991,7 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
       SD_TRY(layernorm<T>(sb.o, Ml, H, w.self.ln_w, w.self.ln_b, eps, h1.s, h1.t_out(), nullptr, s));
       SD_TRY(gemm_T(wfmt, Ml, H, H, h1.t, w.cq, w.cq_b, 0, cq, s));
       const T* kbase = kv_all + static_cast<size_t>(i) * 2 * H;
-      SD_TRY(attention<T>(B, heads, Lq_self, Lk_cross, cq, H, kbase, NL * 2 * H, kbase + H, NL * 2 * H, static_cast<const T*>(nullptr), P, rec_mask, sb.ctx, s, apc));
+      SD_TRY(attention<T>(B, heads, Lq_self, Lk_cross, cq, H, kbase, NL * 2 * H, kbase + H, NL * 2 * H, static_cast<const T*>(nullptr), P, rec_mask, sb.ctx, s, apc, K));
       SD_TRY(gemm_S(wfmt, Ml, H, H, sb.ctx, w.cout, w.cout_b, h1.s, sb.o, s));
       SD_TRY(layernorm<T>(sb.o, Ml, H, w.cln_w, w.cln_b, eps, h2.s, h2.t_out(), nullptr, s));
       SD_TRY(gemm_T(wfmt, Ml, I, H, h2.t, w.inter, w.inter_b, 1, ffn, s));
@@ -1028,39 +1029,41 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
 
 int Model::forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t,
                    const float* lig_angle, const float* lig_mask, const float* rec_seq_in, const float* rec_angle,
-                   const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk, const LoopInv* inv) {
+                   const float* rec_mask, float* logits, cudaStream_t s, const PackInfo* pk, const LoopInv* inv, int K) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
   SD_CHECK(arch == kArchSequence, "handle holds a structure model: use seqdiff_struct_forward");
   SD_CHECK(!pk || precision != SEQDIFF_FP32, "ragged packing runs in the 16-bit modes");
   SD_CHECK(precision >= SEQDIFF_FP32 && precision <= SEQDIFF_FP16, "unknown precision mode");
   SD_CHECK(B > 0 && Ll > 0 && Lr > 0, "empty batch");
   SD_CHECK(!inv || step_ptr, "the sampling-loop invariants are indexed by the device step counter");
+  SD_CHECK(K >= 1 && B % K == 0 && (K == 1 || inv), "shared receptor rows (K > 1) exist in the sampling loop only");
   if (cfg.relative_key) SD_CHECK(Ll <= cfg.max_position_embeddings && Lr <= cfg.max_position_embeddings, "Length exceed");
   SD_CUDA(cudaSetDevice(device));
   SD_TRY(ensure_workspace(workspace_need(precision, B, Ll, Lr)));
   if (g_profiling) profile_mark("__begin__", s);  // host time between two calls is not the first kernel's
-  const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * (Ll + Lr)));
+  const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * Ll + static_cast<long long>(B / K) * Lr));
   switch (precision) {
     case SEQDIFF_FP32:
-      return forward_t<float>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, nullptr, inv);
+      return forward_t<float>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, nullptr, inv, K);
     case SEQDIFF_BF16:
-      return forward_t<bf16>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk, inv);
+      return forward_t<bf16>(1, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk, inv, K);
     default:  // SEQDIFF_FP16
-      return forward_t<f16>(0, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk, inv);
+      return forward_t<f16>(0, B, Ll, Lr, timestep, step_ptr, x_t, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, logits, s, pk, inv, K);
   }
 }
 
 // The per-sampling part of the loop (LoopInv): the kernels forward_t runs on the same inputs, so every value is the one the
 // stand-alone forward computes at every step.  None of them splits K, so a GEMM row's result does not depend on M (T rows of steps
 // here, B rows of one step there), and attention items are per (graph, head), so the receptor graphs give the same result without
-// the ligand graphs next to them.
+// the ligand graphs next to them.  The receptor rows are those of the B / K pockets (forward_t's K).
 template <typename T>
-int Model::loop_invariants_t(int wfmt, int B, int Ll, int Lr, int T_, const float* rec_seq_in, const float* rec_mask, const LoopInv& iv,
+int Model::loop_invariants_t(int wfmt, int B, int K, int Ll, int Lr, int T_, const float* rec_seq_in, const float* rec_mask, const LoopInv& iv,
                              cudaStream_t s, const PackInfo* pk) {
   constexpr bool k16 = !std::is_same<T, float>::value;
   const int H = cfg.hidden_size, heads = cfg.num_attention_heads, P = cfg.max_position_embeddings;
-  const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : B * Lr;
-  const FwdBufs<T> f = carve_forward<T>(ws, s, B, H, cfg.intermediate_size, cfg.num_hidden_layers, B * Ll, B * Lr, Ml, Mr);
+  const int Pk = B / K;  // pockets
+  const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : Pk * Lr;
+  const FwdBufs<T> f = carve_forward<T>(ws, s, B, H, cfg.intermediate_size, cfg.num_hidden_layers, B * Ll, Pk * Lr, Ml, Mr);
   // timestep features of steps 0 .. T-1 (row i: t = i, as (float)*step_ptr gives it) and decoder_normalize's adaLN GEMMs on them
   SD_TRY(timestep_embed(nullptr, nullptr, ts_W, T_, H, iv.te, k16 ? iv.teT : nullptr, Fmt<T>::v, s));
   SD_TRY(gemm_T(wfmt, T_, H, H, static_cast<const T*>(iv.teT), se_dec.ada0, se_dec.ada0_b, 2, static_cast<T*>(iv.u), s));
@@ -1079,7 +1082,7 @@ int Model::loop_invariants_t(int wfmt, int B, int Ll, int Lr, int T_, const floa
   SD_TRY(gemm_T(wfmt, Mr, 3 * H, H, static_cast<const T*>(iv.xrT), a.qkv, a.qkv_b, 0, qkv, s));
   const AttnPack ap = pk ? AttnPack{pk->off_r, pk->off_r, pk->len_r, Mr, Mr, Lr} : AttnPack{};
   const int Lk = pk ? pk->max_r : Lr;
-  SD_TRY(attention<T>(B, heads, Lk, Lk, qkv, 3 * H, qkv + H, 3 * H, qkv + 2 * H, 3 * H, pick<T>(a.E), P, rec_mask, f.sb.ctx, s, pk ? &ap : nullptr));
+  SD_TRY(attention<T>(Pk, heads, Lk, Lk, qkv, 3 * H, qkv + H, 3 * H, qkv + 2 * H, 3 * H, pick<T>(a.E), P, rec_mask, f.sb.ctx, s, pk ? &ap : nullptr));
   SD_TRY(gemm_S(wfmt, Mr, H, H, f.sb.ctx, a.out, a.out_b, iv.xr, iv.o, s));
   return SEQDIFF_OK;
 }
@@ -1088,16 +1091,17 @@ int Model::loop_invariants_t(int wfmt, int B, int Ll, int Lr, int T_, const floa
 // reverse-diffusion loop: one captured CUDA graph per step shape, replayed T times
 // =====================================================================================================
 // Ragged packing: lengths from the (prefix-ones) masks, row maps, offsets.  *usable = false when a mask is not a prefix of ones
-// (the caller then stays on the padded path) or a graph has no valid ligand / receptor token.
-int Model::build_pack(int B, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable) {
+// (the caller then stays on the padded path) or a graph has no valid ligand / receptor token.  B ligand graphs, B / K pockets.
+int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable) {
   *usable = false;
-  std::vector<float> hl(static_cast<size_t>(B) * Ll), hr(static_cast<size_t>(B) * Lr);
+  const int P = B / K;
+  std::vector<float> hl(static_cast<size_t>(B) * Ll), hr(static_cast<size_t>(P) * Lr);
   SD_CUDA(cudaMemcpyAsync(hl.data(), lig_mask, hl.size() * 4, cudaMemcpyDefault, s));
   SD_CUDA(cudaMemcpyAsync(hr.data(), rec_mask, hr.size() * 4, cudaMemcpyDefault, s));
   SD_CUDA(cudaStreamSynchronize(s));
-  std::vector<int> len_l(B), len_r(B);
-  auto lengths = [&](const std::vector<float>& m, int L, std::vector<int>& len) -> bool {
-    for (int b = 0; b < B; ++b) {
+  std::vector<int> len_l(B), len_r(P);
+  auto lengths = [&](const std::vector<float>& m, int G, int L, std::vector<int>& len) -> bool {
+    for (int b = 0; b < G; ++b) {
       int n = 0;
       while (n < L && m[static_cast<size_t>(b) * L + n] == 1.0f) ++n;
       for (int i = n; i < L; ++i)
@@ -1107,31 +1111,35 @@ int Model::build_pack(int B, int Ll, int Lr, const float* lig_mask, const float*
     }
     return true;
   };
-  if (!lengths(hl, Ll, len_l) || !lengths(hr, Lr, len_r)) return SEQDIFF_OK;
+  if (!lengths(hl, B, Ll, len_l) || !lengths(hr, P, Lr, len_r)) return SEQDIFF_OK;
   int Ml = 0, Mr = 0, max_l = 0, max_r = 0;
-  std::vector<int> off_l(B), off_r(B);
+  std::vector<int> off_l(B), off_r(P);
   for (int b = 0; b < B; ++b) {
     off_l[b] = Ml; Ml += len_l[b];
-    off_r[b] = Mr; Mr += len_r[b];
     max_l = len_l[b] > max_l ? len_l[b] : max_l;
-    max_r = len_r[b] > max_r ? len_r[b] : max_r;
   }
-  // block layout (ints): src_l[Ml] | src_r[Mr] | graph[Ml+Mr] | off_l[B] | off_r[B] | len_l[B] | len_r[B] | off_cat[2B] | len_cat[2B]
+  for (int p = 0; p < P; ++p) {
+    off_r[p] = Mr; Mr += len_r[p];
+    max_r = len_r[p] > max_r ? len_r[p] : max_r;
+  }
+  // block layout (ints): src_l[Ml] | src_r[Mr] | graph[Ml+Mr] | off_l[B] | off_r[P] | len_l[B] | len_r[P] | off_cat[B+P] | len_cat[B+P]
   std::vector<int> blk;
-  blk.reserve(2 * (static_cast<size_t>(Ml) + Mr) + 8 * B);
+  blk.reserve(2 * (static_cast<size_t>(Ml) + Mr) + 4 * (static_cast<size_t>(B) + P));
   for (int b = 0; b < B; ++b) for (int l = 0; l < len_l[b]; ++l) blk.push_back(b * Ll + l);
-  for (int b = 0; b < B; ++b) for (int l = 0; l < len_r[b]; ++l) blk.push_back(b * Lr + l);
+  for (int p = 0; p < P; ++p) for (int l = 0; l < len_r[p]; ++l) blk.push_back(p * Lr + l);
   for (int b = 0; b < B; ++b) for (int l = 0; l < len_l[b]; ++l) blk.push_back(b);
-  for (int b = 0; b < B; ++b) for (int l = 0; l < len_r[b]; ++l) blk.push_back(b);
+  for (int p = 0; p < P; ++p) for (int l = 0; l < len_r[p]; ++l) blk.push_back(p);
   for (int b = 0; b < B; ++b) blk.push_back(off_l[b]);
-  for (int b = 0; b < B; ++b) blk.push_back(off_r[b]);
+  for (int p = 0; p < P; ++p) blk.push_back(off_r[p]);
   for (int b = 0; b < B; ++b) blk.push_back(len_l[b]);
-  for (int b = 0; b < B; ++b) blk.push_back(len_r[b]);
+  for (int p = 0; p < P; ++p) blk.push_back(len_r[p]);
   for (int b = 0; b < B; ++b) blk.push_back(off_l[b]);
-  for (int b = 0; b < B; ++b) blk.push_back(Ml + off_r[b]);
+  for (int p = 0; p < P; ++p) blk.push_back(Ml + off_r[p]);
   for (int b = 0; b < B; ++b) blk.push_back(len_l[b]);
-  for (int b = 0; b < B; ++b) blk.push_back(len_r[b]);
-  uint64_t hsh = 1469598103934665603ull;  // FNV-1a over the block: a changed batch composition re-captures the step graph
+  for (int p = 0; p < P; ++p) blk.push_back(len_r[p]);
+  // FNV-1a over K and the block: a changed batch composition re-captures the step graph
+  uint64_t hsh = 1469598103934665603ull;
+  hsh ^= static_cast<uint32_t>(K); hsh *= 1099511628211ull;
   for (int v : blk) { hsh ^= static_cast<uint32_t>(v); hsh *= 1099511628211ull; }
   bool fresh = false;
   if (blk.size() > pack_cap) {
@@ -1140,32 +1148,33 @@ int Model::build_pack(int B, int Ll, int Lr, const float* lig_mask, const float*
     pack_cap = blk.size();
     fresh = true;
   }
-  if (fresh || hsh != pack.hash || pack.B != B) {
+  if (fresh || hsh != pack.hash || pack.B != B || pack.P != P) {
     SD_CUDA(cudaMemcpyAsync(d_pack, blk.data(), blk.size() * sizeof(int), cudaMemcpyHostToDevice, s));
     SD_CUDA(cudaStreamSynchronize(s));  // blk is a stack-lifetime host buffer
   }
   PackInfo pi;
-  pi.B = B; pi.Ml = Ml; pi.Mr = Mr; pi.max_l = max_l; pi.max_r = max_r; pi.hash = hsh;
+  pi.B = B; pi.P = P; pi.Ml = Ml; pi.Mr = Mr; pi.max_l = max_l; pi.max_r = max_r; pi.hash = hsh;
   const int* p = d_pack;
   pi.src_l = p; p += Ml;
   pi.src_r = p; p += Mr;
   pi.graph = p; p += Ml + Mr;
   pi.off_l = p; p += B;
-  pi.off_r = p; p += B;
+  pi.off_r = p; p += P;
   pi.len_l = p; p += B;
-  pi.len_r = p; p += B;
-  pi.off_cat = p; p += 2 * B;
+  pi.len_r = p; p += P;
+  pi.off_cat = p; p += B + P;
   pi.len_cat = p;
   pack = pi;
   *usable = true;
   return SEQDIFF_OK;
 }
 
-int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
+int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
                   const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, int diverse,
                   const float* noise_E, uint64_t seed, uint64_t gid0, float* final_out, cudaStream_t caller, int flags) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
-  SD_CHECK(T >= 1 && B > 0 && Ll > 0 && Lr > 0, "bad sampling arguments");
+  SD_CHECK(T >= 1 && P > 0 && K > 0 && Ll > 0 && Lr > 0, "bad sampling arguments");
+  const int B = P * K;  // ligand graphs: sample j of pocket p is graph p * K + j
   SD_CHECK(cfg.feature_size == SEQDIFF_NUM_CLASSES, "sampling needs feature_size == 20");
   SD_CUDA(cudaSetDevice(device));  // before the stream / events are created: they belong to the handle's device
   if (!loop_stream) {
@@ -1177,7 +1186,7 @@ int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_ta
   cudaStream_t s = loop_stream;
   SD_CUDA(cudaEventRecord(ev_in, caller));
   SD_CUDA(cudaStreamWaitEvent(s, ev_in, 0));
-  const size_t Nl = static_cast<size_t>(B) * Ll, Nr = static_cast<size_t>(B) * Lr;
+  const size_t Nl = static_cast<size_t>(B) * Ll, Nr = static_cast<size_t>(P) * Lr;
   // persistent inputs: x_cur | logits | lig_angle | lig_mask | rec_seq | rec_angle | rec_mask
   const size_t need_in = align256(Nl * 20 * 4) * 2 + align256(Nl * 8 * 4) + align256(Nl * 4) + align256(Nr * 20 * 4) +
                          align256(Nr * 8 * 4) + align256(Nr * 4);
@@ -1212,15 +1221,16 @@ int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_ta
   const PackInfo* pk = nullptr;
   if ((flags & 1) && precision != SEQDIFF_FP32) {
     bool usable = false;
-    SD_TRY(build_pack(B, Ll, Lr, c_lmask, c_rmask, s, &usable));
+    SD_TRY(build_pack(B, K, Ll, Lr, c_lmask, c_rmask, s, &usable));
     if (usable) {
       pk = &pack;
       SD_CUDA(cudaMemsetAsync(logits, 0, Nl * 20 * 4, s));  // padded positions are never written in packed mode: defined as 0
     }
   }
 
+  const long long rows = pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(Nl + Nr);  // token rows of a step
   // The per-sampling invariants (LoopInv), computed here by every call, outside the graph: the graph only holds their addresses.
-  // Receptor rows first (B * Lr, the packed rows are a prefix), then the step tables with a grow-only capacity, so a cached graph
+  // Receptor rows first (P * Lr, the packed rows are a prefix), then the step tables with a grow-only capacity, so a cached graph
   // serves any T up to it.
   {
     inv.rows = T > inv.rows ? T : inv.rows;
@@ -1240,23 +1250,23 @@ int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_ta
     inv.teT = es == 2 ? static_cast<void*>(bi.take<uint16_t>(tH)) : inv.te;
     inv.u = bi.take<uint8_t>(tH * es);
     inv.mod = bi.take<uint8_t>(tH * 6 * es);
-    const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * (Ll + Lr)));
+    const PdlScope pdl_scope(pdl_auto_mode(rows));
     switch (precision) {
-      case SEQDIFF_FP32: SD_TRY(loop_invariants_t<float>(1, B, Ll, Lr, T, c_rseq, c_rmask, inv, s, nullptr)); break;
-      case SEQDIFF_BF16: SD_TRY(loop_invariants_t<bf16>(1, B, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
-      default: SD_TRY(loop_invariants_t<f16>(0, B, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
+      case SEQDIFF_FP32: SD_TRY(loop_invariants_t<float>(1, B, K, Ll, Lr, T, c_rseq, c_rmask, inv, s, nullptr)); break;
+      case SEQDIFF_BF16: SD_TRY(loop_invariants_t<bf16>(1, B, K, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
+      default: SD_TRY(loop_invariants_t<f16>(0, B, K, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
     }
   }
 
   GraphKey key;
   key.pack_hash = pk ? pk->hash : 0;
-  key.precision = precision; key.B = B; key.Ll = Ll; key.Lr = Lr; key.diverse = diverse; key.noise = noise_E;
+  key.precision = precision; key.B = B; key.K = K; key.Ll = Ll; key.Lr = Lr; key.diverse = diverse; key.noise = noise_E;
   key.ws_ptr = ws; key.in_ptr = samp_in; key.tab_ptr = d_tables;  // (seed, gid0) are NOT part of the key: device memory, see arm_loop_kernel
   key.inv_ptr = samp_inv; key.inv_rows = inv.rows;
   uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
   auto one_step = [&](cudaStream_t st) -> int {
-    const PdlScope pdl_scope(pdl_auto_mode(pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(B) * (Ll + Lr)));
-    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, st, pk, &inv));
+    const PdlScope pdl_scope(pdl_auto_mode(rows));
+    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, st, pk, &inv, K));
     SD_TRY(reverse_step(d_tables, 1, B, Ll, x_cur, logits, diverse, noise_E, 0, 0, 0, d_step, x_cur, nullptr, st, d_step + 1, d_rng));
     return SEQDIFF_OK;
   };
@@ -1265,7 +1275,7 @@ int Model::sample(int precision, int B, int Ll, int Lr, int T, const float* q_ta
     // un-captured dry run of the forward: sets kernel attributes and fills the TMA descriptor cache
     SD_CUDA(launch_k(set_int_kernel, dim3(1), dim3(1), 0, s, d_step, T - 1));
     SD_LAUNCHED("set_int", s);
-    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, s, pk, &inv));
+    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, s, pk, &inv, K));
     SD_CUDA(cudaStreamSynchronize(s));
     cudaGraph_t graph = nullptr;
     const uint64_t l0 = g_launches.load();

@@ -73,27 +73,29 @@ int profile_begin(cudaStream_t s);
 int profile_end(char* tags, int tag_stride, float* ms, int* counts, int cap);
 
 // Ragged packing of a sampling batch (DESIGN.md "Ragged batches"): only the valid prefix of every graph is computed.  Token rows of
-// graph b occupy rows [off[b], off[b] + len[b]) of every [rows, H] matrix; all index arrays live in one device block.
+// graph b occupy rows [off[b], off[b] + len[b]) of every [rows, H] matrix; all index arrays live in one device block.  A sampling
+// of K samples per pocket has B = P * K ligand graphs and P receptor graphs (sample b reads pocket b / K).
 struct PackInfo {
-  int B = 0, Ml = 0, Mr = 0;      // packed ligand / receptor row counts
+  int B = 0, P = 0, Ml = 0, Mr = 0;  // ligand / receptor graphs, packed ligand / receptor row counts
   int max_l = 0, max_r = 0;       // largest ligand / receptor length
   const int* src_l = nullptr;     // [Ml] packed ligand row -> padded row index b * Ll + l
   const int* src_r = nullptr;     // [Mr]
-  const int* graph = nullptr;     // [Ml + Mr] graph of a stacked row
+  const int* graph = nullptr;     // [Ml + Mr] graph of a stacked row (receptor rows: the pocket)
   const int* off_l = nullptr;     // [B] first ligand row of graph b
-  const int* off_r = nullptr;     // [B] first receptor row of graph b, relative to the receptor block
+  const int* off_r = nullptr;     // [P] first receptor row of pocket p, relative to the receptor block
   const int* len_l = nullptr;     // [B]
-  const int* len_r = nullptr;     // [B]
-  const int* off_cat = nullptr;   // [2B] ligand offsets, then receptor offsets + Ml (stacked matrix)
-  const int* len_cat = nullptr;   // [2B]
-  uint64_t hash = 0;              // of the length vectors (part of the CUDA-graph key)
+  const int* len_r = nullptr;     // [P]
+  const int* off_cat = nullptr;   // [B + P] ligand offsets, then receptor offsets + Ml (stacked matrix)
+  const int* len_cat = nullptr;   // [B + P]
+  uint64_t hash = 0;              // of K and the length vectors (part of the CUDA-graph key)
 };
 
 // What the sequence model's sampling loop computes once per sampling instead of once per step (Model::sample).  Every graph of the
 // batch shares the step index and x_t is the only other input that changes between steps, so the receptor embedding, the receptor
 // half of ligand_feature_emb's attention sublayer (its input is the receptor embedding alone), the timestep features and
 // decoder_normalize's modulation (a function of the timestep features alone) are the same at every step.  The buffers are carved
-// from the handle's samp_inv block; receptor rows are [Mr, H] in the row order of the step's token matrix (packed or padded).
+// from the handle's samp_inv block; receptor rows are [Mr, H] in the row order of the step's token matrix (packed or padded), one
+// set per pocket: the K samples of a pocket share them.
 struct LoopInv {
   int rows = 0;          // table capacity in steps (>= T of the sampling)
   float* xr = nullptr;   // [Mr, H] receptor embedding, fp32 stream
@@ -144,18 +146,18 @@ struct Model {
   cudaStream_t loop_stream = nullptr;  // private stream: graphs cannot be captured on the legacy default stream
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
   struct GraphKey {
-    int precision = -1, B = 0, Ll = 0, Lr = 0, diverse = 0;
+    int precision = -1, B = 0, K = 0, Ll = 0, Lr = 0, diverse = 0;
     const float* noise = nullptr;
     const void* ws_ptr = nullptr;
     const void* in_ptr = nullptr;
     const void* tab_ptr = nullptr;
     const void* aux_ptr = nullptr;
     const void* inv_ptr = nullptr;
-    int inv_rows = 0;  // with B, Lr and the precision: the layout of the LoopInv buffers
+    int inv_rows = 0;  // with B, K, Lr and the precision: the layout of the LoopInv buffers
     int T = 0;
     uint64_t pack_hash = 0;
     bool operator==(const GraphKey& o) const {
-      return pack_hash == o.pack_hash && aux_ptr == o.aux_ptr && T == o.T && precision == o.precision && B == o.B && Ll == o.Ll && Lr == o.Lr && diverse == o.diverse && noise == o.noise &&
+      return pack_hash == o.pack_hash && aux_ptr == o.aux_ptr && T == o.T && precision == o.precision && B == o.B && K == o.K && Ll == o.Ll && Lr == o.Lr && diverse == o.diverse && noise == o.noise &&
              ws_ptr == o.ws_ptr && in_ptr == o.in_ptr && tab_ptr == o.tab_ptr && inv_ptr == o.inv_ptr && inv_rows == o.inv_rows;
     }
   } graph_key;
@@ -165,18 +167,20 @@ struct Model {
   int set_tensor(const char* name, const float* data, int64_t numel, cudaStream_t s);
   int finalize(cudaStream_t s);
   // inv != NULL (sampling loop, with step_ptr): the step reads what loop_invariants_t() left in `inv` instead of recomputing it;
-  // rec_seq is not read then
+  // rec_seq is not read then.  K > 1 (with inv only): the receptor inputs hold B / K pockets and ligand graph b uses pocket b / K.
   int forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t,
               const float* lig_angle, const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask,
-              float* logits, cudaStream_t s, const PackInfo* pk = nullptr, const LoopInv* inv = nullptr);
-  // flags bit 0: ragged packing (valid positions bit-identical to the padded computation; padded positions of final_out are 0)
-  int sample(int precision, int B, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
+              float* logits, cudaStream_t s, const PackInfo* pk = nullptr, const LoopInv* inv = nullptr, int K = 1);
+  // P pockets x K samples per pocket: ligand inputs / x_T / final_out hold B = P * K graphs (sample j of pocket p is graph
+  // p * K + j), receptor inputs hold P.  flags bit 0: ragged packing (valid positions bit-identical to the padded computation;
+  // padded positions of final_out are 0)
+  int sample(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
              const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, int diverse,
              const float* noise_E, uint64_t seed, uint64_t gid0, float* final_out, cudaStream_t s, int flags = 0);
   int* d_pack = nullptr;  // device block behind PackInfo (grow-only)
   size_t pack_cap = 0;
   PackInfo pack;
-  int build_pack(int B, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable);
+  int build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable);
 
   // ---- training (train.cu) ------------------------------------------------------------------------------------------
   std::vector<ParamSlot> slots;            // trainable tensors in flat-buffer order (fused groups contiguous)
@@ -235,11 +239,11 @@ struct Model {
   template <typename T>
   int forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* x_t, const float* lig_angle,
                 const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, float* logits,
-                cudaStream_t s, const PackInfo* pk, const LoopInv* inv);
+                cudaStream_t s, const PackInfo* pk, const LoopInv* inv, int K);
   // fills `inv` for a sampling of T_ <= inv.rows steps (Model::sample); scratch from the forward's workspace
   template <typename T>
-  int loop_invariants_t(int wfmt, int B, int Ll, int Lr, int T_, const float* rec_seq, const float* rec_mask, const LoopInv& inv, cudaStream_t s,
-                        const PackInfo* pk);
+  int loop_invariants_t(int wfmt, int B, int K, int Ll, int Lr, int T_, const float* rec_seq, const float* rec_mask, const LoopInv& inv,
+                        cudaStream_t s, const PackInfo* pk);
 };
 
 }  // namespace seqdiff

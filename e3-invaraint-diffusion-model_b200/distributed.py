@@ -56,11 +56,15 @@ def denoise_sharded(batch, model, noise_schedule, transition, diverse, denoise_f
     all-gathered in rank order, so each rank returns exactly what a single-GPU call on the whole batch returns:
     the start state x_T of the WHOLE batch is drawn once (rank 0's `generate_discrete_noise`, broadcast as class indices --
     a one-off B*L-byte exchange before the loop, not a data-path collective) unless the caller passes `x_T`, and the Philox
-    noise is keyed by global graph ids taken as ONE block from the process-wide stream on every rank."""
+    noise is keyed by global graph ids taken as ONE block from the process-wide stream on every rank.
+    `num_samples=K > 1` (K sequences per pocket): the ranks share out the POCKETS -- rank r samples pockets [lo, hi), which are graphs
+    [lo*K, hi*K) of the one-GPU call: its slice of x_T and noise_E_steps and its graph ids start there."""
     import torch.distributed as dist
     from . import _cabi
+    from .sample import check_num_samples
     if denoise_fn is None:
         from .sample import denoise as denoise_fn
+    K = check_num_samples(kw.get("num_samples", 1))
     if not (dist.is_available() and dist.is_initialized()):
         return denoise_fn(batch, model, noise_schedule, transition, diverse, **kw)
     world, rank = dist.get_world_size(group), dist.get_rank(group)
@@ -69,12 +73,14 @@ def denoise_sharded(batch, model, noise_schedule, transition, diverse, denoise_f
     hi = lo + sub["ligand_seq"].shape[0]
     x_T = kw.pop("x_T", None)
     if x_T is None:
-        box = [torch.randint(0, C, (n, L)).to(torch.uint8) if rank == 0 else None]
+        box = [torch.randint(0, C, (n * K, L)).to(torch.uint8) if rank == 0 else None]
         dist.broadcast_object_list(box, src=0, group=group)
         x_T = torch.nn.functional.one_hot(box[0].long(), C).float()
-    kw["x_T"] = x_T[lo:hi]
+    kw["x_T"] = x_T[lo * K:hi * K]
+    if K > 1 and kw.get("noise_E_steps") is not None:
+        kw["noise_E_steps"] = kw["noise_E_steps"][:, lo * K * L:hi * K * L]
     base = kw.pop("graph_id0", None)
-    gid0 = lo + (_cabi.GRAPH_IDS.take(n) if base is None else base)
+    gid0 = lo * K + (_cabi.GRAPH_IDS.take(n * K) if base is None else base)
     part = denoise_fn(sub, model, noise_schedule, transition, diverse, graph_id0=gid0, **kw) if sub["ligand_seq"].shape[0] else ([], [], [], [])
     parts = [None] * world
     dist.all_gather_object(parts, part, group=group)

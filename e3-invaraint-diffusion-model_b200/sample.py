@@ -100,19 +100,32 @@ def sample_p_zs_given_zt_discrete(t, s, noised_data, pred_noise, noise_schedule,
     return out
 
 
+def check_num_samples(num_samples) -> int:
+    """The number of sequences sampled per pocket: a positive int (ValueError otherwise)."""
+    if isinstance(num_samples, bool) or not isinstance(num_samples, int) or num_samples < 1:
+        raise ValueError(f"num_samples must be a positive int, got {num_samples!r}")
+    return num_samples
+
+
 @torch.no_grad()
 def denoise_tensors(batch, model, noise_schedule, transition, diverse, timesteps=None, x_T=None, noise_E_steps=None,
-                    graph_id0=None, seed=None, packed=False):
+                    graph_id0=None, seed=None, packed=False, num_samples=1):
     """The T-step loop of reference denoise() (sample.py:184-207) as one C call.  Returns the final
     [B,L,20] tensor (raw logits of the last step, quirk Q4) on the model's device.
     `graph_id0` = global id of the batch's first graph in the Philox noise stream; None (default) continues the process-wide
     stream (`_cabi.GRAPH_IDS`), so consecutive batches and repeated calls never share noise.
     `packed=True`: ragged packing (seqdiff_sample_ex, SEQDIFF_SAMPLE_PACKED) -- only the valid prefix of every graph is computed;
-    the result is bit-identical at the valid positions (all that denoise() reads) and 0 at the padded ones."""
+    the result is bit-identical at the valid positions (all that denoise() reads) and 0 at the padded ones.
+    `num_samples=K > 1`: K sequences per pocket of the batch (seqdiff_sample_multi).  The batch holds P pockets; the result, x_T and
+    the graph ids cover B = P*K graphs, sample j of pocket p being graph p*K + j, and noise_E_steps is [T, P*K*L, 20].  Each pocket's
+    receptor rows are computed once per step for its K samples; the result equals the K = 1 call on the batch whose entries are
+    repeated K times per pocket."""
+    K = check_num_samples(num_samples)
     T = CONFIG["timesteps"] if timesteps is None else timesteps
     h = model._sync_handle()
     dev = model._handle_dev  # the handle's device owns the stream, the workspace and every tensor of this call
-    batch_size, max_len, num_class = batch["ligand_seq"].shape
+    n_pockets, max_len, num_class = batch["ligand_seq"].shape
+    batch_size = n_pockets * K
     if graph_id0 is None:
         graph_id0 = _cabi.GRAPH_IDS.take(batch_size)
     if x_T is None:
@@ -123,6 +136,10 @@ def denoise_tensors(batch, model, noise_schedule, transition, diverse, timesteps
 
     x_T = dv(x_T)
     ligand_mask, ligand_angles = dv(batch["ligand_attn_mask"]), dv(batch["ligand_angles"])
+    if K > 1:
+        if tuple(x_T.shape) != (batch_size, max_len, num_class):
+            raise ValueError(f"x_T must be [P*K, L, {num_class}] = {(batch_size, max_len, num_class)}, got {tuple(x_T.shape)}")
+        ligand_mask, ligand_angles = ligand_mask.repeat_interleave(K, dim=0), ligand_angles.repeat_interleave(K, dim=0)
     receptor_seq, receptor_angles = dv(batch["receptor_seq"]), dv(batch["receptor_angles"])
     receptor_attn_mask = dv(batch["receptor_attn_mask"])
     Lr = receptor_seq.shape[1]
@@ -132,10 +149,17 @@ def denoise_tensors(batch, model, noise_schedule, transition, diverse, timesteps
     tables = tables.to(dev)
     E = None if noise_E_steps is None else dv(noise_E_steps)
     if E is not None and tuple(E.shape) != (T, batch_size * max_len, 20):
-        raise ValueError("noise_E_steps must be [T, B*L, 20]")
+        raise ValueError("noise_E_steps must be [T, B*L, 20]" if K == 1 else "noise_E_steps must be [T, P*K*L, 20]")
     out = torch.empty((batch_size, max_len, num_class), device=dev, dtype=torch.float32)
     with torch.cuda.device(dev):
         stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        if K > 1:
+            _cabi.check(_cabi.lib().seqdiff_sample_multi(h, model._precision_code(), n_pockets, K, max_len, Lr, T, _cabi.ptr(tables),
+                                                         _cabi.ptr(x_T), _cabi.ptr(ligand_angles), _cabi.ptr(ligand_mask),
+                                                         _cabi.ptr(receptor_seq), _cabi.ptr(receptor_angles), _cabi.ptr(receptor_attn_mask),
+                                                         int(bool(diverse)), _cabi.ptr(E), SEED if seed is None else seed, graph_id0,
+                                                         1 if packed else 0, _cabi.ptr(out), stream))
+            return out
         _cabi.check(_cabi.lib().seqdiff_sample_ex(h, model._precision_code(), batch_size, max_len, Lr, T, _cabi.ptr(tables), _cabi.ptr(x_T),
                                                   _cabi.ptr(ligand_angles), _cabi.ptr(ligand_mask), _cabi.ptr(receptor_seq),
                                                   _cabi.ptr(receptor_angles), _cabi.ptr(receptor_attn_mask), int(bool(diverse)),
@@ -164,17 +188,23 @@ def decode_tensors(final, ligand_seq, ligand_mask):
 
 
 @torch.no_grad()
-def denoise(batch, model: PeptideDiff, noise_schedule, transition, diverse, **kw):
-    """reference sample.py:181-229: returns (structure_ids, true_sequences, pred_sequences, recovery_rates)."""
-    batch_size = batch["ligand_seq"].shape[0]
-    final = denoise_tensors(batch, model, noise_schedule, transition, diverse, **kw)
+def denoise(batch, model: PeptideDiff, noise_schedule, transition, diverse, num_samples=1, **kw):
+    """reference sample.py:181-229: returns (structure_ids, true_sequences, pred_sequences, recovery_rates).
+    `num_samples=K`: K sequences per pocket of the batch (denoise_tensors); the lists then hold P*K entries in (pocket, sample)
+    order, with each pocket's structure id and true sequence repeated for its samples."""
+    K = check_num_samples(num_samples)
+    batch_size = batch["ligand_seq"].shape[0] * K
+    final = denoise_tensors(batch, model, noise_schedule, transition, diverse, num_samples=K, **kw)
+    ligand_seq, ligand_mask = batch["ligand_seq"], batch["ligand_attn_mask"]
+    if K > 1:
+        ligand_seq, ligand_mask = ligand_seq.repeat_interleave(K, dim=0), ligand_mask.repeat_interleave(K, dim=0)
     # sample.py:208-224 in one kernel: argmax decode of both sequences + per-graph (matches, valid) counts; the host gets
     # 2 x [B,L] bytes + [B,2] ints in one synchronising copy (the reference syncs once per graph) and only joins letters
-    pred_idx, true_idx, counts = decode_tensors(final, batch["ligand_seq"], batch["ligand_attn_mask"])
+    pred_idx, true_idx, counts = decode_tensors(final, ligand_seq, ligand_mask)
     pred_idx, true_idx, counts = pred_idx.cpu(), true_idx.cpu(), counts.cpu()
     n_valid = counts[:, 1].tolist()
     rates = (counts[:, 0] / counts[:, 1]).tolist()  # int64 / int64 -> float32 true division, as recovery_rate.sum()/mask.sum()
-    masks = batch["ligand_attn_mask"].bool().cpu()
+    masks = ligand_mask.bool().cpu()
     recovery_rates, pred_sequences, true_sequences, structure_ids = [], [], [], []
     for i in range(batch_size):
         mask = masks[i]
@@ -185,7 +215,7 @@ def denoise(batch, model: PeptideDiff, noise_schedule, transition, diverse, **kw
         pred_sequences.append("".join(AA_VOCAB[j] for j in pred_seq))
         true_sequences.append("".join(AA_VOCAB[j] for j in true_seq))
         ids = batch.get("structure_ids")
-        structure_ids.append(f'{ids["pdb_id"][i]}_{ids["ligand_chain"][i]}' if ids is not None else str(i))
+        structure_ids.append(f'{ids["pdb_id"][i // K]}_{ids["ligand_chain"][i // K]}' if ids is not None else str(i // K))
     print(sum(recovery_rates) / len(recovery_rates))
     return structure_ids, true_sequences, pred_sequences, recovery_rates
 
@@ -217,12 +247,15 @@ def denoise_with_generated_angles(batch, generated_angles, model, noise_schedule
 
 
 def sample_dataset(dataloader, model, noise_schedule=None, transition=None, diverse=True, output_path=None, denoise_fn=None,
-                   generated_angles=None, **kw):
+                   generated_angles=None, num_samples=1, **kw):
     """The `__main__` block of the reference (sample.py:231-257): every batch of `dataloader` through `denoise`, results
     collected in the reference's DataFrame (columns structure_ids / true_sequence / predict_sequence / recovery_rate) and, when
     `output_path` is given, pickled exactly like `res.to_pickle(OUTPUT_PATH)`.  Returns the DataFrame.  `generated_angles` (chunks
-    from `load_generated_angles`) turns it into the main block of sample_by_generated_angles.py:247-278."""
+    from `load_generated_angles`) turns it into the main block of sample_by_generated_angles.py:247-278.  `num_samples=K > 1`:
+    K sequences per pocket, rows in (pocket, sample) order."""
     import pandas as pd
+    if check_num_samples(num_samples) > 1:
+        kw["num_samples"] = num_samples
     if noise_schedule is None:
         noise_schedule = PredefinedNoiseScheduleDiscrete(CONFIG["noise_schedule"], CONFIG["timesteps"])
     if transition is None:

@@ -151,6 +151,21 @@ SEQDIFF_API int seqdiff_sample_ex(seqdiff_model_t* m, int precision, int B, int 
                       const float* receptor_mask, int diverse, const float* noise_E_steps, uint64_t seed,
                       uint64_t graph_id0, int flags, float* final_out, void* stream);
 
+/* The same loop for P pockets x K samples per pocket (peptide design: many candidate sequences for one binding pocket).  Ligand-side
+ * arrays hold B = P*K graphs, sample j of pocket p being graph p*K + j with global graph id graph_id0 + p*K + j in the Philox stream:
+ * x_T / final_out [P*K,L_lig,20], ligand_angle [P*K,L_lig,8], ligand_mask [P*K,L_lig], noise_E_steps [T,P*K*L_lig,20] or NULL.
+ * Receptor-side arrays hold the P pockets once: receptor_seq [P,L_rec,20], receptor_angle [P,L_rec,8], receptor_mask [P,L_rec].
+ * The receptor rows of a step (angle embedding, ligand_feature_emb's adaLN + MLP, all decoder layers' cross K|V) depend on the
+ * pocket and the step only, so they are computed once per pocket and the K samples' cross-attention reads them.  final_out equals,
+ * bit for bit, what seqdiff_sample_ex returns for the batch whose receptor arrays are repeated K times per pocket (packed mode:
+ * at the valid positions, padded ones 0).  K = 1 is seqdiff_sample_ex.  P < 1, K < 1 or P*K*max(L_lig, L_rec) > INT32_MAX:
+ * SEQDIFF_ERR_INVALID. */
+SEQDIFF_API int seqdiff_sample_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T,
+                         const float* q_tables_steps, const float* x_T, const float* ligand_angle,
+                         const float* ligand_mask, const float* receptor_seq, const float* receptor_angle,
+                         const float* receptor_mask, int diverse, const float* noise_E_steps, uint64_t seed,
+                         uint64_t graph_id0, int flags, float* final_out, void* stream);
+
 /* ---- output decode: replaces the per-graph loop of denoise(), sequence_model/sample.py:208-224 --------------------
  * final_seq [B,L,20] (the loop's result: raw logits of the last step), true_seq [B,L,20] one-hot, ligand_mask [B,L] {0,1}.
  * pred_idx / true_idx [B,L] u8 = argmax over classes (first maximum, like torch.argmax); counts [B,2] i32 =
