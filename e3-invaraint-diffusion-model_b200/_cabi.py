@@ -62,7 +62,6 @@ PROTOTYPES = {
     "seqdiff_struct_p_sample": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _u64, _u64, _i, _vp, _vp]),
     "seqdiff_struct_sample": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u64, _vp, _vp, _vp]),
     "seqdiff_op_gemm": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
-    "seqdiff_op_gemm_ln": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, C.c_float, _vp, _vp, _vp, _vp]),
     "seqdiff_op_attention": (_i, [_i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _vp]),
     "seqdiff_op_attention_train_fwd": (_i, [_i, _i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, C.c_float, _u64, _u32, _u32, _vp, _vp]),
     "seqdiff_op_attention_train_bwd": (_i, [_i, _i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, C.c_float, _u64, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),

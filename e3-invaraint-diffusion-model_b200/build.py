@@ -16,28 +16,19 @@ CSRC = os.path.join(HERE, "csrc")
 # SEQDIFF_VARIANT=<name> with SEQDIFF_EXTRA_FLAGS="-D..." builds an experiment library libseqdiff_b200_<name>.so next to the product one
 # (own object directory); python loads it when SEQDIFF_LIB names its path (_cabi.py).  A/B measurements only.
 VARIANT = os.environ.get("SEQDIFF_VARIANT", "")
-OBJ = os.path.join(HERE, "build" + ("_ab" if os.environ.get("SEQDIFF_AB_KERNELS") == "1" else "") + ("_dbg" if os.environ.get("SEQDIFF_DEBUG_BOUNDS") == "1" else "") + (f"_{VARIANT}" if VARIANT else ""))
+OBJ = os.path.join(HERE, "build" + ("_dbg" if os.environ.get("SEQDIFF_DEBUG_BOUNDS") == "1" else "") + (f"_{VARIANT}" if VARIANT else ""))
 LIB = os.path.join(HERE, f"libseqdiff_b200_{VARIANT}.so" if VARIANT else ("libseqdiff_b200_dbg.so" if os.environ.get("SEQDIFF_DEBUG_BOUNDS") == "1" else "libseqdiff_b200.so"))
 SOURCES = ["gemm.cu", "rowwise.cu", "attention.cu", "attention_pipe.cu", "reverse_step.cu", "gauss_step.cu", "decode_loss.cu", "collate.cu", "train_kernels.cu", "attention_train.cu", "attention_train_tc.cu", "attention_bwd_pipe.cu", "train.cu", "model.cu", "cabi.cu"]
-# SEQDIFF_AB_KERNELS=1: also build the superseded attention kernels (attention_tc.cu, the mma.sync kernel in attention.cu) as A/B
-# references selectable with SEQDIFF_ATTN=tc|mma.  SEQDIFF_DEBUG_BOUNDS=1: device-side bounds / invariant asserts in every kernel
-# (the stand-in for compute-sanitizer, which the GPU pool does not allow); both change the object directory, not the sources.
-AB_KERNELS = os.environ.get("SEQDIFF_AB_KERNELS") == "1"
+# SEQDIFF_DEBUG_BOUNDS=1: device-side bounds / invariant asserts in every kernel (the stand-in for compute-sanitizer, which the GPU
+# pool does not allow); it changes the object directory and the library name, not the sources.
 DEBUG_BOUNDS = os.environ.get("SEQDIFF_DEBUG_BOUNDS") == "1"
-if AB_KERNELS:
-    SOURCES.insert(3, "attention_tc.cu")
 HEADERS = ["common.cuh", "kernels.h", "model.cuh", "philox.cuh", "skew.cuh", os.path.join("..", "..", "include", "seqdiff_b200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-Xptxas", "-v",
 ]
-
-
-
 FLAGS += os.environ.get("SEQDIFF_EXTRA_FLAGS", "").split()
-if AB_KERNELS:
-    FLAGS.append("-DSEQDIFF_AB_KERNELS")
 if DEBUG_BOUNDS:
     FLAGS.append("-DSEQDIFF_DEBUG_BOUNDS")
 

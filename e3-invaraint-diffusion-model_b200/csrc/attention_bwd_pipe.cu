@@ -425,9 +425,8 @@ template <> struct BwdFmt<bf16> { static constexpr int v = 1; };
 
 // usable(...) = the shapes this kernel covers; everything else stays on attention_bwd_tc (wmma)
 bool attention_bwd_pipe_usable(int Lq, int Lk, const void* dist_emb, float p_drop) {
-  static const bool off = [] { const char* e = getenv("SEQDIFF_TRAIN_ATTN"); return e && (std::string(e) == "wmma" || std::string(e) == "simt"); }();
   (void)dist_emb;
-  return !off && Lq <= 128 && Lk <= 128 && Lq >= 1 && Lk >= 1 && (p_drop <= 0.f || Lk % 4 == 0);
+  return Lq <= 128 && Lk <= 128 && Lq >= 1 && Lk >= 1 && (p_drop <= 0.f || Lk % 4 == 0);
 }
 
 template <typename T, bool REL>

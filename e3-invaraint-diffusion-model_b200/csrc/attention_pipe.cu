@@ -1,9 +1,9 @@
-// attention_pipe.cu -- persistent, warp-specialised tcgen05 attention core (same math as attention.cu / attention_tc.cu,
+// attention_pipe.cu -- persistent, warp-specialised tcgen05 attention core (same math as attention.cu's fp32 kernel,
 // SURVEY.md Appendix A; reference call sites sequence_model/model.py:61 and 226-231 through HF BertSelfAttention):
 //
 //   S[l,r] = ( q_l . k_r + q_l . E[l - r + P - 1] ) / 8 + (1 - mask[r]) * -10000 ;  out_l = softmax_r(S[l,:]) @ V
 //
-// attention_tc.cu runs ONE (graph, head, query block) per CTA as a serial chain  TMA -> MMA -> softmax -> MMA -> store; at
+// The round-1 tcgen05 kernel ran ONE (graph, head, query block) per CTA as a serial chain TMA -> MMA -> softmax -> MMA -> store; at
 // L = 128 that chain is pure latency (25-41 us per launch for 3-6 GFLOP).  Here one CTA per SM walks a list of work items
 // (graph, head, 128-query block) x key blocks ("steps") with three roles that only meet at mbarriers:
 //   warp 0      TMA producer : Q (double-buffered per item), K (+ the 256-row window of E a step can touch), V (double-buffered)

@@ -104,7 +104,7 @@ __global__ void __launch_bounds__(kAtThreads) attention_train_kernel(int heads, 
                                                                      DropSpec dr, T* __restrict__ out, const T* __restrict__ dout,
                                                                      T* __restrict__ dq, int lddq, T* __restrict__ dk, int lddk,
                                                                      T* __restrict__ dv, int lddv, float* __restrict__ dE) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   extern __shared__ float sm[];
   const int h = blockIdx.x, b = blockIdx.y;
   const int t = threadIdx.x;

@@ -93,7 +93,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) attention_train_tc_kernel(int h
                                                                           DropSpec dr, T* __restrict__ out, const T* __restrict__ dout,
                                                                           T* __restrict__ dq, int lddq, T* __restrict__ dk, int lddk,
                                                                           T* __restrict__ dv, int lddv, float* __restrict__ dE, int n_items) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   extern __shared__ __align__(128) uint8_t smraw[];
   uint8_t* sm = smraw + ((128u - (smem_u32(smraw) & 127u)) & 127u);
   // (nvcuda::wmma's load_matrix_sync lowers to state-space-less wmma.load: 17 % of the executed instructions are generic LD on

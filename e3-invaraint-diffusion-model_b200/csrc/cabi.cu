@@ -355,17 +355,6 @@ int seqdiff_op_gemm(int precision, int M, int N, int K, const void* A, const voi
   SD_GUARD_END
 }
 
-int seqdiff_op_gemm_ln(int precision, int M, int N, int K, const void* A, const void* W, const float* bias, const float* resid,
-                       const float* ln_w, const float* ln_b, float eps, float* C, void* h, float* stats, void* stream) {
-  SD_GUARD_BEGIN
-  SD_CHECK(A && W && bias && resid && ln_w && ln_b && C && h && stats, "null argument");
-  SD_CHECK(precision == SEQDIFF_BF16 || precision == SEQDIFF_FP16, "fused GEMM + LayerNorm exists in the 16-bit modes only");
-  const int fmt = precision == SEQDIFF_FP16 ? 0 : 1;
-  const LnOut lo{ln_w, ln_b, eps, h, reinterpret_cast<float2*>(stats)};
-  return gemm_16(M, N, K, A, fmt, W, fmt, bias, resid, 0, C, 2, static_cast<cudaStream_t>(stream), 0, nullptr, &lo);
-  SD_GUARD_END
-}
-
 int seqdiff_op_attention(int precision, int B, int heads, int Lq, int Lk, const void* q, int ldq, const void* k, int ldk,
                          const void* v, int ldv, const void* dist_emb, int P, const float* key_mask, void* out, void* stream) {
   SD_GUARD_BEGIN

@@ -213,42 +213,6 @@ __device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, const void* s
                "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2)
                : "memory");
 }
-// L2 eviction-priority policies for bulk tensor copies (createpolicy): a streaming output larger than L2 is stored evict_first
-// so that it does not push the GEMM's re-read operands out of L2, which are loaded evict_last
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* m, const void* smem_src, int c0, int c1, uint64_t policy) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;" ::"l"(
-                   reinterpret_cast<uint64_t>(m)),
-               "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "l"(policy)
-               : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_e_hint(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint64_t policy) {
-  asm volatile(
-      "{\n\t.reg .pred e;\n\t"
-      "elect.sync _|e, 0xffffffff;\n\t"
-      "@e cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;\n\t}" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "l"(policy)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_cg2_e_hint(void* smem_dst, const CUtensorMap* m, uint32_t bar_cluster_addr, int c0, int c1, uint64_t policy) {
-  asm volatile(
-      "{\n\t.reg .pred e;\n\t"
-      "elect.sync _|e, 0xffffffff;\n\t"
-      "@e cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5;\n\t}" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "l"(policy)
-      : "memory");
-}
 // 2-D tile store shared -> global (bulk async group); rows / columns outside the tensor are clipped
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(reinterpret_cast<uint64_t>(m)),
@@ -316,27 +280,6 @@ __device__ __forceinline__ void tmem_st_32x32(uint32_t taddr, const uint32_t (&r
       : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-// ---- cluster-scope helpers for epilogue-only exchanges between the CTAs of a cluster (distributed shared memory) ------
-__device__ __forceinline__ void st_cluster_f32x2(uint32_t cluster_addr, float a, float b) {
-  asm volatile("st.shared::cluster.v2.f32 [%0], {%1, %2};" ::"r"(cluster_addr), "f"(a), "f"(b) : "memory");
-}
-// wait for a phase completed by (possibly remote) release.cluster arrivals; makes the peers' prior DSMEM writes visible
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done;
-  uint32_t spins = 0;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (!done && ++spins > (1u << 24)) __trap();
-  } while (!done);
-}
 
 // ---- PTX: CTA pairs (cta_group::2) -- one tcgen05.mma spans the two SMs of a cluster of 2 -------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -516,19 +459,11 @@ int debug_guard_check(cudaStream_t s, int* n_bands, int* n_broken);
 // Every kernel of the path is launched with cudaLaunchAttributeProgrammaticStreamSerialization: it may become resident
 // while its predecessor drains, runs its prologue (smem carve-up, mbarrier init, TMEM alloc, descriptor prefetch), and then
 // blocks in pdl_wait() until the predecessor grid has completed and flushed -- before its first dependent global access.
-// pdl_trigger() lets the successor start being scheduled.  Both are no-ops without the attribute (SEQDIFF_PDL=0).
+// pdl_trigger() lets the successor start being scheduled.  Both are no-ops without the attribute.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// first statement of every kernel of the training step: nothing but the wait (a no-op unless the launch carries the programmatic
-// stream serialization attribute, SEQDIFF_TRAIN_PDL); -DSEQDIFF_TRAIN_TRIGGER also lets the successor's CTAs become resident early
-#ifdef SEQDIFF_TRAIN_TRIGGER
-#define SD_TRAIN_PDL_PROLOGUE() do { ::seqdiff::pdl_trigger(); ::seqdiff::pdl_wait(); } while (0)
-#else
-#define SD_TRAIN_PDL_PROLOGUE() ::seqdiff::pdl_wait()
-#endif
-bool pdl_enabled();
 int pdl_scope_exchange(int mode);  // sets the calling thread's scope mode (0 = none), returns the previous one
-int pdl_mode();  // effective mode of this launch: 0 off, 1 every launch, 2 only light successors (< 64 KB of shared memory), 3 only heavy ones
+int pdl_mode();  // effective mode of this launch: 0 off, 1 every launch, 3 only heavy successors (>= 64 KB of shared memory)
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_kc(int cluster_x, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
   cudaLaunchConfig_t cfg{};
@@ -538,8 +473,8 @@ inline cudaError_t launch_kc(int cluster_x, void (*kernel)(KArgs...), dim3 grid,
   cfg.stream = s;
   cudaLaunchAttribute attr[2];
   int n = 0;
-  const int pm = pdl_mode();  // 0 off | 1 every launch | 2 light successors only | 3 heavy successors only (model.cu)
-  if (pm == 1 || (pm == 2 && smem < 65536) || (pm == 3 && smem >= 65536)) {
+  const int pm = pdl_mode();  // 0 off | 1 every launch | 3 heavy successors only (model.cu)
+  if (pm == 1 || (pm == 3 && smem >= 65536)) {
     attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[n].val.programmaticStreamSerializationAllowed = 1;
     ++n;

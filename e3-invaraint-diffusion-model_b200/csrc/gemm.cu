@@ -172,29 +172,16 @@ constexpr int kGemmThreads = 320;
 // of A and HALF of the B tile (the MMA reads both halves across the pair), so a CTA pulls 16 KB + BN/2 * 128 B per k-block
 // from L2 for 128 x BN x 64 MACs -- 2/3 of the 1-CTA traffic at BN = 256.  The mainloop of this model's GEMMs is bound by
 // exactly that L2 -> SM operand stream (profiles/prof_gemm_r01.summary.txt).
-// BN = 384 / 512 (CTA pairs only): the tile is wider than one UMMA (N <= 256), so every k-step issues kNSub = 2 MMAs of
-// kSubN = BN / 2 columns into adjacent TMEM column ranges.  The accumulator then fills most of TMEM (one stage: the epilogue
-// is not overlapped with a next tile) -- these shapes exist for the M = 8192 GEMMs with N = 768 / 1024, where 256 x 384 /
-// 256 x 512 pair tiles cover the whole problem in ONE wave of 128 CTAs (vs 2 ragged waves of 128 x 192) and pull 40 / 48 KB
-// per CTA per k-block for 3 / 4 x the MACs of a 128 x 128 tile.
-template <int BN, bool CG2, bool LN = false> struct GemmCfg {
-  static constexpr int kNSub = BN > 256 ? 2 : 1;
-  static constexpr int kSubN = BN / kNSub;                         // N of one tcgen05.mma
-  static constexpr int kBoxRows = CG2 ? kSubN / 2 : kSubN;         // rows of one B TMA box (per CTA)
-  static constexpr int kBRows = kBoxRows * kNSub;                  // B rows staged per CTA per k-block
-  static constexpr int kAccStages = BN > 256 ? 1 : 2;
+template <int BN, bool CG2> struct GemmCfg {
+  static_assert(BN <= 256, "one tcgen05.mma per k-step: N <= 256");
+  static constexpr int kBoxRows = CG2 ? BN / 2 : BN;  // B rows staged per CTA per k-block (one TMA box)
   static constexpr int kABytes = kBM * kBK * 2;
-  static constexpr int kBBytes = kBRows * kBK * 2;
+  static constexpr int kBBytes = kBoxRows * kBK * 2;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  // (the fused-LayerNorm instantiations give one stage of the deepest rings to their 10 KB exchange area)
-  static constexpr int kStages = BN > 256 ? 4 : (CG2 ? 6 : (BN == 256 ? (LN ? 3 : 4) : (BN == 192 ? 4 : (LN ? 5 : 6))));
-  static constexpr int kTmemCols = BN == 128 ? 256 : 512;  // accumulator stage(s), rounded up to a power of two
+  static constexpr int kStages = (CG2 || BN == 128) ? 6 : 4;
+  static constexpr int kTmemCols = BN == 128 ? 256 : 512;  // 2 accumulator stages, rounded up to a power of two
   static constexpr int kStagingBytes = 8 * 32 * 32 * 4;  // one 32x32 fp32 transpose panel per epilogue warp
-  // fused-LayerNorm exchange area (used by the LNOUT instantiations only; 10.3 KB): [2 halves][128] float2 CTA-local partials,
-  // [2 tile parities][4 source CTAs][128] float2 cluster partials, 2 mbarriers
-  static constexpr int kLnBytes = 2 * 128 * 8 + 2 * 4 * 128 * 8 + 64;
-  static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/ + kStagingBytes + (LN ? kLnBytes : 0);
-  static_assert(BN <= 256 || CG2, "tiles wider than one UMMA are built for CTA pairs only");
+  static constexpr int kSmemBytes = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/ + kStagingBytes;
   static_assert(kSmemBytes <= 232448, "over the 227 KB shared-memory limit");
 };
 
@@ -207,38 +194,36 @@ template <> __device__ __forceinline__ void store4<f16>(f16* p, const float4& v)
   *reinterpret_cast<uint2*>(p) = make_uint2(pack_f16x2(v.x, v.y), pack_f16x2(v.z, v.w));
 }
 
+// Epilogue operand loads (the bias of the 16-bit epilogue, the fp32 residual): coherent loads, deliberately not ld.global.nc.  They
+// cannot move above the fences and barrier waits around them, so each chunk's registers stay local to its chunk.  With non-coherent
+// loads the scheduler hoists them across the unrolled chunk loop: the 16-bit epilogue grows from 86 to 168 registers and spills at
+// BN = 256, and the residual epilogue spills more at its 168-register cap.
+__device__ __forceinline__ float4 ld_f4(const float* p) {
+  float4 v;
+  asm volatile("ld.global.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
+  return v;
+}
+
 // split-K partial products: one 128-bit vector atomic per 4 outputs (fp32 C only; the other instantiations never reach it)
 template <typename T> __device__ __forceinline__ void add4(T*, const float4&) {}
 template <> __device__ __forceinline__ void add4<float>(float* p, const float4& v) { atomicAdd(reinterpret_cast<float4*>(p), v); }
 
 // TOut: bf16 / f16 (operand for the next GEMM or attention) or float (LayerNorm input); resid is always fp32.
 // RESID: 0 none, 1 fp32 residual tensor, 2 residual = LayerNorm(resid) rebuilt from per-row (mean, rstd) + affine (g, b)
-// TH != void: fused output LayerNorm (LnOut in kernels.h).  The grid is then made of clusters of kLnCl = 4 CTAs; CTA r of a
-// cluster owns column quarter r (N == 4 * BN) of the cluster's row blocks.
-constexpr int kLnCl = 4;
-struct LnOutArgs {
-  const float* g;
-  const float* b;
-  float eps;
-  void* h;
-  float2* stats;
-};
 // TN: C[M,N] = At^T Bt with At [K, M] and Bt [K, N] row-major (both operands MN-major for the MMA): the weight-gradient product
 // dW = dY^T X straight from the row-major activations / gradients -- no transposed copies.  tmA / tmB then carry boxes of
 // 64 k-rows x 64 columns; K (the token count) may be ragged, rows past it are zero-filled by TMA.
-template <int BN, int EPI, int RESID, typename TOut, bool CG2, typename TH = void, bool TN = false>
+template <int BN, int EPI, int RESID, typename TOut, bool CG2, bool TN = false>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC,
                     const float* __restrict__ bias, const float* __restrict__ resid, TOut* __restrict__ C, int M, int N, int K,
                     uint32_t idesc, const float2* __restrict__ ln_stats, const float* __restrict__ ln_g, const float* __restrict__ ln_b,
-                    unsigned long long* __restrict__ trace, const LnOutArgs lno, int l2_stream, int ksplit) {
+                    unsigned long long* __restrict__ trace, int ksplit) {
   // ksplit > 1 (fp32 C without residual only): split-K.  A scheduled tile is (output tile, k-range); every split ADDS its partial
   // product into C with vector atomics (C pre-zeroed by the caller, bias added by split 0).  For the weight-gradient products
   // dW[N,K] = dY^T X of the training step, whose outputs are a few dozen tiles with a contraction over every token of the batch.
-  constexpr bool LNOUT = !std::is_void<TH>::value;
-  using Cfg = GemmCfg<BN, CG2, LNOUT>;
-  static_assert(!LNOUT || (!CG2 && RESID != 0 && EPI == 0 && std::is_same<TOut, float>::value), "fused LayerNorm: 1-CTA MMA, fp32 C with residual");
-  static_assert(!TN || (!CG2 && !LNOUT && RESID == 0 && EPI == 0 && std::is_same<TOut, float>::value && BN % 64 == 0 && BN <= 256), "TN: 1-CTA MMA, fp32 C");
+  using Cfg = GemmCfg<BN, CG2>;
+  static_assert(!TN || (!CG2 && RESID == 0 && EPI == 0 && std::is_same<TOut, float>::value && BN % 64 == 0), "TN: 1-CTA MMA, fp32 C");
   constexpr int STAGES = Cfg::kStages;
   constexpr int TILE_M = CG2 ? 2 * kBM : kBM;  // rows per scheduled tile (per CTA pair / per CTA)
   extern __shared__ uint8_t smem_raw[];
@@ -261,12 +246,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   const int num_kb = (K + kBK - 1) / kBK;
   auto kb_lo = [&](int ks) { return static_cast<int>(static_cast<long long>(num_kb) * ks / ksplit); };
   const uint32_t cta_rank = CG2 ? cluster_ctarank() : 0u;  // 0 = leader (issues the MMAs), 1 = peer
-  // LNOUT: CTA r of cluster c walks tiles (m = c, c + #clusters, ...; n = r) -- with num_n == kLnCl that is tile c * 4 + r, step 4 * #clusters
   const int tile0 = CG2 ? static_cast<int>(blockIdx.x >> 1) : static_cast<int>(blockIdx.x);
   const int tile_step = CG2 ? static_cast<int>(gridDim.x >> 1) : static_cast<int>(gridDim.x);
-  float2* ln_cpart = reinterpret_cast<float2*>(smem + STAGES * Cfg::kStageBytes + 256 + Cfg::kStagingBytes);  // [2][128]
-  float2* ln_xpart = ln_cpart + 2 * 128;                                                                       // [2][4][128]
-  uint64_t* ln_bar = reinterpret_cast<uint64_t*>(ln_xpart + 2 * 4 * 128);                                      // [2]
 
   // optional timeline (debug, seqdiff_debug_attn_trace): CTA 0, lane 0 of the TMA / MMA / two epilogue warps
   int tr_n = 0;
@@ -287,7 +268,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tfull_bar[i], 1);
       mbar_init(&tempty_bar[i], CG2 ? 16 : 8);  // one arrival per epilogue warp (of both CTAs of a pair)
-      if (LNOUT) mbar_init(&ln_bar[i], kLnCl * 128);  // 128 row-owner threads of each CTA of the cluster
     }
     fence_mbar_init();
   }
@@ -301,7 +281,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     }
   }
   tc_fence_before();
-  if (CG2 || LNOUT) cluster_sync_all(); else __syncthreads();  // barriers of every CTA of the cluster initialised before any remote arrive / TMA signal
+  if (CG2) cluster_sync_all(); else __syncthreads();  // barriers of both CTAs of a pair initialised before any remote arrive / TMA signal
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   TR(41);
@@ -313,8 +293,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // ------------------------------- TMA producer -------------------------------
     // (whole warp runs the loop; one elected lane issues -- see common.cuh "warp-uniform single-issuer variants")
     {
-      // l2_stream: the output is larger than L2 -- operands are loaded evict_last, the output stored evict_first (below)
-      const uint64_t pol_keep = l2_stream ? l2_policy_evict_last() : 0ull;
       int stage = 0;
       uint32_t phase = 0;
       for (int tile = tile0; tile < num_tiles; tile += tile_step) {
@@ -328,17 +306,9 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             // both CTAs' tiles complete on the LEADER's full barrier, which the leader arms for the bytes of the pair
             if (cta_rank == 0) mbar_expect_tx_e(&full_bar[stage], 2 * Cfg::kStageBytes);
             const uint32_t bar = mapa_u32(smem_u32(&full_bar[stage]), 0);
-            if (l2_stream) tma_load_2d_cg2_e_hint(sA + stage * Cfg::kABytes, &tmA, bar, kb * kBK, a_row, pol_keep);
-            else tma_load_2d_cg2_e(sA + stage * Cfg::kABytes, &tmA, bar, kb * kBK, a_row);
-#pragma unroll
-            for (int j = 0; j < Cfg::kNSub; ++j) {  // half of each UMMA's B tile lives in each CTA of the pair
-              if (l2_stream)
-                tma_load_2d_cg2_e_hint(sB + stage * Cfg::kBBytes + j * Cfg::kBoxRows * kBK * 2, &tmB, bar, kb * kBK,
-                                       n_blk * BN + j * Cfg::kSubN + static_cast<int>(cta_rank) * Cfg::kBoxRows, pol_keep);
-              else
-                tma_load_2d_cg2_e(sB + stage * Cfg::kBBytes + j * Cfg::kBoxRows * kBK * 2, &tmB, bar, kb * kBK,
-                                  n_blk * BN + j * Cfg::kSubN + static_cast<int>(cta_rank) * Cfg::kBoxRows);
-            }
+            tma_load_2d_cg2_e(sA + stage * Cfg::kABytes, &tmA, bar, kb * kBK, a_row);
+            // half of the UMMA's B tile lives in each CTA of the pair
+            tma_load_2d_cg2_e(sB + stage * Cfg::kBBytes, &tmB, bar, kb * kBK, n_blk * BN + static_cast<int>(cta_rank) * Cfg::kBoxRows);
           } else if (TN) {
             mbar_expect_tx_e(&full_bar[stage], Cfg::kStageBytes);
 #pragma unroll
@@ -349,13 +319,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
               tma_load_2d_e(sB + stage * Cfg::kBBytes + j * 8192, &tmB, &full_bar[stage], n_blk * BN + 64 * j, kb * kBK);
           } else {
             mbar_expect_tx_e(&full_bar[stage], Cfg::kStageBytes);
-            if (l2_stream) {
-              tma_load_2d_e_hint(sA + stage * Cfg::kABytes, &tmA, &full_bar[stage], kb * kBK, a_row, pol_keep);
-              tma_load_2d_e_hint(sB + stage * Cfg::kBBytes, &tmB, &full_bar[stage], kb * kBK, n_blk * BN, pol_keep);
-            } else {
-              tma_load_2d_e(sA + stage * Cfg::kABytes, &tmA, &full_bar[stage], kb * kBK, a_row);
-              tma_load_2d_e(sB + stage * Cfg::kBBytes, &tmB, &full_bar[stage], kb * kBK, n_blk * BN);
-            }
+            tma_load_2d_e(sA + stage * Cfg::kABytes, &tmA, &full_bar[stage], kb * kBK, a_row);
+            tma_load_2d_e(sB + stage * Cfg::kBBytes, &tmB, &full_bar[stage], kb * kBK, n_blk * BN);
           }
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
@@ -382,13 +347,9 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
           for (int k = 0; k < kBK / kUmmaK; ++k) {
             const uint64_t adesc = TN ? umma_desc_mnmajor_sw128(a_addr + k * 2048, 8192) : umma_desc_kmajor_sw128(a_addr + k * kUmmaK * 2);
-#pragma unroll
-            for (int j = 0; j < Cfg::kNSub; ++j) {
-              const uint64_t bdesc = TN ? umma_desc_mnmajor_sw128(b_addr + k * 2048, 8192)
-                                        : umma_desc_kmajor_sw128(b_addr + j * Cfg::kBoxRows * kBK * 2 + k * kUmmaK * 2);
-              if (CG2) umma_cg2_e(tmem_d + j * Cfg::kSubN, adesc, bdesc, idesc, ((kb - kb_begin) | k) != 0 ? 1u : 0u);
-              else umma_bf16_e(tmem_d + j * Cfg::kSubN, adesc, bdesc, idesc, ((kb - kb_begin) | k) != 0 ? 1u : 0u);
-            }
+            const uint64_t bdesc = TN ? umma_desc_mnmajor_sw128(b_addr + k * 2048, 8192) : umma_desc_kmajor_sw128(b_addr + k * kUmmaK * 2);
+            if (CG2) umma_cg2_e(tmem_d, adesc, bdesc, idesc, ((kb - kb_begin) | k) != 0 ? 1u : 0u);
+            else umma_bf16_e(tmem_d, adesc, bdesc, idesc, ((kb - kb_begin) | k) != 0 ? 1u : 0u);
           }
           // smem slot reusable once these MMAs have read it (in both CTAs of a pair)
           if (CG2) umma_commit_mc_e(&empty_bar[stage], 3); else umma_commit_e(&empty_bar[stage]);
@@ -396,7 +357,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
         if (CG2) umma_commit_mc_e(&tfull_bar[as], 3); else umma_commit_e(&tfull_bar[as]);  // accumulator complete -> epilogue(s)
         TR(12);
-        if (++as == Cfg::kAccStages) { as = 0; aphase ^= 1; }
+        if (++as == 2) { as = 0; aphase ^= 1; }
       }
     }
   } else {
@@ -412,13 +373,9 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const int lr = lane >> 3, lc = lane & 7;
     int as = 0;
     uint32_t aphase = 0;
-    int ln_it = 0;  // tiles finished by this CTA (fused LayerNorm exchange parity / phase)
-    (void)ln_it;
     constexpr bool kTmaOut = !std::is_same<TOut, float>::value && RESID == 0;  // 16-bit output tiles leave through TMA stores
     int pcount = 0;  // staging panels used so far (they alternate across chunks AND tiles)
     (void)pcount;
-    const uint64_t pol_stream = (kTmaOut && l2_stream) ? l2_policy_evict_first() : 0ull;
-    (void)pol_stream;
     constexpr int NCH = BN / 64;  // 32-column chunks per warp and tile
     for (int tile = tile0; tile < num_tiles; tile += tile_step) {
       const int ks = tile % ksplit, mn = tile / ksplit;
@@ -428,12 +385,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(as * BN) + half * (BN / 2);
       const int col0 = n_blk * BN + half * (BN / 2) + 4 * lc;  // this lane's 4 columns of chunk 0; chunk ci adds 32 ci
       const bool full = row_base + 32 <= M;                    // warp-uniform: no row of this warp's slab is out of range
-      float rs[LNOUT ? 8 : 1], rq[LNOUT ? 8 : 1];  // fused LayerNorm: this lane's partial row sums / sums of squares (8 rows x 4 cols x NCH chunks)
-      if (LNOUT) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { rs[i] = 0.f; rq[i] = 0.f; }
-      }
-      (void)rs; (void)rq;
       if constexpr (kTmaOut) {
         // ---- 16-bit outputs without residual: no transpose.  Each thread owns one accumulator row (TMEM lane) and 32
         // columns per chunk: bias (broadcast loads) / activation / pack, 64 B per row into a SWIZZLE_64B panel, one TMA
@@ -453,7 +404,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           const int cur = ci & 1;
           float4 bv[8];
 #pragma unroll
-          for (int j4 = 0; j4 < 8; ++j4) bv[j4] = __ldg(reinterpret_cast<const float4*>(bias + colw + 32 * ci + 4 * j4));  // same address in every lane
+          for (int j4 = 0; j4 < 8; ++j4) bv[j4] = ld_f4(bias + colw + 32 * ci + 4 * j4);  // same address in every lane
           tmem_ld_wait();
           if (ci + 1 < NCH) tmem_ld_32x32(t_row + static_cast<uint32_t>(32 * (ci + 1)), r[cur ^ 1]);
           uint32_t pk[16];
@@ -480,8 +431,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           fence_proxy_async_smem();  // generic-proxy writes -> visible to the TMA store (async proxy)
           __syncwarp();
           if (lane == 0) {
-            if (l2_stream) tma_store_2d_hint(&tmC, panel, colw + 32 * ci, row_base, pol_stream);
-            else tma_store_2d(&tmC, panel, colw + 32 * ci, row_base);
+            tma_store_2d(&tmC, panel, colw + 32 * ci, row_base);
             tma_store_commit();
           }
           ++pcount;
@@ -511,7 +461,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       };
       auto fetch_resid_row = [&](int ci, int i) {
         const int row = row_base + 4 * i + lr;
-        rres[i] = (full || row < M) ? __ldg(reinterpret_cast<const float4*>(resid + static_cast<size_t>(row) * N + col0 + 32 * ci))
+        rres[i] = (full || row < M) ? ld_f4(resid + static_cast<size_t>(row) * N + col0 + 32 * ci)
                                     : make_float4(0.f, 0.f, 0.f, 0.f);
       };
       fetch_small(0, 0);
@@ -571,10 +521,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 }
                 v[u].x += rv.x; v[u].y += rv.y; v[u].z += rv.z; v[u].w += rv.w;
               }
-              if (LNOUT) {
-                rs[i] += (v[u].x + v[u].y) + (v[u].z + v[u].w);
-                rq[i] = fmaf(v[u].x, v[u].x, fmaf(v[u].y, v[u].y, fmaf(v[u].z, v[u].z, fmaf(v[u].w, v[u].w, rq[i]))));
-              }
             }
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
@@ -597,90 +543,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         if (CG2 && cta_rank != 0) mbar_arrive_cluster(mapa_u32(smem_u32(&tempty_bar[as]), 0));  // the leader's MMA thread waits on it
         else mbar_arrive(&tempty_bar[as]);
       }
-      if constexpr (LNOUT) {
-        // ---- fused LayerNorm of the rows just written (C = pre-LN tensor o; see LnOut in kernels.h) ----
-        // (1) row sums of this warp's 32 x BN/2 slab: reduce over the 8 lanes that share a row, park them in smem
-        const int et = static_cast<int>(threadIdx.x) - 64;  // epilogue thread 0..255
-        const int par = ln_it & 1;                          // exchange buffers alternate per tile
-        // (0) re-read of the tile's pre-LN values for the normalisation pass, issued NOW so that its L2 round trip runs under
-        //     the reduction and the cluster exchange.  Each lane reads back exactly the elements it stored in pass A
-        //     (program order makes them visible; C is not read through the non-coherent path).
-        float4 vc[NCH][8];
-#pragma unroll
-        for (int ci = 0; ci < NCH; ++ci)
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int row = row_base + 4 * i + lr;
-            vc[ci][i] = (full || row < M) ? *reinterpret_cast<const float4*>(C + static_cast<size_t>(row) * N + col0 + 32 * ci)
-                                          : make_float4(0.f, 0.f, 0.f, 0.f);
-          }
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-#pragma unroll
-          for (int off = 1; off < 8; off <<= 1) {
-            rs[i] += __shfl_xor_sync(0xffffffffu, rs[i], off);
-            rq[i] += __shfl_xor_sync(0xffffffffu, rq[i], off);
-          }
-        if (lc == 0) {
-#pragma unroll
-          for (int i = 0; i < 8; ++i) ln_cpart[half * 128 + q * 32 + 4 * i + lr] = make_float2(rs[i], rq[i]);
-        }
-        asm volatile("bar.sync 1, 256;" ::: "memory");  // the 8 epilogue warps
-        // (2) one thread per row adds the two column halves and pushes the CTA's partial into every CTA of the cluster
-        if (et < 128) {
-          const float2 a = ln_cpart[et], b2 = ln_cpart[128 + et];
-          const uint32_t my = cluster_ctarank();
-#pragma unroll
-          for (uint32_t pr = 0; pr < kLnCl; ++pr) {
-            st_cluster_f32x2(mapa_u32(smem_u32(&ln_xpart[(par * kLnCl + static_cast<int>(my)) * 128 + et]), pr), a.x + b2.x, a.y + b2.y);
-            mbar_arrive_cluster(mapa_u32(smem_u32(&ln_bar[par]), pr));  // release.cluster: orders the store above
-          }
-        }
-        TR(24);
-        // (3) all four column quarters of these 128 rows have arrived
-        mbar_wait_cluster(&ln_bar[par], static_cast<uint32_t>(ln_it >> 1) & 1u);
-        TR(25);
-        // (4) statistics of this lane's 8 rows (fp32 sums over N; variance as E[x^2] - mean^2, clamped at 0)
-        float mean8[8], rstd8[8];
-        const float inv_n = 1.0f / static_cast<float>(N);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int rl = q * 32 + 4 * i + lr;
-          float sx = 0.f, sq = 0.f;
-#pragma unroll
-          for (int pr = 0; pr < kLnCl; ++pr) {
-            const float2 t2 = ln_xpart[(par * kLnCl + pr) * 128 + rl];
-            sx += t2.x;
-            sq += t2.y;
-          }
-          mean8[i] = sx * inv_n;
-          const float var = fmaxf(fmaf(-mean8[i], mean8[i], sq * inv_n), 0.f);
-          rstd8[i] = 1.0f / sqrtf(var + lno.eps);
-          if (n_blk == 0 && half == 0 && lc == 0 && row_base + 4 * i + lr < M) lno.stats[row_base + 4 * i + lr] = make_float2(mean8[i], rstd8[i]);
-        }
-        // (5) normalise the values prefetched above
-        TH* hout = static_cast<TH*>(lno.h);
-#pragma unroll
-        for (int ci = 0; ci < NCH; ++ci) {
-          const int col = col0 + 32 * ci;
-          const float4 gg = __ldg(reinterpret_cast<const float4*>(lno.g + col));
-          const float4 bb = __ldg(reinterpret_cast<const float4*>(lno.b + col));
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int row = row_base + 4 * i + lr;
-            const float4 vv = vc[ci][i];
-            float4 hv;
-            hv.x = (vv.x - mean8[i]) * rstd8[i] * gg.x + bb.x;
-            hv.y = (vv.y - mean8[i]) * rstd8[i] * gg.y + bb.y;
-            hv.z = (vv.z - mean8[i]) * rstd8[i] * gg.z + bb.z;
-            hv.w = (vv.w - mean8[i]) * rstd8[i] * gg.w + bb.w;
-            if (full || row < M) store4<TH>(hout + static_cast<size_t>(row) * N + col, hv);
-          }
-        }
-        TR(26);
-        ++ln_it;
-      }
-      if (++as == Cfg::kAccStages) { as = 0; aphase ^= 1; }
+      if (++as == 2) { as = 0; aphase ^= 1; }
     }
     if (kTmaOut && lane == 0) tma_store_wait_all();  // bulk stores complete (and visible) before the CTA exits
   }
@@ -688,7 +551,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   TR(43);
   if (tr_on) trace[tr_base] = static_cast<unsigned long long>(tr_n);
   tc_fence_before();
-  if (CG2 || LNOUT) cluster_sync_all(); else __syncthreads();  // cluster: nobody frees TMEM / exits while a peer may still signal, read or write here
+  if (CG2) cluster_sync_all(); else __syncthreads();  // pair: nobody frees TMEM / exits while the peer may still signal, read or write here
   if (warp == 1) {
     tc_fence_after();
     if (CG2) tmem_dealloc_cg2(tmem_base, Cfg::kTmemCols); else tmem_dealloc(tmem_base, Cfg::kTmemCols);
@@ -708,68 +571,17 @@ static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtenso
   const int tiles = ceil_div(M, CG2 ? 2 * kBM : kBM) * (N / BN) * ksplit;
   const int slots = CG2 ? num_sms() / 2 : num_sms();
   const int grid = (tiles < slots ? tiles : slots) * (CG2 ? 2 : 1);
-  // SEQDIFF_GEMM_L2HINT=1: a 16-bit output that cannot stay in L2 anyway (> 64 MB) is stored evict_first and the operands are
-  // loaded evict_last.  Measured neutral on B200 (tile cadence, per-shape sweep and bench all within noise), so off by default.
-  static const int hint_on = [] { const char* e = getenv("SEQDIFF_GEMM_L2HINT"); return e ? atoi(e) : 0; }();
-  const int l2_stream = (hint_on && !std::is_same<TOut, float>::value && RESID == 0 && static_cast<double>(M) * N * 2 > 64e6) ? 1 : 0;
   SD_CUDA(launch_kc(CG2 ? 2 : 1, kfn, dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, s, ta, tb, tc, bias, resid, static_cast<TOut*>(C), M, N, K,
-                    idesc, ln ? ln->stats : nullptr, ln ? ln->g : nullptr, ln ? ln->b : nullptr, g_attn_trace, LnOutArgs{}, l2_stream, ksplit));
+                    idesc, ln ? ln->stats : nullptr, ln ? ln->g : nullptr, ln ? ln->b : nullptr, g_attn_trace, ksplit));
   SD_LAUNCHED(ksplit > 1 ? (CG2 ? "gemm_tcgen05_2cta_splitk" : "gemm_tcgen05_splitk") : (CG2 ? "gemm_tcgen05_2cta" : "gemm_tcgen05"), s);
   return SEQDIFF_OK;
-}
-
-// fused GEMM + residual + LayerNorm: clusters of 4 CTAs (one per column quarter), each cluster walks its row blocks
-template <int BN, int RESID, typename TH>
-static int launch_tc_ln(const CUtensorMap& ta, const CUtensorMap& tb, const float* bias, const float* resid, float* C, int M, int N, int K,
-                        uint32_t idesc, cudaStream_t s, const LnResid* ln, const LnOut& lo) {
-  using Cfg = GemmCfg<BN, false, true>;
-  auto kfn = gemm_tcgen05_kernel<BN, 0, RESID, float, false, TH>;
-  static bool configured = false;
-  if (!configured) {
-    SD_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
-    configured = true;
-  }
-  const int num_m = ceil_div(M, kBM);
-  // A cluster needs its 4 SMs inside one GPC, so fewer clusters are co-resident than num_sms / 4 (32, not 37, on a 148-SM
-  // B200); persistent clusters beyond that number would only start after the first wave has finished all of its tiles.
-  static int max_cl = 0;
-  if (!max_cl) {
-    cudaLaunchConfig_t qc{};
-    qc.gridDim = dim3(num_sms() / kLnCl * kLnCl);
-    qc.blockDim = dim3(kGemmThreads);
-    qc.dynamicSmemBytes = Cfg::kSmemBytes;
-    cudaLaunchAttribute qa[1];
-    qa[0].id = cudaLaunchAttributeClusterDimension;
-    qa[0].val.clusterDim.x = kLnCl;
-    qa[0].val.clusterDim.y = 1;
-    qa[0].val.clusterDim.z = 1;
-    qc.attrs = qa;
-    qc.numAttrs = 1;
-    int n = 0;
-    SD_CUDA(cudaOccupancyMaxActiveClusters(&n, kfn, &qc));
-    max_cl = n > 0 ? n : 1;
-  }
-  // equal tile counts per cluster: the smallest cluster count that keeps the wave count of the full-occupancy schedule
-  const int waves = ceil_div(num_m, max_cl);
-  const int clusters = ceil_div(num_m, waves);
-  const LnOutArgs a{lo.g, lo.b, lo.eps, lo.h, lo.stats};
-  SD_CUDA(launch_kc(kLnCl, kfn, dim3(clusters * kLnCl), dim3(kGemmThreads), Cfg::kSmemBytes, s, ta, tb, ta /*unused store map*/, bias, resid, C, M, N, K, idesc,
-                    ln ? ln->stats : nullptr, ln ? ln->g : nullptr, ln ? ln->b : nullptr, g_attn_trace, a, 0, 1));
-  SD_LAUNCHED("gemm_tcgen05_ln", s);
-  return SEQDIFF_OK;
-}
-template <int BN, typename TH>
-static int dispatch_tc_ln(const CUtensorMap& ta, const CUtensorMap& tb, const float* bias, const float* resid, float* C, int M, int N, int K,
-                          uint32_t idesc, cudaStream_t s, const LnResid* ln, const LnOut& lo) {
-  if (ln) return launch_tc_ln<BN, 2, TH>(ta, tb, bias, resid, C, M, N, K, idesc, s, ln, lo);
-  return launch_tc_ln<BN, 1, TH>(ta, tb, bias, resid, C, M, N, K, idesc, s, ln, lo);
 }
 
 // C[M,N] (+)= At^T Bt: At [K, M], Bt [K, N] row-major 16-bit (fmt 0 = fp16, 1 = bf16), fp32 C.  split_k as in gemm_16 (C pre-zeroed when != 1).
 template <int BN>
 static int launch_tn(const CUtensorMap& ta, const CUtensorMap& tb, const float* bias, float* C, int M, int N, int K, uint32_t idesc, int ksplit, cudaStream_t s) {
   using Cfg = GemmCfg<BN, false>;
-  auto kfn = gemm_tcgen05_kernel<BN, 0, 0, float, false, void, true>;
+  auto kfn = gemm_tcgen05_kernel<BN, 0, 0, float, false, true>;
   static bool configured = false;
   if (!configured) {
     SD_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
@@ -778,7 +590,7 @@ static int launch_tn(const CUtensorMap& ta, const CUtensorMap& tb, const float* 
   const int tiles = ceil_div(M, kBM) * (N / BN) * ksplit;
   const int grid = tiles < num_sms() ? tiles : num_sms();
   SD_CUDA(launch_kc(1, kfn, dim3(grid), dim3(kGemmThreads), Cfg::kSmemBytes, s, ta, tb, ta, bias, static_cast<const float*>(nullptr), C, M, N, K, idesc,
-                    static_cast<const float2*>(nullptr), static_cast<const float*>(nullptr), static_cast<const float*>(nullptr), g_attn_trace, LnOutArgs{}, 0, ksplit));
+                    static_cast<const float2*>(nullptr), static_cast<const float*>(nullptr), static_cast<const float*>(nullptr), g_attn_trace, ksplit));
   SD_LAUNCHED(ksplit > 1 ? "gemm_tcgen05_tn_splitk" : "gemm_tcgen05_tn", s);
   return SEQDIFF_OK;
 }
@@ -812,11 +624,10 @@ int gemm_16_tn(int M, int N, int K, const void* At, const void* Bt, int fmt, con
 //    256 tiles of 128x192 (2 waves of 3/4-size tiles);
 //  * CTA pairs (cta_group::2, 256x256 per pair, 32 KB per CTA for the same MACs) gain 5-7 % on the largest GEMMs
 //    (ada2 1.21, cross-KV 1.23 PFLOP/s) and nothing on the small ones, whose time is ramp / tail: used from 2.5e10 MACs up.
-// SEQDIFF_GEMM_CG2=0 disables the pair kernel.  Returns bn | (cg2 << 16).
+// Returns bn | (cg2 << 16).
 static int pick_cfg(int M, int N, int K) {
-  static const int allow_cg2 = [] { const char* e = getenv("SEQDIFF_GEMM_CG2"); return e ? atoi(e) : 1; }();
   if (M <= 64) return 128;
-  if (allow_cg2 && N % 256 == 0 && static_cast<double>(M) * N * K >= 2.5e10) return 256 | (1 << 16);
+  if (N % 256 == 0 && static_cast<double>(M) * N * K >= 2.5e10) return 256 | (1 << 16);
   const int sms = num_sms();
   const int m_tiles = ceil_div(M, kBM);
   int best = 0;
@@ -849,11 +660,11 @@ static int dispatch_tc(const CUtensorMap& ta, const CUtensorMap& tb, const CUten
 // a_fmt / w_fmt: 0 = fp16, 1 = bf16.  out_kind: 0 = fp16, 1 = bf16, 2 = fp32 (identity epilogue only; implied by resid).
 // force_cfg: 0 = auto, else  bn | (cg2 << 16)  with bn in {128,192,256} (tests / sweeps).
 int gemm_16(int M, int N, int K, const void* A, int a_fmt, const void* W, int w_fmt, const float* bias, const float* resid, int epi,
-            void* C, int out_kind, cudaStream_t s, int force_cfg, const LnResid* ln_resid, const LnOut* ln_out, int split_k) {
+            void* C, int out_kind, cudaStream_t s, int force_cfg, const LnResid* ln_resid, int split_k) {
   SD_CHECK(M > 0 && N > 0 && K > 0, "empty GEMM");
   // split_k: 1 = off; n > 1 = n k-ranges per output tile; -1 = as many as fill the GPU (>= 4 k-blocks each).  C must be pre-zeroed.
   SD_CHECK(split_k >= -1 && split_k != 0, "split_k must be -1 (auto), 1 (off) or the number of k-ranges");
-  SD_CHECK(split_k == 1 || (out_kind == 2 && !resid && !ln_out && epi == 0), "split-K accumulates into an fp32 C without residual");
+  SD_CHECK(split_k == 1 || (out_kind == 2 && !resid && epi == 0), "split-K accumulates into an fp32 C without residual");
   SD_CHECK(N % 128 == 0, "tcgen05 GEMM needs N % 128 == 0");
   SD_CHECK(K % 8 == 0, "tcgen05 GEMM needs K % 8 == 0 (16B TMA pitch)");
   SD_CHECK(epi >= 0 && epi <= 2, "unknown GEMM epilogue");
@@ -864,24 +675,6 @@ int gemm_16(int M, int N, int K, const void* A, int a_fmt, const void* W, int w_
   SD_CHECK((a_fmt | 1) == 1 && out_kind >= 0 && out_kind <= 2, "bad operand format");
   // measured on B200: tcgen05.mma.kind::f16 with a_format != b_format faults as an illegal instruction
   SD_CHECK(a_fmt == w_fmt, "A and W must share one 16-bit format");
-  if (ln_out) {  // fused output LayerNorm: fixed tile width N / 4, clusters of 4 CTAs
-    SD_CHECK(resid && out_kind == 2 && epi == 0, "fused LayerNorm needs the fp32 residual form");
-    SD_CHECK(N == 512 || N == 768 || N == 1024, "fused LayerNorm: N must be 512, 768 or 1024 (4 column quarters of 128/192/256)");
-    SD_CHECK(ln_out->g && ln_out->b && ln_out->h && ln_out->stats, "fused LayerNorm: null argument");
-    const int bq = N / kLnCl;
-    CUtensorMap ta, tb;
-    SD_TRY(make_tmap(A, a_fmt, M, K, kBM, &ta));
-    SD_TRY(make_tmap(W, w_fmt, N, K, bq, &tb));
-    const uint32_t idesc = umma_idesc_16(kBM, bq, static_cast<uint32_t>(a_fmt), static_cast<uint32_t>(w_fmt));
-    float* Cf = static_cast<float*>(C);
-#define SD_LN_DISPATCH(BN_)                                                                                                   \
-  return a_fmt == 1 ? dispatch_tc_ln<BN_, bf16>(ta, tb, bias, resid, Cf, M, N, K, idesc, s, ln_resid, *ln_out)                \
-                    : dispatch_tc_ln<BN_, f16>(ta, tb, bias, resid, Cf, M, N, K, idesc, s, ln_resid, *ln_out)
-    if (bq == 128) { SD_LN_DISPATCH(128); }
-    if (bq == 192) { SD_LN_DISPATCH(192); }
-    SD_LN_DISPATCH(256);
-#undef SD_LN_DISPATCH
-  }
   int cfg = force_cfg;
   int ksplit = split_k;
   if (ksplit != 1 && !cfg) cfg = pick_cfg(M, N, K);  // the tuner replays launches on the caller's C: not idempotent under accumulation
@@ -924,13 +717,7 @@ int gemm_16(int M, int N, int K, const void* A, int a_fmt, const void* W, int w_
         SD_CUDA(cudaStreamSynchronize(s));  // the operands are ready
         float best_ms = 0.f;
         constexpr int kReps = 8;
-        // (the 256 x 384 / 256 x 512 pair tiles of round 1 were never / once selected over cfg 1 / 2 / 3, the structure model and the
-        //  training shapes -- profiles/gemm_tune_selections_r02.log -- and are no longer built: SEQDIFF_WIDE_TILES brings them back)
-        for (int cand : {128, 192, 256, 128 | (1 << 16), 192 | (1 << 16), 256 | (1 << 16)
-#ifdef SEQDIFF_WIDE_TILES
-                         , 384 | (1 << 16), 512 | (1 << 16)
-#endif
-             }) {
+        for (int cand : {128, 192, 256, 128 | (1 << 16), 192 | (1 << 16), 256 | (1 << 16)}) {
           if (N % (cand & 0xffff)) continue;
           // eager warm-up launch: kernel attributes and the descriptor cache are set outside the capture
           SD_TRY(gemm_16(M, N, K, A, a_fmt, W, w_fmt, bias, resid, epi, C, out_kind, ts, cand, ln_resid));
@@ -975,14 +762,13 @@ int gemm_16(int M, int N, int K, const void* A, int a_fmt, const void* W, int w_
   }
   const int bn = cfg & 0xffff;
   const bool cg2 = (cfg >> 16) != 0;
-  SD_CHECK((bn == 128 || bn == 192 || bn == 256 || ((bn == 384 || bn == 512) && cg2)) && N % bn == 0, "bad tile width");
+  SD_CHECK((bn == 128 || bn == 192 || bn == 256) && N % bn == 0, "bad tile width");
   CUtensorMap ta, tb;
   SD_TRY(make_tmap(A, a_fmt, M, K, kBM, &ta));
-  const int sub_n = bn > 256 ? bn / 2 : bn;  // N of one tcgen05.mma
-  SD_TRY(make_tmap(W, w_fmt, N, K, cg2 ? sub_n / 2 : sub_n, &tb));
+  SD_TRY(make_tmap(W, w_fmt, N, K, cg2 ? bn / 2 : bn, &tb));
   CUtensorMap tc = ta;  // store map of 16-bit outputs (unused for fp32 C)
   if (out_kind != 2) SD_TRY(make_tmap_store16(C, out_kind, M, N, &tc));
-  const uint32_t idesc = umma_idesc_16(cg2 ? 2 * kBM : kBM, sub_n, static_cast<uint32_t>(a_fmt), static_cast<uint32_t>(w_fmt));
+  const uint32_t idesc = umma_idesc_16(cg2 ? 2 * kBM : kBM, bn, static_cast<uint32_t>(a_fmt), static_cast<uint32_t>(w_fmt));
   if (ksplit != 1) {
     const int nkb = ceil_div(K, kBK);
     if (ksplit < 0) {  // auto: one scheduled tile per CTA slot, at least 4 k-blocks per k-range
@@ -997,12 +783,6 @@ int gemm_16(int M, int N, int K, const void* A, int a_fmt, const void* W, int w_
 #define SD_DISPATCH(BN_)                                                                                          \
   return cg2 ? dispatch_tc<BN_, true>(ta, tb, tc, bias, resid, epi, C, out_kind, M, N, K, idesc, s, ln_resid, ksplit) \
              : dispatch_tc<BN_, false>(ta, tb, tc, bias, resid, epi, C, out_kind, M, N, K, idesc, s, ln_resid, ksplit)
-#ifdef SEQDIFF_WIDE_TILES
-  if (bn == 512) return dispatch_tc<512, true>(ta, tb, tc, bias, resid, epi, C, out_kind, M, N, K, idesc, s, ln_resid, ksplit);
-  if (bn == 384) return dispatch_tc<384, true>(ta, tb, tc, bias, resid, epi, C, out_kind, M, N, K, idesc, s, ln_resid, ksplit);
-#else
-  SD_CHECK(bn <= 256, "the 384 / 512-wide pair tiles are not in this build (compile with -DSEQDIFF_WIDE_TILES)");
-#endif
   if (bn == 256) { SD_DISPATCH(256); }
   if (bn == 192) { SD_DISPATCH(192); }
   SD_DISPATCH(128);

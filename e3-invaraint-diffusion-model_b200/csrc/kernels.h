@@ -16,20 +16,8 @@ struct LnResid {
   const float* g;       // [N] LayerNorm weight
   const float* b;       // [N] LayerNorm bias
 };
-// ln_out != NULL (needs resid, fp32 C, N in {512, 768, 1024}): the kernel also applies the LayerNorm that FOLLOWS this
-// Linear -- h = LN(C) * g + b written as the 16-bit operand of the next GEMM, (mean, rstd) per row for a later LnResid
-// rebuild -- so the separate layernorm() launch and its re-read of C disappear.  Four CTAs of a cluster cover the 4 column
-// quarters of a 128-row block and exchange per-row partial sums through distributed shared memory.
-struct LnOut {
-  const float* g;   // [N] LayerNorm weight
-  const float* b;   // [N] LayerNorm bias
-  float eps;
-  void* h;          // [M, N] 16-bit output (format = a_fmt)
-  float2* stats;    // [M] (mean, rstd)
-};
 int gemm_16(int M, int N, int K, const void* A, int a_fmt, const void* W, int w_fmt, const float* bias, const float* resid, int epi,
-            void* C, int out_kind, cudaStream_t s, int force_bn = 0, const LnResid* ln_resid = nullptr, const LnOut* ln_out = nullptr,
-            int split_k = 1);  // split_k: 1 off | n k-ranges per tile | -1 auto; partial products are ADDED into a pre-zeroed fp32 C
+            void* C, int out_kind, cudaStream_t s, int force_bn = 0, const LnResid* ln_resid = nullptr, int split_k = 1);  // split_k: 1 off | n k-ranges per tile | -1 auto; partial products are ADDED into a pre-zeroed fp32 C
 // C[M,N] (+)= At^T Bt + bias: At [K, M], Bt [K, N] row-major 16-bit (both MN-major for the MMA: no transposed copies); fp32 C.
 // The weight-gradient product dW[N_out, N_in] = dY^T X of the training step (At = dY [tokens, N_out], Bt = X [tokens, N_in]).
 int gemm_16_tn(int M, int N, int K, const void* At, const void* Bt, int fmt, const float* bias, float* C, cudaStream_t s, int split_k = 1);
@@ -126,10 +114,6 @@ int attention(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k,
 int collate(int G, const int* offsets, const uint8_t* lig_mask, const uint8_t* poc_mask, const float* ang, const float* aa, int ext, int L,
             float* lig_ang, float* lig_seq, float* lig_attn, float* rec_ang, float* rec_seq, float* rec_attn, int* lengths, cudaStream_t s);
 
-// ---- attention_tc.cu: tcgen05 attention (S, Q.E^T and P.V on UMMA, accumulators in TMEM) ------------------------------
-template <typename T>
-int attention_tc(int B, int heads, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const T* dist_emb,
-                 int P, const float* key_mask, T* out, cudaStream_t s);
 extern unsigned long long* g_attn_trace;  // debug timeline buffer of the pipelined kernel (NULL = off)
 // ---- attention_pipe.cu: persistent, warp-specialised version (TMA / MMA / softmax roles pipelined over work items) -----
 template <typename T>

@@ -76,15 +76,14 @@ int profile_end(char* tags, int tag_stride, float* ms, int* counts, int cap) {
   return n;
 }
 
-// Programmatic dependent launch.  SEQDIFF_PDL=0 / 1 / 2 / 3 forces a mode for every launch (off / every launch / only light successors /
-// only heavy successors, i.e. kernels with >= 64 KB of shared memory: the GEMM and attention kernels).  Unset: chosen per call from the
-// measured behaviour on B200 inside the replayed CUDA graph --
+// Programmatic dependent launch.  Modes: 0 off, 1 every launch, 3 only heavy successors, i.e. kernels with >= 64 KB of shared memory
+// (the GEMM and attention kernels).  Chosen per call from the measured behaviour on B200 inside the replayed CUDA graph --
 //   structure model (M = 4096 steps, 146 kernels of ~10 us): every launch, +2.5 .. 2.7 % (profiles/struct_bench_r01.json);
 //   sequence path, <= 2048 stacked token rows (grids of a few CTAs): every launch, B = 1 685 -> 616 us per step (profiles/pdl_small_r02.log);
 //   sequence path, <= 32768 rows (cfg 2: 16384 padded, ~7000 packed): heavy successors only, +1.1 % padded / +5.3 % packed; every launch
 //     costs 3 % there (the early-launched light kernels take registers next to the persistent CTAs), profiles/pdl_mode3_ab_r02.log;
 //   larger batches (cfg 3): off (+1.7 % padded but -7.6 % packed).
-static thread_local int g_pdl_scope = 0;   // 0 = none, else the mode (1 / 2 / 3) of the innermost scope
+static thread_local int g_pdl_scope = 0;   // 0 = none, else the mode (1 / 3) of the innermost scope
 struct PdlScope {
   const int prev;
   explicit PdlScope(int mode = 1) : prev(g_pdl_scope) { if (mode) g_pdl_scope = mode; }
@@ -100,11 +99,7 @@ int pdl_scope_exchange(int mode) {  // for the other translation units (train.cu
 // measured on B200 (profiles/pdl_small_r02.log) B = 1: 685 -> 616 us, B = 4: 711 -> 665 us per step; from B = 16 on the persistent
 // kernels fill every SM and the early launch only costs (846 -> 919 us).  Hence: on up to 2048 stacked token rows.
 static int pdl_auto_mode(long long rows) { return rows <= 2048 ? 1 : (rows <= 32768 ? 3 : 0); }
-int pdl_mode() {
-  static const int env = [] { const char* e = getenv("SEQDIFF_PDL"); return e ? (e[0] >= '0' && e[0] <= '3' ? e[0] - '0' : 0) : -1; }();
-  return env >= 0 ? env : g_pdl_scope;
-}
-bool pdl_enabled() { return pdl_mode() == 1; }
+int pdl_mode() { return g_pdl_scope; }
 
 // ---- debug-build guard bands (see common.cuh) -------------------------------------------------------------------------------
 #ifdef SEQDIFF_DEBUG_BOUNDS
@@ -202,26 +197,15 @@ static int gemm_S(int, int M, int N, int K, const float* A, const Wt& W, const f
 }
 template <typename T>
 static int gemm_S(int wfmt, int M, int N, int K, const T* A, const Wt& W, const float* bias, const float* resid, float* C, cudaStream_t s,
-                  const LnResid* ln = nullptr, const LnOut* lo = nullptr) {
+                  const LnResid* ln = nullptr) {
   const void* w = wfmt == 1 ? static_cast<const void*>(W.h) : static_cast<const void*>(W.g);
-  return gemm_16(M, N, K, A, Fmt<T>::v, w, wfmt, bias, resid, 0, C, 2, s, 0, ln, lo);
+  return gemm_16(M, N, K, A, Fmt<T>::v, w, wfmt, bias, resid, 0, C, 2, s, 0, ln);
 }
-// Linear + residual followed by its LayerNorm.  SEQDIFF_LN_FUSE=1 runs them as ONE launch (gemm.cu, LnOut: 4-CTA clusters
-// exchange row statistics through DSMEM).  Measured at cfg 2 (profiles/ln_fuse_ab_r01.txt) the fused kernel is 2 % SLOWER end
-// to end than GEMM + layernorm(): its 8 epilogue warps per SM do three memory passes (residual in, o out, o back in, h out)
-// that the stand-alone LayerNorm kernel streams with 64 warps per SM, and the epilogue (14 k cycles per tile) becomes the
-// bound of a K = 768 mainloop (4.6 k).  So it stays opt-in until the epilogue keeps the tile in TMEM (DESIGN.md section 9).
-static bool ln_fuse_enabled(int H) {
-  static const bool on = [] { const char* e = getenv("SEQDIFF_LN_FUSE"); return e && e[0] == '1'; }();
-  return on && (H == 512 || H == 768 || H == 1024);
-}
+// Linear + residual (o, the fp32 stream) followed by its LayerNorm (h, the operand of the next GEMM; stats for a later LnResid rebuild).
+// Fusing the LayerNorm into the GEMM epilogue was measured 2 % slower end to end at cfg 2 (DESIGN.md section 5c).
 template <typename T>
 static int gemm_ln(int wfmt, int M, int H, int K, const T* A, const Wt& W, const float* bias, const float* resid, float* o, const LnResid* lr,
                    const float* ln_w, const float* ln_b, float eps, T* h, float2* stats, cudaStream_t s) {
-  if (ln_fuse_enabled(H)) {
-    const LnOut lo{ln_w, ln_b, eps, h, stats};
-    return gemm_S(wfmt, M, H, K, A, W, bias, resid, o, s, lr, &lo);
-  }
   SD_TRY(gemm_S(wfmt, M, H, K, A, W, bias, resid, o, s, lr));
   return layernorm<T>(o, M, H, ln_w, ln_b, eps, nullptr, h, stats, s);
 }
@@ -1496,7 +1480,7 @@ int Model::struct_forward(int precision, int B, int Ll, int Lr, const float* tim
                           int phases, cudaStream_t s) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
   SD_CHECK(arch == kArchStructure, "handle holds a sequence model: use seqdiff_forward");
-  const PdlScope pdl_on(3);  // launch-bound path: programmatic dependent launch of the heavy kernels (42.3 -> 43.0 k graph-steps/s against every launch) unless SEQDIFF_PDL overrides
+  const PdlScope pdl_on(3);  // launch-bound path: programmatic dependent launch of the heavy kernels (42.3 -> 43.0 k graph-steps/s against every launch)
   SD_CHECK(precision >= SEQDIFF_FP32 && precision <= SEQDIFF_FP16, "unknown precision mode");
   SD_CHECK(B > 0 && Ll > 0 && Lr > 0, "empty batch");
   if (cfg.relative_key) SD_CHECK(Ll <= cfg.max_position_embeddings && Lr <= cfg.max_position_embeddings, "Length exceed");

@@ -105,6 +105,13 @@ __device__ __forceinline__ void write_onehot(float* __restrict__ row, int idx) {
   }
 }
 
+// The same shared-memory pointer, with its address computed at run time (shared window -> generic).  The fast kernel passes its tables
+// through this to the cold-path helper below: with one caller left, the compiler would otherwise specialise the helper on the three
+// static table addresses, and that shifts the caller's register allocation into 88 B of spills.
+__device__ __forceinline__ const float* opaque_smem(const float* p) {
+  return static_cast<const float*>(__cvta_shared_to_generic(__cvta_generic_to_shared(p)));
+}
+
 // Cold path: a row of x_t that is not exactly one-hot (never produced by the sampler itself; sample.py:129-138 accepts it).
 // Kept out of line and fed from global/shared memory so that the hot path's per-class arrays stay in registers.
 //   left[j] = Qt[j,:].x ; den[i] = Qtb[i,:].x (0 -> 1e-6) ; un[j] = sum_i p_i * left[j] * Qsb[i,j] / den[i]
@@ -350,7 +357,8 @@ __global__ void __launch_bounds__(THREADS, MINB) reverse_step_kernel(const float
         if (!live[r]) continue;
         int idx = best[r];
         if (!onehot[r])  // cold: a row of x_t that is not exactly one-hot (never produced by the sampler itself)
-          idx = soft_row_class<true>(logits + nr[r] * C, x_t + nr[r] * C, sQt, sQsb, sQtb, true, nullptr, seed, graph, static_cast<uint32_t>(lr[r]), step);
+          idx = soft_row_class<true>(logits + nr[r] * C, x_t + nr[r] * C, opaque_smem(sQt), opaque_smem(sQsb), opaque_smem(sQtb), true, nullptr, seed, graph,
+                                     static_cast<uint32_t>(lr[r]), step);
         write_onehot(x_s + nr[r] * C, idx);
         if (idx_out) idx_out[nr[r]] = static_cast<uint8_t>(idx);
       }
@@ -437,31 +445,12 @@ int reverse_step(const float* q_tables, int n_tab, int B, int L, const float* x_
                  uint8_t* idx_out, cudaStream_t s, int* advance, const uint64_t* rng) {
   SD_CHECK(B > 0 && L > 0, "empty reverse step");
   SD_CHECK(n_tab == 1 || n_tab == B, "q_tables must hold 1 or B (Qt,Qsb,Qtb) triples");
-  // launch shape of the production (fast) kernel: SEQDIFF_REV_CFG = threads per CTA * 100 + min CTAs per SM * 10 + residues per thread
-  // (sweep on B200: profiles/revstep_r01.log)
-  static const int cfg = [] { const char* e = getenv("SEQDIFF_REV_CFG"); return e ? atoi(e) : 25622; }();
-  if (diverse && !noise_E) {
-#define SD_REV_LAUNCH(T_, MB_)                                                                                                              \
-  {                                                                                                                                         \
-    const dim3 grid(ceil_div(L, (cfg % 10) * T_), B);                                                                                       \
-    SD_CUDA(launch_k(reverse_step_kernel<true, T_, MB_>, dim3(grid), dim3(T_), 0, s, q_tables, n_tab, L, x_t, logits, diverse, noise_E, seed, \
-                     graph_id0, step, step_ptr, x_s, idx_out, advance, rng));                                                               \
-  }
-    SD_CHECK(cfg % 10 >= 1, "SEQDIFF_REV_CFG: residues per thread must be >= 1");
-    switch (cfg / 10) {
-      case 2562: SD_REV_LAUNCH(256, 2); break;
-      case 2563: SD_REV_LAUNCH(256, 3); break;
-      case 1284: SD_REV_LAUNCH(128, 4); break;
-      case 1285: SD_REV_LAUNCH(128, 5); break;
-      case 1286: SD_REV_LAUNCH(128, 6); break;
-      case 643: SD_REV_LAUNCH(64, 3); break;
-      default: SD_CHECK(false, "SEQDIFF_REV_CFG: unknown launch shape");
-    }
-#undef SD_REV_LAUNCH
-  } else {
-    const dim3 grid(ceil_div(L, 2 * kRevThreads), B);
+  // 256 threads per CTA, 2 residues per thread; the fast kernel with 2 CTAs per SM (launch-shape sweep on B200: profiles/revstep_r01.log)
+  const dim3 grid(ceil_div(L, 2 * kRevThreads), B);
+  if (diverse && !noise_E)
+    SD_CUDA(launch_k(reverse_step_kernel<true, 256, 2>, dim3(grid), dim3(kRevThreads), 0, s, q_tables, n_tab, L, x_t, logits, diverse, noise_E, seed, graph_id0, step, step_ptr, x_s, idx_out, advance, rng));
+  else
     SD_CUDA(launch_k(reverse_step_kernel<false>, dim3(grid), dim3(kRevThreads), 0, s, q_tables, n_tab, L, x_t, logits, diverse, noise_E, seed, graph_id0, step, step_ptr, x_s, idx_out, advance, rng));
-  }
   SD_LAUNCHED("reverse_step", s);
   return SEQDIFF_OK;
 }

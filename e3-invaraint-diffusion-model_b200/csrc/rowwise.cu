@@ -287,22 +287,9 @@ __global__ void __launch_bounds__(THREADS) layernorm_kernel(const float* __restr
 
 template <typename T>
 int layernorm(const float* in, int M, int H, const float* w, const float* b, float eps, float* out32, T* outT, float2* stats, cudaStream_t s) {
-  // launch shape: SEQDIFF_LN_VAR = threads per CTA * 10 + rows per warp (sweep on B200: profiles/ln_sweep_r01.log)
-  static const int var = [] { const char* e = getenv("SEQDIFF_LN_VAR"); return e ? atoi(e) : 2561; }();
-#define SD_LN_LAUNCH(TH_, RPW_)                                                                                                           \
-  {                                                                                                                                       \
-    const int grid = ceil_div(ceil_div(M, RPW_) * 32, TH_);                                                                               \
-    SD_VPL_DISPATCH(H, SD_CUDA(launch_k(layernorm_kernel<T, VPL, TH_, RPW_>, dim3(grid), dim3(TH_), 0, s, in, M, H, w, b, eps, out32, outT, stats))); \
-  }
-  switch (var) {
-    case 1281: SD_LN_LAUNCH(128, 1); break;
-    case 5121: SD_LN_LAUNCH(512, 1); break;
-    case 2562: SD_LN_LAUNCH(256, 2); break;
-    case 1282: SD_LN_LAUNCH(128, 2); break;
-    case 641: SD_LN_LAUNCH(64, 1); break;
-    default: SD_LN_LAUNCH(256, 1); break;
-  }
-#undef SD_LN_LAUNCH
+  // 256 threads per CTA, one row per warp (launch-shape sweep on B200: profiles/ln_sweep_r01.log)
+  const int grid = ceil_div(M * 32, kRowThreads);
+  SD_VPL_DISPATCH(H, SD_CUDA(launch_k(layernorm_kernel<T, VPL, kRowThreads, 1>, dim3(grid), dim3(kRowThreads), 0, s, in, M, H, w, b, eps, out32, outT, stats)));
   SD_LAUNCHED("layernorm", s);
   return SEQDIFF_OK;
 }

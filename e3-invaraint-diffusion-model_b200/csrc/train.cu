@@ -55,7 +55,7 @@ static int gemm_any(int M, int N, int K, const T* A, const void* Bw, const float
   if constexpr (std::is_same<T, float>::value) {
     return gemm_f32(M, N, K, A, static_cast<const float*>(Bw), bias, resid, 0, static_cast<float*>(C), s);
   } else {
-    return gemm_16(M, N, K, A, TFmt<T>::v, Bw, TFmt<T>::v, bias, resid, 0, C, (out_f32 || resid) ? 2 : TFmt<T>::v, s, 0, nullptr, nullptr, split_k);
+    return gemm_16(M, N, K, A, TFmt<T>::v, Bw, TFmt<T>::v, bias, resid, 0, C, (out_f32 || resid) ? 2 : TFmt<T>::v, s, 0, nullptr, split_k);
   }
 }
 template <typename T> static const void* wsel(const Wt& w) {
@@ -68,7 +68,7 @@ template <typename T> static const void* wsel(const Wt& w) {
 template <typename T>
 __global__ void __launch_bounds__(256) embed_post_kernel(float* __restrict__ v, const float* __restrict__ te, int L, int H, size_t n8, DropSpec dr,
                                                          float* __restrict__ out32, T* __restrict__ outT) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   for (size_t i = static_cast<size_t>(blockIdx.x) * 256 + threadIdx.x; i < n8; i += static_cast<size_t>(gridDim.x) * 256) {
     float x[8], keep[8];
     load8<float>(v + 8 * i, x);
@@ -95,7 +95,7 @@ static int embed_post(float* v, const float* te, int L, int H, size_t n, DropSpe
   return SEQDIFF_OK;
 }
 __global__ void concat_masks_kernel(float* dst, const float* a, int na, const float* b, int nb) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < na + nb; i += gridDim.x * blockDim.x) dst[i] = i < na ? a[i] : b[i - na];
 }
 
@@ -286,10 +286,6 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
   auto hid = [&]() { return DropSpec{a.p_hidden, site++, a.step, a.seed}; };
   auto att = [&]() { return DropSpec{a.p_attn, site++, a.step, a.seed}; };
   const DropSpec nodrop{0.f, 0u, 0u, 0ull};
-  // SEQDIFF_TRAIN_ATTN=simt: the fp32 SIMT attention kernels in the 16-bit modes as well (A/B reference of the tensor-core kernels)
-  static const bool simt_attn = [] { const char* e = getenv("SEQDIFF_TRAIN_ATTN"); return e && std::string(e) == "simt"; }();
-  // SEQDIFF_TRAIN_ATTN=wmma: the wmma forward kernel instead of the pipelined tcgen05 one (A/B reference; the backward is wmma either way)
-  static const bool wmma_fwd = [] { const char* e = getenv("SEQDIFF_TRAIN_ATTN"); return e && std::string(e) == "wmma"; }();
 
   // ---- workspace ----------------------------------------------------------------------------------
   const size_t es = sizeof(T);
@@ -327,11 +323,10 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
     return dropout_add(O, resid, static_cast<size_t>(M) * N, dr, s);
   };
   // o = dropout(x W^T + b) + resid and h = LayerNorm(o): with dropout on, the residual add cannot ride in the GEMM epilogue (the mask sits
-  // between the two), so it is folded into the LayerNorm pass instead of a pass of its own.  SEQDIFF_DROP_LN_FUSE=0: separate launches.
-  static const bool drop_ln_fuse = [] { const char* e = getenv("SEQDIFF_DROP_LN_FUSE"); return !e || e[0] != '0'; }();
+  // between the two), so it is folded into the LayerNorm pass instead of a pass of its own.
   auto lin_res_ln = [&](int M, int N, int K, const T* X, const Wt& W, const float* bias, const float* resid, float* O, const DropSpec& dr,
                         const float* ln_w, const float* ln_b, const Act2<T>& h, uint8_t* keep_bits) -> int {
-    if (dr.p > 0.f && drop_ln_fuse) {
+    if (dr.p > 0.f) {
       SD_TRY(gemm_any<T>(M, N, K, X, wsel<T>(W), bias, nullptr, O, true, s));
       return dropout_add_layernorm<T>(O, resid, dr, M, N, ln_w, ln_b, eps, h.s, h.t_out(), keep_bits, s);
     }
@@ -341,7 +336,7 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
   // the attention dropout mask travels from the forward to the backward kernel as bits (2 KB per (graph, head)) when both run on the
   // tcgen05 kernels; every other combination regenerates it from the Philox stream
   auto keep_buf = [&](int nb, int Lq, int Lk) -> uint32_t* {
-    if (!k16 || simt_attn || wmma_fwd || a.p_attn <= 0.f || Lk % 4 != 0 || !attention_bwd_pipe_usable(Lq, Lk, nullptr, a.p_attn)) return nullptr;
+    if (!k16 || a.p_attn <= 0.f || Lk % 4 != 0 || !attention_bwd_pipe_usable(Lq, Lk, nullptr, a.p_attn)) return nullptr;
     return ar.take<uint32_t>(static_cast<size_t>(nb) * heads * 128 * 4);
   };
   auto attn_fwd = [&](int nb, int Lq, int Lk, const T* q, int ldq, const T* k, int ldk, const T* v, int ldv, const Wt* E, const float* mask,
@@ -350,10 +345,11 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
     if (dr.p <= 0.f) return attention<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, out, s);
     if constexpr (k16) {
       // the pipelined tcgen05 kernel of the inference path with the dropout mask applied to P (7x faster than the wmma forward)
-      if (!simt_attn && !wmma_fwd && Lk % 4 == 0) return attention_pipe_dropout<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, out, s, keep);
-      if (!simt_attn) return attention_train_fwd_tc<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, out, s);
+      if (Lk % 4 == 0) return attention_pipe_dropout<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, out, s, keep);
+      return attention_train_fwd_tc<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, out, s);
+    } else {
+      return attention_train_fwd<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, out, s);
     }
-    return attention_train_fwd<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, out, s);
   };
 
   // ---- forward ------------------------------------------------------------------------------------
@@ -471,7 +467,7 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
     tp.d_cattn = att();
     tp.d_o2 = hid();
     tp.d_o3 = hid();
-    if (k16 && a.p_hidden > 0.f && drop_ln_fuse) {  // written by dropout_add_layernorm, read by the fused LayerNorm backward
+    if (k16 && a.p_hidden > 0.f) {  // written by dropout_add_layernorm, read by the fused LayerNorm backward
       tp.kb1 = ar.take<uint8_t>(MlH / 8);
       tp.kb2 = ar.take<uint8_t>(MlH / 8);
       tp.kb3 = ar.take<uint8_t>(MlH / 8);
@@ -533,19 +529,14 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
 
   // backward of y = x W^T + b.  dY: T [M,N]; X: T [M,K].  dx_kind 0: none; 1: T [M,K]; 2: fp32 [M,K] (+ resid)
   // 16-bit modes: dW = dY^T X straight from the row-major tensors (both operands MN-major for the MMA, gemm_16_tn), db by a column-sum
-  // kernel -- the two 16-bit transposes per Linear (11 % of the step) are gone.  SEQDIFF_WGRAD_TN=0 restores the transposed form.
-  static const bool wgrad_tn = [] { const char* e = getenv("SEQDIFF_WGRAD_TN"); return !e || e[0] != '0'; }();
-  auto tn_ok = [&](int N, int K) { return k16 && wgrad_tn && N % 8 == 0 && K % 128 == 0; };
-  // LayerNorm backward that also emits the 16-bit dY operand and the bias gradient of the Linear in front of it (one launch instead of
-  // layernorm_bwd + grad_cast + colsum).  SEQDIFF_LN_BWD_FUSE=0 restores the three launches.
-  static const bool ln_bwd_fuse = [] { const char* e = getenv("SEQDIFF_LN_BWD_FUSE"); return !e || e[0] != '0'; }();
+  // kernel -- the two 16-bit transposes per Linear (11 % of the step) are gone.  fp32 mode and shapes failing tn_ok take the transposed form.
+  auto tn_ok = [&](int N, int K) { return k16 && N % 8 == 0 && K % 128 == 0; };
   auto linear_bwd = [&](int M, int N, int K, const T* dY, const T* X, const Wt& W, float* gW, float* gb, int dx_kind, void* dX,
                         const float* resid, bool db_done = false) -> int {
     if constexpr (k16) {
       if (tn_ok(N, K)) {
-        static const bool splitk_tn = [] { const char* e = getenv("SEQDIFF_WGRAD_SPLITK"); return !e || e[0] != '0'; }();
         if (!db_done) SD_TRY(colsum_add<T>(dY, M, N, gb, s));
-        SD_TRY(gemm_16_tn(N, K, M, dY, X, TFmt<T>::v, d_zero_bias, gW, s, splitk_tn ? -1 : 1));
+        SD_TRY(gemm_16_tn(N, K, M, dY, X, TFmt<T>::v, d_zero_bias, gW, s, -1));  // split-K as below
         if (dx_kind) SD_TRY(gemm_any<T>(M, K, N, dY, W.t, d_zero_bias, resid, dX, dx_kind == 2, s));
         return SEQDIFF_OK;
       }
@@ -555,9 +546,8 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
     SD_TRY(transpose_colsum<T>(dY, M, N, trA, gb, s, Mp));
     SD_TRY(transpose_colsum<T>(X, M, K, trB, nullptr, s, Mp));
     // dW [N,K]: a few dozen output tiles with a contraction over every token -> split-K over all SMs, partial products added
-    // into the gradient buffer (zeroed at the start of the backward pass); SEQDIFF_WGRAD_SPLITK=0 keeps one CTA per tile
-    static const bool splitk = [] { const char* e = getenv("SEQDIFF_WGRAD_SPLITK"); return !e || e[0] != '0'; }();
-    SD_TRY(gemm_any<T>(N, K, Mp, trA, trB, d_zero_bias, nullptr, gW, true, s, splitk ? -1 : 1));
+    // into the gradient buffer (zeroed at the start of the backward pass)
+    SD_TRY(gemm_any<T>(N, K, Mp, trA, trB, d_zero_bias, nullptr, gW, true, s, -1));
     if (dx_kind) SD_TRY(gemm_any<T>(M, K, N, dY, W.t, d_zero_bias, resid, dX, dx_kind == 2, s));
     return SEQDIFF_OK;
   };
@@ -565,11 +555,12 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
                       const DropSpec& dr, const T* dctx, T* dq, int lddq, T* dk, int lddk, T* dv, int lddv, float* gE, const uint32_t* keep) -> int {
     const T* e = E ? static_cast<const T*>(wsel<T>(*E)) : nullptr;
     if constexpr (k16) {
-      if (!simt_attn && attention_bwd_pipe_usable(Lq, Lk, e, dr.p))  // tcgen05 backward
+      if (attention_bwd_pipe_usable(Lq, Lk, e, dr.p))  // tcgen05 backward
         return attention_bwd_pipe<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, dctx, dq, lddq, dk, lddk, dv, lddv, gE, s, keep);
-      if (!simt_attn) return attention_bwd_tc<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, dctx, dq, lddq, dk, lddk, dv, lddv, gE, s);
+      return attention_bwd_tc<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, dctx, dq, lddq, dk, lddk, dv, lddv, gE, s);
+    } else {
+      return attention_bwd<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, dctx, dq, lddq, dk, lddk, dv, lddv, gE, s);
     }
-    return attention_bwd<T>(nb, heads, Lq, Lk, q, ldq, k, ldk, v, ldv, e, P, mask, dr, dctx, dq, lddq, dk, lddk, dv, lddv, gE, s);
   };
 
   // SELayer backward (model.py:52-63).  dout = gradient of tp.out.  Result: gradient of tp.x in s1; gradient of c in dc (if non-null).
@@ -636,7 +627,8 @@ int Model::train_t(int wfmt, const TrainArgs& a, cudaStream_t s) {
   float *cur = dA, *s1 = dB, *s2 = dC;
   // post-LN sublayer h = LN(o), o = dropout(x W^T + b) + resid: d(o) in fp32 (it is also the gradient of resid) and, as the Linear's dY,
   // masked by the dropout site `dr` in the operand type (gT).  K = fan-in of that Linear (decides the weight-gradient form, tn_ok).
-  auto ln_fused = [&](int K) { return ln_bwd_fuse && tn_ok(H, K); };
+  // (one launch: layernorm_bwd_cast also emits the 16-bit dY operand and the bias gradient of the Linear in front of it)
+  auto ln_fused = [&](int K) { return tn_ok(H, K); };
   auto ln_bwd = [&](const float* dh, const float* o, const float* gamma, float* d_o, float* dgam, float* dbet, const DropSpec& dr, float* dbias,
                     int K, const uint8_t* keep_bits) -> int {
     if constexpr (k16) {
@@ -717,13 +709,12 @@ int Model::train_step(const TrainArgs& a, cudaStream_t s) {
   // Programmatic dependent launch of the heavy kernels of the step (mode 3: tcgen05 GEMMs and attention -- their prologue, i.e. barrier
   // init, TMEM allocation, descriptor prefetch, runs under the predecessor's tail).  Every kernel launched inside this call starts with
   // griddepcontrol.wait, so any mode is safe.  Measured on B200 (profiles/train_pdl_ab_r02.log): 128 graphs 15.15 -> 14.64 ms per step,
-  // 16 graphs 5.00 -> 4.55 ms; every launch (mode 1) 14.72 / 4.76 ms.  SEQDIFF_TRAIN_PDL=0 | 1 | 2 | 3 overrides.
-  static const int train_pdl = [] { const char* e = getenv("SEQDIFF_TRAIN_PDL"); return e && e[0] >= '0' && e[0] <= '3' ? e[0] - '0' : 3; }();
+  // 16 graphs 5.00 -> 4.55 ms; every launch (mode 1) 14.72 / 4.76 ms.
   struct Scope {
     const int prev;
     explicit Scope(int m) : prev(pdl_scope_exchange(m)) {}
     ~Scope() { pdl_scope_exchange(prev); }
-  } pdl_scope(train_pdl);
+  } pdl_scope(3);
   switch (a.precision) {
     case SEQDIFF_FP32: return train_t<float>(1, a, s);
     case SEQDIFF_BF16: return train_t<bf16>(1, a, s);

@@ -81,7 +81,7 @@ __device__ __forceinline__ void ln_bwd_core(const float (&xhat)[VPL][8], float (
 template <typename T>
 __global__ void __launch_bounds__(256) transpose_colsum_kernel(const T* __restrict__ in, int rows, int cols, T* __restrict__ out, int pitch,
                                                                float* __restrict__ colsum) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   __shared__ float tile[64][65];
   const int r0 = blockIdx.y * 64, c0 = blockIdx.x * 64;
   const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;  // 64 x 4
@@ -142,7 +142,7 @@ __device__ __forceinline__ void atomic_add4(float* dst, float a, float b, float 
 // meet in shared memory, one atomic per column and CTA.
 template <typename T>
 __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ in, int rows, int cols, float* __restrict__ colsum) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   __shared__ float part[8][256];
   const int oct = threadIdx.x & 31, rl = threadIdx.x >> 5;
   const int c0 = blockIdx.x * 256 + oct * 8;
@@ -196,7 +196,7 @@ template int colsum_add<f16>(const f16*, int, int, float*, cudaStream_t);
 // fp32 [rows, cols] -> T [cols, rows] (weights: the fp32 master -> the transposed operand copy the dgrad GEMMs read)
 template <typename T>
 __global__ void __launch_bounds__(256) transpose_cast_kernel(const float* __restrict__ in, int rows, int cols, T* __restrict__ out) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   __shared__ float tile[64][65];
   const int r0 = blockIdx.y * 64, c0 = blockIdx.x * 64;
   const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;
@@ -237,7 +237,7 @@ __device__ __forceinline__ float silu_grad(float x) {
 // a = dropout(act(z)); kind 1 = erf-GELU, 2 = SiLU.  8 elements per thread.
 template <typename T>
 __global__ void __launch_bounds__(256) act_fwd_kernel(const T* __restrict__ z, size_t n8, int kind, DropSpec dr, T* __restrict__ a) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   for (size_t i = static_cast<size_t>(blockIdx.x) * 256 + threadIdx.x; i < n8; i += static_cast<size_t>(gridDim.x) * 256) {
     float v[8];
     load8<T>(z + 8 * i, v);
@@ -261,7 +261,7 @@ int act_fwd(const T* z, size_t n, int kind, DropSpec dr, T* a, cudaStream_t s) {
 template <typename T, typename TG>
 __global__ void __launch_bounds__(256) act_bwd_kernel(const TG* __restrict__ da, const T* __restrict__ z, size_t n8, int kind, DropSpec dr,
                                                       T* __restrict__ dz) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   for (size_t i = static_cast<size_t>(blockIdx.x) * 256 + threadIdx.x; i < n8; i += static_cast<size_t>(gridDim.x) * 256) {
     float g[8], v[8], keep[8];
     load8<TG>(da + 8 * i, g);
@@ -283,7 +283,7 @@ int act_bwd(const TG* da, const T* z, size_t n, int kind, DropSpec dr, T* dz, cu
 }
 // o = dropout(d) + resid (fp32, in place on d): the hidden-state dropout that sits between a Linear and its residual add
 __global__ void __launch_bounds__(256) dropout_add_kernel(float* __restrict__ d, const float* __restrict__ resid, size_t n8, DropSpec dr) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   for (size_t i = static_cast<size_t>(blockIdx.x) * 256 + threadIdx.x; i < n8; i += static_cast<size_t>(gridDim.x) * 256) {
     float v[8], r[8], keep[8];
     load8<float>(d + 8 * i, v);
@@ -317,7 +317,7 @@ __global__ void __launch_bounds__(kTrThreads) dropout_add_layernorm_kernel(float
                                                                            int H, const float* __restrict__ w, const float* __restrict__ b, float eps,
                                                                            float* __restrict__ out32, T* __restrict__ outT,
                                                                            uint8_t* __restrict__ keep_bits) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   const int lane = threadIdx.x & 31;
   const int row = (blockIdx.x * kTrThreads + threadIdx.x) >> 5;
   if (row >= M) return;
@@ -368,7 +368,7 @@ template int dropout_add_layernorm<f16>(float*, const float*, DropSpec, int, int
 // gT = T(g * keep): the fp32 gradient of a (dropout-ed) Linear output as the 16-bit operand of its backward GEMMs
 template <typename T>
 __global__ void __launch_bounds__(256) grad_cast_kernel(const float* __restrict__ g, size_t n8, DropSpec dr, T* __restrict__ out) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   for (size_t i = static_cast<size_t>(blockIdx.x) * 256 + threadIdx.x; i < n8; i += static_cast<size_t>(gridDim.x) * 256) {
     float v[8], keep[8];
     load8<float>(g + 8 * i, v);
@@ -434,7 +434,7 @@ __global__ void __launch_bounds__(kTrThreads) layernorm_bwd_kernel(const float* 
                                                                    float* __restrict__ dgamma, float* __restrict__ dbeta, DropSpec dr,
                                                                    T* __restrict__ gT, float* __restrict__ dbias,
                                                                    const uint8_t* __restrict__ keep_bits) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   constexpr int NACC = FUSE ? 3 : 2;
   extern __shared__ float sacc[];  // [NACC][H]
   for (int e = threadIdx.x; e < NACC * H; e += kTrThreads) sacc[e] = 0.f;
@@ -548,7 +548,7 @@ __global__ void __launch_bounds__(kTrThreads) ln_modulate_bwd_kernel(const float
                                                                      const T* __restrict__ mod, int mod_div, int chunk0, float* __restrict__ din,
                                                                      float* __restrict__ sum_out, T* __restrict__ dmodT, float* __restrict__ dmod32,
                                                                      float* __restrict__ dgamma, float* __restrict__ dbeta, int rpw) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   extern __shared__ float sacc[];  // [2][H] (AFF only)
   if (AFF) {
     for (int e = threadIdx.x; e < 2 * H; e += kTrThreads) sacc[e] = 0.f;
@@ -716,7 +716,7 @@ __global__ void __launch_bounds__(kTrThreads) embed_bwd_kernel(const float* __re
                                                                const float* __restrict__ Wt, const float* __restrict__ b,
                                                                const float* __restrict__ gamma, float eps, DropSpec dr, float* __restrict__ dW,
                                                                float* __restrict__ db, float* __restrict__ dgamma, float* __restrict__ dbeta) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   constexpr int NW = kTrThreads / 32;
   extern __shared__ float sacc[];  // sparse: [fin + 3][H] = dW^T rows | db | dgamma | dbeta;  DENSE: [3][H] sums | [NW][H] g rows | [NW][8] x rows
   const int n_acc = DENSE ? 3 : fin + 3, base_acc = DENSE ? 0 : fin;
@@ -874,9 +874,7 @@ int embed_bwd(const float* dout, const float* x, int M, int fin, int H, const fl
   SD_CHECK(fin >= 1 && fin <= 32, "embed_bwd: fin in [1,32]");
   const int need = ceil_div(M, kTrThreads / 32);
   const int grid = need < num_sms() ? need : num_sms();
-  // SEQDIFF_EMBED_BWD_DENSE=0: shared atomics for every input width (the form that stays for the one-hot sequence embeddings)
-  static const bool dense_ok = [] { const char* e = getenv("SEQDIFF_EMBED_BWD_DENSE"); return !e || e[0] != '0'; }();
-  const bool dense = dense_ok && fin <= 8;
+  const bool dense = fin <= 8;  // the one-hot sequence embeddings (fin = 20) take the shared-atomic form
   const size_t smem = dense ? (static_cast<size_t>(3 + kTrThreads / 32) * H + (kTrThreads / 32) * 8) * sizeof(float)
                             : static_cast<size_t>(fin + 3) * H * sizeof(float);
 #define SD_EB_LAUNCH_(DENSE_)                                                                                       \
@@ -901,113 +899,17 @@ int embed_bwd(const float* dout, const float* x, int M, int fin, int H, const fl
 // AminoAcidPredictor tail backward (forward: predictor_tail_kernel): logits = LN(y; g, b) W2^T + b2
 // dlogits [M,F] fp32 -> dy [M,H] fp32; dW2 [F,H], db2 [F], dg [H], db [H] accumulated.
 // =====================================================================================================
-template <typename T, int VPL>
-__global__ void __launch_bounds__(kTrThreads) predictor_tail_bwd_kernel(const float* __restrict__ dlogits, const T* __restrict__ y, int M, int H,
-                                                                        const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                                                                        const float* __restrict__ W2, int F, float* __restrict__ dy,
-                                                                        float* __restrict__ dW2, float* __restrict__ db2, float* __restrict__ dgamma,
-                                                                        float* __restrict__ dbeta) {
-  SD_TRAIN_PDL_PROLOGUE();
-  extern __shared__ float smem[];
-  float* sW = smem;                                   // [F][H]  W2
-  float* sdW = sW + static_cast<size_t>(F) * H;       // [F][H]  dW2 accumulators
-  float* sG = sdW + static_cast<size_t>(F) * H;       // [2][H]  dgamma | dbeta
-  float* sB = sG + 2 * H;                             // [32]    db2
-  for (int i = threadIdx.x; i < F * H; i += kTrThreads) { sW[i] = W2[i]; sdW[i] = 0.f; }
-  for (int i = threadIdx.x; i < 2 * H; i += kTrThreads) sG[i] = 0.f;
-  if (threadIdx.x < 32) sB[threadIdx.x] = 0.f;
-  __syncthreads();
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int row = blockIdx.x * (kTrThreads / 32) + warp; row < M; row += gridDim.x * (kTrThreads / 32)) {
-    float v[VPL][8], g[VPL][8], ln[VPL][8];
-    ld_row<T, VPL>(y + static_cast<size_t>(row) * H, lane, v);
-    float mean, rstd;
-    stats_of<VPL>(v, H, eps, mean, rstd);
-    const float dl = lane < F ? dlogits[static_cast<size_t>(row) * F + lane] : 0.f;
-    if (lane < F && dl != 0.f) atomicAdd(sB + lane, dl);
-#pragma unroll
-    for (int i = 0; i < VPL; ++i) {
-      float w8[8], b8[8];
-      load8<float>(gamma + (i * 32 + lane) * 8, w8);
-      load8<float>(beta + (i * 32 + lane) * 8, b8);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        v[i][j] = (v[i][j] - mean) * rstd;
-        ln[i][j] = v[i][j] * w8[j] + b8[j];
-        g[i][j] = 0.f;
-      }
-    }
-    bool any = false;
-    for (int f = 0; f < F; ++f) {
-      const float d = __shfl_sync(0xffffffffu, dl, f);
-      if (d == 0.f) continue;  // rows outside the noised set carry a zero gradient: skip them entirely
-      any = true;
-#pragma unroll
-      for (int i = 0; i < VPL; ++i) {
-        float w8[8];
-        load8<float>(sW + static_cast<size_t>(f) * H + (i * 32 + lane) * 8, w8);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          g[i][j] = fmaf(d, w8[j], g[i][j]);
-          atomicAdd(sdW + static_cast<size_t>(f) * H + acc_slot(i, lane, j), d * ln[i][j]);
-        }
-      }
-    }
-    if (any) {
-#pragma unroll
-      for (int i = 0; i < VPL; ++i) {
-        float w8[8];
-        load8<float>(gamma + (i * 32 + lane) * 8, w8);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int e = acc_slot(i, lane, j);
-          atomicAdd(sG + e, g[i][j] * v[i][j]);
-          atomicAdd(sG + H + e, g[i][j]);
-          g[i][j] *= w8[j];
-        }
-      }
-      ln_bwd_core<VPL>(v, g, H, rstd);
-    }
-    st_row<float, VPL>(dy + static_cast<size_t>(row) * H, lane, g);
-  }
-  __syncthreads();
-  if (aligned16(dW2) && aligned16(dgamma) && aligned16(dbeta)) {  // H % 4 == 0: four consecutive columns per 128-bit atomic
-    for (int i = 4 * threadIdx.x; i < F * H; i += 4 * kTrThreads) {
-      const int f = i / H, c = i - f * H;
-      const float x0 = sdW[f * H + acc_slot_of_col(c)], x1 = sdW[f * H + acc_slot_of_col(c + 1)], x2 = sdW[f * H + acc_slot_of_col(c + 2)],
-                  x3 = sdW[f * H + acc_slot_of_col(c + 3)];
-      if (x0 != 0.f || x1 != 0.f || x2 != 0.f || x3 != 0.f) atomic_add4(dW2 + i, x0, x1, x2, x3);
-    }
-    for (int i = 4 * threadIdx.x; i < H; i += 4 * kTrThreads) {
-      const int s0 = acc_slot_of_col(i), s1 = acc_slot_of_col(i + 1), s2 = acc_slot_of_col(i + 2), s3 = acc_slot_of_col(i + 3);
-      atomic_add4(dgamma + i, sG[s0], sG[s1], sG[s2], sG[s3]);
-      atomic_add4(dbeta + i, sG[H + s0], sG[H + s1], sG[H + s2], sG[H + s3]);
-    }
-  } else {
-    for (int i = threadIdx.x; i < F * H; i += kTrThreads) {
-      const int f = i / H, c = i - f * H;
-      const float x = sdW[f * H + acc_slot_of_col(c)];
-      if (x != 0.f) atomicAdd(dW2 + i, x);
-    }
-    for (int i = threadIdx.x; i < H; i += kTrThreads) {
-      const int sl = acc_slot_of_col(i);
-      atomicAdd(dgamma + i, sG[sl]);
-      atomicAdd(dbeta + i, sG[H + sl]);
-    }
-  }
-  if (threadIdx.x < F) atomicAdd(db2 + threadIdx.x, sB[threadIdx.x]);
-}
-// The same for F == 20 (the amino-acid head; seqdiff_train_step requires it) without the F * H / 32 = 480 shared atomics per lane and live row
-// that bound the kernel above (284 us per launch at 16384 rows): the eight warps of a CTA park LN(y) and dlogits of their rows in shared
-// memory, and after a barrier every THREAD owns H / 256 columns of dW2 for all 20 classes in registers (60 accumulators, plain FMAs on
-// conflict-free reads); dgamma / dbeta accumulate in per-warp registers and meet once per CTA (flush_feature_sums).
+// F == 20 (the amino-acid head; seqdiff_train_step requires it).  A warp per row accumulating dW2 through F * H / 32 = 480 shared atomics
+// per lane was bound by them (284 us per launch at 16384 rows).  Here the eight warps of a CTA park LN(y) and dlogits of their rows in
+// shared memory, and after a barrier every THREAD owns H / 256 columns of dW2 for all 20 classes in registers (60 accumulators, plain FMAs
+// on conflict-free reads); dgamma / dbeta accumulate in per-warp registers and meet once per CTA (flush_feature_sums).
 template <typename T, int VPL>
 __global__ void __launch_bounds__(kTrThreads) predictor_tail_bwd20_kernel(const float* __restrict__ dlogits, const T* __restrict__ y, int M, int H,
                                                                           const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
                                                                           const float* __restrict__ W2, float* __restrict__ dy,
                                                                           float* __restrict__ dW2, float* __restrict__ db2, float* __restrict__ dgamma,
                                                                           float* __restrict__ dbeta) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   constexpr int F = 20, NW = kTrThreads / 32;
   extern __shared__ float smem[];
   float* sW = smem;                                   // [F][H]   W2
@@ -1113,24 +1015,10 @@ __global__ void __launch_bounds__(kTrThreads) predictor_tail_bwd20_kernel(const 
 template <typename T>
 int predictor_tail_bwd(const float* dlogits, const T* y, int M, int H, const float* gamma, const float* beta, float eps, const float* W2, int F,
                        float* dy, float* dW2, float* db2, float* dgamma, float* dbeta, cudaStream_t s) {
-  SD_CHECK(F <= 32, "feature_size > 32 not supported");
+  SD_CHECK(F == 20, "predictor_tail_bwd: feature_size must be 20");
   const int need = ceil_div(M, kTrThreads / 32);
   const int grid = need < num_sms() ? need : num_sms();
-  const size_t smem = (2 * static_cast<size_t>(F) * H + 2 * H + 32) * sizeof(float);
-#define SD_PTB_LAUNCH()                                                                                              \
-  {                                                                                                                  \
-    auto kfn = predictor_tail_bwd_kernel<T, VPL>;                                                                    \
-    static bool configured = false;                                                                                  \
-    if (!configured) {                                                                                               \
-      SD_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));                   \
-      configured = true;                                                                                             \
-    }                                                                                                                \
-    SD_CUDA(launch_k(kfn, dim3(grid), dim3(kTrThreads), smem, s, dlogits, y, M, H, gamma, beta, eps, W2, F, dy, dW2, db2, dgamma, dbeta)); \
-  }
-  // SEQDIFF_PTB_DENSE=0: the generic (shared-atomic) kernel also for F == 20
-  static const bool dense_ok = [] { const char* e = getenv("SEQDIFF_PTB_DENSE"); return !e || e[0] != '0'; }();
-  if (dense_ok && F == 20) {
-    const size_t smem20 = (static_cast<size_t>(20 + 2 + kTrThreads / 32) * H + (kTrThreads / 32) * 32 + 32) * sizeof(float);
+  const size_t smem = (static_cast<size_t>(20 + 2 + kTrThreads / 32) * H + (kTrThreads / 32) * 32 + 32) * sizeof(float);
 #define SD_PTB20_LAUNCH()                                                                                            \
   {                                                                                                                  \
     auto kfn = predictor_tail_bwd20_kernel<T, VPL>;                                                                  \
@@ -1139,15 +1027,10 @@ int predictor_tail_bwd(const float* dlogits, const T* y, int M, int H, const flo
       SD_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));                   \
       configured = true;                                                                                             \
     }                                                                                                                \
-    SD_CUDA(launch_k(kfn, dim3(grid), dim3(kTrThreads), smem20, s, dlogits, y, M, H, gamma, beta, eps, W2, dy, dW2, db2, dgamma, dbeta)); \
+    SD_CUDA(launch_k(kfn, dim3(grid), dim3(kTrThreads), smem, s, dlogits, y, M, H, gamma, beta, eps, W2, dy, dW2, db2, dgamma, dbeta)); \
   }
-    SD_VPL_DISPATCH(H, SD_PTB20_LAUNCH());
+  SD_VPL_DISPATCH(H, SD_PTB20_LAUNCH());
 #undef SD_PTB20_LAUNCH
-    SD_LAUNCHED("predictor_tail_bwd", s);
-    return SEQDIFF_OK;
-  }
-  SD_VPL_DISPATCH(H, SD_PTB_LAUNCH());
-#undef SD_PTB_LAUNCH
   SD_LAUNCHED("predictor_tail_bwd", s);
   return SEQDIFF_OK;
 }
@@ -1167,7 +1050,7 @@ template int predictor_tail_bwd<f16>(const float*, const f16*, int, int, const f
 // =====================================================================================================
 __global__ void __launch_bounds__(256) loss_bwd_kernel(int N, const float* __restrict__ logits, const float* __restrict__ x0,
                                                        const float* __restrict__ x_t, const double* __restrict__ terms, float* __restrict__ dlogits) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   constexpr int C = SEQDIFF_NUM_CLASSES;
   const double n_noised = terms[1];
   const float inv_n = n_noised > 0.0 ? static_cast<float>(1.0 / n_noised) : 0.f;
@@ -1234,7 +1117,7 @@ int loss_bwd(int N, const float* logits, const float* x0, const float* x_t, cons
 // sum of squares of the flat gradient, fp64 accumulation, fixed-order fold by the last CTA
 __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, size_t n, double* __restrict__ partial, unsigned* __restrict__ arrive,
                                                     double* __restrict__ out) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   double acc = 0.0;
   const size_t n4 = n / 4;
   // four independent 16-byte loads per thread and pass: 2 CTAs x 256 threads per SM with one load each keep ~1 MB in flight on the whole
@@ -1301,7 +1184,7 @@ __device__ __forceinline__ void adamw_one(float& p, float& mi, float& vi, float 
 __global__ void __launch_bounds__(256) adamw_kernel(AdamSlots sl, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                                                     size_t total, const double* __restrict__ sumsq, float grad_scale, float max_norm, float lr,
                                                     float beta1, float beta2, float eps, float wd, float bc1, float bc2, float* __restrict__ norm_out) {
-  SD_TRAIN_PDL_PROLOGUE();
+  pdl_wait();
   // torch.nn.utils.clip_grad_norm_: coef = max_norm / (total_norm + 1e-6), clamped to 1
   const float total_norm = sqrtf(static_cast<float>(*sumsq)) * grad_scale;
   float coef = 1.0f;

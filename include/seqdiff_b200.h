@@ -265,12 +265,6 @@ SEQDIFF_API int seqdiff_struct_sample(seqdiff_model_t* m, int precision, int B, 
  * (tcgen05 + TMA kernel); resid (optional) is f32 and makes C f32, otherwise C has A's 16-bit type. */
 SEQDIFF_API int seqdiff_op_gemm(int precision, int M, int N, int K, const void* A, const void* W, const float* bias,
                     const void* resid, int epilogue, void* C, void* stream);
-/* Linear + residual + the LayerNorm that follows it (HF BertSelfOutput / BertOutput, modeling_bert: dense -> dropout ->
- * LayerNorm(hidden + input)) in one launch, 16-bit modes only, N in {512, 768, 1024}:
- *   C[M,N] (f32) = A * W^T + bias + resid ;  h[M,N] (16-bit) = LayerNorm(C) * ln_w + ln_b ;  stats[M] = (mean, rstd) as float2 */
-SEQDIFF_API int seqdiff_op_gemm_ln(int precision, int M, int N, int K, const void* A, const void* W, const float* bias,
-                       const float* resid, const float* ln_w, const float* ln_b, float eps, float* C, void* h, float* stats,
-                       void* stream);
 /* multi-head attention core of HF BertSelfAttention (4.38.2 relative_key semantics, SURVEY.md App. A):
  * q [B,Lq,*] k,v [B,Lk,*] with row strides (elements) ldq/ldk/ldv, heads x 64; dist_emb [2P-1,64] or NULL;
  * key_mask [B,Lk] {0,1} -> additive (1-m)*-10000; out [B,Lq,heads*64].  Element type by precision. */

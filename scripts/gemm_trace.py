@@ -12,16 +12,7 @@ stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 A = torch.randn(M, K, device=dev).bfloat16(); W = (torch.randn(N, K, device=dev) / math.sqrt(K)).bfloat16()
 bias = torch.randn(N, device=dev); R = torch.randn(M, N, device=dev) if resid else None
 C = torch.empty(M, N, device=dev, dtype=torch.float32 if resid else torch.bfloat16)
-LN = int(os.environ.get("TLN", 0))
-if LN:
-    R = torch.randn(M, N, device=dev); C = torch.empty(M, N, device=dev)
-    lw, lb = torch.ones(N, device=dev), torch.zeros(N, device=dev)
-    hh = torch.empty(M, N, device=dev, dtype=torch.bfloat16); stt = torch.empty(M, 2, device=dev)
 def call():
-    if LN:
-        rc = lib.seqdiff_op_gemm_ln(1, M, N, K, p(A), p(W), p(bias), p(R), p(lw), p(lb), 1e-12, p(C), p(hh), p(stt), stream)
-        assert rc == 0, lib.seqdiff_last_error()
-        return
     rc = lib.seqdiff_op_gemm(1 | (bn << 8) | (cg2 << 20), M, N, K, p(A), p(W), p(bias), p(R), 0, p(C), stream)
     assert rc == 0, lib.seqdiff_last_error()
 for _ in range(3): call()
@@ -29,7 +20,7 @@ buf = torch.zeros(4 * 1024, dtype=torch.int64, device=dev)
 lib.seqdiff_debug_attn_trace(p(buf)); call(); torch.cuda.synchronize(); lib.seqdiff_debug_attn_trace(None)
 t = buf.cpu().tolist()
 names = {40: "kernel entry", 41: "prologue done", 42: "pdl_wait done", 43: "role done", 1: "tma slot free", 11: "mma stage full", 12: "mma tile committed",
-         20: "epi wait acc", 21: "epi acc ready", 23: "epi tile stored", 24: "ln partial pushed", 25: "ln exchange done", 26: "ln pass C done"}
+         20: "epi wait acc", 21: "epi acc ready", 23: "epi tile stored"}
 ev = []
 for role in range(4):
     n = t[role * 1024]
