@@ -318,7 +318,19 @@ int seqdiff_struct_sample(seqdiff_model_t* m, int precision, int B, int L_lig, i
   SD_GUARD_BEGIN
   SD_CHECK(m && coef_steps && x_T && ligand_mask && receptor_seq && receptor_angles && receptor_mask && final_out, "null argument");
   return m->impl.struct_sample(precision, B, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
-                               noise_steps, seed, graph_id0, steps_out, final_out, static_cast<cudaStream_t>(stream));
+                               noise_steps, seed, graph_id0, steps_out, final_out, static_cast<cudaStream_t>(stream), 0);
+  SD_GUARD_END
+}
+
+int seqdiff_struct_sample_ex(seqdiff_model_t* m, int precision, int B, int L_lig, int L_rec, int T, const float* coef_steps, const float* x_T,
+                             const float* ligand_mask, const float* receptor_seq, const float* receptor_angles, const float* receptor_mask,
+                             const float* noise_steps, uint64_t seed, uint64_t graph_id0, int flags, float* steps_out, float* final_out,
+                             void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(m && coef_steps && x_T && ligand_mask && receptor_seq && receptor_angles && receptor_mask && final_out, "null argument");
+  SD_CHECK((flags & ~1) == 0, "unknown sampling flag");
+  return m->impl.struct_sample(precision, B, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
+                               noise_steps, seed, graph_id0, steps_out, final_out, static_cast<cudaStream_t>(stream), flags);
   SD_GUARD_END
 }
 

@@ -54,11 +54,17 @@ __device__ __forceinline__ float gauss_update(float x, float out, float a, float
 }
 
 // One thread per group of 4 consecutive elements of one graph (per = L * F elements per graph, groups = ceil(per / 4)).
+// PACKED (ragged batch): graph g holds len[g] valid residues of F features, element e of the graph is valid iff e / F < len[g], i.e.
+// iff e < len[g] * F.  Valid elements are computed exactly as in the padded kernel, with the Philox counter of their group inside the
+// PADDED graph, so they draw the same noise; padded elements are written as 0 without being read, and a group with no valid element
+// draws nothing.  With F % 4 != 0 a group can straddle the end of the valid prefix: its valid part is loaded element by element.
+template <bool PACKED>
 __global__ void __launch_bounds__(kGaussThreads) gauss_step_kernel(const float* __restrict__ coef, int T, int per, const float* x_t,
                                                                    const float* __restrict__ model_out, const float* __restrict__ noise,
                                                                    uint64_t seed, uint64_t graph_id0, int step, const int* __restrict__ step_ptr,
                                                                    float* x_out, float* __restrict__ steps_out,
-                                                                   int* __restrict__ advance, int wrap, const uint64_t* __restrict__ rng) {
+                                                                   int* __restrict__ advance, int wrap, const uint64_t* __restrict__ rng,
+                                                                   const int* __restrict__ len, int F) {
   // x_t / x_out carry no __restrict__: the sampling loop updates the angles in place (each thread reads its 4 elements before it writes them)
   pdl_trigger();
   pdl_wait();
@@ -94,25 +100,42 @@ __global__ void __launch_bounds__(kGaussThreads) gauss_step_kernel(const float* 
   for (int q = blockIdx.x * kGaussThreads + threadIdx.x; q < groups; q += gridDim.x * kGaussThreads) {
     const size_t base = static_cast<size_t>(g) * per + 4 * static_cast<size_t>(q);
     const int cnt = min(4, per - 4 * q);
+    int nv = cnt;  // valid elements of the group: a prefix of it
+    if constexpr (PACKED) {
+      nv = min(cnt, max(0, __ldg(len + g) * F - 4 * q));
+      if (nv == 0) {
+        if (vec) {
+          *reinterpret_cast<float4*>(x_out + base) = make_float4(0.f, 0.f, 0.f, 0.f);
+          if (steps_out) *reinterpret_cast<float4*>(steps_out + base) = make_float4(0.f, 0.f, 0.f, 0.f);
+        } else {
+          for (int e = 0; e < cnt; ++e) {
+            x_out[base + e] = 0.f;
+            if (steps_out) steps_out[base + e] = 0.f;
+          }
+        }
+        continue;
+      }
+    }
+    const bool vload = PACKED ? vec && nv == 4 : vec;
     float xv[4], ov[4], zv[4] = {0.f, 0.f, 0.f, 0.f};
-    if (vec) {
+    if (vload) {
       const float4 x4 = *reinterpret_cast<const float4*>(x_t + base);
       const float4 o4 = *reinterpret_cast<const float4*>(model_out + base);
       xv[0] = x4.x; xv[1] = x4.y; xv[2] = x4.z; xv[3] = x4.w;
       ov[0] = o4.x; ov[1] = o4.y; ov[2] = o4.z; ov[3] = o4.w;
     } else {
       for (int e = 0; e < 4; ++e) {
-        xv[e] = e < cnt ? x_t[base + e] : 0.f;
-        ov[e] = e < cnt ? model_out[base + e] : 0.f;
+        xv[e] = e < nv ? x_t[base + e] : 0.f;
+        ov[e] = e < nv ? model_out[base + e] : 0.f;
       }
     }
     if (!last) {
       if (noise) {
-        if (vec) {
+        if (vload) {
           const float4 z4 = *reinterpret_cast<const float4*>(noise + base);
           zv[0] = z4.x; zv[1] = z4.y; zv[2] = z4.z; zv[3] = z4.w;
         } else {
-          for (int e = 0; e < cnt; ++e) zv[e] = noise[base + e];
+          for (int e = 0; e < nv; ++e) zv[e] = noise[base + e];
         }
       } else {
         const uint64_t graph = graph_id0 + static_cast<uint64_t>(g);
@@ -125,6 +148,11 @@ __global__ void __launch_bounds__(kGaussThreads) gauss_step_kernel(const float* 
     float r[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) r[e] = gauss_update(xv[e], ov[e], a, b, c, sd, zv[e], last, wrap != 0);
+    if constexpr (PACKED) {
+#pragma unroll
+      for (int e = 0; e < 4; ++e)
+        if (e >= nv) r[e] = 0.f;
+    }
     if (vec) {
       const float4 r4 = make_float4(r[0], r[1], r[2], r[3]);
       *reinterpret_cast<float4*>(x_out + base) = r4;
@@ -140,13 +168,19 @@ __global__ void __launch_bounds__(kGaussThreads) gauss_step_kernel(const float* 
 
 int gauss_step(const float* coef, int T, int B, int per_graph, const float* x_t, const float* model_out, const float* noise, uint64_t seed,
                uint64_t graph_id0, int step, const int* step_ptr, float* x_out, float* steps_out, cudaStream_t s, int* advance, bool wrap,
-               const uint64_t* rng) {
+               const uint64_t* rng, const int* len, int F) {
   SD_CHECK(B > 0 && per_graph > 0 && T > 0, "empty Gaussian reverse step");
   SD_CHECK(step_ptr != nullptr || (step >= 0 && step < T), "step index out of range");
+  SD_CHECK(!len || (F > 0 && per_graph % F == 0), "packed Gaussian step: per_graph must be a multiple of F");
   const int groups = (per_graph + 3) / 4;
   const dim3 grid(ceil_div(groups, kGaussThreads), B);
-  SD_CUDA(launch_k(gauss_step_kernel, dim3(grid), dim3(kGaussThreads), 0, s, coef, T, per_graph, x_t, model_out, noise, seed, graph_id0, step, step_ptr,
-                   x_out, steps_out, advance, wrap ? 1 : 0, rng));
+  if (len) {
+    SD_CUDA(launch_k(gauss_step_kernel<true>, dim3(grid), dim3(kGaussThreads), 0, s, coef, T, per_graph, x_t, model_out, noise, seed, graph_id0, step,
+                     step_ptr, x_out, steps_out, advance, wrap ? 1 : 0, rng, len, F));
+  } else {
+    SD_CUDA(launch_k(gauss_step_kernel<false>, dim3(grid), dim3(kGaussThreads), 0, s, coef, T, per_graph, x_t, model_out, noise, seed, graph_id0, step,
+                     step_ptr, x_out, steps_out, advance, wrap ? 1 : 0, rng, static_cast<const int*>(nullptr), 0));
+  }
   SD_LAUNCHED("gauss_step", s);
   return SEQDIFF_OK;
 }

@@ -164,9 +164,11 @@ size_t loss_terms_scratch_bytes();
 // noise: N(0,1) values (one [B*per_graph] block; with step_ptr a [T, B*per_graph] table indexed by the step) or NULL ->
 // in-kernel Philox + Box-Muller.  step_ptr / advance as in reverse_step().  steps_out (optional) [T, B*per_graph]: the result
 // is also stored at entry T-1-step (the reference's per-step history).  wrap = false: p_sample's un-wrapped value.
+// len != NULL (ragged packing, per_graph = L * F): graph b has len[b] valid residues of F features; only they are computed (same
+// values and noise as the padded step), every padded element of x_out and steps_out is written as 0.
 int gauss_step(const float* coef, int T, int B, int per_graph, const float* x_t, const float* model_out, const float* noise, uint64_t seed,
                uint64_t graph_id0, int step, const int* step_ptr, float* x_out, float* steps_out, cudaStream_t s, int* advance = nullptr, bool wrap = true,
-               const uint64_t* rng = nullptr);  // rng / in-place (x_out == x_t) as in reverse_step()
+               const uint64_t* rng = nullptr, const int* len = nullptr, int F = 0);  // rng / in-place (x_out == x_t) as in reverse_step()
 
 // ---- train_kernels.cu / attention_train.cu: the training step (reference model.py:313-367 under autograd) ------------
 // out[c][r] = in[r][c] for row-major [rows, cols]; colsum (optional, fp32 [cols]) += column sums (bias gradients); out may be NULL.

@@ -1323,13 +1323,15 @@ static int bert_layer_plain(const Model& m, int wfmt, const LayerW& w, bool cros
 // epilogue from the fp32 pre-LN tensor, the per-row (mean, rstd) and the affine -- the LayerNorm kernels skip their fp32 copy.
 // Pre-LN buffers with fixed roles: obuf[0] self-output, obuf[1] cross-output, obuf[2] FFN-output (every GEMM reads its residual from
 // a different buffer than the one it writes).  *out = 16-bit output of the last layer (all the consumers of a stack read).
+// M token rows.  Ragged packing: aps / apc address the graphs of the self- / cross-attention (AttnPack), Lq / Lk are then the largest
+// lengths and M the packed row count; without them M = B * Lq.
 template <typename T>
-static int bert_stack_lnresid(const Model& m, int wfmt, const std::vector<LayerW>& Ls, bool cross, int B, int Lq, int Lk, const Act<T>& h0,
+static int bert_stack_lnresid(const Model& m, int wfmt, const std::vector<LayerW>& Ls, bool cross, int B, int Lq, int Lk, int M, const Act<T>& h0,
                               const float* q_mask, const float* k_mask, const T* kv_all, int ldkv, T* qkv, T* ctx, T* cq, T* ffn,
-                              float* const (&obuf)[3], float2* lnstats, T* hT0, T* hT1, const T** out, cudaStream_t s) {
+                              float* const (&obuf)[3], float2* lnstats, T* hT0, T* hT1, const T** out, cudaStream_t s,
+                              const AttnPack* aps = nullptr, const AttnPack* apc = nullptr) {
   const int H = m.cfg.hidden_size, I = m.cfg.intermediate_size, heads = m.cfg.num_attention_heads, P = m.cfg.max_position_embeddings;
   const float eps = m.cfg.layer_norm_eps;
-  const int M = B * Lq;
   float2* stA = lnstats;
   float2* stB = lnstats + M;
   float2* stC = lnstats + 2 * static_cast<size_t>(M);
@@ -1339,7 +1341,7 @@ static int bert_stack_lnresid(const Model& m, int wfmt, const std::vector<LayerW
   for (size_t i = 0; i < Ls.size(); ++i) {
     const LayerW& w = Ls[i];
     SD_TRY(gemm_T(wfmt, M, 3 * H, H, h, w.self.qkv, w.self.qkv_b, 0, qkv, s));
-    SD_TRY(attention<T>(B, heads, Lq, Lq, qkv, 3 * H, qkv + H, 3 * H, qkv + 2 * H, 3 * H, pick<T>(w.self.E), P, q_mask, ctx, s));
+    SD_TRY(attention<T>(B, heads, Lq, Lq, qkv, 3 * H, qkv + H, 3 * H, qkv + 2 * H, 3 * H, pick<T>(w.self.E), P, q_mask, ctx, s, aps));
     SD_TRY(gemm_ln<T>(wfmt, M, H, H, ctx, w.self.out, w.self.out_b, i == 0 ? h0.s : o_prev, obuf[0], i == 0 ? nullptr : &prev, w.self.ln_w,
                       w.self.ln_b, eps, hT0, stA, s));
     const T* cur = hT0;
@@ -1348,7 +1350,7 @@ static int bert_stack_lnresid(const Model& m, int wfmt, const std::vector<LayerW
     if (cross) {
       SD_TRY(gemm_T(wfmt, M, H, H, hT0, w.cq, w.cq_b, 0, cq, s));
       const T* kbase = kv_all + i * 2 * static_cast<size_t>(H);
-      SD_TRY(attention<T>(B, heads, Lq, Lk, cq, H, kbase, ldkv, kbase + H, ldkv, static_cast<const T*>(nullptr), P, k_mask, ctx, s));
+      SD_TRY(attention<T>(B, heads, Lq, Lk, cq, H, kbase, ldkv, kbase + H, ldkv, static_cast<const T*>(nullptr), P, k_mask, ctx, s, apc));
       SD_TRY(gemm_ln<T>(wfmt, M, H, H, ctx, w.cout, w.cout_b, obuf[0], obuf[1], &rc, w.cln_w, w.cln_b, eps, hT1, stB, s));
       cur = hT1;
       o_cur = obuf[1];
@@ -1382,14 +1384,24 @@ size_t Model::struct_workspace_need(int precision, int B, int Ll, int Lr) const 
 template <typename T>
 int Model::struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* noised,
                             const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, float* out,
-                            int phases, cudaStream_t s) {
+                            int phases, cudaStream_t s, const PackInfo* pk) {
   constexpr bool k16 = !std::is_same<T, float>::value;
   const int H = cfg.hidden_size, I = cfg.intermediate_size, NL = cfg.num_hidden_layers;
   const float eps = cfg.layer_norm_eps;
-  const int Ml = B * Ll, Mr = B * Lr, Mx = Ml > Mr ? Ml : Mr;
+  // packed (ragged) batch: only the valid prefix of every graph is a row; the buffers keep their padded sizes, inputs, masks and
+  // the output their padded layouts
+  const int Mlp = B * Ll, Mrp = B * Lr, Mx = Mlp > Mrp ? Mlp : Mrp;
+  const int Ml = pk ? pk->Ml : Mlp, Mr = pk ? pk->Mr : Mrp;
+  const int Lq = pk ? pk->max_l : Ll, Lk = pk ? pk->max_r : Lr;  // attention: largest ligand / receptor length
+  AttnPack ap_l{}, ap_r{}, ap_x{};
+  if (pk) {
+    ap_l = AttnPack{pk->off_l, pk->off_l, pk->len_l, Ml, Ml, Ll};
+    ap_r = AttnPack{pk->off_r, pk->off_r, pk->len_r, Mr, Mr, Lr};
+    ap_x = AttnPack{pk->off_l, pk->off_r, pk->len_l, Ml, Mr, Lr};
+  }
   const size_t MxH = static_cast<size_t>(Mx) * H;
   Bump bp(ws, s);
-  T* kv_all = bp.take<T>(static_cast<size_t>(Mr) * NL * 2 * H);  // first: same address for every (B, Ll, Lr) of a loop
+  T* kv_all = bp.take<T>(static_cast<size_t>(Mrp) * NL * 2 * H);  // first: same address for every (B, Ll, Lr) of a loop
   float* te = bp.take<float>(static_cast<size_t>(B) * H);
   T* teT = k16 ? bp.take<T>(static_cast<size_t>(B) * H) : reinterpret_cast<T*>(te);
   Act<T> x = take_act<T>(bp, MxH);
@@ -1408,10 +1420,14 @@ int Model::struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timest
   sb.qkv = bp.take<T>(MxH * 3);
   sb.m1 = bp.take<T>(MxH * 4);
   T* ffn = bp.take<T>(static_cast<size_t>(Mx) * I);
-  auto job = [&](const float* in, int M, const EmbW& e, int L, float* o32, T* oT) {
+  auto job = [&](const float* in, int M, const EmbW& e, int L, float* o32, T* oT, bool lig) {
     EmbedJob jb{};
     jb.x = in; jb.Wt = e.Wt_; jb.b = e.b; jb.lnw = e.ln_w; jb.lnb = e.ln_b; jb.te = nullptr;
     jb.out32 = o32; jb.outT = oT; jb.M = M; jb.fin = e.fin; jb.L = L;
+    if (pk) {
+      jb.src_rows = lig ? pk->src_l : pk->src_r;
+      jb.row_graph = lig ? pk->graph : pk->graph + pk->Ml;
+    }
     return jb;
   };
 
@@ -1419,16 +1435,17 @@ int Model::struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timest
     // receptor branch (model.py:192-202): x = LN(Linear(angles)), c = LN(Linear(seq)); receptor_emb; 12 x (self-attn, FFN)
     EmbedJobs jobs{};
     jobs.n = 2;
-    jobs.j[0] = job(rec_angle, Mr, rec_ang, Lr, x.s, x.t_out());
-    jobs.j[1] = job(rec_seq_in, Mr, rec_seq, Lr, k16 ? nullptr : reinterpret_cast<float*>(cT), k16 ? cT : nullptr);
+    jobs.j[0] = job(rec_angle, Mr, rec_ang, Lr, x.s, x.t_out(), false);
+    jobs.j[1] = job(rec_seq_in, Mr, rec_seq, Lr, k16 ? nullptr : reinterpret_cast<float*>(cT), k16 ? cT : nullptr, false);
     SD_TRY(embed_ln_multi<T>(jobs, eps, H, s));
-    std::vector<Segment> rseg{{0, B, Lr, rec_mask}};
-    SD_TRY(se_layer<T>(*this, wfmt, se_lig, x, cT, Mr, 1, Mr, rseg, sb, x2, s));
+    std::vector<Segment> rseg{{0, B, Lk, rec_mask}};
+    const std::vector<AttnPack> rpack{ap_r};
+    SD_TRY(se_layer<T>(*this, wfmt, se_lig, x, cT, Mr, 1, Mr, rseg, sb, x2, s, pk ? &rpack : nullptr));
     const T* enc_out = nullptr;
     if constexpr (k16) {
       float* const obuf[3] = {sb.o, sb.m2, hb[0].s};
-      SD_TRY(bert_stack_lnresid<T>(*this, wfmt, enc_layers, false, B, Lr, Lr, x2, rec_mask, nullptr, nullptr, 0, sb.qkv, sb.ctx, cq, ffn, obuf,
-                                   reinterpret_cast<float2*>(hb[1].s), hb[0].t, hb[1].t, &enc_out, s));
+      SD_TRY(bert_stack_lnresid<T>(*this, wfmt, enc_layers, false, B, Lk, Lk, Mr, x2, rec_mask, nullptr, nullptr, 0, sb.qkv, sb.ctx, cq, ffn, obuf,
+                                   reinterpret_cast<float2*>(hb[1].s), hb[0].t, hb[1].t, &enc_out, s, pk ? &ap_r : nullptr));
     } else {
       Act<T> h = x2;
       for (int i = 0; i < NL; ++i) {
@@ -1449,16 +1466,18 @@ int Model::struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timest
   {
     EmbedJobs jobs{};
     jobs.n = 1;
-    jobs.j[0] = job(noised, Ml, lig_ang, Ll, x.s, x.t_out());
+    jobs.j[0] = job(noised, Ml, lig_ang, Ll, x.s, x.t_out(), true);
     SD_TRY(embed_ln_multi<T>(jobs, eps, H, s));
   }
-  std::vector<Segment> lseg{{0, B, Ll, lig_mask}};
-  SD_TRY(se_layer<T>(*this, wfmt, se_dec, x, teT, B, Ll, Ml, lseg, sb, x2, s));  // timestep_emb: c broadcast over L
+  // timestep_emb: c broadcast over L (packed: every row takes the timestep features of its graph)
+  std::vector<Segment> lseg{{0, B, Lq, lig_mask}};
+  const std::vector<AttnPack> lpack{ap_l};
+  SD_TRY(se_layer<T>(*this, wfmt, se_dec, x, teT, B, Ll, Ml, lseg, sb, x2, s, pk ? &lpack : nullptr, pk ? pk->graph : nullptr));
   const T* dec_out = nullptr;
   if constexpr (k16) {
     float* const obuf[3] = {sb.o, sb.m2, hb[0].s};
-    SD_TRY(bert_stack_lnresid<T>(*this, wfmt, layers, true, B, Ll, Lr, x2, lig_mask, rec_mask, kv_all, NL * 2 * H, sb.qkv, sb.ctx, cq, ffn, obuf,
-                                 reinterpret_cast<float2*>(hb[1].s), hb[0].t, hb[1].t, &dec_out, s));
+    SD_TRY(bert_stack_lnresid<T>(*this, wfmt, layers, true, B, Lq, Lk, Ml, x2, lig_mask, rec_mask, kv_all, NL * 2 * H, sb.qkv, sb.ctx, cq, ffn, obuf,
+                                 reinterpret_cast<float2*>(hb[1].s), hb[0].t, hb[1].t, &dec_out, s, pk ? &ap_l : nullptr, pk ? &ap_x : nullptr));
   } else {
     Act<T> h = x2;
     for (int i = 0; i < NL; ++i) {
@@ -1471,17 +1490,18 @@ int Model::struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timest
     dec_out = h.t;
   }
   SD_TRY(gemm_T(wfmt, Ml, H, H, dec_out, p1, p1_b, 1, y, s));
-  SD_TRY(predictor_tail<T>(y, Ml, H, p_ln_w, p_ln_b, 1e-12f, p2_w, p2_b, cfg.feature_size, out, s));
+  SD_TRY(predictor_tail<T>(y, Ml, H, p_ln_w, p_ln_b, 1e-12f, p2_w, p2_b, cfg.feature_size, out, s, pk ? pk->src_l : nullptr));
   return SEQDIFF_OK;
 }
 
 int Model::struct_forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* noised,
                           const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, float* out,
-                          int phases, cudaStream_t s) {
+                          int phases, cudaStream_t s, const PackInfo* pk) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
   SD_CHECK(arch == kArchStructure, "handle holds a sequence model: use seqdiff_forward");
   const PdlScope pdl_on(3);  // launch-bound path: programmatic dependent launch of the heavy kernels (42.3 -> 43.0 k graph-steps/s against every launch)
   SD_CHECK(precision >= SEQDIFF_FP32 && precision <= SEQDIFF_FP16, "unknown precision mode");
+  SD_CHECK(!pk || precision != SEQDIFF_FP32, "ragged packing runs in the 16-bit modes");
   SD_CHECK(B > 0 && Ll > 0 && Lr > 0, "empty batch");
   if (cfg.relative_key) SD_CHECK(Ll <= cfg.max_position_embeddings && Lr <= cfg.max_position_embeddings, "Length exceed");
   SD_CUDA(cudaSetDevice(device));
@@ -1489,11 +1509,11 @@ int Model::struct_forward(int precision, int B, int Ll, int Lr, const float* tim
   if (g_profiling) profile_mark("__begin__", s);
   switch (precision) {
     case SEQDIFF_FP32:
-      return struct_forward_t<float>(1, B, Ll, Lr, timestep, step_ptr, noised, lig_mask, rec_seq_in, rec_angle, rec_mask, out, phases, s);
+      return struct_forward_t<float>(1, B, Ll, Lr, timestep, step_ptr, noised, lig_mask, rec_seq_in, rec_angle, rec_mask, out, phases, s, nullptr);
     case SEQDIFF_BF16:
-      return struct_forward_t<bf16>(1, B, Ll, Lr, timestep, step_ptr, noised, lig_mask, rec_seq_in, rec_angle, rec_mask, out, phases, s);
+      return struct_forward_t<bf16>(1, B, Ll, Lr, timestep, step_ptr, noised, lig_mask, rec_seq_in, rec_angle, rec_mask, out, phases, s, pk);
     default:
-      return struct_forward_t<f16>(0, B, Ll, Lr, timestep, step_ptr, noised, lig_mask, rec_seq_in, rec_angle, rec_mask, out, phases, s);
+      return struct_forward_t<f16>(0, B, Ll, Lr, timestep, step_ptr, noised, lig_mask, rec_seq_in, rec_angle, rec_mask, out, phases, s, pk);
   }
 }
 
@@ -1501,7 +1521,7 @@ int Model::struct_forward(int precision, int B, int Ll, int Lr, const float* tim
 // it every step); each step replays one captured graph: ligand branch + Gaussian reverse step + wrap.
 int Model::struct_sample(int precision, int B, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
                          const float* rec_seq_in, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
-                         uint64_t gid0, float* steps_out, float* final_out, cudaStream_t caller) {
+                         uint64_t gid0, float* steps_out, float* final_out, cudaStream_t caller, int flags) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
   SD_CHECK(arch == kArchStructure, "handle holds a sequence model: use seqdiff_sample");
   const PdlScope pdl_on(3);
@@ -1544,8 +1564,17 @@ int Model::struct_sample(int precision, int B, int Ll, int Lr, int T, const floa
   SD_CUDA(cudaMemcpyAsync(c_rseq, rec_seq_in, Nr * 20 * 4, cudaMemcpyDefault, s));
   SD_CUDA(cudaMemcpyAsync(c_rang, rec_angle, Nr * F * 4, cudaMemcpyDefault, s));
   SD_CUDA(cudaMemcpyAsync(c_rmask, rec_mask, Nr * 4, cudaMemcpyDefault, s));
+  // ragged packing (flags bit 0): valid prefixes only, one receptor per ligand graph; needs the 16-bit kernels and prefix masks,
+  // otherwise the padded path runs.  The Gaussian step writes the padded positions of x_cur and steps_out as 0.
+  const PackInfo* pk = nullptr;
+  if ((flags & 1) && precision != SEQDIFF_FP32) {
+    bool usable = false;
+    SD_TRY(build_pack(B, 1, Ll, Lr, c_lmask, c_rmask, s, &usable));
+    if (usable) pk = &pack;
+  }
 
   GraphKey key;
+  key.pack_hash = pk ? pk->hash : 0;
   key.precision = precision; key.B = B; key.Ll = Ll; key.Lr = Lr; key.diverse = 0; key.noise = noise_steps;
   key.ws_ptr = ws; key.in_ptr = samp_in; key.tab_ptr = d_tables; key.aux_ptr = steps_out; key.T = T;
   uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
@@ -1553,10 +1582,11 @@ int Model::struct_sample(int precision, int B, int Ll, int Lr, int T, const floa
   SD_CUDA(launch_k(arm_loop_kernel, dim3(1), dim3(1), 0, s, d_step, T - 1, d_rng, seed, gid0));
   SD_LAUNCHED("arm_loop", s);
   const bool cached = graph_exec && key == graph_key;
-  SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lmask, c_rseq, c_rang, c_rmask, mout, cached ? 1 : 3, s));
+  SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lmask, c_rseq, c_rang, c_rmask, mout, cached ? 1 : 3, s, pk));
   auto one_step = [&](cudaStream_t st) -> int {
-    SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lmask, c_rseq, c_rang, c_rmask, mout, 2, st));
-    SD_TRY(gauss_step(d_tables, T, B, Ll * F, x_cur, mout, noise_steps, 0, 0, 0, d_step, x_cur, steps_out, st, d_step + 1, true, d_rng));
+    SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lmask, c_rseq, c_rang, c_rmask, mout, 2, st, pk));
+    SD_TRY(gauss_step(d_tables, T, B, Ll * F, x_cur, mout, noise_steps, 0, 0, 0, d_step, x_cur, steps_out, st, d_step + 1, true, d_rng,
+                      pk ? pk->len_l : nullptr, F));
     return SEQDIFF_OK;
   };
   if (!cached) {

@@ -219,13 +219,15 @@ struct Model {
   // structure_model/model.py:180-215.  phases: bit 0 = run the receptor branch, bit 1 = the ligand branch.  The receptor branch (embeddings,
   // receptor_emb, encoder, all decoder layers' cross K|V) depends on neither the timestep nor the ligand, so the sampling loop runs it
   // once and keeps the K|V block.
+  // pk (16-bit modes, sampling loop): ragged packing with one receptor per ligand graph (build_pack with K = 1)
   int struct_forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* noised_angles,
                      const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, float* out, int phases,
-                     cudaStream_t s);
-  // structure_model/sample.py:104-144 (STEP = 1): T x (forward, Gaussian reverse step, angle wrap) from one captured graph
+                     cudaStream_t s, const PackInfo* pk = nullptr);
+  // structure_model/sample.py:104-144 (STEP = 1): T x (forward, Gaussian reverse step, angle wrap) from one captured graph.
+  // flags bit 0: ragged packing (valid positions bit-identical to the padded loop; padded positions of steps_out / final_out are 0)
   int struct_sample(int precision, int B, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
                     const float* rec_seq, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
-                    uint64_t gid0, float* steps_out, float* final_out, cudaStream_t s);
+                    uint64_t gid0, float* steps_out, float* final_out, cudaStream_t s, int flags = 0);
 
  public:
   void* dalloc(size_t bytes);
@@ -233,7 +235,7 @@ struct Model {
   template <typename T>
   int struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* noised_angles,
                        const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, float* out, int phases,
-                       cudaStream_t s);
+                       cudaStream_t s, const PackInfo* pk);
   size_t workspace_need(int precision, int B, int Ll, int Lr) const;
   int ensure_workspace(size_t bytes);
   template <typename T>

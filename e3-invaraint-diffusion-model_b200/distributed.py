@@ -96,7 +96,8 @@ def p_sample_loop_sharded(model, ligand_mask, ligand_angle_noise, receptor_seq, 
     """structure_model p_sample_loop (reference structure_model/sample.py:104-144) over the ranks of `group`: every rank samples
     its contiguous block of complexes on its own GPU (noise keyed by the global graph id), then the CPU [T, b_r, L, F] histories
     are all-gathered and concatenated along the batch axis in rank order -- each rank returns what one GPU returns for the
-    whole batch.  No collective on the data path; the only exchange is the result tensor the reference returns anyway."""
+    whole batch.  No collective on the data path; the only exchange is the result tensor the reference returns anyway.
+    Further keywords (`packed`, `seed`, `keep_history`, ...) reach every rank's loop function unchanged."""
     import torch.distributed as dist
     if sample_fn is None:
         from .structure_model import p_sample_loop as sample_fn

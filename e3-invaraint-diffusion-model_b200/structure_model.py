@@ -213,13 +213,16 @@ def p_sample_wrapped(model, ligand_mask, ligand_angle_noise, receptor_seq, recep
 @torch.no_grad()
 def p_sample_loop(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor_mask, receptor_angle, total_timesteps: int, betas,
                   disable_pbar: bool = True, noise_steps: Optional[torch.Tensor] = None, graph_id0: Optional[int] = None, seed: Optional[int] = None,
-                  keep_history: bool = True) -> torch.Tensor:
+                  keep_history: bool = True, packed: bool = False) -> torch.Tensor:
     """reference structure_model/sample.py:104-144: returns a CPU tensor [timesteps, B, L, F] (entry k = wrapped angles after
-    the k-th reverse step).  The whole loop is ONE C call (`seqdiff_struct_sample`): the receptor branch is evaluated once, every
+    the k-th reverse step).  The whole loop is ONE C call (`seqdiff_struct_sample_ex`): the receptor branch is evaluated once, every
     step replays a captured CUDA graph (ligand branch + Gaussian step + wrap), and the history is written by the step kernel --
     one device->host copy at the end instead of one per step.  `keep_history=False` returns only the final [1,B,L,F] entry.
     `noise_steps` [T,B,L,F]: entry i = the N(0,1) draw used at step index i (entry 0 unused).  `graph_id0` = None continues the
-    process-wide Philox noise stream, so successive batches / calls draw fresh noise like the reference's `torch.randn_like`."""
+    process-wide Philox noise stream, so successive batches / calls draw fresh noise like the reference's `torch.randn_like`.
+    `packed=True`: ragged packing (SEQDIFF_SAMPLE_PACKED) -- only the valid prefix of every complex is computed; values at valid
+    positions are bit-identical to `packed=False`, padded positions come back as 0 (the reference computes values there, which
+    `sample()` trims away).  Masks that are not prefixes of ones, or fp32 precision, run the padded loop."""
     h = model._sync_handle()
     dev = model._handle_dev
     T = int(total_timesteps)
@@ -240,9 +243,10 @@ def p_sample_loop(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor
     final = torch.empty((B, Ll, Fs), device=dev, dtype=torch.float32)
     with torch.cuda.device(dev):
         stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _cabi.check(_cabi.lib().seqdiff_struct_sample(h, model._precision_code(), B, Ll, Lr, T, _cabi.ptr(coef), _cabi.ptr(x), _cabi.ptr(lm),
-                                                      _cabi.ptr(rs), _cabi.ptr(ra), _cabi.ptr(rm), _cabi.ptr(z), SEED if seed is None else seed,
-                                                      graph_id0, _cabi.ptr(hist), _cabi.ptr(final), stream))
+        _cabi.check(_cabi.lib().seqdiff_struct_sample_ex(h, model._precision_code(), B, Ll, Lr, T, _cabi.ptr(coef), _cabi.ptr(x),
+                                                         _cabi.ptr(lm), _cabi.ptr(rs), _cabi.ptr(ra), _cabi.ptr(rm), _cabi.ptr(z),
+                                                         SEED if seed is None else seed, graph_id0, 1 if packed else 0, _cabi.ptr(hist),
+                                                         _cabi.ptr(final), stream))
     return (hist if keep_history else final[None]).cpu()
 
 
@@ -251,7 +255,8 @@ def sample(model, test_angle_ds, first_batch_only: bool = True, loop_fn=None, **
     noise with the dataset's own `sample_noise`, run `p_sample_loop`, and trim every complex to its ligand length -> a list of numpy
     arrays [timesteps, len_i, n_ft].  `test_angle_ds` is duck-typed like the reference's NoisedAnglesDataset (`__len__`,
     `__getitem__` -> dict of tensors, `sample_noise`, `timesteps`, `alpha_beta_terms["betas"]`).  The reference stops after the
-    first batch (the `break` at sample.py:228); `first_batch_only=False` samples the whole dataset."""
+    first batch (the `break` at sample.py:228); `first_batch_only=False` samples the whole dataset.  Further keywords go to the loop
+    function, e.g. `packed=True` (ragged packing, see `p_sample_loop`): the trimmed arrays are the same, bit for bit."""
     fn = p_sample_loop if loop_fn is None else loop_fn
     bs = CONFIG["batch_size"]
 

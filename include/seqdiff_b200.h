@@ -259,6 +259,18 @@ SEQDIFF_API int seqdiff_struct_sample(seqdiff_model_t* m, int precision, int B, 
                           const float* receptor_mask, const float* noise_steps, uint64_t seed, uint64_t graph_id0,
                           float* steps_out, float* final_out, void* stream);
 
+/* The same loop with options.  flags bit 0 (SEQDIFF_SAMPLE_PACKED): ragged packing -- only the valid prefix of every complex
+ * (ligand_mask / receptor_mask must be prefixes of ones, as the reference's dataset builds them) is carried through the GEMMs /
+ * LayerNorms / attention of both stacks and through the Gaussian step: M = sum of lengths instead of B * L.  Values at valid
+ * positions of final_out and steps_out are bit-identical to the padded loop (a padded key's probability underflows to exactly 0,
+ * every other operator is row-local, and a valid element draws the same noise); padded positions of both are 0 (the reference
+ * computes values there, which sample() trims away).  Non-prefix masks, a complex with no valid ligand or receptor token, or fp32
+ * mode silently take the padded path.  Other flag bits: SEQDIFF_ERR_INVALID. */
+SEQDIFF_API int seqdiff_struct_sample_ex(seqdiff_model_t* m, int precision, int B, int L_lig, int L_rec, int T, const float* coef_steps,
+                             const float* x_T, const float* ligand_mask, const float* receptor_seq, const float* receptor_angles,
+                             const float* receptor_mask, const float* noise_steps, uint64_t seed, uint64_t graph_id0, int flags,
+                             float* steps_out, float* final_out, void* stream);
+
 /* ---- operator-level entry points (used by the parity tests and the micro benchmarks) --------------
  * C[M,N] = epilogue(A[M,K] * W[N,K]^T + bias[N] (+ resid[M,N])); epilogue: 0 none, 1 erf-GELU, 2 SiLU.
  * precision FP32: all f32 (SIMT kernel).  BF16 / FP16: A and W are 16-bit in the mode's formats
