@@ -317,7 +317,7 @@ int seqdiff_struct_sample(seqdiff_model_t* m, int precision, int B, int L_lig, i
                           const float* noise_steps, uint64_t seed, uint64_t graph_id0, float* steps_out, float* final_out, void* stream) {
   SD_GUARD_BEGIN
   SD_CHECK(m && coef_steps && x_T && ligand_mask && receptor_seq && receptor_angles && receptor_mask && final_out, "null argument");
-  return m->impl.struct_sample(precision, B, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
+  return m->impl.struct_sample(precision, B, 1, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
                                noise_steps, seed, graph_id0, steps_out, final_out, static_cast<cudaStream_t>(stream), 0);
   SD_GUARD_END
 }
@@ -326,10 +326,21 @@ int seqdiff_struct_sample_ex(seqdiff_model_t* m, int precision, int B, int L_lig
                              const float* ligand_mask, const float* receptor_seq, const float* receptor_angles, const float* receptor_mask,
                              const float* noise_steps, uint64_t seed, uint64_t graph_id0, int flags, float* steps_out, float* final_out,
                              void* stream) {
+  return seqdiff_struct_sample_multi(m, precision, B, 1, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles,
+                                     receptor_mask, noise_steps, seed, graph_id0, flags, steps_out, final_out, stream);
+}
+
+int seqdiff_struct_sample_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T, const float* coef_steps,
+                                const float* x_T, const float* ligand_mask, const float* receptor_seq, const float* receptor_angles,
+                                const float* receptor_mask, const float* noise_steps, uint64_t seed, uint64_t graph_id0, int flags,
+                                float* steps_out, float* final_out, void* stream) {
   SD_GUARD_BEGIN
   SD_CHECK(m && coef_steps && x_T && ligand_mask && receptor_seq && receptor_angles && receptor_mask && final_out, "null argument");
+  SD_CHECK(P >= 1 && K >= 1, "need at least one pocket and one sample per pocket");
+  SD_CHECK(L_lig > 0 && L_rec > 0 && static_cast<int64_t>(P) * K * (L_lig > L_rec ? L_lig : L_rec) <= INT32_MAX,
+           "pockets x samples x length overflows the row counts");
   SD_CHECK((flags & ~1) == 0, "unknown sampling flag");
-  return m->impl.struct_sample(precision, B, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
+  return m->impl.struct_sample(precision, P, K, L_lig, L_rec, T, coef_steps, x_T, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
                                noise_steps, seed, graph_id0, steps_out, final_out, static_cast<cudaStream_t>(stream), flags);
   SD_GUARD_END
 }

@@ -219,23 +219,26 @@ struct Model {
   // structure_model/model.py:180-215.  phases: bit 0 = run the receptor branch, bit 1 = the ligand branch.  The receptor branch (embeddings,
   // receptor_emb, encoder, all decoder layers' cross K|V) depends on neither the timestep nor the ligand, so the sampling loop runs it
   // once and keeps the K|V block.
-  // pk (16-bit modes, sampling loop): ragged packing with one receptor per ligand graph (build_pack with K = 1)
+  // pk (16-bit modes, sampling loop): ragged packing (build_pack(B, K, ...)).  K > 1 (sampling loop): the receptor inputs hold B / K
+  // pockets, the receptor branch runs over them once, and ligand graph b cross-attends to pocket b / K.
   int struct_forward(int precision, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* noised_angles,
                      const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, float* out, int phases,
-                     cudaStream_t s, const PackInfo* pk = nullptr);
+                     cudaStream_t s, const PackInfo* pk = nullptr, int K = 1);
   // structure_model/sample.py:104-144 (STEP = 1): T x (forward, Gaussian reverse step, angle wrap) from one captured graph.
+  // P pockets x K samples per pocket: ligand inputs / x_T / noise / steps_out / final_out hold B = P * K graphs (sample j of pocket p
+  // is graph p * K + j), receptor inputs hold P.
   // flags bit 0: ragged packing (valid positions bit-identical to the padded loop; padded positions of steps_out / final_out are 0)
-  int struct_sample(int precision, int B, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
+  int struct_sample(int precision, int P, int K, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
                     const float* rec_seq, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
                     uint64_t gid0, float* steps_out, float* final_out, cudaStream_t s, int flags = 0);
 
  public:
   void* dalloc(size_t bytes);
-  size_t struct_workspace_need(int precision, int B, int Ll, int Lr) const;
+  size_t struct_workspace_need(int precision, int B, int Ll, int Lr, int K = 1) const;
   template <typename T>
   int struct_forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, const int* step_ptr, const float* noised_angles,
                        const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, float* out, int phases,
-                       cudaStream_t s, const PackInfo* pk);
+                       cudaStream_t s, const PackInfo* pk, int K);
   size_t workspace_need(int precision, int B, int Ll, int Lr) const;
   int ensure_workspace(size_t bytes);
   template <typename T>

@@ -119,7 +119,8 @@ def denoise_tensors(batch, model, noise_schedule, transition, diverse, timesteps
     `num_samples=K > 1`: K sequences per pocket of the batch (seqdiff_sample_multi).  The batch holds P pockets; the result, x_T and
     the graph ids cover B = P*K graphs, sample j of pocket p being graph p*K + j, and noise_E_steps is [T, P*K*L, 20].  Each pocket's
     receptor rows are computed once per step for its K samples; the result equals the K = 1 call on the batch whose entries are
-    repeated K times per pocket."""
+    repeated K times per pocket.  The batch's ligand_angles / ligand_attn_mask are [P, ...] and repeated for the K samples, or
+    already [P*K, ...]: one entry per sample (e.g. a different generated backbone for each sample, design.py)."""
     K = check_num_samples(num_samples)
     T = CONFIG["timesteps"] if timesteps is None else timesteps
     h = model._sync_handle()
@@ -139,7 +140,13 @@ def denoise_tensors(batch, model, noise_schedule, transition, diverse, timesteps
     if K > 1:
         if tuple(x_T.shape) != (batch_size, max_len, num_class):
             raise ValueError(f"x_T must be [P*K, L, {num_class}] = {(batch_size, max_len, num_class)}, got {tuple(x_T.shape)}")
-        ligand_mask, ligand_angles = ligand_mask.repeat_interleave(K, dim=0), ligand_angles.repeat_interleave(K, dim=0)
+        def per_sample(x, name):
+            if x.shape[0] == batch_size:
+                return x
+            if x.shape[0] != n_pockets:
+                raise ValueError(f"{name} must hold P = {n_pockets} or P*K = {batch_size} entries, got {x.shape[0]}")
+            return x.repeat_interleave(K, dim=0)
+        ligand_mask, ligand_angles = per_sample(ligand_mask, "ligand_attn_mask"), per_sample(ligand_angles, "ligand_angles")
     receptor_seq, receptor_angles = dv(batch["receptor_seq"]), dv(batch["receptor_angles"])
     receptor_attn_mask = dv(batch["receptor_attn_mask"])
     Lr = receptor_seq.shape[1]
@@ -193,11 +200,21 @@ def denoise(batch, model: PeptideDiff, noise_schedule, transition, diverse, num_
     `num_samples=K`: K sequences per pocket of the batch (denoise_tensors); the lists then hold P*K entries in (pocket, sample)
     order, with each pocket's structure id and true sequence repeated for its samples."""
     K = check_num_samples(num_samples)
-    batch_size = batch["ligand_seq"].shape[0] * K
     final = denoise_tensors(batch, model, noise_schedule, transition, diverse, num_samples=K, **kw)
+    structure_ids, true_sequences, pred_sequences, recovery_rates = decode_batch(final, batch, K)
+    print(sum(recovery_rates) / len(recovery_rates))
+    return structure_ids, true_sequences, pred_sequences, recovery_rates
+
+
+def decode_batch(final, batch, K=1):
+    """The result lists of denoise() for the final tensor of P*K graphs of `batch` (K per pocket, in (pocket, sample) order):
+    (structure_ids, true_sequences, pred_sequences, recovery_rates), each pocket's id and native sequence repeated for its samples."""
+    batch_size = batch["ligand_seq"].shape[0] * K
     ligand_seq, ligand_mask = batch["ligand_seq"], batch["ligand_attn_mask"]
     if K > 1:
-        ligand_seq, ligand_mask = ligand_seq.repeat_interleave(K, dim=0), ligand_mask.repeat_interleave(K, dim=0)
+        ligand_seq = ligand_seq.repeat_interleave(K, dim=0)
+        if ligand_mask.shape[0] != batch_size:  # per-pocket mask (denoise_tensors also takes one per sample)
+            ligand_mask = ligand_mask.repeat_interleave(K, dim=0)
     # sample.py:208-224 in one kernel: argmax decode of both sequences + per-graph (matches, valid) counts; the host gets
     # 2 x [B,L] bytes + [B,2] ints in one synchronising copy (the reference syncs once per graph) and only joins letters
     pred_idx, true_idx, counts = decode_tensors(final, ligand_seq, ligand_mask)
@@ -216,7 +233,6 @@ def denoise(batch, model: PeptideDiff, noise_schedule, transition, diverse, num_
         true_sequences.append("".join(AA_VOCAB[j] for j in true_seq))
         ids = batch.get("structure_ids")
         structure_ids.append(f'{ids["pdb_id"][i // K]}_{ids["ligand_chain"][i // K]}' if ids is not None else str(i // K))
-    print(sum(recovery_rates) / len(recovery_rates))
     return structure_ids, true_sequences, pred_sequences, recovery_rates
 
 

@@ -17,6 +17,7 @@ from torch import nn
 from torch.nn import functional as F
 
 from . import _cabi
+from .sample import check_num_samples
 from .model import (BertEmbeddings, BertEncoder, ConditionalBertForDiffusionBase as _SeqBase, GaussianFourierProjection, SELayer,
                     _Container, _BertLayer, BertAttention, _Intermediate, _SelfOutput)
 
@@ -129,12 +130,16 @@ class ConditionalBertForDiffusionBase(_SeqBase):
     def initialize_weights(self):  # the structure model keeps torch's default init (no initialize_weights in the reference)
         return None
 
-    def _inputs(self, noised_ligand_angles, ligand_attention_masks, receptor_seq, receptor_angles, receptor_attention_masks):
+    def _inputs(self, noised_ligand_angles, ligand_attention_masks, receptor_seq, receptor_angles, receptor_attention_masks, K: int = 1):
+        """K > 1: the receptor tensors hold B / K pockets (sampling loop, sample j of pocket p = ligand graph p*K + j)."""
         dev = self._handle_dev
         B, Ll, Fs = noised_ligand_angles.shape
         Lr = receptor_seq.shape[1]
         if Fs != self.feature_size:
             raise ValueError(f"expected {self.feature_size} angle features, got {Fs}")
+        if B % K:
+            raise ValueError(f"{B} ligand graphs are not {K} samples for each pocket")
+        P = B // K
 
         def prep(x, shape):
             x = x.to(device=dev, dtype=torch.float32).contiguous()
@@ -142,8 +147,8 @@ class ConditionalBertForDiffusionBase(_SeqBase):
                 raise ValueError(f"expected shape {shape}, got {tuple(x.shape)}")
             return x
 
-        return (B, Ll, Lr, prep(noised_ligand_angles, (B, Ll, Fs)), prep(ligand_attention_masks, (B, Ll)), prep(receptor_seq, (B, Lr, 20)),
-                prep(receptor_angles, (B, Lr, Fs)), prep(receptor_attention_masks, (B, Lr)))
+        return (B, Ll, Lr, prep(noised_ligand_angles, (B, Ll, Fs)), prep(ligand_attention_masks, (B, Ll)), prep(receptor_seq, (P, Lr, 20)),
+                prep(receptor_angles, (P, Lr, Fs)), prep(receptor_attention_masks, (P, Lr)))
 
     def forward(self, timestep, noised_ligand_angles, ligand_attention_masks, receptor_seq, receptor_angles, receptor_attention_masks,
                 ligand_pos_ids=None, receptor_pos_ids=None):
@@ -211,22 +216,21 @@ def p_sample_wrapped(model, ligand_mask, ligand_angle_noise, receptor_seq, recep
 
 
 @torch.no_grad()
-def p_sample_loop(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor_mask, receptor_angle, total_timesteps: int, betas,
-                  disable_pbar: bool = True, noise_steps: Optional[torch.Tensor] = None, graph_id0: Optional[int] = None, seed: Optional[int] = None,
-                  keep_history: bool = True, packed: bool = False) -> torch.Tensor:
-    """reference structure_model/sample.py:104-144: returns a CPU tensor [timesteps, B, L, F] (entry k = wrapped angles after
-    the k-th reverse step).  The whole loop is ONE C call (`seqdiff_struct_sample_ex`): the receptor branch is evaluated once, every
-    step replays a captured CUDA graph (ligand branch + Gaussian step + wrap), and the history is written by the step kernel --
-    one device->host copy at the end instead of one per step.  `keep_history=False` returns only the final [1,B,L,F] entry.
-    `noise_steps` [T,B,L,F]: entry i = the N(0,1) draw used at step index i (entry 0 unused).  `graph_id0` = None continues the
-    process-wide Philox noise stream, so successive batches / calls draw fresh noise like the reference's `torch.randn_like`.
-    `packed=True`: ragged packing (SEQDIFF_SAMPLE_PACKED) -- only the valid prefix of every complex is computed; values at valid
-    positions are bit-identical to `packed=False`, padded positions come back as 0 (the reference computes values there, which
-    `sample()` trims away).  Masks that are not prefixes of ones, or fp32 precision, run the padded loop."""
+def p_sample_loop_tensors(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor_mask, receptor_angle, total_timesteps: int, betas,
+                          noise_steps: Optional[torch.Tensor] = None, graph_id0: Optional[int] = None, seed: Optional[int] = None,
+                          keep_history: bool = True, packed: bool = False, num_samples: int = 1):
+    """`p_sample_loop` without the copy to the host: returns (history [T,B,L,F] or None when keep_history=False, final [B,L,F]), both
+    on the model's device."""
+    K = check_num_samples(num_samples)
     h = model._sync_handle()
     dev = model._handle_dev
     T = int(total_timesteps)
-    B, Ll, Lr, x, lm, rs, ra, rm = model._inputs(ligand_angle_noise, ligand_mask, receptor_seq, receptor_angle, receptor_mask)
+    n_pockets = receptor_seq.shape[0]
+    if K > 1 and ligand_mask.shape[0] == n_pockets:
+        ligand_mask = ligand_mask.repeat_interleave(K, dim=0)
+    if ligand_angle_noise.shape[0] != n_pockets * K:
+        raise ValueError(f"ligand_angle_noise must hold P*K = {n_pockets * K} graphs, got {ligand_angle_noise.shape[0]}")
+    B, Ll, Lr, x, lm, rs, ra, rm = model._inputs(ligand_angle_noise, ligand_mask, receptor_seq, receptor_angle, receptor_mask, K)
     if graph_id0 is None:
         graph_id0 = _cabi.GRAPH_IDS.take(B)
     Fs = model.feature_size
@@ -238,25 +242,52 @@ def p_sample_loop(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor
     if noise_steps is not None:
         z = noise_steps.to(device=dev, dtype=torch.float32).contiguous()
         if tuple(z.shape) != (T, B, Ll, Fs):
-            raise ValueError("noise_steps must be [T, B, L, F]")
+            raise ValueError("noise_steps must be [T, B, L, F]" if K == 1 else "noise_steps must be [T, P*K, L, F]")
     hist = torch.empty((T, B, Ll, Fs), device=dev, dtype=torch.float32) if keep_history else None
     final = torch.empty((B, Ll, Fs), device=dev, dtype=torch.float32)
     with torch.cuda.device(dev):
         stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _cabi.check(_cabi.lib().seqdiff_struct_sample_ex(h, model._precision_code(), B, Ll, Lr, T, _cabi.ptr(coef), _cabi.ptr(x),
-                                                         _cabi.ptr(lm), _cabi.ptr(rs), _cabi.ptr(ra), _cabi.ptr(rm), _cabi.ptr(z),
-                                                         SEED if seed is None else seed, graph_id0, 1 if packed else 0, _cabi.ptr(hist),
-                                                         _cabi.ptr(final), stream))
+        _cabi.check(_cabi.lib().seqdiff_struct_sample_multi(h, model._precision_code(), n_pockets, K, Ll, Lr, T, _cabi.ptr(coef), _cabi.ptr(x),
+                                                            _cabi.ptr(lm), _cabi.ptr(rs), _cabi.ptr(ra), _cabi.ptr(rm), _cabi.ptr(z),
+                                                            SEED if seed is None else seed, graph_id0, 1 if packed else 0, _cabi.ptr(hist),
+                                                            _cabi.ptr(final), stream))
+    return hist, final
+
+
+@torch.no_grad()
+def p_sample_loop(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor_mask, receptor_angle, total_timesteps: int, betas,
+                  disable_pbar: bool = True, noise_steps: Optional[torch.Tensor] = None, graph_id0: Optional[int] = None, seed: Optional[int] = None,
+                  keep_history: bool = True, packed: bool = False, num_samples: int = 1) -> torch.Tensor:
+    """reference structure_model/sample.py:104-144: returns a CPU tensor [timesteps, B, L, F] (entry k = wrapped angles after
+    the k-th reverse step).  The whole loop is ONE C call (`seqdiff_struct_sample_multi`): the receptor branch is evaluated once, every
+    step replays a captured CUDA graph (ligand branch + Gaussian step + wrap), and the history is written by the step kernel --
+    one device->host copy at the end instead of one per step.  `keep_history=False` returns only the final [1,B,L,F] entry.
+    `noise_steps` [T,B,L,F]: entry i = the N(0,1) draw used at step index i (entry 0 unused).  `graph_id0` = None continues the
+    process-wide Philox noise stream, so successive batches / calls draw fresh noise like the reference's `torch.randn_like`.
+    `packed=True`: ragged packing (SEQDIFF_SAMPLE_PACKED) -- only the valid prefix of every complex is computed; values at valid
+    positions are bit-identical to `packed=False`, padded positions come back as 0 (the reference computes values there, which
+    `sample()` trims away).  Masks that are not prefixes of ones, or fp32 precision, run the padded loop.
+    `num_samples=K > 1`: K backbones per pocket.  The receptor tensors hold P pockets; ligand_angle_noise, noise_steps, the graph ids
+    and the result cover B = P*K graphs, sample j of pocket p being graph p*K + j; ligand_mask is [P*K, L], or [P, L] and repeated.
+    The receptor branch runs once per pocket; the result equals the K = 1 loop on the batch whose pockets are repeated K times."""
+    hist, final = p_sample_loop_tensors(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor_mask, receptor_angle, total_timesteps,
+                                        betas, noise_steps=noise_steps, graph_id0=graph_id0, seed=seed, keep_history=keep_history,
+                                        packed=packed, num_samples=num_samples)
     return (hist if keep_history else final[None]).cpu()
 
 
-def sample(model, test_angle_ds, first_batch_only: bool = True, loop_fn=None, **kw):
+def sample(model, test_angle_ds, first_batch_only: bool = True, loop_fn=None, num_samples: int = 1, **kw):
     """reference structure_model/sample.py:191-229: chunk the dataset's features into batches of CONFIG["batch_size"], draw the start
     noise with the dataset's own `sample_noise`, run `p_sample_loop`, and trim every complex to its ligand length -> a list of numpy
     arrays [timesteps, len_i, n_ft].  `test_angle_ds` is duck-typed like the reference's NoisedAnglesDataset (`__len__`,
     `__getitem__` -> dict of tensors, `sample_noise`, `timesteps`, `alpha_beta_terms["betas"]`).  The reference stops after the
     first batch (the `break` at sample.py:228); `first_batch_only=False` samples the whole dataset.  Further keywords go to the loop
-    function, e.g. `packed=True` (ragged packing, see `p_sample_loop`): the trimmed arrays are the same, bit for bit."""
+    function, e.g. `packed=True` (ragged packing, see `p_sample_loop`): the trimmed arrays are the same, bit for bit.
+    `num_samples=K > 1`: K backbones per complex (see `p_sample_loop`), the start noise drawn for all P*K of a batch at once; the list
+    then holds the arrays in (complex, sample) order."""
+    K = check_num_samples(num_samples)
+    if K > 1:
+        kw["num_samples"] = K
     fn = p_sample_loop if loop_fn is None else loop_fn
     bs = CONFIG["batch_size"]
 
@@ -274,11 +305,11 @@ def sample(model, test_angle_ds, first_batch_only: bool = True, loop_fn=None, **
     for idx, this_lengths in enumerate(ligand_len):
         print(f"Generating Batch {idx}/{len(ligand_len)}")
         batch = len(this_lengths)
-        noise = test_angle_ds.sample_noise(torch.zeros((batch, pad, feature_size), dtype=torch.float32))
+        noise = test_angle_ds.sample_noise(torch.zeros((batch * K, pad, feature_size), dtype=torch.float32))
         sampled = fn(model=model, ligand_mask=ligand_mask[idx], ligand_angle_noise=noise, receptor_seq=receptor_seq[idx],
                      receptor_mask=receptor_mask[idx], receptor_angle=receptor_angle[idx], total_timesteps=test_angle_ds.timesteps,
                      betas=test_angle_ds.alpha_beta_terms["betas"], disable_pbar=False, **kw)
-        retval.extend(sampled[:, i, :int(l), :].numpy() for i, l in enumerate(this_lengths))
+        retval.extend(sampled[:, i, :int(this_lengths[i // K]), :].numpy() for i in range(batch * K))
         if first_batch_only:
             break
     return retval

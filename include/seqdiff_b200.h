@@ -271,6 +271,20 @@ SEQDIFF_API int seqdiff_struct_sample_ex(seqdiff_model_t* m, int precision, int 
                              const float* receptor_mask, const float* noise_steps, uint64_t seed, uint64_t graph_id0, int flags,
                              float* steps_out, float* final_out, void* stream);
 
+/* The same loop for P pockets x K samples per pocket (peptide design: several candidate backbones for one binding pocket).  Ligand-side
+ * arrays hold B = P*K graphs, sample j of pocket p being graph p*K + j with global graph id graph_id0 + p*K + j in the Philox stream:
+ * x_T / final_out [P*K,L_lig,F], ligand_mask [P*K,L_lig], noise_steps [T,P*K*L_lig*F] or NULL, steps_out [T,P*K*L_lig*F] or NULL.
+ * Receptor-side arrays hold the P pockets once: receptor_seq [P,L_rec,20], receptor_angles [P,L_rec,F], receptor_mask [P,L_rec].
+ * The receptor branch (embeddings, receptor_emb, the encoder and every decoder layer's cross K|V) runs once per sampling over the
+ * P pockets, and the K samples' cross-attention reads their pocket's K|V.  steps_out and final_out equal, bit for bit, what
+ * seqdiff_struct_sample_ex returns for the batch whose receptor arrays are repeated K times per pocket (packed mode: at the valid
+ * positions, padded ones 0).  K = 1 is seqdiff_struct_sample_ex.  P < 1, K < 1, P*K*max(L_lig, L_rec) > INT32_MAX or an unknown
+ * flag bit: SEQDIFF_ERR_INVALID. */
+SEQDIFF_API int seqdiff_struct_sample_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T,
+                                const float* coef_steps, const float* x_T, const float* ligand_mask, const float* receptor_seq,
+                                const float* receptor_angles, const float* receptor_mask, const float* noise_steps, uint64_t seed,
+                                uint64_t graph_id0, int flags, float* steps_out, float* final_out, void* stream);
+
 /* ---- operator-level entry points (used by the parity tests and the micro benchmarks) --------------
  * C[M,N] = epilogue(A[M,K] * W[N,K]^T + bias[N] (+ resid[M,N])); epilogue: 0 none, 1 erf-GELU, 2 SiLU.
  * precision FP32: all f32 (SIMT kernel).  BF16 / FP16: A and W are 16-bit in the mode's formats
