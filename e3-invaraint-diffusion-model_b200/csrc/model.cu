@@ -843,7 +843,9 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
   const int P = cfg.max_position_embeddings;
   const float eps = cfg.layer_norm_eps;
   // packed (ragged) batch: only the valid prefix of every graph is a row; inputs, masks and logits keep their padded layouts.
-  // The receptor rows are those of the B / K pockets.
+  // The receptor rows are those of the B / K pockets.  A receptor-only pack (pk->lig_padded, sampling loop) packs the receptor
+  // rows alone: pl, the pack the ligand side uses, is then NULL and the ligand rows run the padded path.
+  const PackInfo* pl = pk && !pk->lig_padded ? pk : nullptr;
   const int Ml = pk ? pk->Ml : B * Ll, Mr = pk ? pk->Mr : B / K * Lr, Mt = Ml + Mr;
   const int Mlp = B * Ll, Mrp = B / K * Lr;  // padded row counts (input tensors, key masks)
   const size_t MlH = static_cast<size_t>(Ml) * H;
@@ -868,7 +870,7 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
       jb.x = in; jb.Wt = e.Wt_; jb.b = e.b; jb.lnw = e.ln_w; jb.lnb = e.ln_b; jb.te = cond ? te_ : nullptr;
       jb.te_row = cond && inv ? step_ptr : nullptr;
       jb.out32 = o32; jb.outT = oT; jb.M = M; jb.fin = e.fin; jb.L = L;
-      if (pk) {
+      if (lig ? pl : pk) {
         jb.src_rows = lig ? pk->src_l : pk->src_r;
         jb.row_graph = lig ? pk->graph : pk->graph + pk->Ml;
       }
@@ -892,13 +894,14 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
   std::vector<Segment> segs;
   std::vector<AttnPack> packs;
   AttnPack pk_self{}, pk_cross{};
-  if (pk) {
+  if (pk) {  // receptor-only pack: the cross-attention's queries are the padded ligand rows (off_l[b] = b * Ll, len_l[b] = Ll)
     pk_self = AttnPack{pk->off_l, pk->off_l, pk->len_l, Ml, Ml, Ll};
     pk_cross = AttnPack{pk->off_l, pk->off_r, pk->len_l, Ml, Mr, Lr};
   }
+  SD_CHECK(pl == pk || inv, "a receptor-only pack exists in the sampling loop only");
   if (inv) {
-    segs.push_back({0, B, pk ? pk->max_l : Ll, lig_mask});
-    if (pk) packs.push_back(pk_self);
+    segs.push_back({0, B, pl ? pl->max_l : Ll, lig_mask});
+    if (pl) packs.push_back(pk_self);
   } else if (pk) {
     // offsets are absolute rows of the stacked matrix, so every segment starts at row 0
     if (Ll == Lr) {
@@ -916,11 +919,11 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
     segs.push_back({0, B, Ll, lig_mask});
     segs.push_back({Ml, B, Lr, rec_mask});
   }
-  const int Lq_self = pk ? pk->max_l : Ll, Lk_cross = pk ? pk->max_r : Lr;
-  const AttnPack* aps = pk ? &pk_self : nullptr;
+  const int Lq_self = pl ? pl->max_l : Ll, Lk_cross = pk ? pk->max_r : Lr;
+  const AttnPack* aps = pl ? &pk_self : nullptr;
   const AttnPack* apc = pk ? &pk_cross : nullptr;
   const SEHoist<T> hz_lig{Ml, inv ? inv->o : nullptr, inv ? inv->xr : nullptr, nullptr, nullptr};
-  SD_TRY(se_layer<T>(*this, wfmt, se_lig, x, ccat, Mt, 1, Mt, segs, sb, x2, s, pk ? &packs : nullptr, nullptr, inv ? &hz_lig : nullptr));
+  SD_TRY(se_layer<T>(*this, wfmt, se_lig, x, ccat, Mt, 1, Mt, segs, sb, x2, s, pl ? &packs : nullptr, nullptr, inv ? &hz_lig : nullptr));
   const T* rec = x2.t + MlH;
 
   // decoder: 6 x (self-attn -> cross-attn -> FFN), post-LN (HF BertLayer; model.py:226-231)
@@ -989,9 +992,9 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
   // modulation is row *step_ptr of inv->mod.
   std::vector<Segment> lseg{{0, B, Lq_self, lig_mask}};
   std::vector<AttnPack> lpack;
-  if (pk) lpack.push_back(pk_self);
+  if (pl) lpack.push_back(pk_self);
   const SEHoist<T> hz_dec{Ml, nullptr, nullptr, inv ? static_cast<const T*>(inv->mod) : nullptr, step_ptr};
-  SD_TRY(se_layer<T>(*this, wfmt, se_dec, h, teT, B, Ll, Ml, lseg, sb, x, s, pk ? &lpack : nullptr, pk ? pk->graph : nullptr, inv ? &hz_dec : nullptr));
+  SD_TRY(se_layer<T>(*this, wfmt, se_dec, h, teT, B, Ll, Ml, lseg, sb, x, s, pl ? &lpack : nullptr, pl ? pl->graph : nullptr, inv ? &hz_dec : nullptr));
 
   // AminoAcidPredictor (model.py:148-153)
   if constexpr (std::is_same<T, bf16>::value) {
@@ -1003,11 +1006,11 @@ int Model::forward_t(int wfmt, int B, int Ll, int Lr, const float* timestep, con
     f16* yh = reinterpret_cast<f16*>(y);
     SD_TRY(f32_to_16<f16>(x.s, static_cast<size_t>(Ml) * H, xh, s));
     SD_TRY(gemm_16(Ml, H, H, xh, 0, p1.g, 0, p1_b, nullptr, 1, yh, 0, s));
-    SD_TRY(predictor_tail<f16>(yh, Ml, H, p_ln_w, p_ln_b, 1e-12f, p2_w, p2_b, cfg.feature_size, logits, s, pk ? pk->src_l : nullptr));
+    SD_TRY(predictor_tail<f16>(yh, Ml, H, p_ln_w, p_ln_b, 1e-12f, p2_w, p2_b, cfg.feature_size, logits, s, pl ? pl->src_l : nullptr));
     return SEQDIFF_OK;
   }
   SD_TRY(gemm_T(wfmt, Ml, H, H, x.t, p1, p1_b, 1, y, s));
-  SD_TRY(predictor_tail<T>(y, Ml, H, p_ln_w, p_ln_b, 1e-12f, p2_w, p2_b, cfg.feature_size, logits, s, pk ? pk->src_l : nullptr));
+  SD_TRY(predictor_tail<T>(y, Ml, H, p_ln_w, p_ln_b, 1e-12f, p2_w, p2_b, cfg.feature_size, logits, s, pl ? pl->src_l : nullptr));
   return SEQDIFF_OK;
 }
 
@@ -1076,14 +1079,16 @@ int Model::loop_invariants_t(int wfmt, int B, int K, int Ll, int Lr, int T_, con
 // =====================================================================================================
 // Ragged packing: lengths from the (prefix-ones) masks, row maps, offsets.  *usable = false when a mask is not a prefix of ones
 // (the caller then stays on the padded path) or a graph has no valid ligand / receptor token.  B ligand graphs, B / K pockets.
-int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable) {
+// lig_padded: every ligand length is Ll whatever the ligand mask says, so only the receptor masks are read and checked.
+int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable,
+                      bool lig_padded) {
   *usable = false;
   const int P = B / K;
-  std::vector<float> hl(static_cast<size_t>(B) * Ll), hr(static_cast<size_t>(P) * Lr);
-  SD_CUDA(cudaMemcpyAsync(hl.data(), lig_mask, hl.size() * 4, cudaMemcpyDefault, s));
+  std::vector<float> hl(lig_padded ? 0 : static_cast<size_t>(B) * Ll), hr(static_cast<size_t>(P) * Lr);
+  if (!lig_padded) SD_CUDA(cudaMemcpyAsync(hl.data(), lig_mask, hl.size() * 4, cudaMemcpyDefault, s));
   SD_CUDA(cudaMemcpyAsync(hr.data(), rec_mask, hr.size() * 4, cudaMemcpyDefault, s));
   SD_CUDA(cudaStreamSynchronize(s));
-  std::vector<int> len_l(B), len_r(P);
+  std::vector<int> len_l(B, Ll), len_r(P);
   auto lengths = [&](const std::vector<float>& m, int G, int L, std::vector<int>& len) -> bool {
     for (int b = 0; b < G; ++b) {
       int n = 0;
@@ -1095,7 +1100,7 @@ int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const
     }
     return true;
   };
-  if (!lengths(hl, B, Ll, len_l) || !lengths(hr, P, Lr, len_r)) return SEQDIFF_OK;
+  if ((!lig_padded && !lengths(hl, B, Ll, len_l)) || !lengths(hr, P, Lr, len_r)) return SEQDIFF_OK;
   int Ml = 0, Mr = 0, max_l = 0, max_r = 0;
   std::vector<int> off_l(B), off_r(P);
   for (int b = 0; b < B; ++b) {
@@ -1121,9 +1126,10 @@ int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const
   for (int p = 0; p < P; ++p) blk.push_back(Ml + off_r[p]);
   for (int b = 0; b < B; ++b) blk.push_back(len_l[b]);
   for (int p = 0; p < P; ++p) blk.push_back(len_r[p]);
-  // FNV-1a over K and the block: a changed batch composition re-captures the step graph
+  // FNV-1a over K, the kind of pack and the block: a changed batch composition re-captures the step graph
   uint64_t hsh = 1469598103934665603ull;
   hsh ^= static_cast<uint32_t>(K); hsh *= 1099511628211ull;
+  hsh ^= lig_padded ? 1u : 0u; hsh *= 1099511628211ull;
   for (int v : blk) { hsh ^= static_cast<uint32_t>(v); hsh *= 1099511628211ull; }
   bool fresh = false;
   if (blk.size() > pack_cap) {
@@ -1137,7 +1143,7 @@ int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const
     SD_CUDA(cudaStreamSynchronize(s));  // blk is a stack-lifetime host buffer
   }
   PackInfo pi;
-  pi.B = B; pi.P = P; pi.Ml = Ml; pi.Mr = Mr; pi.max_l = max_l; pi.max_r = max_r; pi.hash = hsh;
+  pi.B = B; pi.P = P; pi.Ml = Ml; pi.Mr = Mr; pi.max_l = max_l; pi.max_r = max_r; pi.hash = hsh; pi.lig_padded = lig_padded;
   const int* p = d_pack;
   pi.src_l = p; p += Ml;
   pi.src_r = p; p += Mr;
@@ -1210,6 +1216,14 @@ int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const floa
       pk = &pack;
       SD_CUDA(cudaMemsetAsync(logits, 0, Nl * 20 * 4, s));  // padded positions are never written in packed mode: defined as 0
     }
+  }
+  // padded path, 16-bit modes: the receptor rows are still packed (PackInfo::lig_padded), since no output reads a padded one.  It
+  // needs prefix receptor masks with at least one valid token per pocket: a pocket without one attends uniformly over its padded
+  // keys, whose values are then read.  Otherwise (and in fp32 mode) every receptor row is computed.
+  if (!pk && precision != SEQDIFF_FP32) {
+    bool usable = false;
+    SD_TRY(build_pack(B, K, Ll, Lr, nullptr, c_rmask, s, &usable, true));
+    if (usable) pk = &pack;
   }
 
   const long long rows = pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(Nl + Nr);  // token rows of a step

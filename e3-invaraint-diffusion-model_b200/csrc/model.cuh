@@ -87,7 +87,11 @@ struct PackInfo {
   const int* len_r = nullptr;     // [P]
   const int* off_cat = nullptr;   // [B + P] ligand offsets, then receptor offsets + Ml (stacked matrix)
   const int* len_cat = nullptr;   // [B + P]
-  uint64_t hash = 0;              // of K and the length vectors (part of the CUDA-graph key)
+  uint64_t hash = 0;              // of K, lig_padded and the length vectors (part of the CUDA-graph key)
+  // Receptor-only pack (the padded sampling loop): the ligand rows keep their padded layout -- every ligand length is Ll, so
+  // Ml = B * Ll, src_l is the identity and off_l[b] = b * Ll -- and only the receptor rows are packed.  No output reads a padded
+  // receptor row (DESIGN.md section 9), so the result is the padded computation's at every position, padded ones included.
+  bool lig_padded = false;
 };
 
 // What the sequence model's sampling loop computes once per sampling instead of once per step (Model::sample).  Every graph of the
@@ -180,7 +184,9 @@ struct Model {
   int* d_pack = nullptr;  // device block behind PackInfo (grow-only)
   size_t pack_cap = 0;
   PackInfo pack;
-  int build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable);
+  // lig_padded: the receptor-only pack (PackInfo::lig_padded); lig_mask is not read then
+  int build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const float* rec_mask, cudaStream_t s, bool* usable,
+                 bool lig_padded = false);
 
   // ---- training (train.cu) ------------------------------------------------------------------------------------------
   std::vector<ParamSlot> slots;            // trainable tensors in flat-buffer order (fused groups contiguous)

@@ -7,9 +7,9 @@ template arguments.  Prints one JSON object: per mode the library's launch count
 per kernel name the time, launches and share per step.  The library's own event profiler marks only eager launches, so it
 sees the stand-alone forward, not the loop's step.
 K > 1: the workload's B graphs become B / K pockets x K samples, profiled both as the replicated batch ("<mode>_replicated",
-seqdiff_sample_ex) and with the pockets shared ("<mode>_shared", seqdiff_sample_multi).  Every kernel of the step is then also
-listed by its position in the step ("by_position": the kernel trace cut at each reverse_step_kernel, mean device time over the
-full steps), which tells apart launches of the same kernel, e.g. the cross K|V GEMM from the decoder's GEMMs."""
+seqdiff_sample_ex) and with the pockets shared ("<mode>_shared", seqdiff_sample_multi).  Every kernel of the step is also listed
+by its position in the step ("by_position": the kernel trace cut at each reverse_step_kernel, mean device time over the full
+steps), which tells apart launches of the same kernel, e.g. the cross K|V GEMM from the decoder's GEMMs."""
 import json
 import os
 import re
@@ -77,16 +77,15 @@ for packed, form in forms:
         "launches_per_sampling": launches, "us_per_step": round(tot / T, 1),
         "kernels": {n: {"us_per_step": round(v[0] / T, 2), "launches_per_step": round(v[1] / T, 2), "share": round(v[0] / tot, 4)}
                     for n, v in sorted(agg.items(), key=lambda kv: -kv[1][0])}}
-    if K > 1:
-        with tempfile.TemporaryDirectory() as d:
-            p.export_chrome_trace(os.path.join(d, "trace.json"))
-            events = json.load(open(os.path.join(d, "trace.json")))["traceEvents"]
-        kern = sorted((e for e in events if e.get("cat") == "kernel"), key=lambda e: e["ts"])
-        cuts = [i for i, e in enumerate(kern) if "reverse_step_kernel" in e["name"]]
-        steps = [kern[a + 1:b + 1] for a, b in zip(cuts, cuts[1:])]  # full steps: after one reverse step up to the next
-        n = len(steps[0])
-        assert all(len(st) == n for st in steps), "steps of different kernel counts"
-        rec["by_position"] = [{"kernel": re.split(r"[<(]", re.sub(r"^(void )?seqdiff::", "", steps[0][i]["name"]))[0],
-                               "grid": steps[0][i]["args"]["grid"], "us": round(sum(st[i]["dur"] for st in steps) / len(steps), 2)}
-                              for i in range(n)]
+    with tempfile.TemporaryDirectory() as d:
+        p.export_chrome_trace(os.path.join(d, "trace.json"))
+        events = json.load(open(os.path.join(d, "trace.json")))["traceEvents"]
+    kern = sorted((e for e in events if e.get("cat") == "kernel"), key=lambda e: e["ts"])
+    cuts = [i for i, e in enumerate(kern) if "reverse_step_kernel" in e["name"]]
+    steps = [kern[a + 1:b + 1] for a, b in zip(cuts, cuts[1:])]  # full steps: after one reverse step up to the next
+    n = len(steps[0])
+    assert all(len(st) == n for st in steps), "steps of different kernel counts"
+    rec["by_position"] = [{"kernel": re.split(r"[<(]", re.sub(r"^(void )?seqdiff::", "", steps[0][i]["name"]))[0],
+                           "grid": steps[0][i]["args"]["grid"], "us": round(sum(st[i]["dur"] for st in steps) / len(steps), 2)}
+                          for i in range(n)]
 print(json.dumps(out, indent=1))
