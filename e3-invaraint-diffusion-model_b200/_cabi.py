@@ -69,6 +69,8 @@ PROTOTYPES = {
     "seqdiff_op_attention_train_bwd": (_i, [_i, _i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, C.c_float, _u64, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "seqdiff_op_layernorm": (_i, [_i, _i, _i, _vp, _vp, _vp, C.c_float, _vp, _vp, _vp, _vp]),
     "seqdiff_op_philox_u32": (_i, [_u64, _u64, _u32, _i, _i, _vp, _vp]),
+    "seqdiff_op_gemm_ex": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "seqdiff_op_attention_packed": (_i, [_i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
 }
 
 _LIB = None

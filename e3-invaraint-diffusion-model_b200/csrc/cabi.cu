@@ -475,4 +475,39 @@ int seqdiff_op_philox_u32(uint64_t seed, uint64_t graph_id0, uint32_t step, int 
   SD_GUARD_END
 }
 
+int seqdiff_op_gemm_ex(int precision, int M, int N, int K, const void* A, const void* W, const float* bias, const float* resid, const float* ln_stats,
+                       const float* ln_g, const float* ln_b, int epilogue, int out_f32, int split_k, void* C, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(A && W && bias && C, "null argument");
+  const int force_bn = ((precision >> 8) & 0xfff) | (((precision >> 20) & 1) << 16);
+  const int mode = precision & 0xff;
+  SD_CHECK(mode == SEQDIFF_BF16 || mode == SEQDIFF_FP16, "the tcgen05 GEMM forms exist for the 16-bit modes");
+  const int fmt = mode == SEQDIFF_FP16 ? 0 : 1;
+  const LnResid ln{reinterpret_cast<const float2*>(ln_stats), ln_g, ln_b};
+  return gemm_16(M, N, K, A, fmt, W, fmt, bias, resid, epilogue, C, out_f32 ? 2 : fmt, static_cast<cudaStream_t>(stream), force_bn,
+                 ln_stats ? &ln : nullptr, split_k);
+  SD_GUARD_END
+}
+
+int seqdiff_op_attention_packed(int precision, int B, int heads, int Lq, int Lk, const void* q, int ldq, const void* k, int ldk, const void* v,
+                                int ldv, const void* dist_emb, int P, const float* key_mask, int Lk_mask, const int* q_off, const int* k_off,
+                                const int* q_len, int q_rows, int k_rows, int kv_div, void* out, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(q && k && v && key_mask && out, "null argument");
+  SD_CHECK(q_off || (!k_off && !q_len && Lk_mask == Lk), "padded form (q_off NULL): no k_off / q_len, and the key-mask pitch is Lk");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const AttnPack pk{q_off, k_off, q_len, q_rows, k_rows, Lk_mask};
+  const AttnPack* pack = q_off ? &pk : nullptr;
+  if (precision == SEQDIFF_FP32)
+    return attention<float>(B, heads, Lq, Lk, static_cast<const float*>(q), ldq, static_cast<const float*>(k), ldk, static_cast<const float*>(v),
+                            ldv, static_cast<const float*>(dist_emb), P, key_mask, static_cast<float*>(out), s, pack, kv_div);
+  if (precision == SEQDIFF_FP16)
+    return attention<f16>(B, heads, Lq, Lk, static_cast<const f16*>(q), ldq, static_cast<const f16*>(k), ldk, static_cast<const f16*>(v), ldv,
+                          static_cast<const f16*>(dist_emb), P, key_mask, static_cast<f16*>(out), s, pack, kv_div);
+  SD_CHECK(precision == SEQDIFF_BF16, "bad precision");
+  return attention<bf16>(B, heads, Lq, Lk, static_cast<const bf16*>(q), ldq, static_cast<const bf16*>(k), ldk, static_cast<const bf16*>(v), ldv,
+                         static_cast<const bf16*>(dist_emb), P, key_mask, static_cast<bf16*>(out), s, pack, kv_div);
+  SD_GUARD_END
+}
+
 }  // extern "C"

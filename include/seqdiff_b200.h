@@ -317,6 +317,27 @@ SEQDIFF_API int seqdiff_op_layernorm(int precision, int M, int H, const float* i
                          float* out32, void* out16, float* stats, void* stream);
 /* Philox4x32-10 stream the sampler uses: out[n*20+j] = raw u32 for (seed, graph, residue, step, class) */
 SEQDIFF_API int seqdiff_op_philox_u32(uint64_t seed, uint64_t graph_id0, uint32_t step, int B, int L, uint32_t* out, void* stream);
+/* Every form of the 16-bit tcgen05 GEMM the model and the training step run (operator-level entry for tests).  precision: BF16 / FP16,
+ * with the tile bits of seqdiff_op_gemm (bn << 8, cta_pair << 20; 0 = the tuner / cost model).
+ *   ln_stats == NULL: C = epilogue(A W^T + bias) (+ resid), as seqdiff_op_gemm.
+ *   ln_stats != NULL: the residual is LayerNorm(resid) = (resid - mean) * rstd * ln_g + ln_b, rebuilt in the epilogue from the [M] (mean, rstd)
+ *   pairs seqdiff_op_layernorm writes to its `stats` argument (the decoder's residual GEMMs).
+ * out_f32: C is fp32 (implied by resid), else C has A's 16-bit type.  split_k (fp32 C, no residual, identity epilogue): 1 off, n > 1 k-ranges per
+ * output tile, -1 auto; the number of k-ranges is clamped to the k-blocks (K / 64 rounded up), and when more than one remains every k-range
+ * ADDS its partial product into C (bias added once) -- pre-zero C for C = A W^T + bias.  Illegal combinations: SEQDIFF_ERR_INVALID. */
+SEQDIFF_API int seqdiff_op_gemm_ex(int precision, int M, int N, int K, const void* A, const void* W, const float* bias, const float* resid,
+                                   const float* ln_stats, const float* ln_g, const float* ln_b, int epilogue, int out_f32, int split_k, void* C,
+                                   void* stream);
+/* The attention core of seqdiff_op_attention in its packed and shared-key forms (operator-level entry for tests).
+ *   q_off != NULL (16-bit modes): packed batch.  q_off / k_off / q_len are DEVICE arrays of B ints: graph b's query rows are q_off[b] ..
+ *   q_off[b] + q_len[b] - 1 of q (q_rows rows in all) and of out ([q_rows, heads*64]), its key rows start at k_off[b / kv_div] of k / v (k_rows
+ *   rows).  Lq / Lk are the largest query / key lengths; key_mask rows have the pitch Lk_mask >= Lk.  Output rows past q_len[b] are not written.
+ *   q_off == NULL: the padded layout of seqdiff_op_attention (k_off and q_len NULL, Lk_mask == Lk; q_rows / k_rows unused), every precision.
+ * kv_div >= 1, B % kv_div == 0: query graph b reads the keys, values and key-mask row of key graph b / kv_div. */
+SEQDIFF_API int seqdiff_op_attention_packed(int precision, int B, int heads, int Lq, int Lk, const void* q, int ldq, const void* k, int ldk,
+                                            const void* v, int ldv, const void* dist_emb, int P, const float* key_mask, int Lk_mask,
+                                            const int* q_off, const int* k_off, const int* q_len, int q_rows, int k_rows, int kv_div, void* out,
+                                            void* stream);
 
 #ifdef __cplusplus
 }

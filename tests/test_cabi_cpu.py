@@ -26,6 +26,51 @@ def test_library_exports_every_declared_symbol():
     assert lib.seqdiff_abi_version() == 1
 
 
+def test_operator_entry_points_reject_illegal_forms():
+    """seqdiff_op_gemm_ex / seqdiff_op_attention_packed reject the forms no kernel implements before anything reaches the device
+    (stand-in pointers, never dereferenced)"""
+    import ctypes
+    import seqdiff_b200 as sd
+    lib = sd.lib()
+    buf = ctypes.create_string_buffer(64)
+    p = ctypes.cast(buf, ctypes.c_void_p)
+    BF16, FP16, FP32 = 1, 2, 0
+    gemm_bad = {
+        "split-K with a residual": (BF16, p, None, None, None, 0, 1, 2),
+        "split-K into a 16-bit C": (BF16, None, None, None, None, 0, 0, 4),
+        "auto split-K into a 16-bit C": (FP16, None, None, None, None, 0, 0, -1),
+        "split-K with GELU": (BF16, None, None, None, None, 1, 1, 2),
+        "split_k = 0": (BF16, None, None, None, None, 0, 1, 0),
+        "LayerNorm residual without resid": (BF16, None, p, p, p, 0, 1, 1),
+        "LayerNorm residual without its affine": (BF16, p, p, None, p, 0, 1, 1),
+        "LayerNorm residual with split-K": (BF16, p, p, p, p, 0, 1, 3),
+        "residual into a 16-bit C": (BF16, p, None, None, None, 0, 0, 1),
+        "fp32 mode": (FP32, None, None, None, None, 0, 1, 1),
+    }
+    for what, (prec, resid, st, g, b, epi, out_f32, split) in gemm_bad.items():
+        rc = lib.seqdiff_op_gemm_ex(prec, 256, 768, 768, p, p, p, resid, st, g, b, epi, out_f32, split, p, None)
+        assert rc == 1, what  # SEQDIFF_ERR_INVALID
+        assert lib.seqdiff_last_error()
+
+    def attn(prec, B, kv_div, q_off=None, k_off=None, q_len=None, Lk_mask=64):
+        return lib.seqdiff_op_attention_packed(prec, B, 2, 64, 64, p, 384, p, 384, p, 384, None, 128, p, Lk_mask, q_off, k_off, q_len,
+                                               B * 64, B * 64, kv_div, p, None)
+    attn_bad = {
+        "a pack in fp32 mode": attn(FP32, 4, 1, p, p, p),
+        "B % kv_div != 0 (bf16, padded)": attn(BF16, 4, 3),
+        "B % kv_div != 0 (fp16, packed)": attn(FP16, 4, 3, p, p, p),
+        "B % kv_div != 0 (fp32)": attn(FP32, 4, 3),
+        "kv_div = 0": attn(BF16, 4, 0),
+        "a pack without k_off": attn(BF16, 4, 1, p, None, p),
+        "key-mask pitch below Lk": attn(BF16, 4, 1, p, p, p, Lk_mask=32),
+        "padded form with a pack array": attn(BF16, 4, 1, None, p, None),
+        "padded form with another mask pitch": attn(FP32, 4, 1, Lk_mask=128),
+    }
+    for what, rc in attn_bad.items():
+        assert rc == 1, what
+        assert lib.seqdiff_last_error()
+
+
 def test_state_dict_schema_is_the_reference_schema():
     import seqdiff_b200 as sd
     for L, rel in ((128, True), (64, True), (64, False)):
