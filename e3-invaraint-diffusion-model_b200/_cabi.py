@@ -57,6 +57,8 @@ PROTOTYPES = {
     "seqdiff_train_step": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_float, C.c_float, _u64, _u32, _vp, _vp, _vp, _vp]),
     "seqdiff_adamw_step": (_i, [_vp, _vp, _vp, _vp, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _i, _vp, _vp]),
     "seqdiff_model_get_tensor": (_i, [_vp, C.c_char_p, _vp, _i64, _vp]),
+    "seqdiff_struct_train_step": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_float, C.c_float, _u64, _u32, _vp, _vp, _vp, _vp]),
+    "seqdiff_struct_loss_terms": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp]),
     "seqdiff_struct_model_create": (_i, [C.POINTER(SeqdiffConfig), _i, C.POINTER(_vp)]),
     "seqdiff_struct_forward": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "seqdiff_struct_p_sample": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _u64, _u64, _i, _vp, _vp]),

@@ -229,6 +229,30 @@ int seqdiff_train_step(seqdiff_model_t* m, int precision, int B, int L_lig, int 
   SD_GUARD_END
 }
 
+int seqdiff_struct_train_step(seqdiff_model_t* m, int precision, int B, int L_lig, int L_rec, const float* timestep, const float* corrupted,
+                              const float* known_noise, const float* ligand_mask, const float* receptor_seq, const float* receptor_angles,
+                              const float* receptor_mask, float p_hidden, float p_attn, uint64_t seed, uint32_t step, float* grads_out,
+                              double* terms_out, float* pred_out, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(m && timestep && corrupted && known_noise && ligand_mask && receptor_seq && receptor_angles && receptor_mask && grads_out && terms_out,
+           "null argument");
+  StructTrainArgs a{};
+  a.precision = precision; a.B = B; a.Ll = L_lig; a.Lr = L_rec;
+  a.t = timestep; a.corrupted = corrupted; a.known_noise = known_noise; a.lig_mask = ligand_mask;
+  a.rec_seq = receptor_seq; a.rec_angle = receptor_angles; a.rec_mask = receptor_mask;
+  a.p_hidden = p_hidden; a.p_attn = p_attn; a.seed = seed; a.step = step;
+  a.grads = grads_out; a.terms = terms_out; a.pred_out = pred_out;
+  return m->impl.struct_train_step(a, static_cast<cudaStream_t>(stream));
+  SD_GUARD_END
+}
+
+int seqdiff_struct_loss_terms(int N, int F, const float* pred, const float* known_noise, const float* ligand_mask, double* terms, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(pred && known_noise && ligand_mask && terms, "null argument");
+  return angle_loss_terms(N, F, pred, known_noise, ligand_mask, terms, static_cast<cudaStream_t>(stream));
+  SD_GUARD_END
+}
+
 int seqdiff_adamw_step(seqdiff_model_t* m, const float* grads, float* exp_avg, float* exp_avg_sq, float grad_scale, float max_grad_norm, float lr,
                        float beta1, float beta2, float eps, float weight_decay, int step, float* grad_norm_out, void* stream) {
   SD_GUARD_BEGIN

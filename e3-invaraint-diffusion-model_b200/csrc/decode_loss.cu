@@ -184,33 +184,34 @@ __global__ void __launch_bounds__(kLossThreads) loss_terms_kernel(int N, const f
 }
 
 size_t loss_terms_scratch_bytes() { return (static_cast<size_t>(kLossMaxCtas) * kLossTerms + 2) * sizeof(double); }
+// per-CTA partials + arrival counter.  The training steps hand in scratch from their own workspace: a cudaMallocAsync per optimizer
+// step can stall the launching thread for milliseconds whenever the pool has been trimmed at a synchronisation (seen as 3 - 90 ms
+// gaps in front of this launch in the per-kernel profiles of the training step).  The stand-alone entry points keep stream-ordered
+// scratch, so concurrent calls on different streams never share it, with the pool told to keep what it has instead of returning it
+// to the OS at every synchronisation.
+static cudaError_t stream_scratch(double** out, size_t bytes, cudaStream_t s) {
+  static const bool pool_kept = [] {
+    int dev = 0;
+    cudaMemPool_t pool;
+    if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess) {
+      uint64_t keep = 64ull << 20;  // bytes the pool may hold across synchronisations (this scratch is 24 KB)
+      uint64_t cur = 0;
+      if (cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &cur) == cudaSuccess && cur < keep)
+        cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
+    }
+    cudaGetLastError();
+    return true;
+  }();
+  (void)pool_kept;
+  return cudaMallocAsync(reinterpret_cast<void**>(out), bytes, s);
+}
 int loss_terms(int N, const float* logits, const float* x0, const float* x_t, const float* mask, double* terms, cudaStream_t s, double* scratch_in) {
   SD_CHECK(N > 0, "empty loss");
   int ctas = ceil_div(N, kLossThreads);
   if (ctas > kLossMaxCtas) ctas = kLossMaxCtas;
   const size_t bytes = (static_cast<size_t>(ctas) * kLossTerms + 2) * sizeof(double);
-  // per-CTA partials + arrival counter.  The training step hands in scratch from its own workspace (loss_terms_scratch_bytes()): a
-  // cudaMallocAsync per optimizer step can stall the launching thread for milliseconds whenever the pool has been trimmed at a
-  // synchronisation (seen as 3 - 90 ms gaps in front of this launch in the per-kernel profiles of the training step).  The stand-alone
-  // entry point keeps stream-ordered scratch, so concurrent calls on different streams never share it, with the pool told to keep
-  // what it has instead of returning it to the OS at every synchronisation.
   double* scratch = scratch_in;
-  if (!scratch) {
-    static const bool pool_kept = [] {
-      int dev = 0;
-      cudaMemPool_t pool;
-      if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess) {
-        uint64_t keep = 64ull << 20;  // bytes the pool may hold across synchronisations (this scratch is 24 KB)
-        uint64_t cur = 0;
-        if (cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &cur) == cudaSuccess && cur < keep)
-          cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
-      }
-      cudaGetLastError();
-      return true;
-    }();
-    (void)pool_kept;
-    SD_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&scratch), bytes, s));
-  }
+  if (!scratch) SD_CUDA(stream_scratch(&scratch, bytes, s));
   unsigned* arrive = reinterpret_cast<unsigned*>(scratch + static_cast<size_t>(ctas) * kLossTerms);
   cudaError_t e = cudaMemsetAsync(arrive, 0, 2 * sizeof(double), s);
   if (e == cudaSuccess) e = launch_k(loss_terms_kernel, dim3(ctas), dim3(kLossThreads), 0, s, N, logits, x0, x_t, mask, scratch, arrive, terms);
@@ -218,6 +219,120 @@ int loss_terms(int N, const float* logits, const float* x0, const float* x_t, co
   SD_CUDA(e);
   SD_CUDA(ef);
   SD_LAUNCHED("loss_terms", s);
+  return SEQDIFF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Objective of the structure (angle) model: wrapped smooth-L1 on the predicted noise, per feature, over the valid ligand positions.
+//   d = wrap(known_noise - pred) into [-pi, pi);  h(d) = 0.5 d^2 / beta (|d| < beta), |d| - 0.5 beta otherwise;  beta = pi / 10.
+// terms[i] = sum of h over the valid positions of feature i (i < F), terms[F] = number of valid positions; loss = mean_i terms[i] / terms[F].
+__device__ __forceinline__ float wrap_angle(float v) {  // modulo_with_wrapped_range(v, -pi, pi) with the bounds as fp32 values (gauss_step.cu)
+  constexpr float kMin = -3.14159274101257324f, kTop = 6.28318548202514648f;
+  float m = fmodf(__fsub_rn(v, kMin), kTop);
+  if (m != 0.f && m < 0.f) m = __fadd_rn(m, kTop);
+  return __fadd_rn(m, kMin);
+}
+constexpr float kAngleBeta = 0.314159265358979f;
+
+template <int F>
+__global__ void __launch_bounds__(kLossThreads) angle_loss_terms_kernel(int N, const float* __restrict__ pred, const float* __restrict__ noise,
+                                                                        const float* __restrict__ mask, double* __restrict__ partial,
+                                                                        unsigned* __restrict__ arrive, double* __restrict__ terms) {
+  pdl_trigger();
+  pdl_wait();
+  constexpr int NT = F + 1;
+  double acc[NT];
+#pragma unroll
+  for (int k = 0; k < NT; ++k) acc[k] = 0.0;
+  for (int n = blockIdx.x * kLossThreads + threadIdx.x; n < N; n += gridDim.x * kLossThreads) {
+    if (mask[n] == 0.f) continue;
+    acc[F] += 1.0;
+#pragma unroll
+    for (int i = 0; i < F; ++i) {
+      const size_t e = static_cast<size_t>(n) * F + i;
+      const float d = wrap_angle(__fsub_rn(noise[e], pred[e]));
+      const float ad = fabsf(d);
+      acc[i] += ad < kAngleBeta ? 0.5f * d * d / kAngleBeta : ad - 0.5f * kAngleBeta;
+    }
+  }
+  // fixed-order reduction (deterministic run to run): warp shuffles, warps in order, then the last CTA folds the partials in CTA order
+  __shared__ double s_acc[kLossThreads / 32][NT];
+#pragma unroll
+  for (int k = 0; k < NT; ++k) {
+    double v = acc[k];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) s_acc[threadIdx.x >> 5][k] = v;
+  }
+  __syncthreads();
+  __shared__ bool s_last;
+  if (threadIdx.x < NT) {
+    double v = 0.0;
+    for (int w = 0; w < kLossThreads / 32; ++w) v += s_acc[w][threadIdx.x];
+    partial[static_cast<size_t>(blockIdx.x) * NT + threadIdx.x] = v;
+  }
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(arrive, 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (s_last) {
+    __threadfence();
+    if (threadIdx.x < NT) {
+      double v = 0.0;
+      for (unsigned c = 0; c < gridDim.x; ++c) v += reinterpret_cast<const volatile double*>(partial)[static_cast<size_t>(c) * NT + threadIdx.x];
+      terms[threadIdx.x] = v;
+    }
+    if (threadIdx.x == 0) *arrive = 0u;
+  }
+}
+
+// dL/dpred = -h'(d) / (F * n_valid) at valid positions, 0 elsewhere; h'(d) = d / beta or sign(d).  n_valid = terms[F], read on the
+// device (no host synchronisation); a batch without a valid position (n_valid = 0) gets a zero gradient.
+template <int F>
+__global__ void __launch_bounds__(256) angle_loss_bwd_kernel(int N, const float* __restrict__ pred, const float* __restrict__ noise,
+                                                             const float* __restrict__ mask, const double* __restrict__ terms,
+                                                             float* __restrict__ dpred) {
+  pdl_wait();
+  const double n_valid = terms[F];
+  const float scale = n_valid > 0.0 ? static_cast<float>(-1.0 / (static_cast<double>(F) * n_valid)) : 0.f;
+  for (int e = blockIdx.x * 256 + threadIdx.x; e < N * F; e += gridDim.x * 256) {
+    float g = 0.f;
+    if (mask[e / F] != 0.f) {
+      const float d = wrap_angle(__fsub_rn(noise[e], pred[e]));
+      g = scale * (fabsf(d) < kAngleBeta ? d / kAngleBeta : (d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f)));
+    }
+    dpred[e] = g;
+  }
+}
+
+size_t angle_loss_scratch_bytes() { return (static_cast<size_t>(kLossMaxCtas) * (kAngleMaxF + 1) + 2) * sizeof(double); }
+int angle_loss_terms(int N, int F, const float* pred, const float* noise, const float* mask, double* terms, cudaStream_t s, double* scratch_in) {
+  SD_CHECK(N > 0, "empty loss");
+  SD_CHECK(F == 8 || F == 20, "angle loss: feature_size must be 8 or 20");
+  int ctas = ceil_div(N, kLossThreads);
+  if (ctas > kLossMaxCtas) ctas = kLossMaxCtas;
+  const size_t bytes = (static_cast<size_t>(ctas) * (F + 1) + 2) * sizeof(double);
+  double* scratch = scratch_in;
+  if (!scratch) SD_CUDA(stream_scratch(&scratch, bytes, s));
+  unsigned* arrive = reinterpret_cast<unsigned*>(scratch + static_cast<size_t>(ctas) * (F + 1));
+  cudaError_t e = cudaMemsetAsync(arrive, 0, 2 * sizeof(double), s);
+  if (e == cudaSuccess) {
+    if (F == 8) e = launch_k(angle_loss_terms_kernel<8>, dim3(ctas), dim3(kLossThreads), 0, s, N, pred, noise, mask, scratch, arrive, terms);
+    else e = launch_k(angle_loss_terms_kernel<20>, dim3(ctas), dim3(kLossThreads), 0, s, N, pred, noise, mask, scratch, arrive, terms);
+  }
+  const cudaError_t ef = scratch_in ? cudaSuccess : cudaFreeAsync(scratch, s);
+  SD_CUDA(e);
+  SD_CUDA(ef);
+  SD_LAUNCHED("angle_loss_terms", s);
+  return SEQDIFF_OK;
+}
+int angle_loss_bwd(int N, int F, const float* pred, const float* noise, const float* mask, const double* terms, float* dpred, cudaStream_t s) {
+  SD_CHECK(N > 0, "empty loss");
+  SD_CHECK(F == 8 || F == 20, "angle loss: feature_size must be 8 or 20");
+  const int grid = ceil_div(N * F, 256);
+  if (F == 8) SD_CUDA(launch_k(angle_loss_bwd_kernel<8>, dim3(grid), dim3(256), 0, s, N, pred, noise, mask, terms, dpred));
+  else SD_CUDA(launch_k(angle_loss_bwd_kernel<20>, dim3(grid), dim3(256), 0, s, N, pred, noise, mask, terms, dpred));
+  SD_LAUNCHED("angle_loss_bwd", s);
   return SEQDIFF_OK;
 }
 

@@ -157,6 +157,15 @@ int decode_sequences(int B, int L, const float* final_seq, const float* true_seq
 int loss_terms(int N, const float* logits, const float* x0, const float* x_t, const float* mask, double* terms, cudaStream_t s,
                double* scratch = nullptr);  // scratch (optional): loss_terms_scratch_bytes() of caller-owned, stream-private memory
 size_t loss_terms_scratch_bytes();
+// Structure-model objective (wrapped smooth-L1 on the predicted noise, beta = pi / 10) over N rows of F in {8, 20} features:
+// terms [F + 1] = per-feature fp64 sums of the loss over the rows with mask != 0, then the number of such rows (fixed reduction order).
+// scratch (optional): angle_loss_scratch_bytes() of caller-owned, stream-private memory; else stream-ordered pool memory.
+constexpr int kAngleMaxF = 20;
+int angle_loss_terms(int N, int F, const float* pred, const float* noise, const float* mask, double* terms, cudaStream_t s,
+                     double* scratch = nullptr);
+size_t angle_loss_scratch_bytes();
+// d(mean over features of the per-feature mean loss)/d(pred) [N, F]; the row count is read from terms[F] on the device
+int angle_loss_bwd(int N, int F, const float* pred, const float* noise, const float* mask, const double* terms, float* dpred, cudaStream_t s);
 
 // ---- gauss_step.cu ----------------------------------------------------------------------------------
 // Gaussian reverse step + angle wrap of the structure model (structure_model/sample.py:92-101,139-141) on B graphs of
@@ -203,6 +212,7 @@ int ln_modulate_bwd(const float* dout, const float* in, int M, int H, bool affin
                     cudaStream_t s);
 int embed_bwd(const float* dout, const float* x, int M, int fin, int H, const float* Wt, const float* b, const float* gamma, float eps, DropSpec dr,
               float* dW, float* db, float* dgamma, float* dbeta, cudaStream_t s);
+// (F = 20: the amino-acid head; F = 8: the structure model's angle head)
 template <typename T>
 int predictor_tail_bwd(const float* dlogits, const T* y, int M, int H, const float* gamma, const float* beta, float eps, const float* W2, int F,
                        float* dy, float* dW2, float* db2, float* dgamma, float* dbeta, cudaStream_t s);

@@ -64,6 +64,18 @@ struct TrainArgs {
   float* logits_out; // optional [B, Ll, feature_size]
 };
 
+// arguments of one training step of the structure model (forward + wrapped smooth-L1 loss + backward)
+struct StructTrainArgs {
+  int precision, B, Ll, Lr;
+  const float *t, *corrupted, *known_noise, *lig_mask, *rec_seq, *rec_angle, *rec_mask;
+  float p_hidden, p_attn;
+  uint64_t seed;
+  uint32_t step;
+  float* grads;     // flat fp32 [train_param_count()], overwritten
+  double* terms;    // [feature_size + 1]: per-feature loss sums, then the number of valid ligand positions
+  float* pred_out;  // optional [B, Ll, feature_size]
+};
+
 struct Segment {  // a run of graphs sharing one padded length inside a token matrix
   int row0, B, L;
   const float* mask;
@@ -216,11 +228,14 @@ struct Model {
   size_t tws_bytes = 0;
   int build_slots();
   int64_t train_param_count();
+  int train_prologue(int precision, int B, int Ll, int Lr, float p_hidden, float p_attn, cudaStream_t s);
   int train_step(const TrainArgs& a, cudaStream_t s);
+  int struct_train_step(const StructTrainArgs& a, cudaStream_t s);
   int adamw(const float* grads, float* m, float* v, float grad_scale, float max_norm, float lr, float beta1, float beta2, float eps, float wd,
             int step, float* norm_out, cudaStream_t s);
   int get_tensor(const char* name, float* out, int64_t numel, cudaStream_t s);
   template <typename T> int train_t(int wfmt, const TrainArgs& a, cudaStream_t s);
+  template <typename T> int struct_train_t(const StructTrainArgs& a, cudaStream_t s);
 
   // structure_model/model.py:180-215.  phases: bit 0 = run the receptor branch, bit 1 = the ligand branch.  The receptor branch (embeddings,
   // receptor_emb, encoder, all decoder layers' cross K|V) depends on neither the timestep nor the ligand, so the sampling loop runs it

@@ -899,18 +899,19 @@ int embed_bwd(const float* dout, const float* x, int M, int fin, int H, const fl
 // AminoAcidPredictor tail backward (forward: predictor_tail_kernel): logits = LN(y; g, b) W2^T + b2
 // dlogits [M,F] fp32 -> dy [M,H] fp32; dW2 [F,H], db2 [F], dg [H], db [H] accumulated.
 // =====================================================================================================
-// F == 20 (the amino-acid head; seqdiff_train_step requires it).  A warp per row accumulating dW2 through F * H / 32 = 480 shared atomics
-// per lane was bound by them (284 us per launch at 16384 rows).  Here the eight warps of a CTA park LN(y) and dlogits of their rows in
-// shared memory, and after a barrier every THREAD owns H / 256 columns of dW2 for all 20 classes in registers (60 accumulators, plain FMAs
-// on conflict-free reads); dgamma / dbeta accumulate in per-warp registers and meet once per CTA (flush_feature_sums).
-template <typename T, int VPL>
-__global__ void __launch_bounds__(kTrThreads) predictor_tail_bwd20_kernel(const float* __restrict__ dlogits, const T* __restrict__ y, int M, int H,
+// F = 20 (the amino-acid head) or 8 (the structure model's angle head).  A warp per row accumulating dW2 through F * H / 32 = 480 shared
+// atomics per lane (F = 20) was bound by them (284 us per launch at 16384 rows).  Here the eight warps of a CTA park LN(y) and dlogits of
+// their rows in shared memory, and after a barrier every THREAD owns H / 256 columns of dW2 for all F outputs in registers (60 accumulators
+// at F = 20, plain FMAs on conflict-free reads); dgamma / dbeta accumulate in per-warp registers and meet once per CTA (flush_feature_sums).
+template <typename T, int F, int VPL>
+__global__ void __launch_bounds__(kTrThreads) predictor_tail_bwd_kernel(const float* __restrict__ dlogits, const T* __restrict__ y, int M, int H,
                                                                           const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
                                                                           const float* __restrict__ W2, float* __restrict__ dy,
                                                                           float* __restrict__ dW2, float* __restrict__ db2, float* __restrict__ dgamma,
                                                                           float* __restrict__ dbeta) {
   pdl_wait();
-  constexpr int F = 20, NW = kTrThreads / 32;
+  constexpr int NW = kTrThreads / 32;
+  static_assert(F <= 32, "one lane per output");
   extern __shared__ float smem[];
   float* sW = smem;                                   // [F][H]   W2
   float* sG = sW + static_cast<size_t>(F) * H;        // [2][H]   dgamma | dbeta (flush)
@@ -1015,13 +1016,13 @@ __global__ void __launch_bounds__(kTrThreads) predictor_tail_bwd20_kernel(const 
 template <typename T>
 int predictor_tail_bwd(const float* dlogits, const T* y, int M, int H, const float* gamma, const float* beta, float eps, const float* W2, int F,
                        float* dy, float* dW2, float* db2, float* dgamma, float* dbeta, cudaStream_t s) {
-  SD_CHECK(F == 20, "predictor_tail_bwd: feature_size must be 20");
+  SD_CHECK(F == 20 || F == 8, "predictor_tail_bwd: feature_size must be 20 or 8");
   const int need = ceil_div(M, kTrThreads / 32);
   const int grid = need < num_sms() ? need : num_sms();
-  const size_t smem = (static_cast<size_t>(20 + 2 + kTrThreads / 32) * H + (kTrThreads / 32) * 32 + 32) * sizeof(float);
-#define SD_PTB20_LAUNCH()                                                                                            \
+  const size_t smem = (static_cast<size_t>(F + 2 + kTrThreads / 32) * H + (kTrThreads / 32) * 32 + 32) * sizeof(float);
+#define SD_PTB_LAUNCH_(F_)                                                                                           \
   {                                                                                                                  \
-    auto kfn = predictor_tail_bwd20_kernel<T, VPL>;                                                                  \
+    auto kfn = predictor_tail_bwd_kernel<T, F_, VPL>;                                                                \
     static bool configured = false;                                                                                  \
     if (!configured) {                                                                                               \
       SD_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));                   \
@@ -1029,8 +1030,10 @@ int predictor_tail_bwd(const float* dlogits, const T* y, int M, int H, const flo
     }                                                                                                                \
     SD_CUDA(launch_k(kfn, dim3(grid), dim3(kTrThreads), smem, s, dlogits, y, M, H, gamma, beta, eps, W2, dy, dW2, db2, dgamma, dbeta)); \
   }
-  SD_VPL_DISPATCH(H, SD_PTB20_LAUNCH());
-#undef SD_PTB20_LAUNCH
+#define SD_PTB_LAUNCH() if (F == 20) SD_PTB_LAUNCH_(20) else SD_PTB_LAUNCH_(8)
+  SD_VPL_DISPATCH(H, SD_PTB_LAUNCH());
+#undef SD_PTB_LAUNCH_
+#undef SD_PTB_LAUNCH
   SD_LAUNCHED("predictor_tail_bwd", s);
   return SEQDIFF_OK;
 }

@@ -321,7 +321,41 @@ def loss_terms(logits, x0, x_t, ligand_mask):
     return out
 
 
-class PeptideDiff(ConditionalBertForDiffusionBase):
+class _FlatTraining:
+    """The optimizer side shared by the trainable models (PeptideDiff, structure_model.ConditionalBertForDiffusion): the handle's flat
+    parameter space, the fused clip + AdamW step and the copy of the trained masters back into the module."""
+
+    def _flat_params(self):
+        from . import train as _train
+        if getattr(self, "_flat", None) is None or self._flat.handle is not self._handle:
+            self._sync_handle()
+            self._flat = _train.FlatParams(self)
+        return self._flat
+
+    def configure_optimizers(self, group=None, grad_comm: str = "fp32"):
+        """reference model.py:416-450: AdamW(lr, weight_decay=l2_lambda) over all parameters -- here the fused clip + AdamW kernel
+        over the handle's flat parameter space, with the data-parallel gradient all-reduce in front of it.  The LinearWarmup
+        schedule (stepped per epoch, as Lightning does with interval="epoch") is applied by train.fit()."""
+        from . import train as _train
+        if self.lr_scheduler not in (None, "OneCycleLR", "LinearWarmup"):
+            raise ValueError(f"Unknown lr scheduler {self.lr_scheduler}")
+        if getattr(self, "_optimizer", None) is None or self._optimizer.flat is not self._flat_params():
+            self._optimizer = _train.FlatAdamW(self._flat_params(), lr=self.lr, weight_decay=self.l2_lambda,
+                                               gradient_clip=getattr(self, "gradient_clip", 1.0), group=group, grad_comm=grad_comm)
+        return {"optimizer": self._optimizer}
+
+    def pull_weights(self):
+        """copies the trained masters from the C handle back into this module's parameters (state_dict / checkpoints)."""
+        from . import train as _train
+        _train.pull_weights(self)
+
+    def state_dict(self, *a, **kw):
+        if getattr(self, "_weights_dirty", False):
+            self.pull_weights()
+        return super().state_dict(*a, **kw)
+
+
+class PeptideDiff(_FlatTraining, ConditionalBertForDiffusionBase):
     """reference model.py:256-450 without the Lightning base class (Trainer is out of scope, SURVEY.md
     section 2).  Inference-side members match the reference; `apply_aa_noise` runs the CUDA q-sample
     kernel; `get_loss` evaluates the reference's loss terms with the CUDA forward and the CUDA reduction
@@ -404,13 +438,6 @@ class PeptideDiff(ConditionalBertForDiffusionBase):
         return torch.mean(loss)
 
     # ---- training (BASELINE configs[3]) ----------------------------------------------------------
-    def _flat_params(self):
-        from . import train as _train
-        if getattr(self, "_flat", None) is None or self._flat.handle is not self._handle:
-            self._sync_handle()
-            self._flat = _train.FlatParams(self)
-        return self._flat
-
     def training_step(self, batch, batch_idx, t_int=None, noise_E=None):
         """reference model.py:347-367.  Draws t (torch.randint, as the reference), q-samples x_t on the GPU, then runs forward
         (dropout active in train() mode) + get_loss + the FULL backward in one C call: the gradients of the 61.06 M live
@@ -436,25 +463,3 @@ class PeptideDiff(ConditionalBertForDiffusionBase):
         self.last_log = {"aa_noise_rate": aa_noise_rate, "aa_recovery_rate": aa_recovery_rate, "avg_timestep": t_int.mean().int(),
                          "train_loss": loss, "train_aa_noised_loss": aa_noised_loss, "train_aa_all_loss": aa_all_loss, "train_elbo_loss": elbo}
         return loss
-
-    def configure_optimizers(self, group=None, grad_comm: str = "fp32"):
-        """reference model.py:416-450: AdamW(lr, weight_decay=l2_lambda) over all parameters -- here the fused clip + AdamW kernel
-        over the handle's flat parameter space, with the data-parallel gradient all-reduce in front of it.  The LinearWarmup
-        schedule (stepped per epoch, as Lightning does with interval="epoch") is applied by train.fit()."""
-        from . import train as _train
-        if self.lr_scheduler not in (None, "OneCycleLR", "LinearWarmup"):
-            raise ValueError(f"Unknown lr scheduler {self.lr_scheduler}")
-        if getattr(self, "_optimizer", None) is None or self._optimizer.flat is not self._flat_params():
-            self._optimizer = _train.FlatAdamW(self._flat_params(), lr=self.lr, weight_decay=self.l2_lambda,
-                                               gradient_clip=getattr(self, "gradient_clip", 1.0), group=group, grad_comm=grad_comm)
-        return {"optimizer": self._optimizer}
-
-    def pull_weights(self):
-        """copies the trained masters from the C handle back into this module's parameters (state_dict / checkpoints)."""
-        from . import train as _train
-        _train.pull_weights(self)
-
-    def state_dict(self, *a, **kw):
-        if getattr(self, "_weights_dirty", False):
-            self.pull_weights()
-        return super().state_dict(*a, **kw)

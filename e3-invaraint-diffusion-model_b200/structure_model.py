@@ -19,7 +19,7 @@ from torch.nn import functional as F
 from . import _cabi
 from .sample import check_num_samples
 from .model import (BertEmbeddings, BertEncoder, ConditionalBertForDiffusionBase as _SeqBase, GaussianFourierProjection, SELayer,
-                    _Container, _BertLayer, BertAttention, _Intermediate, _SelfOutput)
+                    _Container, _BertLayer, BertAttention, _FlatTraining, _Intermediate, _SelfOutput)
 
 SEED = 0          # Philox seed of the in-kernel N(0,1) stream (explicit `noise` tensors override it)
 STEP = 1          # structure_model/sample.py:14; only the reference default is implemented
@@ -170,7 +170,82 @@ class ConditionalBertForDiffusionBase(_SeqBase):
         return out
 
 
-ConditionalBertForDiffusion = ConditionalBertForDiffusionBase  # the Lightning wrapper (model.py:232-403) adds training only
+def _check_valid_ligand(mask):
+    if not bool((mask != 0).any()):
+        raise ValueError("the batch has no valid ligand position (ligand_attn_mask is all zero): its loss is undefined")
+
+
+def angle_loss_terms(pred, known_noise, ligand_mask):
+    """The F+1 fp64 reduction terms of the structure model's objective (include/seqdiff_b200.h: seqdiff_struct_loss_terms) as a device
+    tensor: per-feature sums of the wrapped smooth-L1 over the valid ligand positions, then their count."""
+    dev = pred.device
+    if dev.type != "cuda":
+        raise RuntimeError("angle_loss_terms runs only on a CUDA device (no CPU fallback)")
+    Fs = pred.shape[-1]
+    pr = pred.to(dtype=torch.float32).reshape(-1, Fs).contiguous()
+    kn = known_noise.to(device=dev, dtype=torch.float32).reshape(-1, Fs).contiguous()
+    m = ligand_mask.to(device=dev, dtype=torch.float32).reshape(-1).contiguous()
+    if not (pr.shape[0] == kn.shape[0] == m.shape[0]):
+        raise ValueError("pred, known_noise and ligand_mask must cover the same positions")
+    out = torch.empty(Fs + 1, device=dev, dtype=torch.float64)
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _cabi.check(_cabi.lib().seqdiff_struct_loss_terms(pr.shape[0], Fs, _cabi.ptr(pr), _cabi.ptr(kn), _cabi.ptr(m), _cabi.ptr(out), stream))
+    return out
+
+
+class ConditionalBertForDiffusion(_FlatTraining, ConditionalBertForDiffusionBase):
+    """reference structure_model/model.py:232-403 without the Lightning base class: the angle denoiser plus its training step.
+    `training_step` runs forward (dropout active in train() mode) + the wrapped smooth-L1 loss + the full hand-written backward
+    (csrc/train.cu) in one C call; `configure_optimizers` returns the fused clip + AdamW step over the handle's flat parameter space
+    (train.py), so `train.fit` trains this model as it trains PeptideDiff.  Only loss="smooth_l1" is implemented."""
+
+    def __init__(self, encoder_config, decoder_config, feature_size: int, *, loss: str = "smooth_l1", learning_rate: float = 5e-5,
+                 l2_lambda: float = 0.0, lr_scheduler=None, max_epochs: int = 1, gradient_clip: float = 1.0) -> None:
+        if loss != "smooth_l1":
+            raise ValueError(f"only the 'smooth_l1' objective is implemented in CUDA, got {loss!r}")
+        ConditionalBertForDiffusionBase.__init__(self, encoder_config, decoder_config, feature_size)
+        self.loss = loss
+        self.lr = learning_rate
+        self.l2_lambda = l2_lambda
+        self.lr_scheduler = lr_scheduler
+        self.max_epochs = max_epochs
+        self.gradient_clip = gradient_clip
+        self._noise_seed = 0
+
+    def training_step(self, batch, batch_idx):
+        """One optimizer step's forward + loss + backward on a NoisedAnglesDataset batch (corrupted, t, known_noise and the keys
+        sample() reads).  The gradients land in the flat buffer `self._flat.grads`, ready for `configure_optimizers()["optimizer"].step()`.
+        Returns the loss (device scalar); the per-feature losses are kept in `self.last_log`."""
+        from . import train as _train
+        _check_valid_ligand(batch["ligand_attn_mask"])
+        flat = self._flat_params()
+        self._train_steps = getattr(self, "_train_steps", 0) + 1
+        opt = getattr(self, "_optimizer", None)
+        if opt is not None and opt.flat is flat:
+            opt.arm_overlap()
+        terms, _ = _train.struct_train_step_tensors(self, flat, batch, seed=self._noise_seed, step=self._train_steps)
+        if opt is not None and opt.flat is flat:
+            opt.launch_overlapped_all_reduce()  # bucket k's all-reduce starts when the backward pass has finished bucket k
+        loss, per_feature = _train.angle_loss_from_terms(terms)
+        self.last_log = {"train_loss": loss, "train_loss_per_feature": per_feature}
+        return loss
+
+    @torch.no_grad()
+    def validation_step(self, batch, batch_idx):
+        """The same objective on the eval-mode (dropout-free) forward; returns the loss (device scalar), per-feature losses in `last_log`."""
+        from . import train as _train
+        _check_valid_ligand(batch["ligand_attn_mask"])
+        was_training = self.training
+        self.eval()
+        try:
+            pred = self.forward(batch["t"], batch["corrupted"], batch["ligand_attn_mask"], batch["receptor_seq"], batch["receptor_angles"],
+                                batch["receptor_attn_mask"])
+        finally:
+            self.train(was_training)
+        loss, per_feature = _train.angle_loss_from_terms(angle_loss_terms(pred, batch["known_noise"], batch["ligand_attn_mask"]))
+        self.last_log = {"val_loss": loss, "val_loss_per_feature": per_feature}
+        return loss
 
 
 # ---- structure_model/sample.py -------------------------------------------------------------------------------------

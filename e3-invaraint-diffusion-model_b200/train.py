@@ -227,6 +227,43 @@ def train_step_tensors(model, flat: FlatParams, batch, t_norm, noised_ligand_seq
     return terms, logits
 
 
+def struct_train_step_tensors(model, flat: FlatParams, batch, p_hidden=None, p_attn=None, seed=0, step=0, want_pred=False):
+    """forward + wrapped smooth-L1 loss + backward of one (local) batch of the structure model (structure_model.ConditionalBertForDiffusion):
+    fills flat.grads, returns (terms [F+1] f64 device tensor: per-feature loss sums, then the number of valid ligand positions; the
+    prediction [B,L,F] or None).  `batch`: the NoisedAnglesDataset dict (corrupted, t, known_noise, ligand_attn_mask, receptor_seq,
+    receptor_angles, receptor_attn_mask); t is the integer step, unnormalised."""
+    dev = flat.device
+    cfg = model.decoder_config
+    p_h = float(getattr(cfg, "hidden_dropout_prob", 0.0)) if p_hidden is None else float(p_hidden)
+    p_a = float(getattr(cfg, "attention_probs_dropout_prob", 0.0)) if p_attn is None else float(p_attn)
+    if not model.training:
+        p_h = p_a = 0.0
+    h = model._sync_handle()
+    B, Ll, Lr, x, lm, rs, ra, rm = model._inputs(batch["corrupted"], batch["ligand_attn_mask"], batch["receptor_seq"], batch["receptor_angles"],
+                                                batch["receptor_attn_mask"])
+    Fs = model.feature_size
+    noise = batch["known_noise"].to(device=dev, dtype=torch.float32).contiguous()
+    if tuple(noise.shape) != (B, Ll, Fs):
+        raise ValueError(f"known_noise must be {(B, Ll, Fs)}, got {tuple(noise.shape)}")
+    t = batch["t"].to(device=dev, dtype=torch.float32).reshape(-1).contiguous()
+    if t.numel() != B:
+        raise ValueError("t must hold one step per graph")
+    terms = torch.empty(Fs + 1, device=dev, dtype=torch.float64)
+    pred = torch.empty((B, Ll, Fs), device=dev, dtype=torch.float32) if want_pred else None
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        p = _cabi.ptr
+        _cabi.check(_cabi.lib().seqdiff_struct_train_step(h, model._precision_code(), B, Ll, Lr, p(t), p(x), p(noise), p(lm), p(rs), p(ra), p(rm),
+                                                          p_h, p_a, int(seed), int(step) & 0xFFFFFFFF, p(flat.grads), p(terms), p(pred), stream))
+    return terms, pred
+
+
+def angle_loss_from_terms(terms):
+    """(total loss, per-feature losses) of the structure model's objective from its F+1 reduction terms (device tensors, fp32)."""
+    per_feature = (terms[:-1] / terms[-1]).float()
+    return per_feature.mean(), per_feature
+
+
 def loss_from_terms(terms):
     """the 6-tuple of PeptideDiff.get_loss (model.py:345) from the ten reduction terms."""
     n_mask, n_noised, n_sel, n_same, n_rec, ce_noised, ce_sel, ent, kl = (terms[i] for i in range(9))

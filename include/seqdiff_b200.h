@@ -285,6 +285,29 @@ SEQDIFF_API int seqdiff_struct_sample_multi(seqdiff_model_t* m, int precision, i
                                 const float* receptor_angles, const float* receptor_mask, const float* noise_steps, uint64_t seed,
                                 uint64_t graph_id0, int flags, float* steps_out, float* final_out, void* stream);
 
+/* ==== structure-model training step: replaces autograd over ConditionalBertForDiffusion.training_step (structure_model/model.py)
+ * The flat parameter space, the gradient buckets and the optimizer are those of the sequence model's step: seqdiff_train_param_count /
+ * _param_table / _grad_buckets / _set_bucket_events, seqdiff_adamw_step and seqdiff_model_get_tensor accept a structure handle.  Trainable
+ * tensors = its state_dict minus the `timestep_projector.W` buffer, in forward order: receptor_seq_emb, receptor_angle_emb, receptor_emb,
+ * encoder layers, the fused cross K | V of every decoder layer, ligand_angle_emb, timestep_emb, decoder layers, angles_predictor.
+ * Buckets (NL >= 2): [decoder second half + head] is final first, then [cross K | V + ligand_angle_emb + timestep_emb + decoder first
+ * half], [encoder second half], [receptor embeddings + receptor_emb + encoder first half].
+ *
+ * Objective (FoldingDiff's, which the reference inherits): d = wrap(known_noise - pred) into [-pi, pi), h = smooth-L1 with beta = pi/10;
+ * loss = mean over the F features of (mean of h over the positions with ligand_mask != 0).
+ * timestep [B] = the integer step as float (unnormalised, as the sampler passes it); corrupted, known_noise [B,L_lig,F]; masks and
+ * receptor tensors as seqdiff_struct_forward.  p_hidden / p_attn, seed and step: dropout as in seqdiff_train_step.
+ * grads_out: flat fp32 [param_count], overwritten.  terms_out: double[F+1] on the device = per-feature sums of h over the valid positions,
+ * then the number of valid positions.  pred_out (optional) [B,L_lig,F].  F in {8, 20}; L_lig, L_rec <= 128 and B*L % 8 == 0.
+ * A batch without a valid ligand position is an input error the caller must reject: it gives zero gradients and a count of 0. */
+SEQDIFF_API int seqdiff_struct_train_step(seqdiff_model_t* m, int precision, int B, int L_lig, int L_rec, const float* timestep,
+                              const float* corrupted, const float* known_noise, const float* ligand_mask, const float* receptor_seq,
+                              const float* receptor_angles, const float* receptor_mask, float p_hidden, float p_attn, uint64_t seed,
+                              uint32_t step, float* grads_out, double* terms_out, float* pred_out, void* stream);
+/* the loss terms above (terms[F+1]) for N rows of already computed predictions pred [N,F] (evaluation: validation_step) */
+SEQDIFF_API int seqdiff_struct_loss_terms(int N, int F, const float* pred, const float* known_noise, const float* ligand_mask, double* terms,
+                              void* stream);
+
 /* ---- operator-level entry points (used by the parity tests and the micro benchmarks) --------------
  * C[M,N] = epilogue(A[M,K] * W[N,K]^T + bias[N] (+ resid[M,N])); epilogue: 0 none, 1 erf-GELU, 2 SiLU.
  * precision FP32: all f32 (SIMT kernel).  BF16 / FP16: A and W are 16-bit in the mode's formats
