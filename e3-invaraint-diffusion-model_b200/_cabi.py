@@ -47,6 +47,7 @@ PROTOTYPES = {
     "seqdiff_sample": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _u64, _u64, _vp, _vp]),
     "seqdiff_sample_ex": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _u64, _u64, _i, _vp, _vp]),
     "seqdiff_sample_multi": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _u64, _u64, _i, _vp, _vp]),
+    "seqdiff_score_multi": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u64, _i, _vp, _vp]),
     "seqdiff_decode": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "seqdiff_loss_terms": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "seqdiff_train_param_count": (_i64, [_vp]),

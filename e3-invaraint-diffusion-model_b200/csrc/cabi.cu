@@ -298,6 +298,23 @@ int seqdiff_sample_multi(seqdiff_model_t* m, int precision, int P, int K, int L_
   SD_GUARD_END
 }
 
+int seqdiff_score_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T, const float* q_tables_steps,
+                        const float* x0, const float* ligand_angle, const float* ligand_mask, const float* receptor_seq,
+                        const float* receptor_angle, const float* receptor_mask, const float* noise_E_steps, uint64_t seed, uint64_t graph_id0,
+                        int flags, double* terms_out, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(m && q_tables_steps && x0 && ligand_angle && ligand_mask && receptor_seq && receptor_angle && receptor_mask && terms_out,
+           "null argument");
+  SD_CHECK(P >= 1 && K >= 1 && T >= 1, "need at least one pocket, one sample per pocket and one step");
+  SD_CHECK(L_lig > 0 && L_rec > 0 && static_cast<int64_t>(P) * K * (L_lig > L_rec ? L_lig : L_rec) <= INT32_MAX,
+           "pockets x samples x length overflows the row counts");
+  SD_CHECK((flags & ~1) == 0, "unknown scoring flag");
+  SD_CHECK(m->impl.cfg.feature_size == SEQDIFF_NUM_CLASSES, "scoring needs feature_size == 20");
+  return m->impl.score(precision, P, K, L_lig, L_rec, T, q_tables_steps, x0, ligand_angle, ligand_mask, receptor_seq, receptor_angle,
+                       receptor_mask, noise_E_steps, seed, graph_id0, terms_out, static_cast<cudaStream_t>(stream), flags);
+  SD_GUARD_END
+}
+
 int seqdiff_struct_model_create(const seqdiff_config_t* cfg, int device, seqdiff_model_t** out) {
   SD_GUARD_BEGIN
   SD_CHECK(cfg != nullptr && out != nullptr, "null argument");

@@ -144,8 +144,14 @@ int reverse_step(const float* q_tables, int n_tab, int B, int L, const float* x_
 // rng != NULL: device pointer to (seed, graph_id0), overriding the by-value arguments (kernel parameters are frozen into a captured
 // CUDA graph; device memory is not, so one cached graph serves calls with different seeds / graph offsets).
 // In-place contract: x_s may alias x_t (the loop does that) -- every thread reads its own 20-float row completely before writing it.
+// step_ptr != NULL (scoring loop, with rng): qtb is the [T,3,20,20] step-table array and step k = *step_ptr draws from its Qtb (shared by
+// the B graphs), noise_E (optional) is [T, B*L, 20] and read at entry k, the Philox step is k.  The counter is not advanced.
 int apply_aa_noise(const float* qtb, int B, int L, const float* x0, const float* noise_E, uint64_t seed, uint64_t graph_id0,
-                   uint32_t step, float* x_t, uint8_t* idx_out, cudaStream_t s);
+                   uint32_t step, float* x_t, uint8_t* idx_out, cudaStream_t s, const int* step_ptr = nullptr, const uint64_t* rng = nullptr);
+// Terms of step k = *step_ptr of the scoring loop's bound (see vlb_terms_kernel): acc [B*L, 2] fp64 += (kl_k or, at k = 0, the
+// reconstruction term; ce_k) at the positions with mask != 0; the last CTA to read the counter decrements it (advance as in reverse_step).
+int vlb_terms(const float* q_tables, int B, int L, const float* x0, const float* x_t, const float* logits, const float* mask,
+              const int* step_ptr, int* advance, double* acc, cudaStream_t s);
 int philox_u32(uint64_t seed, uint64_t graph_id0, uint32_t step, int B, int L, uint32_t* out, cudaStream_t s);
 
 // ---- decode_loss.cu ---------------------------------------------------------------------------------

@@ -229,6 +229,7 @@ __global__ void arm_loop_kernel(int* step, int v, uint64_t* rng, uint64_t seed, 
 // =====================================================================================================
 Model::~Model() {
   if (graph_exec) cudaGraphExecDestroy(graph_exec);
+  if (score_exec) cudaGraphExecDestroy(score_exec);
   if (loop_stream) cudaStreamDestroy(loop_stream);
   if (ev_in) cudaEventDestroy(ev_in);
   if (ev_out) cudaEventDestroy(ev_out);
@@ -237,6 +238,7 @@ Model::~Model() {
   if (ws) { debug_guard_begin(ws); cudaFree(ws); }
   if (samp_in) { debug_guard_begin(samp_in); cudaFree(samp_in); }
   if (samp_inv) { debug_guard_begin(samp_inv); cudaFree(samp_inv); }
+  if (score_in) { debug_guard_begin(score_in); cudaFree(score_in); }
   if (d_tables) cudaFree(d_tables);
   if (d_pack) cudaFree(d_pack);
   if (tws) { debug_guard_begin(tws); cudaFree(tws); }
@@ -473,6 +475,11 @@ int Model::finalize(cudaStream_t s) {
       cudaGraphExecDestroy(graph_exec);
       graph_exec = nullptr;
       graph_key = GraphKey();
+    }
+    if (score_exec) {
+      cudaGraphExecDestroy(score_exec);
+      score_exec = nullptr;
+      score_key = GraphKey();
     }
     if (!packed_allocs.empty()) {  // re-finalize after a weight upload: drop the previous packed copies
       SD_CUDA(cudaDeviceSynchronize());
@@ -1159,9 +1166,9 @@ int Model::build_pack(int B, int K, int Ll, int Lr, const float* lig_mask, const
   return SEQDIFF_OK;
 }
 
-int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
-                  const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, int diverse,
-                  const float* noise_E, uint64_t seed, uint64_t gid0, float* final_out, cudaStream_t caller, int flags) {
+int Model::loop_setup(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_in, const float* lig_angle,
+                      const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, cudaStream_t caller,
+                      int flags, bool scoring, LoopIO* io, cudaStream_t* ls) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
   SD_CHECK(T >= 1 && P > 0 && K > 0 && Ll > 0 && Lr > 0, "bad sampling arguments");
   const int B = P * K;  // ligand graphs: sample j of pocket p is graph p * K + j
@@ -1174,6 +1181,7 @@ int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const floa
   }
   // everything below runs on the private stream, ordered after the caller's prior work ...
   cudaStream_t s = loop_stream;
+  *ls = s;
   SD_CUDA(cudaEventRecord(ev_in, caller));
   SD_CUDA(cudaStreamWaitEvent(s, ev_in, 0));
   const size_t Nl = static_cast<size_t>(B) * Ll, Nr = static_cast<size_t>(P) * Lr;
@@ -1193,28 +1201,40 @@ int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const floa
   }
   SD_TRY(ensure_workspace(workspace_need(precision, B, Ll, Lr)));
   Bump bp(samp_in, s);
-  float* x_cur = bp.take<float>(Nl * 20);
-  float* logits = bp.take<float>(Nl * 20);
-  float* c_lang = bp.take<float>(Nl * 8);
-  float* c_lmask = bp.take<float>(Nl);
-  float* c_rseq = bp.take<float>(Nr * 20);
-  float* c_rang = bp.take<float>(Nr * 8);
-  float* c_rmask = bp.take<float>(Nr);
+  io->x_cur = bp.take<float>(Nl * 20);
+  io->logits = bp.take<float>(Nl * 20);
+  io->c_lang = bp.take<float>(Nl * 8);
+  io->c_lmask = bp.take<float>(Nl);
+  io->c_rseq = bp.take<float>(Nr * 20);
+  io->c_rang = bp.take<float>(Nr * 8);
+  io->c_rmask = bp.take<float>(Nr);
+  if (scoring) {  // x0 | fp64 sums in a block of their own: scoring never moves the sampler's buffers (its cached graph stays valid)
+    const size_t need_sc = align256(Nl * 20 * 4) + align256(Nl * 2 * 8) + 4 * kGuardBytes;
+    if (need_sc > score_in_bytes) {
+      if (score_in) { SD_CUDA(cudaDeviceSynchronize()); debug_guard_begin(score_in); SD_CUDA(cudaFree(score_in)); score_in = nullptr; score_in_bytes = 0; }
+      SD_CUDA(cudaMalloc(reinterpret_cast<void**>(&score_in), need_sc));
+      score_in_bytes = need_sc;
+    }
+    Bump bs(score_in, s);
+    io->x0 = bs.take<float>(Nl * 20);
+    io->acc = bs.take<double>(Nl * 2);
+  }
   SD_CUDA(cudaMemcpyAsync(d_tables, q_tables, tab_floats * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(x_cur, x_T, Nl * 20 * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_lang, lig_angle, Nl * 8 * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_lmask, lig_mask, Nl * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_rseq, rec_seq_in, Nr * 20 * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_rang, rec_angle, Nr * 8 * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_rmask, rec_mask, Nr * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(scoring ? io->x0 : io->x_cur, x_in, Nl * 20 * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_lang, lig_angle, Nl * 8 * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_lmask, lig_mask, Nl * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_rseq, rec_seq_in, Nr * 20 * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_rang, rec_angle, Nr * 8 * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_rmask, rec_mask, Nr * 4, cudaMemcpyDefault, s));
+  if (scoring) SD_CUDA(cudaMemsetAsync(io->acc, 0, Nl * 2 * 8, s));
   // ragged packing (flags bit 0): valid prefixes only; needs the 16-bit kernels and prefix masks, otherwise the padded path runs
   const PackInfo* pk = nullptr;
   if ((flags & 1) && precision != SEQDIFF_FP32) {
     bool usable = false;
-    SD_TRY(build_pack(B, K, Ll, Lr, c_lmask, c_rmask, s, &usable));
+    SD_TRY(build_pack(B, K, Ll, Lr, io->c_lmask, io->c_rmask, s, &usable));
     if (usable) {
       pk = &pack;
-      SD_CUDA(cudaMemsetAsync(logits, 0, Nl * 20 * 4, s));  // padded positions are never written in packed mode: defined as 0
+      SD_CUDA(cudaMemsetAsync(io->logits, 0, Nl * 20 * 4, s));  // padded positions are never written in packed mode: defined as 0
     }
   }
   // padded path, 16-bit modes: the receptor rows are still packed (PackInfo::lig_padded), since no output reads a padded one.  It
@@ -1222,11 +1242,12 @@ int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const floa
   // keys, whose values are then read.  Otherwise (and in fp32 mode) every receptor row is computed.
   if (!pk && precision != SEQDIFF_FP32) {
     bool usable = false;
-    SD_TRY(build_pack(B, K, Ll, Lr, nullptr, c_rmask, s, &usable, true));
+    SD_TRY(build_pack(B, K, Ll, Lr, nullptr, io->c_rmask, s, &usable, true));
     if (usable) pk = &pack;
   }
-
+  io->pk = pk;
   const long long rows = pk ? static_cast<long long>(pk->Ml) + pk->Mr : static_cast<long long>(Nl + Nr);  // token rows of a step
+  io->rows = rows;
   // The per-sampling invariants (LoopInv), computed here by every call, outside the graph: the graph only holds their addresses.
   // Receptor rows first (P * Lr, the packed rows are a prefix), then the step tables with a grow-only capacity, so a cached graph
   // serves any T up to it.
@@ -1250,50 +1271,104 @@ int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const floa
     inv.mod = bi.take<uint8_t>(tH * 6 * es);
     const PdlScope pdl_scope(pdl_auto_mode(rows));
     switch (precision) {
-      case SEQDIFF_FP32: SD_TRY(loop_invariants_t<float>(1, B, K, Ll, Lr, T, c_rseq, c_rmask, inv, s, nullptr)); break;
-      case SEQDIFF_BF16: SD_TRY(loop_invariants_t<bf16>(1, B, K, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
-      default: SD_TRY(loop_invariants_t<f16>(0, B, K, Ll, Lr, T, c_rseq, c_rmask, inv, s, pk)); break;
+      case SEQDIFF_FP32: SD_TRY(loop_invariants_t<float>(1, B, K, Ll, Lr, T, io->c_rseq, io->c_rmask, inv, s, nullptr)); break;
+      case SEQDIFF_BF16: SD_TRY(loop_invariants_t<bf16>(1, B, K, Ll, Lr, T, io->c_rseq, io->c_rmask, inv, s, pk)); break;
+      default: SD_TRY(loop_invariants_t<f16>(0, B, K, Ll, Lr, T, io->c_rseq, io->c_rmask, inv, s, pk)); break;
     }
   }
-
-  GraphKey key;
+  GraphKey& key = io->key;
   key.pack_hash = pk ? pk->hash : 0;
-  key.precision = precision; key.B = B; key.K = K; key.Ll = Ll; key.Lr = Lr; key.diverse = diverse; key.noise = noise_E;
+  key.precision = precision; key.B = B; key.K = K; key.Ll = Ll; key.Lr = Lr;
   key.ws_ptr = ws; key.in_ptr = samp_in; key.tab_ptr = d_tables;  // (seed, gid0) are NOT part of the key: device memory, see arm_loop_kernel
   key.inv_ptr = samp_inv; key.inv_rows = inv.rows;
+  if (scoring) key.aux_ptr = score_in;
+  return SEQDIFF_OK;
+}
+
+template <typename Fwd, typename Step>
+int Model::replay_loop(cudaGraphExec_t& exec, GraphKey& cached, int& kernels, const GraphKey& key, int T, uint64_t seed, uint64_t gid0,
+                       cudaStream_t s, const Fwd& fwd, const Step& step) {
   uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
-  auto one_step = [&](cudaStream_t st) -> int {
-    const PdlScope pdl_scope(pdl_auto_mode(rows));
-    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, st, pk, &inv, K));
-    SD_TRY(reverse_step(d_tables, 1, B, Ll, x_cur, logits, diverse, noise_E, 0, 0, 0, d_step, x_cur, nullptr, st, d_step + 1, d_rng));
-    return SEQDIFF_OK;
-  };
-  if (!graph_exec || !(key == graph_key)) {
-    if (graph_exec) { cudaGraphExecDestroy(graph_exec); graph_exec = nullptr; }
+  if (!exec || !(key == cached)) {
+    if (exec) { cudaGraphExecDestroy(exec); exec = nullptr; }
     // un-captured dry run of the forward: sets kernel attributes and fills the TMA descriptor cache
     SD_CUDA(launch_k(set_int_kernel, dim3(1), dim3(1), 0, s, d_step, T - 1));
     SD_LAUNCHED("set_int", s);
-    SD_TRY(forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lang, c_lmask, c_rseq, c_rang, c_rmask, logits, s, pk, &inv, K));
+    SD_TRY(fwd(s));
     SD_CUDA(cudaStreamSynchronize(s));
     cudaGraph_t graph = nullptr;
     const uint64_t l0 = g_launches.load();
     SD_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const int rc = one_step(s);
-    graph_kernels = static_cast<int>(g_launches.load() - l0);  // kernel nodes per replay
+    const int rc = step(s);
+    kernels = static_cast<int>(g_launches.load() - l0);  // kernel nodes per replay
     cudaError_t ce = cudaStreamEndCapture(s, &graph);
     if (rc != SEQDIFF_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
     SD_CUDA(ce);
-    ce = cudaGraphInstantiate(&graph_exec, graph, 0);
+    ce = cudaGraphInstantiate(&exec, graph, 0);
     cudaGraphDestroy(graph);
     SD_CUDA(ce);
-    graph_key = key;
+    cached = key;
   }
   SD_CUDA(launch_k(arm_loop_kernel, dim3(1), dim3(1), 0, s, d_step, T - 1, d_rng, seed, gid0));
   SD_LAUNCHED("arm_loop", s);
-  for (int it = 0; it < T; ++it) SD_CUDA(cudaGraphLaunch(graph_exec, s));
-  g_launches.fetch_add(static_cast<uint64_t>(T) * graph_kernels, std::memory_order_relaxed);  // replayed kernel nodes
-  SD_CUDA(cudaMemcpyAsync(final_out, logits, Nl * 20 * 4, cudaMemcpyDefault, s));
+  for (int it = 0; it < T; ++it) SD_CUDA(cudaGraphLaunch(exec, s));
+  g_launches.fetch_add(static_cast<uint64_t>(T) * kernels, std::memory_order_relaxed);  // replayed kernel nodes
+  return SEQDIFF_OK;
+}
+
+int Model::sample(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
+                  const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, int diverse,
+                  const float* noise_E, uint64_t seed, uint64_t gid0, float* final_out, cudaStream_t caller, int flags) {
+  LoopIO io;
+  cudaStream_t s = nullptr;
+  SD_TRY(loop_setup(precision, P, K, Ll, Lr, T, q_tables, x_T, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, caller, flags, false, &io, &s));
+  const int B = P * K;
+  const PackInfo* pk = io.pk;
+  GraphKey key = io.key;
+  key.diverse = diverse; key.noise = noise_E;
+  uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
+  auto fwd = [&](cudaStream_t st) -> int {
+    return forward(precision, B, Ll, Lr, nullptr, d_step, io.x_cur, io.c_lang, io.c_lmask, io.c_rseq, io.c_rang, io.c_rmask, io.logits, st, pk, &inv, K);
+  };
+  auto one_step = [&](cudaStream_t st) -> int {
+    const PdlScope pdl_scope(pdl_auto_mode(io.rows));
+    SD_TRY(fwd(st));
+    SD_TRY(reverse_step(d_tables, 1, B, Ll, io.x_cur, io.logits, diverse, noise_E, 0, 0, 0, d_step, io.x_cur, nullptr, st, d_step + 1, d_rng));
+    return SEQDIFF_OK;
+  };
+  SD_TRY(replay_loop(graph_exec, graph_key, graph_kernels, key, T, seed, gid0, s, fwd, one_step));
+  SD_CUDA(cudaMemcpyAsync(final_out, io.logits, static_cast<size_t>(B) * Ll * 20 * 4, cudaMemcpyDefault, s));
   // ... and the caller's stream continues only after the loop has finished
+  SD_CUDA(cudaEventRecord(ev_out, s));
+  SD_CUDA(cudaStreamWaitEvent(caller, ev_out, 0));
+  return SEQDIFF_OK;
+}
+
+// One step of the score: x_t ~ q(x_t | x0) at the step's Qtb (the training q-sample), the sampling step's forward on it, then the
+// step's bound terms (vlb_terms, which advances the step counter).  Same invariants, packing and K-per-pocket receptor rows as sample().
+int Model::score(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x0, const float* lig_angle,
+                 const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, const float* noise_E,
+                 uint64_t seed, uint64_t gid0, double* terms_out, cudaStream_t caller, int flags) {
+  LoopIO io;
+  cudaStream_t s = nullptr;
+  SD_TRY(loop_setup(precision, P, K, Ll, Lr, T, q_tables, x0, lig_angle, lig_mask, rec_seq_in, rec_angle, rec_mask, caller, flags, true, &io, &s));
+  const int B = P * K;
+  const PackInfo* pk = io.pk;
+  GraphKey key = io.key;
+  key.noise = noise_E;
+  uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
+  auto fwd = [&](cudaStream_t st) -> int {
+    return forward(precision, B, Ll, Lr, nullptr, d_step, io.x_cur, io.c_lang, io.c_lmask, io.c_rseq, io.c_rang, io.c_rmask, io.logits, st, pk, &inv, K);
+  };
+  auto one_step = [&](cudaStream_t st) -> int {
+    const PdlScope pdl_scope(pdl_auto_mode(io.rows));
+    SD_TRY(apply_aa_noise(d_tables, B, Ll, io.x0, noise_E, 0, 0, 0, io.x_cur, nullptr, st, d_step, d_rng));
+    SD_TRY(fwd(st));
+    SD_TRY(vlb_terms(d_tables, B, Ll, io.x0, io.x_cur, io.logits, io.c_lmask, d_step, d_step + 1, io.acc, st));
+    return SEQDIFF_OK;
+  };
+  SD_TRY(replay_loop(score_exec, score_key, score_kernels, key, T, seed, gid0, s, fwd, one_step));
+  SD_CUDA(cudaMemcpyAsync(terms_out, io.acc, static_cast<size_t>(B) * Ll * 2 * 8, cudaMemcpyDefault, s));
   SD_CUDA(cudaEventRecord(ev_out, s));
   SD_CUDA(cudaStreamWaitEvent(caller, ev_out, 0));
   return SEQDIFF_OK;

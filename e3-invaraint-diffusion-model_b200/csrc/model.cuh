@@ -193,6 +193,37 @@ struct Model {
   int sample(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_T, const float* lig_angle,
              const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, int diverse,
              const float* noise_E, uint64_t seed, uint64_t gid0, float* final_out, cudaStream_t s, int flags = 0);
+  // The same loop scoring given sequences x0 (P * K graphs, one-hot at the valid positions) under the sampler's variational bound:
+  // T x (q-sample x_t ~ q(x_t | x0) with the step's Qtb -> forward -> vlb_terms), replayed from its own captured graph (score_exec),
+  // so that alternating sample / score calls on one handle keep both graphs.  terms_out [P * K, Ll, 2] fp64 (device or host):
+  // per residue (prior-free bound terms summed over the steps, cross-entropy summed over the steps); 0 at masked positions.
+  int score(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x0, const float* lig_angle,
+            const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, const float* noise_E,
+            uint64_t seed, uint64_t gid0, double* terms_out, cudaStream_t s, int flags = 0);
+  uint8_t* score_in = nullptr;  // x0 + the fp64 sums of the scoring loop (grow-only)
+  size_t score_in_bytes = 0;
+  cudaGraphExec_t score_exec = nullptr;
+  int score_kernels = 0;
+  GraphKey score_key;
+  // what sample() and score() share: the loop's buffers in the persistent input block, the packing and the step-graph key
+  struct LoopIO {
+    float *x_cur, *logits, *c_lang, *c_lmask, *c_rseq, *c_rang, *c_rmask;
+    float* x0 = nullptr;     // score only: the scored sequences
+    double* acc = nullptr;   // score only: [B * Ll, 2] fp64 sums (zeroed by loop_setup)
+    const PackInfo* pk = nullptr;
+    long long rows = 0;      // token rows of a step
+    GraphKey key;
+  };
+  // Private stream ordered after `caller`, persistent copies of the inputs (x_in -> x_cur for sampling, -> x0 for scoring), the step
+  // tables, the workspace, the packing (flags bit 0) and the LoopInv of this call.  Returns the loop stream in *ls.
+  int loop_setup(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x_in, const float* lig_angle,
+                 const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, cudaStream_t caller, int flags,
+                 bool scoring, LoopIO* io, cudaStream_t* ls);
+  // (Re)captures `step` into `exec` unless `key` matches the cached key (dry run of `fwd` first), then arms the step counter at T - 1
+  // with the Philox key (seed, gid0) and replays the graph T times on s.
+  template <typename Fwd, typename Step>
+  int replay_loop(cudaGraphExec_t& exec, GraphKey& cached, int& kernels, const GraphKey& key, int T, uint64_t seed, uint64_t gid0, cudaStream_t s,
+                  const Fwd& fwd, const Step& step);
   int* d_pack = nullptr;  // device block behind PackInfo (grow-only)
   size_t pack_cap = 0;
   PackInfo pack;

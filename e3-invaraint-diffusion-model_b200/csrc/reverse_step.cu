@@ -457,14 +457,27 @@ int reverse_step(const float* q_tables, int n_tab, int B, int L, const float* x_
 
 // ---------------------------------------------------------------------------------------------------
 // q-sample (training): prob[i] = Qtb[b][i,:].x0[n]; all-zero rows (padding) -> class 0  (model.py:301-308)
+// step_ptr != NULL (the scoring loop): every graph draws from the step's Qtb = q_tables[k][2] (qtb = the [T,3,20,20] step tables),
+// k = *step_ptr (read only: the step's last kernel advances it), noise entry k of a [T, B*L, 20] noise_E, (seed, graph_id0) from rng.
 __global__ void __launch_bounds__(kRevThreads) apply_aa_noise_kernel(const float* __restrict__ qtb, int L, const float* __restrict__ x0,
                                                                      const float* __restrict__ noise_E, uint64_t seed, uint64_t graph_id0,
-                                                                     uint32_t step, float* __restrict__ x_t, uint8_t* __restrict__ idx_out) {
+                                                                     uint32_t step, float* __restrict__ x_t, uint8_t* __restrict__ idx_out,
+                                                                     const int* __restrict__ step_ptr, const uint64_t* __restrict__ rng) {
   pdl_trigger();
   pdl_wait();  // predecessor grid complete + flushed before any dependent global access
   __shared__ float sQ[C * C];
   const int b = blockIdx.x;
-  for (int i = threadIdx.x; i < C * C; i += kRevThreads) sQ[i] = qtb[static_cast<size_t>(b) * C * C + i];
+  size_t tab = static_cast<size_t>(b) * C * C;
+  if (step_ptr) {
+    const int k = *step_ptr;
+    SD_DEV_ASSERT(k >= 0);
+    tab = static_cast<size_t>(k) * (3 * C * C) + 2 * C * C;
+    step = static_cast<uint32_t>(k);
+    if (noise_E) noise_E += static_cast<size_t>(k) * gridDim.x * L * C;
+    seed = rng[0];
+    graph_id0 = rng[1];
+  }
+  for (int i = threadIdx.x; i < C * C; i += kRevThreads) sQ[i] = qtb[tab + i];
   __syncthreads();
   for (int l = threadIdx.x; l < L; l += kRevThreads) {
     const size_t n = static_cast<size_t>(b) * L + l;
@@ -518,10 +531,134 @@ __global__ void __launch_bounds__(kRevThreads) apply_aa_noise_kernel(const float
 }
 
 int apply_aa_noise(const float* qtb, int B, int L, const float* x0, const float* noise_E, uint64_t seed, uint64_t graph_id0,
-                   uint32_t step, float* x_t, uint8_t* idx_out, cudaStream_t s) {
+                   uint32_t step, float* x_t, uint8_t* idx_out, cudaStream_t s, const int* step_ptr, const uint64_t* rng) {
   SD_CHECK(B > 0 && L > 0, "empty q-sample");
-  SD_CUDA(launch_k(apply_aa_noise_kernel, dim3(B), dim3(kRevThreads), 0, s, qtb, L, x0, noise_E, seed, graph_id0, step, x_t, idx_out));
+  SD_CHECK(!step_ptr || rng, "the in-loop q-sample reads its Philox key from device memory");
+  SD_CUDA(launch_k(apply_aa_noise_kernel, dim3(B), dim3(kRevThreads), 0, s, qtb, L, x0, noise_E, seed, graph_id0, step, x_t, idx_out, step_ptr, rng));
   SD_LAUNCHED("apply_aa_noise", s);
+  return SEQDIFF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Terms of the variational bound at step k of the scoring loop (Model::score), one thread per residue n of graph b, valid ones only:
+//   ce  = -log softmax(z)_a                                    (a = native class: x0 one-hot, z = the step's logits; fp64 from fp32 z)
+//   k >= 1: kl = sum_{j: q_j > 0} q_j (log q_j - log max(p_j, 1e-30))  in fp64, where
+//           p = the reverse step's normalised prob (exact mode above: softmax, sPost with the reference's rounding, 1e-5 rows) and
+//           q = the same with one-hot(a) for softmax(z), i.e. row a of post_x normalised   (x = the drawn class of x_t)
+//   k == 0: kl is replaced by the reconstruction term ce (the step at which the sampler returns the raw logits)
+// acc[n] += (kl or ce, ce).  A thread owns its residue's two fp64 sums and the steps run in sequence: bit-reproducible sums.
+// The step counter is read and advanced as in reverse_step_kernel (advance / step_ptr).
+constexpr int kVlbThreads = 128;
+__global__ void __launch_bounds__(kVlbThreads) vlb_terms_kernel(const float* __restrict__ q_tables, int L, const float* __restrict__ x0,
+                                                                const float* __restrict__ x_t, const float* __restrict__ logits,
+                                                                const float* __restrict__ mask, const int* __restrict__ step_ptr,
+                                                                int* __restrict__ advance, double* __restrict__ acc) {
+  pdl_trigger();
+  pdl_wait();
+  __shared__ int s_sidx;
+  if (threadIdx.x == 0) {
+    s_sidx = *reinterpret_cast<const volatile int*>(step_ptr);
+    __threadfence();
+    const unsigned total = gridDim.x * gridDim.y;
+    if (atomicAdd(reinterpret_cast<unsigned*>(advance), 1u) == total - 1u) {
+      *reinterpret_cast<volatile unsigned*>(advance) = 0u;
+      *const_cast<int*>(step_ptr) = s_sidx - 1;
+    }
+  }
+  __syncthreads();
+  const int k = s_sidx;
+  SD_DEV_ASSERT(k >= 0);
+  constexpr int kXS = C * C + 1;  // odd x-stride, as in the exact reverse step
+  __shared__ float sQt[C * C], sQsb[C * C], sQtb[C * C];
+  __shared__ float sPost[C * kXS];
+  if (k > 0) {
+    const float* tab = q_tables + static_cast<size_t>(k) * (3 * C * C);
+    for (int i = threadIdx.x; i < C * C; i += kVlbThreads) {
+      sQt[i] = tab[i];
+      sQsb[i] = tab[C * C + i];
+      sQtb[i] = tab[2 * C * C + i];
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < C * C; e += kVlbThreads) {
+      const int i = e / C, j = e - i * C;
+      const float qsb = sQsb[e];
+      for (int x = 0; x < C; ++x) {
+        float den = sQtb[i * C + x];
+        if (den == 0.f) den = 1e-6f;
+        sPost[x * kXS + e] = __fdiv_rn(__fmul_rn(sQt[j * C + x], qsb), den);
+      }
+    }
+    __syncthreads();
+  }
+  const int b = blockIdx.y;
+  for (int l = blockIdx.x * kVlbThreads + threadIdx.x; l < L; l += gridDim.x * kVlbThreads) {
+    const size_t n = static_cast<size_t>(b) * L + l;
+    if (mask[n] == 0.f) continue;
+    float lg[C];
+    int a = -1, x = -1;
+#pragma unroll
+    for (int j4 = 0; j4 < C; j4 += 4) {
+      const float4 z = *reinterpret_cast<const float4*>(logits + n * C + j4);
+      const float4 t = *reinterpret_cast<const float4*>(x0 + n * C + j4);
+      const float4 d = *reinterpret_cast<const float4*>(x_t + n * C + j4);
+      lg[j4] = z.x; lg[j4 + 1] = z.y; lg[j4 + 2] = z.z; lg[j4 + 3] = z.w;
+      if (t.x != 0.f) a = j4; if (t.y != 0.f) a = j4 + 1; if (t.z != 0.f) a = j4 + 2; if (t.w != 0.f) a = j4 + 3;
+      if (d.x != 0.f) x = j4; if (d.y != 0.f) x = j4 + 1; if (d.z != 0.f) x = j4 + 2; if (d.w != 0.f) x = j4 + 3;
+    }
+    SD_DEV_ASSERT(a >= 0 && x >= 0);  // valid rows of x0 are one-hot (checked by the caller); x_t is the q-sample's one-hot
+    float mx = lg[0];
+#pragma unroll
+    for (int j = 1; j < C; ++j) mx = fmaxf(mx, lg[j]);
+    double se = 0.0;
+#pragma unroll
+    for (int j = 0; j < C; ++j) se += exp(static_cast<double>(lg[j]) - static_cast<double>(mx));
+    const double ce = log(se) - (static_cast<double>(lg[a]) - static_cast<double>(mx));
+    double t0 = ce;
+    if (k > 0) {
+      float p[C], ps = 0.f;
+#pragma unroll
+      for (int j = 0; j < C; ++j) { p[j] = expf(lg[j] - mx); ps += p[j]; }
+#pragma unroll
+      for (int j = 0; j < C; ++j) p[j] = __fdiv_rn(p[j], ps);
+      const float* post = sPost + x * kXS;
+      float un[C];
+#pragma unroll
+      for (int j = 0; j < C; ++j) un[j] = 0.f;
+#pragma unroll
+      for (int i = 0; i < C; ++i) {
+#pragma unroll
+        for (int j = 0; j < C; ++j) un[j] = __fadd_rn(un[j], __fmul_rn(p[i], post[i * C + j]));
+      }
+      float tot = 0.f, totq = 0.f;
+#pragma unroll
+      for (int j = 0; j < C; ++j) { tot += un[j]; totq += post[a * C + j]; }
+      const bool pz = tot == 0.f, qz = totq == 0.f;
+      float tz = 0.f;  // sample.py:167: an all-zero row becomes 1e-5 everywhere, summed in order as in the reverse step
+#pragma unroll
+      for (int j = 0; j < C; ++j) tz += 1e-5f;
+      if (pz) tot = tz;
+      if (qz) totq = tz;
+      double kl = 0.0;
+#pragma unroll
+      for (int j = 0; j < C; ++j) {
+        const float pj = __fdiv_rn(pz ? 1e-5f : un[j], tot);
+        const float qj = __fdiv_rn(qz ? 1e-5f : post[a * C + j], totq);
+        if (qj > 0.f) kl += static_cast<double>(qj) * (log(static_cast<double>(qj)) - log(static_cast<double>(fmaxf(pj, 1e-30f))));
+      }
+      t0 = kl;
+    }
+    acc[2 * n] += t0;
+    acc[2 * n + 1] += ce;
+  }
+}
+
+int vlb_terms(const float* q_tables, int B, int L, const float* x0, const float* x_t, const float* logits, const float* mask,
+              const int* step_ptr, int* advance, double* acc, cudaStream_t s) {
+  SD_CHECK(B > 0 && L > 0, "empty score step");
+  SD_CHECK(step_ptr && advance, "the score step is indexed by the loop's device step counter");
+  SD_CUDA(launch_k(vlb_terms_kernel, dim3(ceil_div(L, kVlbThreads), B), dim3(kVlbThreads), 0, s, q_tables, L, x0, x_t, logits, mask, step_ptr,
+                   advance, acc));
+  SD_LAUNCHED("vlb_terms", s);
   return SEQDIFF_OK;
 }
 

@@ -23,7 +23,8 @@ from torch.nn import functional as F
 
 from . import _cabi
 from . import structure_model as SM
-from .sample import CONFIG, check_num_samples, decode_batch, denoise_tensors
+from .model import AA_VOCAB
+from .sample import CONFIG, check_num_samples, decode_batch, denoise_tensors, score
 from .utils import DiscreteUniformTransition, PredefinedNoiseScheduleDiscrete
 
 STRUCT_KEYS = ("ligand_attn_mask", "receptor_seq", "receptor_angles", "receptor_attn_mask")
@@ -63,6 +64,39 @@ def start_noise(n: int, L: int, feature_size: int) -> torch.Tensor:
     return SM.modulo_with_wrapped_range(torch.randn(n, L, feature_size))
 
 
+def sequence_schedule(timesteps=None, noise_schedule=None, transition=None):
+    """(T, noise schedule, transition) of the design's sequence sampler: CONFIG["timesteps"] steps of the cosine schedule and
+    DiscreteUniformTransition(20) unless given"""
+    T_q = CONFIG["timesteps"] if timesteps is None else timesteps
+    if noise_schedule is None:
+        noise_schedule = PredefinedNoiseScheduleDiscrete(CONFIG["noise_schedule"], T_q)
+    if transition is None:
+        transition = DiscreteUniformTransition(20)  # as the reference's structure -> sequence script (sample_by_generated_angles.py:253)
+    return T_q, noise_schedule, transition
+
+
+def score_designs(seq_model, batch, K: int, backbone_angles, pred_sequences, packed: bool = True, seed=None, timesteps=None, noise_schedule=None,
+                  transition=None):
+    """(nll_per_residue, perplexity) of design()'s rows of one batch: each predicted sequence scored under its pocket and its own generated
+    backbone (the swapped batch of the sequence sampler: backbone angles zero-padded to the batch length, one entry per row), with the
+    design's sequence schedule, transition and T.  Philox graph ids continue the process-wide stream."""
+    P, Lq, _ = batch["ligand_seq"].shape
+    n = P * K
+    angles = torch.zeros((n, Lq, 8), dtype=torch.float32)
+    seqs = torch.zeros((n, Lq, 20), dtype=torch.float32)
+    for i in range(n):
+        a = torch.as_tensor(backbone_angles[i], dtype=torch.float32)
+        angles[i, :a.shape[0]] = a
+        idx = torch.tensor([AA_VOCAB.index(c) for c in pred_sequences[i]], dtype=torch.long)
+        seqs[i, :idx.numel()] = F.one_hot(idx, 20).float()
+    swapped = dict(batch)
+    swapped["ligand_angles"] = angles
+    T_q, noise_schedule, transition = sequence_schedule(timesteps, noise_schedule, transition)
+    _, _, nll, ppl, _ = score(swapped, seq_model, noise_schedule, transition, sequences=seqs, timesteps=T_q, seed=seed, packed=packed,
+                              num_samples=K)
+    return nll, ppl
+
+
 @torch.no_grad()
 def design_tensors(struct_model, seq_model, batch, num_backbones: int = 1, num_sequences: int = 1, *, packed: bool = True,
                    struct_betas: Optional[torch.Tensor] = None, struct_timesteps: Optional[int] = None, noise_schedule=None,
@@ -96,11 +130,7 @@ def design_tensors(struct_model, seq_model, batch, num_backbones: int = 1, num_s
     backbones = F.pad(torch.where(valid[..., None], angles, torch.zeros((), device=angles.device)), (0, 0, 0, Lq - Ll_s))
     swapped = dict(batch)
     swapped["ligand_angles"] = backbones.repeat_interleave(K2, dim=0)
-    T_q = CONFIG["timesteps"] if timesteps is None else timesteps
-    if noise_schedule is None:
-        noise_schedule = PredefinedNoiseScheduleDiscrete(CONFIG["noise_schedule"], T_q)
-    if transition is None:
-        transition = DiscreteUniformTransition(20)  # as the reference's structure -> sequence script (sample_by_generated_angles.py:253)
+    T_q, noise_schedule, transition = sequence_schedule(timesteps, noise_schedule, transition)
     final = denoise_tensors(swapped, seq_model, noise_schedule, transition, diverse, timesteps=T_q, x_T=seq_x_T, graph_id0=seq_graph_id0,
                             seed=seed, packed=packed, num_samples=K1 * K2)
     return backbones, final
@@ -129,18 +159,25 @@ def design(struct_model, seq_model, batch, num_backbones: int = 1, num_sequences
 
 
 def design_dataset(dataloader, struct_model, seq_model, num_backbones: int = 1, num_sequences: int = 1, output_path=None, design_fn=None,
-                   **kw):
+                   score: bool = False, **kw):
     """Every batch of `dataloader` through `design`; returns sample_dataset's DataFrame (structure_ids / true_sequence /
-    predict_sequence / recovery_rate) plus a `backbone` column, pickled to `output_path` like sample_dataset when given."""
+    predict_sequence / recovery_rate) plus a `backbone` column, pickled to `output_path` like sample_dataset when given.
+    score=True adds `nll_per_residue` and `perplexity`: each predicted sequence scored under its pocket and its own backbone
+    (score_designs), the candidates' model score where no native peptide exists."""
     import pandas as pd
     K1, K2 = _check_counts(num_backbones, num_sequences)
     fn = design if design_fn is None else design_fn
+    skw = {k: kw[k] for k in ("packed", "seed", "timesteps", "noise_schedule", "transition") if k in kw}
     rows = []
     for idx, batch in enumerate(dataloader):
         print(f"Generating Batch {idx}")
-        ids, backbone, _, true_seqs, pred_seqs, rates = fn(struct_model, seq_model, batch, K1, K2, **kw)
-        rows.extend(zip(ids, true_seqs, pred_seqs, rates, backbone))
-    res = pd.DataFrame(rows, columns=["structure_ids", "true_sequence", "predict_sequence", "recovery_rate", "backbone"])
+        ids, backbone, angles, true_seqs, pred_seqs, rates = fn(struct_model, seq_model, batch, K1, K2, **kw)
+        if score:
+            rows.extend(zip(ids, true_seqs, pred_seqs, rates, backbone, *score_designs(seq_model, batch, K1 * K2, angles, pred_seqs, **skw)))
+        else:
+            rows.extend(zip(ids, true_seqs, pred_seqs, rates, backbone))
+    columns = ["structure_ids", "true_sequence", "predict_sequence", "recovery_rate", "backbone"]
+    res = pd.DataFrame(rows, columns=columns + (["nll_per_residue", "perplexity"] if score else []))
     if output_path is not None:
         res.to_pickle(output_path)
     return res

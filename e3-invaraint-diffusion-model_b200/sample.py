@@ -14,6 +14,7 @@ either handed in explicitly (`noise_E`, parity runs) or generated in-kernel by P
 from __future__ import annotations
 
 import ctypes
+import math
 
 import torch
 from torch.nn import functional as F
@@ -173,6 +174,112 @@ def denoise_tensors(batch, model, noise_schedule, transition, diverse, timesteps
                                                   _cabi.ptr(E), SEED if seed is None else seed, graph_id0, 1 if packed else 0,
                                                   _cabi.ptr(out), stream))
     return out
+
+
+def score_prior(tables):
+    """[20] fp64: the prior term KL(r_a || uniform) of native class a, r_a = Qtb of the last step's table column a, normalised.  It does not
+    depend on the model (the bound's L_T)."""
+    qtb = tables[-1, 2].double()
+    r = qtb / qtb.sum(dim=0, keepdim=True)
+    return torch.where(r > 0, r * torch.log(r * r.shape[0]), torch.zeros((), dtype=torch.float64)).sum(dim=0)
+
+
+@torch.no_grad()
+def score_tensors(batch, model, noise_schedule, transition, sequences=None, timesteps=None, noise_E_steps=None, graph_id0=None, seed=None,
+                  packed=False, num_samples=1):
+    """The negative log-likelihood bound of `sequences` for the pockets and backbones of `batch` under the sampler's reverse process
+    (seqdiff_score_multi): T steps of (x_t ~ q(x_t | x0) at the step's Qtb, denoiser forward at step k, per-residue bound terms) from one
+    captured CUDA graph.  Returns (terms [B, L, 2] fp64, prior [B] fp64) on the model's device, B = P*K: terms[..., 0] = sum_{k>=1} kl_k +
+    the reconstruction term of k = 0, terms[..., 1] = sum_k of the x0 cross-entropy -log softmax(z_k)_a, both 0 at masked positions;
+    prior = the sum over the valid positions of the prior term (score_prior).  nll = prior + terms[..., 0].sum(-1).
+    `sequences` (default batch["ligand_seq"], the native peptides) is [P, L, 20] or [P*K, L, 20], one-hot at every valid position;
+    ligand_angles / ligand_attn_mask may be given per pocket or per sample (as denoise_tensors takes them).  `noise_E_steps` [T, P*K*L, 20]:
+    explicit Exp(1) race noise of the q-sample, entry k at step k; else Philox keyed by (seed, graph_id0 + graph, residue, k), graph_id0
+    None continuing the process-wide stream.  `packed` / `num_samples` as in denoise_tensors.  ValueError (before any device work) for
+    disagreeing shapes, a valid position that is not exactly one-hot, or a graph without a valid ligand position."""
+    K = check_num_samples(num_samples)
+    T = CONFIG["timesteps"] if timesteps is None else int(timesteps)
+    n_pockets, max_len, num_class = batch["ligand_seq"].shape
+    if num_class != 20:
+        raise ValueError(f"scoring needs 20 classes, got {num_class}")
+    B = n_pockets * K
+
+    def per_sample(x, name, tail):
+        if tuple(x.shape[1:]) != tail:
+            raise ValueError(f"{name} must be [P or P*K, {', '.join(map(str, tail))}], got {tuple(x.shape)}")
+        if x.shape[0] == B:
+            return x
+        if x.shape[0] != n_pockets:
+            raise ValueError(f"{name} must hold P = {n_pockets} or P*K = {B} entries, got {x.shape[0]}")
+        return x.repeat_interleave(K, dim=0)
+
+    seqs = per_sample(batch["ligand_seq"] if sequences is None else sequences, "sequences", (max_len, 20))
+    ligand_mask = per_sample(batch["ligand_attn_mask"], "ligand_attn_mask", (max_len,))
+    ligand_angles = per_sample(batch["ligand_angles"], "ligand_angles", (max_len, 8))
+    receptor_seq, receptor_angles, receptor_mask = batch["receptor_seq"], batch["receptor_angles"], batch["receptor_attn_mask"]
+    Lr = receptor_seq.shape[1]
+    for x, name, shape in ((receptor_seq, "receptor_seq", (n_pockets, Lr, 20)), (receptor_angles, "receptor_angles", (n_pockets, Lr, 8)),
+                           (receptor_mask, "receptor_attn_mask", (n_pockets, Lr))):
+        if tuple(x.shape) != shape:
+            raise ValueError(f"{name} must be {shape}, got {tuple(x.shape)}")
+    if noise_E_steps is not None and tuple(noise_E_steps.shape) != (T, B * max_len, 20):
+        raise ValueError(f"noise_E_steps must be [T, P*K*L, 20] = {(T, B * max_len, 20)}, got {tuple(noise_E_steps.shape)}")
+    # host-side checks of the scored sequences (the kernels read the native class of a valid position as its one nonzero entry)
+    seqs_h, valid = seqs.detach().float().cpu(), ligand_mask.detach().cpu() != 0
+    rows = seqs_h[valid]
+    if not (((rows == 0) | (rows == 1)).all() and (rows.sum(dim=-1) == 1).all()):
+        raise ValueError("every valid position of the scored sequences must be exactly one-hot")
+    if not valid.any(dim=1).all():
+        raise ValueError("every graph needs at least one valid ligand position to be scored")
+    tables = loop_tables(T, noise_schedule, transition)
+    if tables.shape[0] != T or tables.shape[1:] != (3, 20, 20):
+        raise ValueError("transition tables must be [T,3,20,20] (per-step scalar schedule)")
+    prior = (score_prior(tables)[seqs_h.argmax(dim=-1)] * valid).sum(dim=1)
+
+    h = model._sync_handle()
+    dev = model._handle_dev
+    if graph_id0 is None:
+        graph_id0 = _cabi.GRAPH_IDS.take(B)
+
+    def dv(x):
+        return x.to(device=dev, dtype=torch.float32, non_blocking=True).contiguous()
+
+    E = None if noise_E_steps is None else dv(noise_E_steps)
+    terms = torch.empty((B, max_len, 2), device=dev, dtype=torch.float64)
+    args = [dv(tables), dv(seqs), dv(ligand_angles), dv(ligand_mask), dv(receptor_seq), dv(receptor_angles), dv(receptor_mask)]
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _cabi.check(_cabi.lib().seqdiff_score_multi(h, model._precision_code(), n_pockets, K, max_len, Lr, T, *map(_cabi.ptr, args),
+                                                    _cabi.ptr(E), SEED if seed is None else seed, graph_id0, 1 if packed else 0,
+                                                    _cabi.ptr(terms), stream))
+    return terms, prior.to(dev)
+
+
+@torch.no_grad()
+def score(batch, model, noise_schedule, transition, **kw):
+    """score_tensors on the host: (structure_ids, sequences, nll_per_residue, perplexity, ce_per_residue), one entry per scored graph in
+    (pocket, sample) order.  nll_per_residue = (prior + sum of the bound terms) / valid positions, in nats; perplexity =
+    exp(nll_per_residue); ce_per_residue = the x0 cross-entropy summed over the T steps / (T * valid positions)."""
+    K = check_num_samples(kw.get("num_samples", 1))
+    terms, prior = score_tensors(batch, model, noise_schedule, transition, **kw)
+    T = CONFIG["timesteps"] if kw.get("timesteps") is None else int(kw["timesteps"])
+    seqs = batch["ligand_seq"] if kw.get("sequences") is None else kw["sequences"]
+    mask = batch["ligand_attn_mask"]
+    P = batch["ligand_seq"].shape[0]
+    if seqs.shape[0] != P * K:
+        seqs = seqs.repeat_interleave(K, dim=0)
+    if mask.shape[0] != P * K:
+        mask = mask.repeat_interleave(K, dim=0)
+    valid = mask.detach().cpu() != 0
+    n = valid.sum(dim=1).double()
+    sums = terms.sum(dim=1).cpu()
+    nll = ((prior.cpu() + sums[:, 0]) / n).tolist()
+    ce = (sums[:, 1] / (T * n)).tolist()
+    idx = seqs.detach().float().cpu().argmax(dim=-1)
+    ids = batch.get("structure_ids")
+    structure_ids = [f'{ids["pdb_id"][i // K]}_{ids["ligand_chain"][i // K]}' if ids is not None else str(i // K) for i in range(P * K)]
+    sequences = ["".join(AA_VOCAB[j] for j in idx[i][valid[i]].tolist()) for i in range(P * K)]
+    return structure_ids, sequences, nll, [math.exp(v) for v in nll], ce
 
 
 def decode_tensors(final, ligand_seq, ligand_mask):

@@ -166,6 +166,28 @@ SEQDIFF_API int seqdiff_sample_multi(seqdiff_model_t* m, int precision, int P, i
                          const float* receptor_mask, int diverse, const float* noise_E_steps, uint64_t seed,
                          uint64_t graph_id0, int flags, float* final_out, void* stream);
 
+/* ---- sequence score: the negative log-likelihood bound of given sequences for their pockets and backbones (no reference
+ * counterpart; the model score inverse-folding tools report).  Same batch layout, packing (flags bit 0), K-per-pocket receptor rows,
+ * step tables and Philox keying as seqdiff_sample_multi; x0 [P*K,L_lig,20] = the scored sequences, one-hot at every position with
+ * ligand_mask != 0 (the caller checks this).  One step k (k = T-1 .. 0, tables entry k: t = (k+1)/T, s = k/T) is replayed from a
+ * captured CUDA graph of its own (sampling and scoring on one handle keep both graphs):
+ *   x_t ~ q(x_t | x0): prob[i] = Qtb_k[i, a] (a = native class), exponential race with noise_E_steps[k] [P*K*L_lig, 20] or Philox
+ *         keyed by (seed, graph_id0 + graph, residue, k) -- the training q-sample (seqdiff_apply_aa_noise) at t_int = k+1;
+ *   z   = the denoiser's logits at timestep k (the raw step index, as the sampler feeds it);
+ *   ce_k = -log softmax(z)_a;
+ *   k >= 1: kl_k = sum_{j: q_j > 0} q_j (log q_j - log max(p_j, 1e-30)) in fp64, p = the reverse step's normalised posterior prob
+ *           (sample.py:162-168, from softmax(z) and the drawn x_t) and q = the same with one-hot(a) in place of softmax(z);
+ *   k == 0: the reconstruction term ce_0 takes the place of kl.
+ * terms_out [P*K, L_lig, 2] f64 (device or host): per position (sum_{k>=1} kl_k + ce_0, sum_k ce_k), 0 where ligand_mask == 0.  The
+ * model-independent prior KL(Qtb_{T-1}[:, a] normalised || uniform) is the caller's (sample.py: score_tensors).  Qt is the reference's
+ * row-normalised Qsb / Qtb (quirk Q5), not a one-step matrix, so this is the D3PM bound under the sampler's own posterior: a consistent
+ * ranking score for what the sampler generates, not a calibrated likelihood.  Sums are per position in step order: bit-reproducible.
+ * P < 1, K < 1, T < 1, P*K*max(L_lig, L_rec) > INT32_MAX, unknown flag bits or feature_size != 20: SEQDIFF_ERR_INVALID. */
+SEQDIFF_API int seqdiff_score_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T,
+                        const float* q_tables_steps, const float* x0, const float* ligand_angle, const float* ligand_mask,
+                        const float* receptor_seq, const float* receptor_angle, const float* receptor_mask,
+                        const float* noise_E_steps, uint64_t seed, uint64_t graph_id0, int flags, double* terms_out, void* stream);
+
 /* ---- output decode: replaces the per-graph loop of denoise(), sequence_model/sample.py:208-224 --------------------
  * final_seq [B,L,20] (the loop's result: raw logits of the last step), true_seq [B,L,20] one-hot, ligand_mask [B,L] {0,1}.
  * pred_idx / true_idx [B,L] u8 = argmax over classes (first maximum, like torch.argmax); counts [B,2] i32 =
