@@ -66,6 +66,7 @@ PROTOTYPES = {
     "seqdiff_struct_sample": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u64, _vp, _vp, _vp]),
     "seqdiff_struct_sample_ex": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u64, _i, _vp, _vp, _vp]),
     "seqdiff_struct_sample_multi": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u64, _i, _vp, _vp, _vp]),
+    "seqdiff_struct_score_multi": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u64, _i, _vp, _vp]),
     "seqdiff_op_gemm": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "seqdiff_op_attention": (_i, [_i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _vp]),
     "seqdiff_op_attention_train_fwd": (_i, [_i, _i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, C.c_float, _u64, _u32, _u32, _vp, _vp]),

@@ -386,6 +386,23 @@ int seqdiff_struct_sample_multi(seqdiff_model_t* m, int precision, int P, int K,
   SD_GUARD_END
 }
 
+int seqdiff_struct_score_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T, const float* qs_steps,
+                               const float* x0, const float* ligand_mask, const float* receptor_seq, const float* receptor_angles,
+                               const float* receptor_mask, const float* noise_steps, uint64_t seed, uint64_t graph_id0, int flags,
+                               double* terms_out, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(m && qs_steps && x0 && ligand_mask && receptor_seq && receptor_angles && receptor_mask && terms_out, "null argument");
+  SD_CHECK(P >= 1 && K >= 1 && T >= 1, "need at least one pocket, one backbone per pocket and one step");
+  SD_CHECK(L_lig > 0 && L_rec > 0 && static_cast<int64_t>(P) * K * (L_lig > L_rec ? L_lig : L_rec) <= INT32_MAX,
+           "pockets x backbones x length overflows the row counts");
+  SD_CHECK(static_cast<int64_t>(P) * K <= 65535, "more than 65535 backbones in one call (the step kernels put one graph per grid row)");
+  SD_CHECK((flags & ~1) == 0, "unknown scoring flag");
+  SD_CHECK(m->impl.arch == kArchStructure, "handle holds a sequence model: use seqdiff_score_multi");
+  return m->impl.struct_score(precision, P, K, L_lig, L_rec, T, qs_steps, x0, ligand_mask, receptor_seq, receptor_angles, receptor_mask,
+                              noise_steps, seed, graph_id0, terms_out, static_cast<cudaStream_t>(stream), flags);
+  SD_GUARD_END
+}
+
 int seqdiff_decode(int B, int L, const float* final_seq, const float* true_seq, const float* ligand_mask, uint8_t* pred_idx,
                    uint8_t* true_idx, int32_t* counts, void* stream) {
   SD_GUARD_BEGIN

@@ -495,6 +495,22 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
   return launch_kc(1, kernel, grid, block, smem, s, args...);
 }
 
+// ---- angles of the structure model: one definition for the sampler, the training loss and the backbone score --------------------
+// modulo_with_wrapped_range(v, -pi, pi) (structure_model/utils.py:20-40): torch `%` is fmod, then + 2pi if the remainder is negative.
+// The python-float bounds enter the fp32 kernels as their nearest fp32 values.
+__device__ __forceinline__ float wrap_angle(float v) {
+  constexpr float kMin = -3.14159274101257324f, kTop = 6.28318548202514648f;
+  float m = fmodf(__fsub_rn(v, kMin), kTop);
+  if (m != 0.f && m < 0.f) m = __fadd_rn(m, kTop);
+  return __fadd_rn(m, kMin);
+}
+// FoldingDiff's smooth-L1 on a wrapped angle difference: h(d) = 0.5 d^2 / beta (|d| < beta), |d| - 0.5 beta otherwise; beta = pi / 10
+constexpr float kAngleBeta = 0.314159265358979f;
+__device__ __forceinline__ float angle_smooth_l1(float d) {
+  const float ad = fabsf(d);
+  return ad < kAngleBeta ? 0.5f * d * d / kAngleBeta : ad - 0.5f * kAngleBeta;
+}
+
 // ---- misc -------------------------------------------------------------------------------------------
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 int num_sms();  // SM count of the current device (cached)

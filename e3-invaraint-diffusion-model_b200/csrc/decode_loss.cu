@@ -226,13 +226,7 @@ int loss_terms(int N, const float* logits, const float* x0, const float* x_t, co
 // Objective of the structure (angle) model: wrapped smooth-L1 on the predicted noise, per feature, over the valid ligand positions.
 //   d = wrap(known_noise - pred) into [-pi, pi);  h(d) = 0.5 d^2 / beta (|d| < beta), |d| - 0.5 beta otherwise;  beta = pi / 10.
 // terms[i] = sum of h over the valid positions of feature i (i < F), terms[F] = number of valid positions; loss = mean_i terms[i] / terms[F].
-__device__ __forceinline__ float wrap_angle(float v) {  // modulo_with_wrapped_range(v, -pi, pi) with the bounds as fp32 values (gauss_step.cu)
-  constexpr float kMin = -3.14159274101257324f, kTop = 6.28318548202514648f;
-  float m = fmodf(__fsub_rn(v, kMin), kTop);
-  if (m != 0.f && m < 0.f) m = __fadd_rn(m, kTop);
-  return __fadd_rn(m, kMin);
-}
-constexpr float kAngleBeta = 0.314159265358979f;
+// wrap_angle and h (angle_smooth_l1) are common.cuh's, shared with the sampler and the backbone score.
 
 template <int F>
 __global__ void __launch_bounds__(kLossThreads) angle_loss_terms_kernel(int N, const float* __restrict__ pred, const float* __restrict__ noise,
@@ -250,9 +244,7 @@ __global__ void __launch_bounds__(kLossThreads) angle_loss_terms_kernel(int N, c
 #pragma unroll
     for (int i = 0; i < F; ++i) {
       const size_t e = static_cast<size_t>(n) * F + i;
-      const float d = wrap_angle(__fsub_rn(noise[e], pred[e]));
-      const float ad = fabsf(d);
-      acc[i] += ad < kAngleBeta ? 0.5f * d * d / kAngleBeta : ad - 0.5f * kAngleBeta;
+      acc[i] += angle_smooth_l1(wrap_angle(__fsub_rn(noise[e], pred[e])));
     }
   }
   // fixed-order reduction (deterministic run to run): warp shuffles, warps in order, then the last CTA folds the partials in CTA order

@@ -41,16 +41,36 @@ __device__ __forceinline__ void box_muller(uint32_t w0, uint32_t w1, float& z0, 
   z1 = r * sn;
 }
 
+// the four N(0,1) values of 4-element group q of global graph `graph` at step `step`
+__device__ __forceinline__ void philox_normal4(uint64_t seed, uint64_t graph, int q, int step, float (&z)[4]) {
+  uint32_t ctr[4] = {static_cast<uint32_t>(q), static_cast<uint32_t>(step), static_cast<uint32_t>(graph), static_cast<uint32_t>(graph >> 32)};
+  philox4(ctr, static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32));
+  box_muller(ctr[0], ctr[1], z[0], z[1]);
+  box_muller(ctr[2], ctr[3], z[2], z[3]);
+}
+
+// the loop step index from the device counter; with `advance`, the last CTA to have read it moves it on (no separate launch)
+__device__ __forceinline__ int loop_step(const int* step_ptr, int* advance) {
+  __shared__ int s_sidx;
+  if (threadIdx.x == 0) {
+    s_sidx = *reinterpret_cast<const volatile int*>(step_ptr);
+    if (advance) {
+      __threadfence();
+      const unsigned total = gridDim.x * gridDim.y;
+      if (atomicAdd(reinterpret_cast<unsigned*>(advance), 1u) == total - 1u) {
+        *reinterpret_cast<volatile unsigned*>(advance) = 0u;
+        *const_cast<int*>(step_ptr) = s_sidx - 1;
+      }
+    }
+  }
+  __syncthreads();
+  return s_sidx;
+}
+
 __device__ __forceinline__ float gauss_update(float x, float out, float a, float b, float c, float sd, float z, bool last, bool wrap) {
   const float mean = __fmul_rn(a, __fsub_rn(x, __fdiv_rn(__fmul_rn(b, out), c)));
   const float v = last ? mean : __fadd_rn(mean, __fmul_rn(sd, z));
-  if (!wrap) return v;  // p_sample alone (sample.py:55-102) returns the un-wrapped value
-  // modulo_with_wrapped_range(v, -pi, pi): the python-float bounds enter the fp32 kernels as their nearest fp32 values
-  constexpr float kMin = -3.14159274101257324f, kTop = 6.28318548202514648f;
-  const float sh = __fsub_rn(v, kMin);
-  float m = fmodf(sh, kTop);
-  if (m != 0.f && m < 0.f) m = __fadd_rn(m, kTop);
-  return __fadd_rn(m, kMin);
+  return wrap ? wrap_angle(v) : v;  // p_sample alone (sample.py:55-102) returns the un-wrapped value
 }
 
 // One thread per group of 4 consecutive elements of one graph (per = L * F elements per graph, groups = ceil(per / 4)).
@@ -74,20 +94,7 @@ __global__ void __launch_bounds__(kGaussThreads) gauss_step_kernel(const float* 
   }
   const size_t n_all = static_cast<size_t>(gridDim.y) * per;
   if (step_ptr) {  // sampling loop: the step index lives on the device; the last CTA to have read it moves it on
-    __shared__ int s_sidx;
-    if (threadIdx.x == 0) {
-      s_sidx = *reinterpret_cast<const volatile int*>(step_ptr);
-      if (advance) {
-        __threadfence();
-        const unsigned total = gridDim.x * gridDim.y;
-        if (atomicAdd(reinterpret_cast<unsigned*>(advance), 1u) == total - 1u) {
-          *reinterpret_cast<volatile unsigned*>(advance) = 0u;
-          *const_cast<int*>(step_ptr) = s_sidx - 1;
-        }
-      }
-    }
-    __syncthreads();
-    step = s_sidx;
+    step = loop_step(step_ptr, advance);
     if (noise) noise += static_cast<size_t>(step) * n_all;
   }
   if (step < 0 || step >= T) return;
@@ -138,11 +145,7 @@ __global__ void __launch_bounds__(kGaussThreads) gauss_step_kernel(const float* 
           for (int e = 0; e < nv; ++e) zv[e] = noise[base + e];
         }
       } else {
-        const uint64_t graph = graph_id0 + static_cast<uint64_t>(g);
-        uint32_t ctr[4] = {static_cast<uint32_t>(q), static_cast<uint32_t>(step), static_cast<uint32_t>(graph), static_cast<uint32_t>(graph >> 32)};
-        philox4(ctr, static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32));
-        box_muller(ctr[0], ctr[1], zv[0], zv[1]);
-        box_muller(ctr[2], ctr[3], zv[2], zv[3]);
+        philox_normal4(seed, graph_id0 + static_cast<uint64_t>(g), q, step, zv);
       }
     }
     float r[4];
@@ -182,6 +185,147 @@ int gauss_step(const float* coef, int T, int B, int per_graph, const float* x_t,
                      step_ptr, x_out, steps_out, advance, wrap ? 1 : 0, rng, static_cast<const int*>(nullptr), 0));
   }
   SD_LAUNCHED("gauss_step", s);
+  return SEQDIFF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Backbone score (Model::struct_score): the structure model's training objective at every step k = T-1 .. 0 of a loop.
+//   x_k = wrap(sqrt_ac[k] * x0 + sqrt_1m_ac[k] * eps_k)      fp32, __fmul_rn, __fmul_rn, __fadd_rn, wrap_angle (NoisedAnglesDataset)
+//   acc += h(wrap(eps_k - pred_k))                           fp64, per element, at the valid positions (angle_loss_terms' arithmetic)
+// Both kernels read k from the loop's step counter and (seed, graph_id0) from its RNG words, and take eps_k of element e of graph g
+// the way gauss_step_kernel takes its z: from the explicit table noise[k] [B * per], or from Philox at the element's 4-element group
+// inside the PADDED graph -- so packed and padded batches draw the same eps at every valid element.  The terms kernel recomputes
+// eps_k rather than reading a buffer.  Same thread layout as the Gaussian step: one thread per group of 4 consecutive elements.
+__device__ __forceinline__ void step_noise4(const float* noise, size_t base, int nv, bool vload, uint64_t seed, uint64_t graph, int q, int step,
+                                            float (&z)[4]) {
+  if (noise) {
+    if (vload) {
+      const float4 z4 = *reinterpret_cast<const float4*>(noise + base);
+      z[0] = z4.x; z[1] = z4.y; z[2] = z4.z; z[3] = z4.w;
+    } else {
+      for (int e = 0; e < nv; ++e) z[e] = noise[base + e];
+    }
+  } else {
+    philox_normal4(seed, graph, q, step, z);
+  }
+}
+
+// x_t [B, per]: padded -> every element; PACKED -> the valid elements (e < len[g] * F), padded ones are neither read nor written.
+template <bool PACKED>
+__global__ void __launch_bounds__(kGaussThreads) angle_qsample_kernel(const float* __restrict__ qs, int per, const float* __restrict__ x0,
+                                                                      const float* __restrict__ noise, const int* __restrict__ step_ptr,
+                                                                      const uint64_t* __restrict__ rng, const int* __restrict__ len, int F,
+                                                                      float* __restrict__ x_t) {
+  pdl_trigger();
+  pdl_wait();
+  const int step = loop_step(step_ptr, nullptr);
+  const uint64_t seed = rng[0], graph_id0 = rng[1];
+  const int g = blockIdx.y;
+  if (noise) noise += static_cast<size_t>(step) * gridDim.y * per;
+  const float sa = __ldg(qs + 2 * step), sb = __ldg(qs + 2 * step + 1);
+  const int groups = (per + 3) >> 2;
+  const bool vec = (per & 3) == 0;
+  for (int q = blockIdx.x * kGaussThreads + threadIdx.x; q < groups; q += gridDim.x * kGaussThreads) {
+    const size_t base = static_cast<size_t>(g) * per + 4 * static_cast<size_t>(q);
+    int nv = min(4, per - 4 * q);
+    if constexpr (PACKED) {
+      nv = min(nv, max(0, __ldg(len + g) * F - 4 * q));
+      if (nv == 0) continue;
+    }
+    const bool vload = vec && nv == 4;
+    float xv[4] = {0.f, 0.f, 0.f, 0.f}, zv[4] = {0.f, 0.f, 0.f, 0.f};
+    if (vload) {
+      const float4 x4 = *reinterpret_cast<const float4*>(x0 + base);
+      xv[0] = x4.x; xv[1] = x4.y; xv[2] = x4.z; xv[3] = x4.w;
+    } else {
+      for (int e = 0; e < nv; ++e) xv[e] = x0[base + e];
+    }
+    step_noise4(noise, base, nv, vload, seed, graph_id0 + static_cast<uint64_t>(g), q, step, zv);
+    float r[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) r[e] = wrap_angle(__fadd_rn(__fmul_rn(sa, xv[e]), __fmul_rn(sb, zv[e])));
+    if (vload) {
+      *reinterpret_cast<float4*>(x_t + base) = make_float4(r[0], r[1], r[2], r[3]);
+    } else {
+      for (int e = 0; e < nv; ++e) x_t[base + e] = r[e];
+    }
+  }
+}
+
+// acc [B, per] fp64 += h(wrap(eps - pred)) at the valid elements: padded -> mask[g * (per / F) + e / F] != 0, PACKED -> e < len[g] * F.
+// Every element is owned by one thread and summed in step order (no atomics): bit-reproducible.  Other elements are never read or
+// written.  The last CTA to have read the step counter moves it on.
+template <bool PACKED>
+__global__ void __launch_bounds__(kGaussThreads) angle_score_terms_kernel(int per, const float* __restrict__ pred, const float* __restrict__ noise,
+                                                                          const float* __restrict__ mask, const int* __restrict__ step_ptr,
+                                                                          int* __restrict__ advance, const uint64_t* __restrict__ rng,
+                                                                          const int* __restrict__ len, int F, double* __restrict__ acc) {
+  pdl_trigger();
+  pdl_wait();
+  const int step = loop_step(step_ptr, advance);
+  const uint64_t seed = rng[0], graph_id0 = rng[1];
+  const int g = blockIdx.y;
+  if (noise) noise += static_cast<size_t>(step) * gridDim.y * per;
+  const int groups = (per + 3) >> 2;
+  const bool vec = (per & 3) == 0;
+  for (int q = blockIdx.x * kGaussThreads + threadIdx.x; q < groups; q += gridDim.x * kGaussThreads) {
+    const size_t base = static_cast<size_t>(g) * per + 4 * static_cast<size_t>(q);
+    const int cnt = min(4, per - 4 * q);
+    bool valid[4] = {false, false, false, false};
+    int nv = 0;  // packed: valid elements form a prefix of the group
+    if constexpr (PACKED) {
+      nv = min(cnt, max(0, __ldg(len + g) * F - 4 * q));
+      for (int e = 0; e < 4; ++e) valid[e] = e < nv;
+    } else {
+      for (int e = 0; e < cnt; ++e) {
+        valid[e] = __ldg(mask + static_cast<size_t>(g) * (per / F) + (4 * q + e) / F) != 0.f;
+        nv += valid[e] ? 1 : 0;
+      }
+    }
+    if (nv == 0) continue;
+    const bool vload = vec && nv == 4;
+    float zv[4] = {0.f, 0.f, 0.f, 0.f};
+    // explicit noise: element-wise loads cover the valid ones only (padded mode may have holes, so nv is not a prefix length there)
+    if (noise && !vload) {
+      for (int e = 0; e < 4; ++e)
+        if (valid[e]) zv[e] = noise[base + e];
+    } else {
+      step_noise4(noise, base, 4, vload, seed, graph_id0 + static_cast<uint64_t>(g), q, step, zv);
+    }
+#pragma unroll
+    for (int e = 0; e < 4; ++e)
+      if (valid[e]) acc[base + e] += static_cast<double>(angle_smooth_l1(wrap_angle(__fsub_rn(zv[e], pred[base + e]))));
+  }
+}
+
+int angle_qsample(const float* qs, int B, int per_graph, const float* x0, const float* noise, const int* step_ptr, const uint64_t* rng,
+                  float* x_t, cudaStream_t s, const int* len, int F) {
+  SD_CHECK(B > 0 && per_graph > 0 && F > 0 && per_graph % F == 0, "angle q-sample: per_graph must be a positive multiple of F");
+  SD_CHECK(step_ptr && rng, "angle q-sample runs inside a loop (step counter and RNG words on the device)");
+  const dim3 grid(ceil_div((per_graph + 3) / 4, kGaussThreads), B);
+  if (len) {
+    SD_CUDA(launch_k(angle_qsample_kernel<true>, grid, dim3(kGaussThreads), 0, s, qs, per_graph, x0, noise, step_ptr, rng, len, F, x_t));
+  } else {
+    SD_CUDA(launch_k(angle_qsample_kernel<false>, grid, dim3(kGaussThreads), 0, s, qs, per_graph, x0, noise, step_ptr, rng,
+                     static_cast<const int*>(nullptr), F, x_t));
+  }
+  SD_LAUNCHED("angle_qsample", s);
+  return SEQDIFF_OK;
+}
+
+int angle_score_terms(int B, int per_graph, const float* pred, const float* noise, const float* mask, const int* step_ptr, int* advance,
+                      const uint64_t* rng, double* acc, cudaStream_t s, const int* len, int F) {
+  SD_CHECK(B > 0 && per_graph > 0 && F > 0 && per_graph % F == 0, "angle score terms: per_graph must be a positive multiple of F");
+  SD_CHECK(step_ptr && advance && rng, "angle score terms run inside a loop (step counter and RNG words on the device)");
+  const dim3 grid(ceil_div((per_graph + 3) / 4, kGaussThreads), B);
+  if (len) {
+    SD_CUDA(launch_k(angle_score_terms_kernel<true>, grid, dim3(kGaussThreads), 0, s, per_graph, pred, noise, mask, step_ptr, advance, rng, len,
+                     F, acc));
+  } else {
+    SD_CUDA(launch_k(angle_score_terms_kernel<false>, grid, dim3(kGaussThreads), 0, s, per_graph, pred, noise, mask, step_ptr, advance, rng,
+                     static_cast<const int*>(nullptr), F, acc));
+  }
+  SD_LAUNCHED("angle_score_terms", s);
   return SEQDIFF_OK;
 }
 

@@ -184,6 +184,15 @@ int angle_loss_bwd(int N, int F, const float* pred, const float* noise, const fl
 int gauss_step(const float* coef, int T, int B, int per_graph, const float* x_t, const float* model_out, const float* noise, uint64_t seed,
                uint64_t graph_id0, int step, const int* step_ptr, float* x_out, float* steps_out, cudaStream_t s, int* advance = nullptr, bool wrap = true,
                const uint64_t* rng = nullptr, const int* len = nullptr, int F = 0);  // rng / in-place (x_out == x_t) as in reverse_step()
+// Backbone score loop (Model::struct_score), step k = *step_ptr, (seed, graph_id0) = rng[0..1], per_graph = L * F:
+// angle_qsample: x_t = wrap(qs[k,0] * x0 + qs[k,1] * eps_k) (qs [T,2] = sqrt(alphabar), sqrt(1 - alphabar)); eps_k from noise [T, B*per_graph]
+// at entry k or from Philox keyed as in gauss_step.  The counter is not advanced.
+// angle_score_terms: acc [B*per_graph] fp64 += h(wrap(eps_k - pred)) at the valid elements (mask != 0; len: e < len[g] * F); the last CTA
+// to read the counter decrements it.  len != NULL (packed): only the valid elements are read or written by either kernel.
+int angle_qsample(const float* qs, int B, int per_graph, const float* x0, const float* noise, const int* step_ptr, const uint64_t* rng,
+                  float* x_t, cudaStream_t s, const int* len, int F);
+int angle_score_terms(int B, int per_graph, const float* pred, const float* noise, const float* mask, const int* step_ptr, int* advance,
+                      const uint64_t* rng, double* acc, cudaStream_t s, const int* len, int F);
 
 // ---- train_kernels.cu / attention_train.cu: the training step (reference model.py:313-367 under autograd) ------------
 // out[c][r] = in[r][c] for row-major [rows, cols]; colsum (optional, fp32 [cols]) += column sums (bias gradients); out may be NULL.

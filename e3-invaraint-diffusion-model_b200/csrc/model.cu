@@ -1170,6 +1170,7 @@ int Model::loop_setup(int precision, int P, int K, int Ll, int Lr, int T, const 
                       const float* lig_mask, const float* rec_seq_in, const float* rec_angle, const float* rec_mask, cudaStream_t caller,
                       int flags, bool scoring, LoopIO* io, cudaStream_t* ls) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
+  SD_CHECK(arch == kArchSequence, "handle holds a structure model: use seqdiff_struct_sample_multi / seqdiff_struct_score_multi");
   SD_CHECK(T >= 1 && P > 0 && K > 0 && Ll > 0 && Lr > 0, "bad sampling arguments");
   const int B = P * K;  // ligand graphs: sample j of pocket p is graph p * K + j
   SD_CHECK(cfg.feature_size == SEQDIFF_NUM_CLASSES, "sampling needs feature_size == 20");
@@ -1608,14 +1609,11 @@ int Model::struct_forward(int precision, int B, int Ll, int Lr, const float* tim
   }
 }
 
-// structure_model/sample.py:104-144.  The receptor branch runs ONCE (it sees neither t nor the ligand; the reference recomputes
-// it every step) and over the P pockets only; each step replays one captured graph: ligand branch + Gaussian reverse step + wrap.
-int Model::struct_sample(int precision, int P, int K, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
-                         const float* rec_seq_in, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
-                         uint64_t gid0, float* steps_out, float* final_out, cudaStream_t caller, int flags) {
+int Model::struct_loop_setup(int precision, int P, int K, int Ll, int Lr, int T, const float* table, const float* x_in, const float* lig_mask,
+                             const float* rec_seq_in, const float* rec_angle, const float* rec_mask, cudaStream_t caller, int flags,
+                             bool scoring, StructIO* io, cudaStream_t* ls) {
   SD_CHECK(finalized, "model not finalised (seqdiff_model_finalize)");
-  SD_CHECK(arch == kArchStructure, "handle holds a sequence model: use seqdiff_sample");
-  const PdlScope pdl_on(3);
+  SD_CHECK(arch == kArchStructure, scoring ? "handle holds a sequence model: use seqdiff_score_multi" : "handle holds a sequence model: use seqdiff_sample");
   SD_CHECK(T >= 1 && P > 0 && K > 0 && Ll > 0 && Lr > 0, "bad sampling arguments");
   const int B = P * K;  // ligand graphs: sample j of pocket p is graph p * K + j
   SD_CUDA(cudaSetDevice(device));
@@ -1624,7 +1622,9 @@ int Model::struct_sample(int precision, int P, int K, int Ll, int Lr, int T, con
     SD_CUDA(cudaEventCreateWithFlags(&ev_in, cudaEventDisableTiming));
     SD_CUDA(cudaEventCreateWithFlags(&ev_out, cudaEventDisableTiming));
   }
+  // everything below runs on the private stream, ordered after the caller's prior work
   cudaStream_t s = loop_stream;
+  *ls = s;
   SD_CUDA(cudaEventRecord(ev_in, caller));
   SD_CUDA(cudaStreamWaitEvent(s, ev_in, 0));
   const int F = cfg.feature_size;
@@ -1636,70 +1636,145 @@ int Model::struct_sample(int precision, int P, int K, int Ll, int Lr, int T, con
     SD_CUDA(cudaMalloc(reinterpret_cast<void**>(&samp_in), need_in + 16 * kGuardBytes));
     samp_in_bytes = need_in + 16 * kGuardBytes;
   }
-  const size_t tab_floats = static_cast<size_t>(T) * 4;
-  if (tab_floats > tables_cap) {
+  const size_t tab_floats = static_cast<size_t>(T) * (scoring ? 2 : 4);
+  if (!scoring && tab_floats > tables_cap) {
     if (d_tables) { SD_CUDA(cudaDeviceSynchronize()); SD_CUDA(cudaFree(d_tables)); d_tables = nullptr; tables_cap = 0; }
     SD_CUDA(cudaMalloc(reinterpret_cast<void**>(&d_tables), tab_floats * 4));
     tables_cap = tab_floats;
   }
   SD_TRY(ensure_workspace(struct_workspace_need(precision, B, Ll, Lr, K)));
   Bump bp(samp_in, s);
-  float* x_cur = bp.take<float>(Nl * F);
-  float* mout = bp.take<float>(Nl * F);
-  float* c_lmask = bp.take<float>(Nl);
-  float* c_rseq = bp.take<float>(Nr * 20);
-  float* c_rang = bp.take<float>(Nr * F);
-  float* c_rmask = bp.take<float>(Nr);
-  SD_CUDA(cudaMemcpyAsync(d_tables, coef_steps, tab_floats * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(x_cur, x_T, Nl * F * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_lmask, lig_mask, Nl * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_rseq, rec_seq_in, Nr * 20 * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_rang, rec_angle, Nr * F * 4, cudaMemcpyDefault, s));
-  SD_CUDA(cudaMemcpyAsync(c_rmask, rec_mask, Nr * 4, cudaMemcpyDefault, s));
+  io->x_cur = bp.take<float>(Nl * F);
+  io->mout = bp.take<float>(Nl * F);
+  io->c_lmask = bp.take<float>(Nl);
+  io->c_rseq = bp.take<float>(Nr * 20);
+  io->c_rang = bp.take<float>(Nr * F);
+  io->c_rmask = bp.take<float>(Nr);
+  // x0 | fp64 sums | q-sample table in a block of their own: scoring never moves the sampler's buffers (its cached graph stays valid).
+  // The table goes last, so the addresses the score's step graph holds depend on (B, Ll) and the block's base only, all in its key: a
+  // cached graph serves any T, and the kernels read the step from the device counter.
+  if (scoring) {
+    const size_t need_sc = align256(Nl * F * 4) + align256(Nl * F * 8) + align256(tab_floats * 4) + 4 * kGuardBytes;
+    if (need_sc > score_in_bytes) {
+      if (score_in) { SD_CUDA(cudaDeviceSynchronize()); debug_guard_begin(score_in); SD_CUDA(cudaFree(score_in)); score_in = nullptr; score_in_bytes = 0; }
+      SD_CUDA(cudaMalloc(reinterpret_cast<void**>(&score_in), need_sc));
+      score_in_bytes = need_sc;
+    }
+    Bump bs(score_in, s);
+    io->x0 = bs.take<float>(Nl * F);
+    io->acc = bs.take<double>(Nl * F);
+    io->qs = bs.take<float>(tab_floats);
+  }
+  SD_CUDA(cudaMemcpyAsync(scoring ? io->qs : d_tables, table, tab_floats * 4, cudaMemcpyDefault, s));
+  // scoring: x_cur starts as x0 too, so that the un-captured dry run of the ligand branch reads defined angles
+  SD_CUDA(cudaMemcpyAsync(io->x_cur, x_in, Nl * F * 4, cudaMemcpyDefault, s));
+  if (scoring) SD_CUDA(cudaMemcpyAsync(io->x0, x_in, Nl * F * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_lmask, lig_mask, Nl * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_rseq, rec_seq_in, Nr * 20 * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_rang, rec_angle, Nr * F * 4, cudaMemcpyDefault, s));
+  SD_CUDA(cudaMemcpyAsync(io->c_rmask, rec_mask, Nr * 4, cudaMemcpyDefault, s));
+  if (scoring) SD_CUDA(cudaMemsetAsync(io->acc, 0, Nl * F * 8, s));
   // ragged packing (flags bit 0): valid prefixes only, ligand offsets per sample and receptor offsets per pocket; needs the 16-bit
-  // kernels and prefix masks, otherwise the padded path runs.  The Gaussian step writes the padded positions of x_cur and steps_out as 0.
+  // kernels and prefix masks with a valid position in every complex, otherwise the padded path runs.
   const PackInfo* pk = nullptr;
   if ((flags & 1) && precision != SEQDIFF_FP32) {
     bool usable = false;
-    SD_TRY(build_pack(B, K, Ll, Lr, c_lmask, c_rmask, s, &usable));
+    SD_TRY(build_pack(B, K, Ll, Lr, io->c_lmask, io->c_rmask, s, &usable));
     if (usable) pk = &pack;
   }
-
-  GraphKey key;
+  io->pk = pk;
+  GraphKey& key = io->key;
   key.pack_hash = pk ? pk->hash : 0;
-  key.precision = precision; key.B = B; key.K = K; key.Ll = Ll; key.Lr = Lr; key.diverse = 0; key.noise = noise_steps;
-  key.ws_ptr = ws; key.in_ptr = samp_in; key.tab_ptr = d_tables; key.aux_ptr = steps_out; key.T = T;
+  key.precision = precision; key.B = B; key.K = K; key.Ll = Ll; key.Lr = Lr; key.diverse = 0;
+  key.ws_ptr = ws; key.in_ptr = samp_in;  // (seed, gid0) are NOT part of the key: device memory, see arm_loop_kernel
+  if (scoring) key.aux_ptr = score_in;
+  else key.tab_ptr = d_tables;
+  return SEQDIFF_OK;
+}
+
+template <typename Step>
+int Model::struct_replay(cudaGraphExec_t& exec, GraphKey& cached, int& kernels, const GraphKey& key, int precision, int K, int Ll, int Lr, int T,
+                         uint64_t seed, uint64_t gid0, const StructIO& io, cudaStream_t s, const Step& step) {
   uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
   // receptor branch once, eagerly (also the un-captured dry run that sets kernel attributes and fills the TMA descriptor cache)
   SD_CUDA(launch_k(arm_loop_kernel, dim3(1), dim3(1), 0, s, d_step, T - 1, d_rng, seed, gid0));
   SD_LAUNCHED("arm_loop", s);
-  const bool cached = graph_exec && key == graph_key;
-  SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lmask, c_rseq, c_rang, c_rmask, mout, cached ? 1 : 3, s, pk, K));
-  auto one_step = [&](cudaStream_t st) -> int {
-    SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, x_cur, c_lmask, c_rseq, c_rang, c_rmask, mout, 2, st, pk, K));
-    SD_TRY(gauss_step(d_tables, T, B, Ll * F, x_cur, mout, noise_steps, 0, 0, 0, d_step, x_cur, steps_out, st, d_step + 1, true, d_rng,
-                      pk ? pk->len_l : nullptr, F));
-    return SEQDIFF_OK;
-  };
-  if (!cached) {
-    if (graph_exec) { cudaGraphExecDestroy(graph_exec); graph_exec = nullptr; }
+  const bool hit = exec && key == cached;
+  SD_TRY(struct_forward(precision, key.B, Ll, Lr, nullptr, d_step, io.x_cur, io.c_lmask, io.c_rseq, io.c_rang, io.c_rmask, io.mout, hit ? 1 : 3, s,
+                        io.pk, K));
+  if (!hit) {
+    if (exec) { cudaGraphExecDestroy(exec); exec = nullptr; }
     SD_CUDA(cudaStreamSynchronize(s));
     cudaGraph_t graph = nullptr;
     const uint64_t l0 = g_launches.load();
     SD_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const int rc = one_step(s);
-    graph_kernels = static_cast<int>(g_launches.load() - l0);
+    const int rc = step(s);
+    kernels = static_cast<int>(g_launches.load() - l0);  // kernel nodes per replay
     cudaError_t ce = cudaStreamEndCapture(s, &graph);
     if (rc != SEQDIFF_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
     SD_CUDA(ce);
-    ce = cudaGraphInstantiate(&graph_exec, graph, 0);
+    ce = cudaGraphInstantiate(&exec, graph, 0);
     cudaGraphDestroy(graph);
     SD_CUDA(ce);
-    graph_key = key;
+    cached = key;
   }
-  for (int it = 0; it < T; ++it) SD_CUDA(cudaGraphLaunch(graph_exec, s));
-  g_launches.fetch_add(static_cast<uint64_t>(T) * graph_kernels, std::memory_order_relaxed);
-  SD_CUDA(cudaMemcpyAsync(final_out, x_cur, Nl * F * 4, cudaMemcpyDefault, s));
+  for (int it = 0; it < T; ++it) SD_CUDA(cudaGraphLaunch(exec, s));
+  g_launches.fetch_add(static_cast<uint64_t>(T) * kernels, std::memory_order_relaxed);  // replayed kernel nodes
+  return SEQDIFF_OK;
+}
+
+// structure_model/sample.py:104-144.  The receptor branch runs ONCE (it sees neither t nor the ligand; the reference recomputes
+// it every step) and over the P pockets only; each step replays one captured graph: ligand branch + Gaussian reverse step + wrap.
+int Model::struct_sample(int precision, int P, int K, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
+                         const float* rec_seq_in, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
+                         uint64_t gid0, float* steps_out, float* final_out, cudaStream_t caller, int flags) {
+  const PdlScope pdl_on(3);
+  StructIO io;
+  cudaStream_t s = nullptr;
+  SD_TRY(struct_loop_setup(precision, P, K, Ll, Lr, T, coef_steps, x_T, lig_mask, rec_seq_in, rec_angle, rec_mask, caller, flags, false, &io, &s));
+  const int B = P * K, F = cfg.feature_size;
+  const PackInfo* pk = io.pk;
+  GraphKey key = io.key;
+  key.noise = noise_steps; key.aux_ptr = steps_out; key.T = T;
+  uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
+  // the Gaussian step writes the padded positions of x_cur and steps_out as 0 in packed mode
+  auto one_step = [&](cudaStream_t st) -> int {
+    SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, io.x_cur, io.c_lmask, io.c_rseq, io.c_rang, io.c_rmask, io.mout, 2, st, pk, K));
+    SD_TRY(gauss_step(d_tables, T, B, Ll * F, io.x_cur, io.mout, noise_steps, 0, 0, 0, d_step, io.x_cur, steps_out, st, d_step + 1, true, d_rng,
+                      pk ? pk->len_l : nullptr, F));
+    return SEQDIFF_OK;
+  };
+  SD_TRY(struct_replay(graph_exec, graph_key, graph_kernels, key, precision, K, Ll, Lr, T, seed, gid0, io, s, one_step));
+  SD_CUDA(cudaMemcpyAsync(final_out, io.x_cur, static_cast<size_t>(B) * Ll * F * 4, cudaMemcpyDefault, s));
+  // ... and the caller's stream continues only after the loop has finished
+  SD_CUDA(cudaEventRecord(ev_out, s));
+  SD_CUDA(cudaStreamWaitEvent(caller, ev_out, 0));
+  return SEQDIFF_OK;
+}
+
+// Backbone score: one step is the training q-sample of x0 at step k (angle_qsample), the sampler's ligand branch at timestep k on it,
+// then the step's objective terms (angle_score_terms, which advances the step counter).  Same staging, packing, K-per-pocket receptor
+// rows and eager receptor branch as struct_sample(), but its own graph, key and input block.
+int Model::struct_score(int precision, int P, int K, int Ll, int Lr, int T, const float* qs_steps, const float* x0, const float* lig_mask,
+                        const float* rec_seq_in, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
+                        uint64_t gid0, double* terms_out, cudaStream_t caller, int flags) {
+  const PdlScope pdl_on(3);
+  StructIO io;
+  cudaStream_t s = nullptr;
+  SD_TRY(struct_loop_setup(precision, P, K, Ll, Lr, T, qs_steps, x0, lig_mask, rec_seq_in, rec_angle, rec_mask, caller, flags, true, &io, &s));
+  const int B = P * K, F = cfg.feature_size;
+  const PackInfo* pk = io.pk;
+  GraphKey key = io.key;
+  key.noise = noise_steps;
+  uint64_t* d_rng = reinterpret_cast<uint64_t*>(d_step + 16);
+  auto one_step = [&](cudaStream_t st) -> int {
+    SD_TRY(angle_qsample(io.qs, B, Ll * F, io.x0, noise_steps, d_step, d_rng, io.x_cur, st, pk ? pk->len_l : nullptr, F));
+    SD_TRY(struct_forward(precision, B, Ll, Lr, nullptr, d_step, io.x_cur, io.c_lmask, io.c_rseq, io.c_rang, io.c_rmask, io.mout, 2, st, pk, K));
+    SD_TRY(angle_score_terms(B, Ll * F, io.mout, noise_steps, io.c_lmask, d_step, d_step + 1, d_rng, io.acc, st, pk ? pk->len_l : nullptr, F));
+    return SEQDIFF_OK;
+  };
+  SD_TRY(struct_replay(score_exec, score_key, score_kernels, key, precision, K, Ll, Lr, T, seed, gid0, io, s, one_step));
+  SD_CUDA(cudaMemcpyAsync(terms_out, io.acc, static_cast<size_t>(B) * Ll * F * 8, cudaMemcpyDefault, s));
   SD_CUDA(cudaEventRecord(ev_out, s));
   SD_CUDA(cudaStreamWaitEvent(caller, ev_out, 0));
   return SEQDIFF_OK;

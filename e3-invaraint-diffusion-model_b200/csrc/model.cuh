@@ -200,7 +200,7 @@ struct Model {
   int score(int precision, int P, int K, int Ll, int Lr, int T, const float* q_tables, const float* x0, const float* lig_angle,
             const float* lig_mask, const float* rec_seq, const float* rec_angle, const float* rec_mask, const float* noise_E,
             uint64_t seed, uint64_t gid0, double* terms_out, cudaStream_t s, int flags = 0);
-  uint8_t* score_in = nullptr;  // x0 + the fp64 sums of the scoring loop (grow-only)
+  uint8_t* score_in = nullptr;  // x0 + the fp64 sums of the scoring loop (grow-only; a structure handle adds the q-sample table)
   size_t score_in_bytes = 0;
   cudaGraphExec_t score_exec = nullptr;
   int score_kernels = 0;
@@ -283,6 +283,33 @@ struct Model {
   int struct_sample(int precision, int P, int K, int Ll, int Lr, int T, const float* coef_steps, const float* x_T, const float* lig_mask,
                     const float* rec_seq, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
                     uint64_t gid0, float* steps_out, float* final_out, cudaStream_t s, int flags = 0);
+  // The same loop scoring given backbones x0 (P * K graphs) under the structure model's training objective: T x (q-sample x_k from x0
+  // at step k -> ligand branch at timestep k -> terms += h(wrap(eps_k - pred))), replayed from its own captured graph (score_exec /
+  // score_key, which a structure handle does not otherwise use), so that alternating sample / score calls keep both graphs.
+  // qs_steps [T, 2] = (sqrt(alphabar), sqrt(1 - alphabar)); terms_out [P * K, Ll, F] fp64 (device or host): per element, the sum over
+  // the steps of the wrapped smooth-L1; 0 at masked positions.  flags bit 0: ragged packing (bit-identical terms at valid positions).
+  int struct_score(int precision, int P, int K, int Ll, int Lr, int T, const float* qs_steps, const float* x0, const float* lig_mask,
+                   const float* rec_seq, const float* rec_angle, const float* rec_mask, const float* noise_steps, uint64_t seed,
+                   uint64_t gid0, double* terms_out, cudaStream_t s, int flags = 0);
+  // what struct_sample() and struct_score() share: the loop's buffers in the persistent input block, the packing and the step-graph key
+  struct StructIO {
+    float *x_cur, *mout, *c_lmask, *c_rseq, *c_rang, *c_rmask;
+    float* x0 = nullptr;    // score only, in score_in: the scored backbones ...
+    double* acc = nullptr;  // ... the [B * Ll, F] fp64 sums (zeroed by struct_loop_setup) ...
+    float* qs = nullptr;    // ... and, last (its size depends on T), the [T, 2] q-sample table
+    const PackInfo* pk = nullptr;
+    GraphKey key;
+  };
+  // Private stream ordered after `caller`, persistent copies of the inputs (x_in -> x_cur, and -> x0 for scoring), the step table
+  // (sampling: coef -> d_tables; scoring: qs -> the score block), the workspace and the packing (flags bit 0).  Returns the stream in *ls.
+  int struct_loop_setup(int precision, int P, int K, int Ll, int Lr, int T, const float* table, const float* x_in, const float* lig_mask,
+                        const float* rec_seq, const float* rec_angle, const float* rec_mask, cudaStream_t caller, int flags, bool scoring,
+                        StructIO* io, cudaStream_t* ls);
+  // Arms the step counter at T - 1 with the Philox key (seed, gid0), runs the receptor branch eagerly (with the ligand branch as the
+  // un-captured dry run when `step` has to be (re)captured into `exec`, i.e. unless `key` matches the cached key), replays T times.
+  template <typename Step>
+  int struct_replay(cudaGraphExec_t& exec, GraphKey& cached, int& kernels, const GraphKey& key, int precision, int K, int Ll, int Lr, int T,
+                    uint64_t seed, uint64_t gid0, const StructIO& io, cudaStream_t s, const Step& step);
 
  public:
   void* dalloc(size_t bytes);

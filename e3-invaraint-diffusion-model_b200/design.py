@@ -75,6 +75,33 @@ def sequence_schedule(timesteps=None, noise_schedule=None, transition=None):
     return T_q, noise_schedule, transition
 
 
+def structure_schedule(struct_betas=None, struct_timesteps=None):
+    """(T, betas) of the design's structure sampler: the cosine schedule of structure_model.CONFIG["timesteps"] steps unless given"""
+    if struct_betas is None:
+        T_s = SM.CONFIG["timesteps"] if struct_timesteps is None else int(struct_timesteps)
+        struct_betas = SM.cosine_beta_schedule(T_s)
+    T_s = len(struct_betas) if struct_timesteps is None else int(struct_timesteps)
+    return T_s, struct_betas
+
+
+def score_design_backbones(struct_model, batch, K: int, backbone_angles, packed: bool = True, seed=None, struct_betas=None,
+                           struct_timesteps=None):
+    """backbone_loss [P*K] of design()'s backbones of one batch: backbone j of pocket p (angles trimmed to the ligand length, zero-padded
+    back to the structure model's length) scored under its pocket with the design's structure schedule (structure_model.score_backbones).
+    Philox graph ids continue the process-wide stream."""
+    Ls = struct_model.encoder_config.max_position_embeddings
+    _, st = structure_inputs(batch, Ls)
+    n, Ll_s = len(backbone_angles), st["ligand_attn_mask"].shape[1]
+    x0 = torch.zeros((n, Ll_s, struct_model.feature_size), dtype=torch.float32)
+    for i, a in enumerate(backbone_angles):
+        a = torch.as_tensor(a, dtype=torch.float32)
+        x0[i, :a.shape[0]] = a
+    T_s, betas = structure_schedule(struct_betas, struct_timesteps)
+    loss, _ = SM.score_backbones(struct_model, st["ligand_attn_mask"], x0, st["receptor_seq"], st["receptor_attn_mask"], st["receptor_angles"],
+                                 T_s, betas, seed=seed, packed=packed, num_samples=K)
+    return loss.tolist()
+
+
 def score_designs(seq_model, batch, K: int, backbone_angles, pred_sequences, packed: bool = True, seed=None, timesteps=None, noise_schedule=None,
                   transition=None):
     """(nll_per_residue, perplexity) of design()'s rows of one batch: each predicted sequence scored under its pocket and its own generated
@@ -112,10 +139,7 @@ def design_tensors(struct_model, seq_model, batch, num_backbones: int = 1, num_s
     lig_len, st = structure_inputs(batch, Ls)
     Ll_s = st["ligand_attn_mask"].shape[1]
     Fs = struct_model.feature_size
-    if struct_betas is None:
-        T_s = SM.CONFIG["timesteps"] if struct_timesteps is None else int(struct_timesteps)
-        struct_betas = SM.cosine_beta_schedule(T_s)
-    T_s = len(struct_betas) if struct_timesteps is None else int(struct_timesteps)
+    T_s, struct_betas = structure_schedule(struct_betas, struct_timesteps)
     if x_T is None:
         x_T = start_noise(P * K1, Ll_s, Fs)
     if graph_id0 is None:
@@ -159,25 +183,32 @@ def design(struct_model, seq_model, batch, num_backbones: int = 1, num_sequences
 
 
 def design_dataset(dataloader, struct_model, seq_model, num_backbones: int = 1, num_sequences: int = 1, output_path=None, design_fn=None,
-                   score: bool = False, **kw):
+                   score: bool = False, score_backbones: bool = False, **kw):
     """Every batch of `dataloader` through `design`; returns sample_dataset's DataFrame (structure_ids / true_sequence /
     predict_sequence / recovery_rate) plus a `backbone` column, pickled to `output_path` like sample_dataset when given.
     score=True adds `nll_per_residue` and `perplexity`: each predicted sequence scored under its pocket and its own backbone
-    (score_designs), the candidates' model score where no native peptide exists."""
+    (score_designs), the candidates' model score where no native peptide exists.
+    score_backbones=True adds `backbone_loss`: each backbone scored once under its pocket by the structure model's training objective
+    averaged over the timesteps (score_design_backbones, with the design's struct_betas / struct_timesteps, seed and packing), repeated
+    over the backbone's num_sequences rows; lower = more native-like to the structure model."""
     import pandas as pd
     K1, K2 = _check_counts(num_backbones, num_sequences)
     fn = design if design_fn is None else design_fn
     skw = {k: kw[k] for k in ("packed", "seed", "timesteps", "noise_schedule", "transition") if k in kw}
+    bkw = {k: kw[k] for k in ("packed", "seed", "struct_betas", "struct_timesteps") if k in kw}
     rows = []
     for idx, batch in enumerate(dataloader):
         print(f"Generating Batch {idx}")
         ids, backbone, angles, true_seqs, pred_seqs, rates = fn(struct_model, seq_model, batch, K1, K2, **kw)
+        cols = [ids, true_seqs, pred_seqs, rates, backbone]
         if score:
-            rows.extend(zip(ids, true_seqs, pred_seqs, rates, backbone, *score_designs(seq_model, batch, K1 * K2, angles, pred_seqs, **skw)))
-        else:
-            rows.extend(zip(ids, true_seqs, pred_seqs, rates, backbone))
+            cols.extend(score_designs(seq_model, batch, K1 * K2, angles, pred_seqs, **skw))
+        if score_backbones:
+            loss = score_design_backbones(struct_model, batch, K1, angles[::K2], **bkw)
+            cols.append([loss[i // K2] for i in range(len(ids))])
+        rows.extend(zip(*cols))
     columns = ["structure_ids", "true_sequence", "predict_sequence", "recovery_rate", "backbone"]
-    res = pd.DataFrame(rows, columns=columns + (["nll_per_residue", "perplexity"] if score else []))
+    res = pd.DataFrame(rows, columns=columns + (["nll_per_residue", "perplexity"] if score else []) + (["backbone_loss"] if score_backbones else []))
     if output_path is not None:
         res.to_pickle(output_path)
     return res

@@ -351,6 +351,95 @@ def p_sample_loop(model, ligand_mask, ligand_angle_noise, receptor_seq, receptor
     return (hist if keep_history else final[None]).cpu()
 
 
+def qsample_coefficients(betas: torch.Tensor) -> torch.Tensor:
+    """[T,2] fp32 table of the training q-sample, indexed by step: (sqrt(alphabar), sqrt(1 - alphabar)) of compute_alphas(betas)"""
+    ab = compute_alphas(betas.detach().float().cpu())
+    return torch.stack([ab["sqrt_alphas_cumprod"], ab["sqrt_one_minus_alphas_cumprod"]], dim=1).contiguous()
+
+
+@torch.no_grad()
+def score_backbones_tensors(model, ligand_mask, backbones, receptor_seq, receptor_mask, receptor_angle, total_timesteps: int, betas, *,
+                            noise_steps: Optional[torch.Tensor] = None, graph_id0: Optional[int] = None, seed: Optional[int] = None,
+                            packed: bool = False, num_samples: int = 1) -> torch.Tensor:
+    """The structure model's training objective for given backbones in their pockets, at every timestep (seqdiff_struct_score_multi):
+    for k = T-1 .. 0, x_k = wrap(sqrt(alphabar_k) x0 + sqrt(1 - alphabar_k) eps_k) (the training q-sample), pred = the denoiser at
+    timestep k, terms += h(wrap(eps_k - pred)) with FoldingDiff's smooth-L1 h (beta = pi/10), from one captured CUDA graph per step.
+    Arguments in p_sample_loop's order; `backbones` [P*K, L, F] are the scored angles x0, `ligand_mask` [P*K, L] or [P, L] (repeated),
+    the receptor tensors hold the P pockets, `betas` [T] is the schedule compute_alphas() turns into the q-sample's coefficients.
+    Returns terms [P*K, L, F] fp64 on the model's device: per position and feature, the sum over the T steps, 0 at masked positions
+    (score_backbones forms the per-backbone loss).  `noise_steps` [T, P*K, L, F]: explicit eps, entry k at step k; else Philox keyed as
+    the sampler's noise, graph_id0 = None continuing the process-wide stream.  `packed` / `num_samples` as in p_sample_loop: packed terms
+    equal the padded ones at the valid positions.  ValueError (before any device work) for disagreeing shapes, betas not of length T,
+    a complex without a valid ligand position, non-finite backbones (padded rows reach the valid ones through 0 * NaN in attention) or
+    a bad num_samples."""
+    K = check_num_samples(num_samples)
+    T = int(total_timesteps)
+    if T < 1:
+        raise ValueError(f"total_timesteps must be >= 1, got {total_timesteps}")
+    Fs = model.feature_size
+    if receptor_seq.dim() != 3 or receptor_seq.shape[2] != 20:
+        raise ValueError(f"receptor_seq must be [P, L_rec, 20], got {tuple(receptor_seq.shape)}")
+    P, Lr = receptor_seq.shape[0], receptor_seq.shape[1]
+    B = P * K
+    if backbones.dim() != 3 or tuple(backbones.shape[::2]) != (B, Fs):
+        raise ValueError(f"backbones must be [P*K, L, F] = [{B}, L, {Fs}], got {tuple(backbones.shape)}")
+    Ll = backbones.shape[1]
+    if K > 1 and tuple(ligand_mask.shape) == (P, Ll):
+        ligand_mask = ligand_mask.repeat_interleave(K, dim=0)
+    for x, name, shape in ((ligand_mask, "ligand_mask", (B, Ll)), (receptor_mask, "receptor_mask", (P, Lr)),
+                           (receptor_angle, "receptor_angle", (P, Lr, Fs))):
+        if tuple(x.shape) != shape:
+            raise ValueError(f"{name} must be {shape}, got {tuple(x.shape)}")
+    betas = torch.as_tensor(betas)
+    if betas.dim() != 1 or betas.shape[0] != T:
+        raise ValueError(f"betas must hold one value per timestep ({T}), got shape {tuple(betas.shape)}")
+    if noise_steps is not None and tuple(noise_steps.shape) != (T, B, Ll, Fs):
+        raise ValueError(f"noise_steps must be [T, P*K, L, F] = {(T, B, Ll, Fs)}, got {tuple(noise_steps.shape)}")
+    if not bool((ligand_mask != 0).any(dim=1).all()):
+        raise ValueError("every backbone needs at least one valid ligand position to be scored")
+    if not bool(torch.isfinite(backbones).all()):
+        raise ValueError("backbones must be finite everywhere, padded positions included")
+    qs = qsample_coefficients(betas)
+
+    h = model._sync_handle()
+    dev = model._handle_dev
+    if graph_id0 is None:
+        graph_id0 = _cabi.GRAPH_IDS.take(B)
+
+    def dv(x):
+        return x.to(device=dev, dtype=torch.float32).contiguous()
+
+    terms = torch.empty((B, Ll, Fs), device=dev, dtype=torch.float64)
+    args = [dv(qs), dv(backbones), dv(ligand_mask), dv(receptor_seq), dv(receptor_angle), dv(receptor_mask)]
+    z = None if noise_steps is None else dv(noise_steps)
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _cabi.check(_cabi.lib().seqdiff_struct_score_multi(h, model._precision_code(), P, K, Ll, Lr, T, *map(_cabi.ptr, args), _cabi.ptr(z),
+                                                           SEED if seed is None else seed, graph_id0, 1 if packed else 0, _cabi.ptr(terms),
+                                                           stream))
+    return terms
+
+
+def backbone_loss(terms: torch.Tensor, ligand_mask: torch.Tensor, total_timesteps: int):
+    """(loss [B], per_feature [B, F]) fp64 on the host from score_backbones_tensors' terms: per_feature[b, f] = sum_l terms[b, l, f] /
+    (T * n_b) over the n_b valid positions, loss = mean_f per_feature -- the training objective averaged over the T timesteps"""
+    t = terms.detach().cpu()
+    n = (ligand_mask.detach().cpu() != 0).sum(dim=1).double()
+    if n.shape[0] != t.shape[0]:
+        n = n.repeat_interleave(t.shape[0] // n.shape[0])
+    per_feature = t.sum(dim=1) / (int(total_timesteps) * n[:, None])
+    return per_feature.mean(dim=-1), per_feature
+
+
+@torch.no_grad()
+def score_backbones(model, ligand_mask, backbones, receptor_seq, receptor_mask, receptor_angle, total_timesteps: int, betas, **kw):
+    """score_backbones_tensors on the host: (loss [P*K], per_feature [P*K, F]) fp64, one entry per backbone in (pocket, backbone) order.
+    loss is the structure model's training objective for the backbone in its pocket, averaged over the T timesteps (one noise draw per
+    step): lower = more native-like to the model.  It is a ranking score, not a likelihood."""
+    terms = score_backbones_tensors(model, ligand_mask, backbones, receptor_seq, receptor_mask, receptor_angle, total_timesteps, betas, **kw)
+    return backbone_loss(terms, ligand_mask, total_timesteps)
+
+
 def sample(model, test_angle_ds, first_batch_only: bool = True, loop_fn=None, num_samples: int = 1, **kw):
     """reference structure_model/sample.py:191-229: chunk the dataset's features into batches of CONFIG["batch_size"], draw the start
     noise with the dataset's own `sample_noise`, run `p_sample_loop`, and trim every complex to its ligand length -> a list of numpy

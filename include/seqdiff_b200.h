@@ -307,6 +307,28 @@ SEQDIFF_API int seqdiff_struct_sample_multi(seqdiff_model_t* m, int precision, i
                                 const float* receptor_angles, const float* receptor_mask, const float* noise_steps, uint64_t seed,
                                 uint64_t graph_id0, int flags, float* steps_out, float* final_out, void* stream);
 
+/* ---- backbone score: the structure model's training objective for given backbones in their pockets, at every timestep (no reference
+ * counterpart).  Same batch layout, packing (flags bit 0), K-per-pocket receptor branch and Philox keying as seqdiff_struct_sample_multi;
+ * x0 [P*K,L_lig,F] = the scored backbone angles (finite everywhere), qs_steps [T,2] = (sqrt_alphas_cumprod, sqrt_one_minus_alphas_cumprod)
+ * of compute_alphas(betas) in fp32.  Step k = T-1 .. 0 is replayed from a captured CUDA graph of its own (sampling and scoring on one
+ * handle keep both graphs):
+ *   eps_k ~ N(0,1) [P*K,L_lig,F]: noise_steps[k] [P*K*L_lig*F], or Philox4x32-10 + Box-Muller keyed like the sampler's z:
+ *           (seed, graph_id0 + graph, 4-element group inside the padded graph, k);
+ *   x_k   = wrap(qs[k,0] * x0 + qs[k,1] * eps_k), fp32, each operation rounded in this order (the training q-sample);
+ *   pred  = the denoiser at timestep k (the raw step index, as the sampler feeds it);
+ *   terms += h(wrap(eps_k - pred)), the training loss's wrapped smooth-L1 (beta = pi/10), in fp64 at every valid position.
+ * terms_out [P*K,L_lig,F] f64 (device or host): per position and feature, the sum over the T steps; 0 where ligand_mask == 0.  The
+ * backbone's score is loss = mean_f sum_l terms[l, f] / (T * n_valid): a Monte-Carlo estimate, stratified over t with one draw per step,
+ * of the training objective E_{t, eps}[loss] for this complex -- lower = more native-like to the model.
+ * A ranking score, not a likelihood.  Sums are per element in step order: bit-reproducible; packed equals padded at the valid positions.
+ * P < 1, K < 1, T < 1, P*K > 65535 (the step kernels put one graph per grid row; split larger batches over calls with offset
+ * graph_id0, which gives the same terms), P*K*max(L_lig, L_rec) > INT32_MAX, unknown flag bits or a sequence-model handle:
+ * SEQDIFF_ERR_INVALID. */
+SEQDIFF_API int seqdiff_struct_score_multi(seqdiff_model_t* m, int precision, int P, int K, int L_lig, int L_rec, int T,
+                               const float* qs_steps, const float* x0, const float* ligand_mask, const float* receptor_seq,
+                               const float* receptor_angles, const float* receptor_mask, const float* noise_steps, uint64_t seed,
+                               uint64_t graph_id0, int flags, double* terms_out, void* stream);
+
 /* ==== structure-model training step: replaces autograd over ConditionalBertForDiffusion.training_step (structure_model/model.py)
  * The flat parameter space, the gradient buckets and the optimizer are those of the sequence model's step: seqdiff_train_param_count /
  * _param_table / _grad_buckets / _set_bucket_events, seqdiff_adamw_step and seqdiff_model_get_tensor accept a structure handle.  Trainable
