@@ -75,6 +75,16 @@ PROTOTYPES = {
     "seqdiff_op_philox_u32": (_i, [_u64, _u64, _u32, _i, _i, _vp, _vp]),
     "seqdiff_op_gemm_ex": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "seqdiff_op_attention_packed": (_i, [_i, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "seqdiff_op_dropout_add_layernorm": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, C.c_float, C.c_float, _u64, _u32, _u32, _vp, _vp, _vp, _vp]),
+    "seqdiff_op_layernorm_bwd": (_i, [_i, _i, _i, _vp, _vp, _vp, C.c_float, _vp, _vp, _vp, C.c_float, _u64, _u32, _u32, _vp, _vp, _vp, _vp]),
+    "seqdiff_op_ln_modulate_bwd": (_i, [_i, _i, _i, _vp, _vp, _i, _vp, _vp, C.c_float, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "seqdiff_op_embed_bwd": (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, C.c_float, C.c_float, _u64, _u32, _u32, _vp, _vp, _vp, _vp, _vp]),
+    "seqdiff_op_predictor_tail_bwd": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, C.c_float, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "seqdiff_op_train_elementwise": (_i, [_i, _i, _i64, _i, _vp, _vp, C.c_float, _u64, _u32, _u32, _vp, _vp]),
+    "seqdiff_op_transpose_colsum": (_i, [_i, _i, _i, _vp, _vp, _i, _vp, _vp]),
+    "seqdiff_op_colsum_add": (_i, [_i, _i, _i, _vp, _vp, _vp]),
+    "seqdiff_op_loss_bwd": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "seqdiff_op_angle_loss_bwd": (_i, [_i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 _LIB = None

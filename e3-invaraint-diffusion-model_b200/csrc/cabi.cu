@@ -568,4 +568,168 @@ int seqdiff_op_attention_packed(int precision, int B, int heads, int Lq, int Lk,
   SD_GUARD_END
 }
 
+// ---- training-step rowwise / elementwise kernels, operator level (train_kernels.cu, decode_loss.cu) ----------------------------------------
+// Thin: every form a kernel does not implement is rejected here, before anything reaches the device; the launchers are called as the training
+// step calls them.  Row-vector operands are read and written 16 bytes at a time, so their pointers must be 16 B aligned; the accumulated
+// parameter gradients may sit at any float offset (the flushes pick 128-bit or scalar atomics from the alignment).
+}  // extern "C"
+namespace {
+bool is_a16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+bool rowwise_h(int H) { return H == 256 || H == 512 || H == 768 || H == 1024; }
+bool mode_ok(int precision) { return precision == SEQDIFF_FP32 || precision == SEQDIFF_BF16 || precision == SEQDIFF_FP16; }
+}  // namespace
+extern "C" {
+
+int seqdiff_op_dropout_add_layernorm(int precision, int M, int H, float* d, const float* resid, const float* ln_w, const float* ln_b, float eps,
+                                     float p, uint64_t seed, uint32_t site, uint32_t step, float* out32, void* out16, uint8_t* keep_bits,
+                                     void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(d && resid && ln_w && ln_b, "null argument");
+  SD_CHECK(mode_ok(precision) && M > 0 && rowwise_h(H), "precision, M > 0 and H in {256, 512, 768, 1024}");
+  SD_CHECK(precision != SEQDIFF_FP32 || !out16, "FP32 has no 16-bit output");
+  SD_CHECK(is_a16(d) && is_a16(resid) && is_a16(ln_w) && is_a16(ln_b) && is_a16(out32) && is_a16(out16), "row pointers must be 16 B aligned");
+  const DropSpec dr{p, site, step, seed};
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (precision == SEQDIFF_FP32) return dropout_add_layernorm<float>(d, resid, dr, M, H, ln_w, ln_b, eps, out32, nullptr, keep_bits, s);
+  if (precision == SEQDIFF_BF16)
+    return dropout_add_layernorm<bf16>(d, resid, dr, M, H, ln_w, ln_b, eps, out32, static_cast<bf16*>(out16), keep_bits, s);
+  return dropout_add_layernorm<f16>(d, resid, dr, M, H, ln_w, ln_b, eps, out32, static_cast<f16*>(out16), keep_bits, s);
+  SD_GUARD_END
+}
+
+int seqdiff_op_layernorm_bwd(int precision, int M, int H, const float* dh, const float* o, const float* gamma, float eps, float* d_o, float* dgamma,
+                             float* dbeta, float p, uint64_t seed, uint32_t site, uint32_t step, const uint8_t* keep_bits, void* g16, float* dbias,
+                             void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(dh && o && gamma && d_o && dgamma && dbeta, "null argument");
+  SD_CHECK(mode_ok(precision) && M > 0 && rowwise_h(H), "precision, M > 0 and H in {256, 512, 768, 1024}");
+  SD_CHECK(is_a16(dh) && is_a16(o) && is_a16(gamma) && is_a16(d_o) && is_a16(g16), "row pointers must be 16 B aligned");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (precision == SEQDIFF_FP32) {
+    SD_CHECK(!g16 && !dbias && !keep_bits && p == 0.f, "FP32: the plain LayerNorm backward (no 16-bit operand, bias gradient or dropout)");
+    return layernorm_bwd(dh, o, M, H, gamma, eps, d_o, dgamma, dbeta, s);
+  }
+  SD_CHECK(g16 && dbias, "16-bit modes: the 16-bit dY operand and the bias gradient are required");
+  const DropSpec dr{p, site, step, seed};
+  if (precision == SEQDIFF_BF16)
+    return layernorm_bwd_cast<bf16>(dh, o, M, H, gamma, eps, d_o, dgamma, dbeta, dr, keep_bits, static_cast<bf16*>(g16), dbias, s);
+  return layernorm_bwd_cast<f16>(dh, o, M, H, gamma, eps, d_o, dgamma, dbeta, dr, keep_bits, static_cast<f16*>(g16), dbias, s);
+  SD_GUARD_END
+}
+
+int seqdiff_op_ln_modulate_bwd(int precision, int M, int H, const float* dout, const float* in, int affine_first, const float* lnw, const float* lnb,
+                               float eps1, const void* mod, int mod_div, int chunk0, float* din, float* sum_out, void* dmodT, float* dmod32,
+                               float* dgamma, float* dbeta, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(dout && in && mod && din, "null argument");
+  SD_CHECK(mode_ok(precision) && M > 0 && rowwise_h(H), "precision, M > 0 and H in {256, 512, 768, 1024}");
+  SD_CHECK(!affine_first || (lnw && lnb && dgamma && dbeta), "affine_first needs the LayerNorm affine and its gradients");
+  SD_CHECK((dmodT != nullptr) != (dmod32 != nullptr), "exactly one of dmodT / dmod32");
+  SD_CHECK(mod_div >= 1 && (!dmodT || mod_div == 1), "mod_div >= 1; per-token rows (dmodT) need mod_div == 1");
+  SD_CHECK(chunk0 >= 0 && chunk0 <= 3, "chunk0: the (shift, scale, gate) triple starts at chunk 0 .. 3 of the 6H row");
+  SD_CHECK(is_a16(dout) && is_a16(in) && is_a16(lnw) && is_a16(lnb) && is_a16(mod) && is_a16(din) && is_a16(sum_out) && is_a16(dmodT),
+           "row pointers must be 16 B aligned");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+#define SD_LMB(T) ln_modulate_bwd<T>(dout, in, M, H, affine_first != 0, lnw, lnb, eps1, static_cast<const T*>(mod), mod_div, chunk0, din, sum_out, \
+                                     static_cast<T*>(dmodT), dmod32, dgamma, dbeta, s)
+  if (precision == SEQDIFF_FP32) return SD_LMB(float);
+  if (precision == SEQDIFF_BF16) return SD_LMB(bf16);
+  return SD_LMB(f16);
+#undef SD_LMB
+  SD_GUARD_END
+}
+
+int seqdiff_op_embed_bwd(int M, int fin, int H, const float* dout, const float* x, const float* Wt, const float* b, const float* gamma, float eps,
+                         float p, uint64_t seed, uint32_t site, uint32_t step, float* dW, float* db, float* dgamma, float* dbeta, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(dout && x && Wt && b && gamma && dW && db && dgamma && dbeta, "null argument");
+  SD_CHECK(M > 0 && rowwise_h(H) && fin >= 1 && fin <= 32, "M > 0, H in {256, 512, 768, 1024} and fin in [1, 32]");
+  SD_CHECK(is_a16(dout) && is_a16(Wt) && is_a16(b) && is_a16(gamma), "row pointers must be 16 B aligned");
+  return embed_bwd(dout, x, M, fin, H, Wt, b, gamma, eps, DropSpec{p, site, step, seed}, dW, db, dgamma, dbeta, static_cast<cudaStream_t>(stream));
+  SD_GUARD_END
+}
+
+int seqdiff_op_predictor_tail_bwd(int precision, int M, int H, int F, const float* dlogits, const void* y, const float* gamma, const float* beta,
+                                  float eps, const float* W2, float* dy, float* dW2, float* db2, float* dgamma, float* dbeta, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(dlogits && y && gamma && beta && W2 && dy && dW2 && db2 && dgamma && dbeta, "null argument");
+  SD_CHECK(mode_ok(precision) && M > 0 && rowwise_h(H) && (F == 8 || F == 20), "precision, M > 0, H in {256, 512, 768, 1024} and F in {8, 20}");
+  SD_CHECK(is_a16(y) && is_a16(gamma) && is_a16(beta) && is_a16(W2) && is_a16(dy), "row pointers must be 16 B aligned");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+#define SD_PTB(T) predictor_tail_bwd<T>(dlogits, static_cast<const T*>(y), M, H, gamma, beta, eps, W2, F, dy, dW2, db2, dgamma, dbeta, s)
+  if (precision == SEQDIFF_FP32) return SD_PTB(float);
+  if (precision == SEQDIFF_BF16) return SD_PTB(bf16);
+  return SD_PTB(f16);
+#undef SD_PTB
+  SD_GUARD_END
+}
+
+int seqdiff_op_train_elementwise(int op, int precision, int64_t n, int kind, const void* in, const void* aux, float p, uint64_t seed, uint32_t site,
+                                 uint32_t step, void* out, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(out && (in || op == 4), "null argument");
+  SD_CHECK(mode_ok(precision) && n > 0 && n % 8 == 0, "precision and n > 0, n % 8 == 0");
+  SD_CHECK(op >= 0 && op <= 4, "op: 0 act_fwd, 1 act_bwd, 2 act_bwd (fp32 gradient), 3 grad_cast, 4 dropout_add");
+  SD_CHECK(op > 2 || kind == 1 || kind == 2, "activation kind: 1 erf-GELU, 2 SiLU");
+  SD_CHECK(op == 0 || op == 3 || op == 4 || aux, "act_bwd needs z");
+  SD_CHECK(op != 4 || precision == SEQDIFF_FP32, "dropout_add is fp32");
+  SD_CHECK(is_a16(in) && is_a16(aux) && is_a16(out), "pointers must be 16 B aligned");
+  const DropSpec dr{p, site, step, seed};
+  const size_t m = static_cast<size_t>(n);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (op == 4) return dropout_add(static_cast<float*>(out), static_cast<const float*>(in), m, dr, s);
+#define SD_EW(T)                                                                                                                          \
+  switch (op) {                                                                                                                           \
+    case 0: return act_fwd<T>(static_cast<const T*>(in), m, kind, dr, static_cast<T*>(out), s);                                          \
+    case 1: return act_bwd<T, T>(static_cast<const T*>(in), static_cast<const T*>(aux), m, kind, dr, static_cast<T*>(out), s);           \
+    case 2: return act_bwd<T, float>(static_cast<const float*>(in), static_cast<const T*>(aux), m, kind, dr, static_cast<T*>(out), s);   \
+    default: return grad_cast<T>(static_cast<const float*>(in), m, dr, static_cast<T*>(out), s);                                        \
+  }
+  if (precision == SEQDIFF_FP32) { SD_EW(float) }
+  if (precision == SEQDIFF_BF16) { SD_EW(bf16) }
+  SD_EW(f16)
+#undef SD_EW
+  SD_GUARD_END
+}
+
+int seqdiff_op_transpose_colsum(int precision, int rows, int cols, const void* in, void* out, int pitch, float* colsum, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(in && (out || colsum), "null argument");
+  SD_CHECK(mode_ok(precision) && rows > 0 && cols > 0, "precision, rows > 0 and cols > 0");
+  SD_CHECK(pitch == 0 || (pitch >= rows && pitch - rows < 64), "pitch: 0 (= rows) or rows rounded up by less than one 64-row tile");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (precision == SEQDIFF_FP32)
+    return transpose_colsum<float>(static_cast<const float*>(in), rows, cols, static_cast<float*>(out), colsum, s, pitch);
+  if (precision == SEQDIFF_BF16) return transpose_colsum<bf16>(static_cast<const bf16*>(in), rows, cols, static_cast<bf16*>(out), colsum, s, pitch);
+  return transpose_colsum<f16>(static_cast<const f16*>(in), rows, cols, static_cast<f16*>(out), colsum, s, pitch);
+  SD_GUARD_END
+}
+
+int seqdiff_op_colsum_add(int precision, int rows, int cols, const void* in, float* colsum, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(in && colsum, "null argument");
+  SD_CHECK(precision == SEQDIFF_BF16 || precision == SEQDIFF_FP16, "the column sum exists for the 16-bit modes");
+  SD_CHECK(rows > 0 && cols > 0 && cols % 8 == 0 && is_a16(in), "rows > 0, cols a multiple of 8, 16 B aligned input");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (precision == SEQDIFF_BF16) return colsum_add<bf16>(static_cast<const bf16*>(in), rows, cols, colsum, s);
+  return colsum_add<f16>(static_cast<const f16*>(in), rows, cols, colsum, s);
+  SD_GUARD_END
+}
+
+int seqdiff_op_loss_bwd(int N, const float* logits, const float* x0, const float* x_t, const double* terms, float* dlogits, void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(logits && x0 && x_t && terms && dlogits, "null argument");
+  SD_CHECK(is_a16(logits) && is_a16(x0) && is_a16(x_t) && is_a16(dlogits), "row pointers must be 16 B aligned");
+  return loss_bwd(N, logits, x0, x_t, terms, dlogits, static_cast<cudaStream_t>(stream));
+  SD_GUARD_END
+}
+
+int seqdiff_op_angle_loss_bwd(int N, int F, const float* pred, const float* noise, const float* mask, const double* terms, float* dpred,
+                              void* stream) {
+  SD_GUARD_BEGIN
+  SD_CHECK(pred && noise && mask && terms && dpred, "null argument");
+  return angle_loss_bwd(N, F, pred, noise, mask, terms, dpred, static_cast<cudaStream_t>(stream));
+  SD_GUARD_END
+}
+
 }  // extern "C"

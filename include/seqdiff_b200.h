@@ -406,6 +406,59 @@ SEQDIFF_API int seqdiff_op_attention_packed(int precision, int B, int heads, int
                                             const int* q_off, const int* k_off, const int* q_len, int q_rows, int k_rows, int kv_div, void* out,
                                             void* stream);
 
+/* The rowwise and elementwise kernels of the training step, one entry each (operator-level, for tests).  Conventions:
+ *   precision FP32 / BF16 / FP16 selects the operand type T of the 16-bit tensors (fp32 in FP32 mode); the residual stream, its gradients and
+ *   every parameter gradient are fp32.  Parameter gradients (dgamma, dbeta, dbias, dW, db, dW2, db2, dmod32) are ADDED into.
+ *   Dropout: keep-scale of flat element e = (Philox word >= p * 2^32) / (1 - p), the word keyed by (seed, site, step, e) as in the training
+ *   step; p = 0: no dropout.  H in {256, 512, 768, 1024}.  Row-vector pointers 16 B aligned.  Illegal forms: SEQDIFF_ERR_INVALID.
+ * d <- o = dropout(d) + resid; out32 / out16 (either may be NULL; out16 not in FP32) = LayerNorm(o) * ln_w + ln_b;
+ * keep_bits [M, H / 8] (optional): bit j of byte k of a row = keep flag of element 8 k + j of that row. */
+SEQDIFF_API int seqdiff_op_dropout_add_layernorm(int precision, int M, int H, float* d, const float* resid, const float* ln_w, const float* ln_b,
+                                                 float eps, float p, uint64_t seed, uint32_t site, uint32_t step, float* out32, void* out16,
+                                                 uint8_t* keep_bits, void* stream);
+/* backward of h = LayerNorm(o) * gamma + beta: d_o, dgamma, dbeta.  FP32: g16, dbias and keep_bits NULL, p = 0.  16-bit modes also write
+ * g16 = T(d_o * keep) and add its column sums into dbias; the mask comes from keep_bits when given (and p > 0), else from Philox. */
+SEQDIFF_API int seqdiff_op_layernorm_bwd(int precision, int M, int H, const float* dh, const float* o, const float* gamma, float eps, float* d_o,
+                                         float* dgamma, float* dbeta, float p, uint64_t seed, uint32_t site, uint32_t step,
+                                         const uint8_t* keep_bits, void* g16, float* dbias, void* stream);
+/* backward of the adaLN residual update y = affine_first ? LayerNorm(in; lnw, lnb, eps1) : in, out = x + gate * (LN(y) * (1 + scale) + shift)
+ * with (shift, scale, gate) = chunks chunk0 .. chunk0 + 2 (0 <= chunk0 <= 3) of mod row row / mod_div ([*, 6H], type T).  din; sum_out
+ * (optional) = din + dout; exactly one of dmodT ([M, 6H] T rows, mod_div == 1; only the three chunks are written) and dmod32 ([M / mod_div
+ * rounded up, 6H] fp32, added into); dgamma / dbeta with affine_first. */
+SEQDIFF_API int seqdiff_op_ln_modulate_bwd(int precision, int M, int H, const float* dout, const float* in, int affine_first, const float* lnw,
+                                           const float* lnb, float eps1, const void* mod, int mod_div, int chunk0, float* din, float* sum_out,
+                                           void* dmodT, float* dmod32, float* dgamma, float* dbeta, void* stream);
+/* backward of the embedding out = dropout(LayerNorm(x Wt + b) * gamma + beta) (fp32): x [M, fin], 1 <= fin <= 32, Wt [fin, H];
+ * dW [H, fin], db, dgamma, dbeta [H] added into. */
+SEQDIFF_API int seqdiff_op_embed_bwd(int M, int fin, int H, const float* dout, const float* x, const float* Wt, const float* b, const float* gamma,
+                                     float eps, float p, uint64_t seed, uint32_t site, uint32_t step, float* dW, float* db, float* dgamma,
+                                     float* dbeta, void* stream);
+/* backward of the prediction head logits = LayerNorm(y; gamma, beta) W2^T + b2, y [M, H] of type T, F in {8, 20}: dy [M, H] fp32;
+ * dW2 [F, H], db2 [F], dgamma, dbeta [H] added into. */
+SEQDIFF_API int seqdiff_op_predictor_tail_bwd(int precision, int M, int H, int F, const float* dlogits, const void* y, const float* gamma,
+                                              const float* beta, float eps, const float* W2, float* dy, float* dW2, float* db2, float* dgamma,
+                                              float* dbeta, void* stream);
+/* n elements (n % 8 == 0) of one elementwise kernel; kind 1 erf-GELU, 2 SiLU:
+ *   op 0 act_fwd:   out = T(dropout(act(in)))               in, out: T
+ *   op 1 act_bwd:   out = T(in * keep * act'(aux))          in (the gradient), aux (z), out: T
+ *   op 2 act_bwd:   the same with an fp32 gradient `in`
+ *   op 3 grad_cast: out = T(in * keep)                      in: fp32
+ *   op 4 dropout_add (FP32 only): out <- dropout(out) + in, in place on out; in (the residual) may be NULL */
+SEQDIFF_API int seqdiff_op_train_elementwise(int op, int precision, int64_t n, int kind, const void* in, const void* aux, float p, uint64_t seed,
+                                             uint32_t site, uint32_t step, void* out, void* stream);
+/* out [cols, pitch] = transpose of in [rows, cols] (type T; columns rows .. pitch - 1 written as zeros; pitch 0 = rows, else
+ * rows <= pitch < rows + 64; out may be NULL); colsum [cols] (optional) += column sums of in. */
+SEQDIFF_API int seqdiff_op_transpose_colsum(int precision, int rows, int cols, const void* in, void* out, int pitch, float* colsum, void* stream);
+/* colsum [cols] += column sums of in [rows, cols] (BF16 / FP16, cols % 8 == 0) */
+SEQDIFF_API int seqdiff_op_colsum_add(int precision, int rows, int cols, const void* in, float* colsum, void* stream);
+/* gradient of the sequence loss with respect to the logits [N, 20]; terms: the device fp64 array seqdiff_loss_terms writes (terms[1] = number
+ * of noised rows) */
+SEQDIFF_API int seqdiff_op_loss_bwd(int N, const float* logits, const float* x0, const float* x_t, const double* terms, float* dlogits,
+                                    void* stream);
+/* gradient of the angle loss with respect to pred [N, F] (F in {8, 20}); terms: device fp64 [F + 1], terms[F] = number of valid rows */
+SEQDIFF_API int seqdiff_op_angle_loss_bwd(int N, int F, const float* pred, const float* noise, const float* mask, const double* terms, float* dpred,
+                                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -71,6 +71,96 @@ def test_operator_entry_points_reject_illegal_forms():
         assert lib.seqdiff_last_error()
 
 
+def test_training_kernel_entry_points_reject_illegal_forms():
+    """the operator entries of the training step's rowwise / elementwise kernels reject every form no kernel implements before anything
+    reaches the device (stand-in pointers, never dereferenced)"""
+    import ctypes
+    import seqdiff_b200 as sd
+    lib = sd.lib()
+    buf = ctypes.create_string_buffer(128)
+    p = ctypes.c_void_p((ctypes.addressof(buf) + 15) // 16 * 16)
+    q = ctypes.c_void_p(p.value + 4)  # not 16 B aligned
+    BF16, FP16, FP32 = 1, 2, 0
+    S = 0x1_2345_6789
+
+    def dal(prec=BF16, M=4, H=768, d=p, out16=p, resid=p):
+        return lib.seqdiff_op_dropout_add_layernorm(prec, M, H, d, resid, p, p, 1e-12, 0.1, S, 3, 5, p, out16, p, None)
+
+    def lnb(prec=BF16, M=4, H=768, g16=p, dbias=p, keep=None, dpr=0.1, dgamma=p):
+        return lib.seqdiff_op_layernorm_bwd(prec, M, H, p, p, p, 1e-12, p, dgamma, p, dpr, S, 3, 5, keep, g16, dbias, None)
+
+    def lnm(prec=BF16, M=4, H=768, aff=1, lnw=p, div=1, chunk0=0, dmodT=p, dmod32=None, sum_out=None):
+        return lib.seqdiff_op_ln_modulate_bwd(prec, M, H, p, p, aff, lnw, p, 1e-12, p, div, chunk0, p, sum_out, dmodT, dmod32, p, p, None)
+
+    def emb(M=4, fin=8, H=768, dW=p, x=p):
+        return lib.seqdiff_op_embed_bwd(M, fin, H, p, x, p, p, p, 1e-12, 0.1, S, 3, 5, dW, p, p, p, None)
+
+    def ptb(prec=BF16, M=4, H=768, F=20, y=p):
+        return lib.seqdiff_op_predictor_tail_bwd(prec, M, H, F, p, y, p, p, 1e-12, p, p, p, p, p, p, None)
+
+    def ew(op=0, prec=BF16, n=64, kind=1, inp=p, aux=p, out=p):
+        return lib.seqdiff_op_train_elementwise(op, prec, n, kind, inp, aux, 0.1, S, 3, 5, out, None)
+
+    bad = {
+        "dropout_add_layernorm: H = 384": dal(H=384),
+        "dropout_add_layernorm: H = 1280": dal(H=1280),
+        "dropout_add_layernorm: H = 300": dal(H=300),
+        "dropout_add_layernorm: M = 0": dal(M=0),
+        "dropout_add_layernorm: FP32 with a 16-bit output": dal(prec=FP32),
+        "dropout_add_layernorm: no residual": dal(resid=None),
+        "dropout_add_layernorm: unaligned rows": dal(d=q),
+        "dropout_add_layernorm: precision 3": dal(prec=3),
+        "layernorm_bwd: FP32 with g16": lnb(prec=FP32, dbias=None, dpr=0.0),
+        "layernorm_bwd: FP32 with dbias": lnb(prec=FP32, g16=None, dpr=0.0),
+        "layernorm_bwd: FP32 with dropout": lnb(prec=FP32, g16=None, dbias=None),
+        "layernorm_bwd: FP32 with keep bits": lnb(prec=FP32, g16=None, dbias=None, dpr=0.0, keep=p),
+        "layernorm_bwd: 16-bit without g16": lnb(g16=None),
+        "layernorm_bwd: 16-bit without dbias": lnb(prec=FP16, dbias=None),
+        "layernorm_bwd: no dgamma": lnb(dgamma=None),
+        "layernorm_bwd: H = 640": lnb(H=640),
+        "ln_modulate_bwd: both dmodT and dmod32": lnm(dmod32=p),
+        "ln_modulate_bwd: neither dmodT nor dmod32": lnm(dmodT=None),
+        "ln_modulate_bwd: dmodT with mod_div 24": lnm(div=24),
+        "ln_modulate_bwd: mod_div 0": lnm(div=0, dmodT=None, dmod32=p),
+        "ln_modulate_bwd: chunk0 4": lnm(chunk0=4),
+        "ln_modulate_bwd: chunk0 -1": lnm(chunk0=-1),
+        "ln_modulate_bwd: affine without lnw": lnm(lnw=None),
+        "ln_modulate_bwd: H = 128": lnm(H=128),
+        "ln_modulate_bwd: unaligned sum_out": lnm(sum_out=q),
+        "embed_bwd: fin 0": emb(fin=0),
+        "embed_bwd: fin 33": emb(fin=33),
+        "embed_bwd: H = 2048": emb(H=2048),
+        "embed_bwd: no dW": emb(dW=None),
+        "embed_bwd: no x": emb(x=None),
+        "predictor_tail_bwd: F 21": ptb(F=21),
+        "predictor_tail_bwd: F 4": ptb(F=4),
+        "predictor_tail_bwd: H = 1536": ptb(H=1536),
+        "predictor_tail_bwd: M = -1": ptb(M=-1),
+        "predictor_tail_bwd: unaligned y": ptb(y=q),
+        "elementwise: n % 8": ew(n=60),
+        "elementwise: n = 0": ew(n=0),
+        "elementwise: op 5": ew(op=5),
+        "elementwise: kind 3": ew(kind=3),
+        "elementwise: act_bwd without z": ew(op=1, aux=None),
+        "elementwise: dropout_add in a 16-bit mode": ew(op=4, prec=FP16),
+        "elementwise: no output": ew(out=None),
+        "elementwise: no input": ew(op=3, inp=None),
+        "elementwise: unaligned output": ew(op=3, out=q),
+        "transpose_colsum: pitch below rows": lib.seqdiff_op_transpose_colsum(BF16, 100, 64, p, p, 99, p, None),
+        "transpose_colsum: pitch a tile past rows": lib.seqdiff_op_transpose_colsum(BF16, 100, 64, p, p, 164, p, None),
+        "transpose_colsum: neither output": lib.seqdiff_op_transpose_colsum(BF16, 100, 64, p, None, 0, None, None),
+        "colsum_add: FP32": lib.seqdiff_op_colsum_add(FP32, 100, 64, p, p, None),
+        "colsum_add: cols % 8": lib.seqdiff_op_colsum_add(BF16, 100, 60, p, p, None),
+        "loss_bwd: N = 0": lib.seqdiff_op_loss_bwd(0, p, p, p, p, p, None),
+        "loss_bwd: no terms": lib.seqdiff_op_loss_bwd(4, p, p, p, None, p, None),
+        "angle_loss_bwd: F 12": lib.seqdiff_op_angle_loss_bwd(4, 12, p, p, p, p, p, None),
+        "angle_loss_bwd: N = 0": lib.seqdiff_op_angle_loss_bwd(0, 8, p, p, p, p, p, None),
+    }
+    for what, rc in bad.items():
+        assert rc == 1, what  # SEQDIFF_ERR_INVALID
+        assert lib.seqdiff_last_error()
+
+
 def test_state_dict_schema_is_the_reference_schema():
     import seqdiff_b200 as sd
     for L, rel in ((128, True), (64, True), (64, False)):

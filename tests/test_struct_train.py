@@ -22,13 +22,14 @@ T_STEPS = 1000
 SMALL_COS = {"bf16": 0.995, "fp16": 0.9999}  # the sequence step's bounds for the small gradient tensors (tests/test_train.py)
 
 
-def _cfg(L, layers, rel=True):
-    return S.OracleConfig(max_position_embeddings=L, num_hidden_layers=layers, feature_size=8, relative_key=rel)
+def _cfg(L, layers, rel=True, feature_size=8):
+    return S.OracleConfig(max_position_embeddings=L, num_hidden_layers=layers, feature_size=feature_size, relative_key=rel)
 
 
-def _noised_batch(B, Ll, Lr, n_lig, n_rec, seed):
+def _noised_batch(B, Ll, Lr, n_lig, n_rec, seed, feature_size=8):
     """A batch the way FoldingDiff's NoisedAnglesDataset builds one: t ~ U{0..T-1}, known_noise ~ N(0,1), corrupted =
-    wrap(sqrt(alphabar_t) x0 + sqrt(1 - alphabar_t) known_noise), on top of the padded dataset tensors."""
+    wrap(sqrt(alphabar_t) x0 + sqrt(1 - alphabar_t) known_noise), on top of the padded dataset tensors.  feature_size != 8: x0 and the
+    receptor angles are that many uniform angles per position (the dataset has 8)."""
     batch = O.synthetic_batch(B, Ll, n_lig, n_rec, seed)
     if Lr != Ll:
         rec = O.synthetic_batch(B, Lr, n_lig, n_rec, seed + 1)
@@ -37,8 +38,11 @@ def _noised_batch(B, Ll, Lr, n_lig, n_rec, seed):
     g = torch.Generator().manual_seed(seed + 2)
     ab = S.compute_alphas(S.cosine_beta_schedule(T_STEPS))
     t = torch.randint(0, T_STEPS, (B,), generator=g)
-    noise = torch.randn(B, Ll, 8, generator=g)
+    noise = torch.randn(B, Ll, feature_size, generator=g)
     x0 = batch["ligand_angles"]
+    if feature_size != 8:
+        x0 = (torch.rand(B, Ll, feature_size, generator=g) * 2 - 1) * math.pi
+        batch["receptor_angles"] = (torch.rand(B, Lr, feature_size, generator=g) * 2 - 1) * math.pi * batch["receptor_attn_mask"][..., None]
     corrupted = S.modulo_with_wrapped_range(ab["sqrt_alphas_cumprod"][t][:, None, None] * x0 +
                                             ab["sqrt_one_minus_alphas_cumprod"][t][:, None, None] * noise)
     return {"corrupted": corrupted, "t": t, "known_noise": noise, "ligand_attn_mask": batch["ligand_attn_mask"],
@@ -172,18 +176,20 @@ def _worst_small_tensor_cosine(flat, m, grads_ref):
     return worst
 
 
-# (Ll, Lr, B, layers, relative_key, n_lig, n_rec, seed).  The seeds are chosen so that no valid known_noise - pred lies within 1e-4 of
-# an odd multiple of pi, where the wrap jumps and the fp32 comparison would depend on rounding; each case asserts it.
-CASES = {"rel-2+2-L64-ragged": (64, 64, 2, 2, True, (10, 64), (20, 64), 1),
-         "abs-Ll!=Lr": (24, 40, 2, 2, False, (5, 24), (12, 40), 2),
-         "rel-12+12-L64": (64, 64, 2, 12, True, (30, 64), (40, 64), 3)}
+# (Ll, Lr, B, layers, relative_key, n_lig, n_rec, seed, feature_size).  The seeds are chosen so that no valid known_noise - pred lies within
+# 1e-4 of an odd multiple of pi, where the wrap jumps and the fp32 comparison would depend on rounding; each case asserts it.
+# feature_size 20: the 20-class head and the fin = 20 dense angle embedding of the structure model.
+CASES = {"rel-2+2-L64-ragged": (64, 64, 2, 2, True, (10, 64), (20, 64), 1, 8),
+         "abs-Ll!=Lr": (24, 40, 2, 2, False, (5, 24), (12, 40), 2, 8),
+         "rel-12+12-L64": (64, 64, 2, 12, True, (30, 64), (40, 64), 3, 8),
+         "rel-2+2-L64-F20": (64, 64, 2, 2, True, (10, 64), (20, 64), 4, 20)}
 
 
 def _oracle_case(case):
-    Ll, Lr, B, NL, rel, n_lig, n_rec, seed = CASES[case]
-    cfg = _cfg(max(Ll, Lr), NL, rel)
+    Ll, Lr, B, NL, rel, n_lig, n_rec, seed, Fs = CASES[case]
+    cfg = _cfg(max(Ll, Lr), NL, rel, Fs)
     state = S.init_struct_state_dict(cfg, seed)
-    batch = _noised_batch(B, Ll, Lr, n_lig, n_rec, seed + 10)
+    batch = _noised_batch(B, Ll, Lr, n_lig, n_rec, seed + 10, Fs)
     return cfg, state, batch
 
 
